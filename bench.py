@@ -2,6 +2,7 @@
 """Benchmark of the k-mer hot path (extract + sort + count, k=31) -- BASELINE.json's metric.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg2|cfg3]
+                  [--dump-outputs DIR]
   (N>1: launched by torchrun, one rank per GPU; rank 0 prints ONE JSON line)
 
 A "step" is one pass of the hot path over one synthetic input (--workload auto):
@@ -25,6 +26,9 @@ A "step" is one pass of the hot path over one synthetic input (--workload auto):
            `sort_lsd8_model_frac` = SURVEY.md §8d's fixed 8-bit LSD model N*W*(2*P8+1) over the same time
 `cpu_baseline` / --impl reference: the oracle's numpy port of the reference algorithm on the
            host cores (bounded sample) -- a reported baseline, not the target.
+--dump-outputs DIR: after the timed steps, the (k-mer, count) table of the last one is written to
+           DIR as float64 .npy files (see dump_outputs; `bench_outputs/` is ignored by git).  The
+           inputs are seeded, so two builds run with the same arguments can be compared file by file.
 """
 from __future__ import annotations
 
@@ -275,6 +279,49 @@ def verify_table(eng, d, tab, n_win_global, world, rank):
             "sum_key_times_count_eq_sum_keys_mod_2_64": kc == ks}
 
 
+DUMP_ROWS = 1 << 20  # 4 float64 arrays of this many rows: 32 MB
+
+
+def dump_rows(n: int) -> np.ndarray:
+    """Rows of an n-row table that --dump-outputs writes: all of them up to DUMP_ROWS, else a fixed
+    seeded sample; ascending."""
+    if n <= DUMP_ROWS:
+        return np.arange(n, dtype=np.int64)
+    return np.sort(np.random.default_rng(1234).choice(n, DUMP_ROWS, replace=False))
+
+
+def dump_outputs(out_dir, eng, tab, world, rank):
+    """Writes the (k-mer, count) table of one step -- the rank-order concatenation of every rank's slice,
+    i.e. the whole job's table, so the files do not depend on N for the same workload -- as float64 .npy
+    files in `out_dir`: `n_rows` (the table's length), the sampled `rows` (dump_rows) and their `keys_hi`,
+    `keys_lo` (the 2k-bit k-mer code split at bit 31, so both halves are exact in float64) and `counts`."""
+    import torch
+    import torch.distributed as dist
+
+    ns = [tab.n]
+    if world > 1:
+        ns = [None] * world
+        dist.all_gather_object(ns, tab.n)
+    off = sum(ns[:rank])
+    rows = dump_rows(sum(ns))
+    mine = torch.from_numpy(rows[(rows >= off) & (rows < off + tab.n)] - off).to(eng.device)
+    keys = tab.keys[: tab.n * 8].view(torch.int64)[mine].cpu().numpy().view(np.uint64)
+    counts = tab.counts[: tab.n * 4].view(torch.int32)[mine].cpu().numpy().view(np.uint32)
+    parts = [(keys, counts)]
+    if world > 1:
+        parts = [None] * world if rank == 0 else None
+        dist.gather_object((keys, counts), parts, dst=0)
+    if rank != 0:
+        return
+    keys = np.concatenate([p[0] for p in parts])
+    counts = np.concatenate([p[1] for p in parts])
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"n_rows": np.array([sum(ns)]), "rows": rows, "keys_hi": keys >> np.uint64(31),
+              "keys_lo": keys & np.uint64((1 << 31) - 1), "counts": counts}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+
+
 # ---- GPU arm --------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -285,7 +332,12 @@ def main():
     ap.add_argument("--workload", default="auto", choices=["auto", "cfg2", "cfg3"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's table to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's table; it is not available with --impl reference")
     if args.workload == "auto":
         # N=1: the configuration the single-GPU path is quoted on; N>1: BASELINE.json's scaling configuration
         args.workload = "cfg2" if args.gpus == 1 else "cfg3"
@@ -373,6 +425,8 @@ def main():
     ls_ns = int(lib.kmg_get_stat(b"local_sort_ns"))
     ls_cnt = int(lib.kmg_get_stat(b"local_sort_count"))
     lib.kmg_set_option(b"time_passes", 0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, eng, tab, world, rank)  # before the N>1 e2e steps overwrite `tab`
     dev_ms = sum(a.elapsed_time(b_) for a, b_ in ev)
     tmax = torch.tensor([dev_ms], dtype=torch.float64, device=eng.device)
     if world > 1:

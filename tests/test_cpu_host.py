@@ -217,6 +217,40 @@ def test_bench_reference_arm_prints_the_contract_line(gpus):
     assert p.returncode == 0 and p.stdout.strip() == ""
 
 
+def test_bench_rejects_zero_steps_and_a_reference_dump(tmp_path):
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=300)
+        assert p.returncode == 2 and "error:" in p.stderr, p.stderr[-2000:]
+
+
+def test_bench_dump_outputs_writes_a_fixed_sample_of_the_table(tmp_path):
+    """bench.py --dump-outputs on a host-resident stand-in for a device table: the same seeded rows every
+    time, float64 files, k-mer codes recovered exactly from their two halves, at most 64 MB."""
+    import types
+
+    import torch
+
+    sys.path.insert(0, ROOT)
+    import bench
+
+    for n in (1000, 3 * bench.DUMP_ROWS):
+        keys = np.sort(np.random.default_rng(0).integers(0, 1 << 62, n, dtype=np.uint64))
+        counts = np.random.default_rng(1).integers(1, 1 << 31, n).astype(np.uint32)
+        tab = types.SimpleNamespace(n=n, keys=torch.from_numpy(keys.view(np.uint8).copy()),
+                                    counts=torch.from_numpy(counts.view(np.uint8).copy()))
+        bench.dump_outputs(str(tmp_path / str(n)), types.SimpleNamespace(device=torch.device("cpu")), tab, 1, 0)
+        files = {f[:-4]: tmp_path / str(n) / f for f in os.listdir(tmp_path / str(n))}
+        assert set(files) == {"n_rows", "rows", "keys_hi", "keys_lo", "counts"}
+        assert sum(os.path.getsize(f) for f in files.values()) <= 64 << 20
+        a = {name: np.load(f) for name, f in files.items()}
+        assert all(v.dtype == np.float64 for v in a.values()) and a["n_rows"].tolist() == [n]
+        rows = a["rows"].astype(np.int64)
+        assert rows.size == min(n, bench.DUMP_ROWS) and (np.diff(rows) > 0).all()
+        assert np.array_equal(rows, bench.dump_rows(n))
+        got = a["keys_hi"].astype(np.uint64) << np.uint64(31) | a["keys_lo"].astype(np.uint64)
+        assert np.array_equal(got, keys[rows]) and np.array_equal(a["counts"], counts[rows])
+
+
 def test_every_option_and_stat_is_documented_in_the_header():
     """kmg_set_option / kmg_get_stat names handled in api.cu must appear in include/kmg.h's
     tuning section (and nothing documented may be unknown to the library)."""
