@@ -93,6 +93,37 @@ int kmg_extract(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, ui
                 void* d_vals_out, int val_bytes, uint64_t pos_offset, uint64_t* d_counts, uint64_t* d_hist_out,
                 void* d_ws, size_t ws_bytes, void* stream);
 
+/* ---- K1+K2 by key range: one pass of a sorted output that does not fit the device at once ----------
+ * With n_parts = 2^b parts (b <= 8), the part of a narrow key is its top b bits, key >> (2k - b) (the
+ * first bases; the same rule as kmg_range_partition and kmg_extract_dest_counts for power-of-two
+ * n_parts).  The part of a wide key follows the merged string order: if its first 4 symbols s are plain
+ * bases it is the narrow part of that 4-mer, otherwise the part of the largest plain 4-mer that sorts
+ * below s.  So every wide key of part p sorts after all narrow keys of parts < p and before all narrow
+ * keys of parts > p, and concatenating the per-part outputs in part order gives the whole sorted output.
+ *
+ * kmg_wide_part_table (host): h_table65536[x] = part of a wide key whose top 16 bits are x (its first
+ * 4 symbols), for DNA (plain ACGT) or RNA (rna != 0, plain ACGU).  Copy it to the device for the calls
+ * below. */
+int kmg_wide_part_table(int rna, int n_parts, uint8_t* h_table65536);
+/* kmg_extract restricted to the keys whose part lies in [part_lo, part_hi) (k >= 4): the kept keys in
+ * the same position order ('+' before '-' per position), so equal keys keep their emission order.
+ * Keys that are not kept are neither stored nor counted: d_counts[0] = keys stored, d_counts[1]
+ * (narrow) = windows of the wide stream in the whole window range.  Output capacity = the exact number
+ * of keys in the range (kmg_extract_dest_counts, kmg_extract_wide_part_counts).  d_wide_parts: device
+ * copy of kmg_wide_part_table's table (required for wide = 1).  d_hist_out must be NULL (KMG_ERR_ARG):
+ * the 4-mer-derived histograms describe every key, not the kept ones.  Workspace:
+ * kmg_extract_workspace_bytes(win_end - win_begin). */
+int kmg_extract_parts(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
+                      int wide, const uint8_t* d_lut256, const uint8_t* d_comp16, int n_parts, int part_lo, int part_hi,
+                      const uint8_t* d_wide_parts, void* d_keys_out, int key_bytes, void* d_vals_out, int val_bytes,
+                      uint64_t pos_offset, uint64_t* d_counts, uint64_t* d_hist_out, void* d_ws, size_t ws_bytes,
+                      void* stream);
+/* Keys of the wide stream per part (count-only launch of the filtered wide extraction, k >= 4):
+ * d_counts[0..n_parts).  d_comp16 is required with rc (the '-' key has its own part). */
+int kmg_extract_wide_part_counts(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k,
+                                 int rc, const uint8_t* d_lut256, const uint8_t* d_comp16, int n_parts,
+                                 const uint8_t* d_wide_parts, uint64_t* d_counts, void* stream);
+
 /* ---- K3: HBM-resident LSD radix sort (batch.py:156-168 + the merge of join.py:63-93) --
  * Stable, sorts on key bits [begin_bit, end_bit).  Ping-pongs between (keys, keys_alt)
  * [and (vals, vals_alt)]; *h_selector_out (host, written before return) is 0 if the

@@ -29,6 +29,10 @@ SIGNATURES = {
     "kmg_ws_status": (i32, [vp, vp]),
     "kmg_extract_workspace_bytes": (sz, [u64]),
     "kmg_extract": (i32, [vp, u64, u64, u64, i32, i32, i32, vp, vp, vp, i32, vp, i32, u64, vp, vp, vp, sz, vp]),
+    "kmg_wide_part_table": (i32, [i32, i32, u8p]),
+    "kmg_extract_parts": (i32, [vp, u64, u64, u64, i32, i32, i32, vp, vp, i32, i32, i32, vp, vp, i32, vp, i32, u64, vp,
+                                vp, vp, sz, vp]),
+    "kmg_extract_wide_part_counts": (i32, [vp, u64, u64, u64, i32, i32, vp, vp, i32, vp, vp, vp]),
     "kmg_radix_sort_workspace_bytes": (sz, [u64, i32, i32, i32, i32]),
     "kmg_radix_sort": (i32, [vp, vp, vp, vp, u64, i32, i32, i32, i32, vp, C.POINTER(i32), vp, sz, vp]),
     "kmg_rle_workspace_bytes": (sz, [u64]),

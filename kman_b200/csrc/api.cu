@@ -197,6 +197,35 @@ extern "C" int kmg_build_lut(const char* symbols, const char* complement, uint8_
     return KMG_OK;
 }
 
+// part of a wide key = part of the largest plain 4-mer m <= s (s = its first 4 symbols; m < s unless s is
+// plain, since s is then not a plain 4-mer).  m keeps the plain prefix of s, replaces the first other
+// symbol by the largest plain base below it (one exists: 'A' is plain and sorts first) and fills up with
+// the largest plain base.
+extern "C" int kmg_wide_part_table(int rna, int n_parts, uint8_t* h_table65536) {
+    KMG_REQUIRE(h_table65536, KMG_ERR_ARG, "null pointer argument");
+    KMG_REQUIRE(n_parts >= 1 && n_parts <= 256 && (n_parts & (n_parts - 1)) == 0, KMG_ERR_ARG,
+                "n_parts must be a power of two <= 256, got %d", n_parts);
+    const char* plain = rna ? "ACGU" : "ACGT";
+    int b = 0;
+    while ((1 << b) < n_parts) ++b;
+    for (uint32_t x = 0; x < 65536; ++x) {
+        uint32_t m = 0;  // packed 2-bit codes of the 4-mer, first symbol in the top bits
+        bool below = false;
+        for (int i = 0; i < 4; ++i) {
+            int code = 3;
+            if (!below) {
+                const char c = kSymbols16[(x >> (12 - 4 * i)) & 0xFu];
+                code = 0;
+                while (code < 3 && plain[code + 1] <= c) ++code;  // largest plain base <= c
+                below = plain[code] != c;
+            }
+            m = (m << 2) | (uint32_t)code;
+        }
+        h_table65536[x] = (uint8_t)(m >> (8 - b));
+    }
+    return KMG_OK;
+}
+
 // read back and clear the error word of a stage workspace (synchronises the stream)
 extern "C" int kmg_ws_status(void* d_ws, void* stream) {
     KMG_REQUIRE(d_ws, KMG_ERR_ARG, "null workspace");

@@ -40,7 +40,19 @@ struct ExtractParams {
     // (key >> digit_shift) & 255; cursors[256] hold the next free element of every region
     unsigned long long* cursors;
     int digit_shift;
+    // range filter (kmg_extract_parts, FILTER instantiations): a key is kept when its part lies in
+    // [part_lo, part_hi).  Narrow part = (key >> part_shift) & part_mask (its top log2(n_parts) bits),
+    // wide part = wide_parts[top 16 bits of the key] (kmg_wide_part_table).  The wide count-only
+    // launch adds every key to part_counts[part] instead.
+    int part_shift;
+    uint32_t part_mask, part_lo, part_hi;
+    const uint8_t* wide_parts;
+    unsigned long long* part_counts;
 };
+
+__device__ __forceinline__ bool in_parts(uint32_t part, const ExtractParams& p) {
+    return part - p.part_lo < p.part_hi - p.part_lo;
+}
 
 constexpr int EX_MAX_OFF = 2 * MAX_PASSES;
 
@@ -96,10 +108,13 @@ __device__ __forceinline__ ValT make_val(uint64_t pos, uint32_t strand) {
 //         slots in the 256 digit regions with one global atomic per digit and writes digit runs
 //         -- no compaction in position order, no tile prefix, no waiting for other tiles, and the
 //         keys never make the extra round trip through HBM in extraction order.
-template <typename KeyT, int PPT, bool RC, int VAL_BYTES, bool HIST, int MODE, int EX_BLOCK>
+// FILTER (MODE 0 only): keep only the keys whose part lies in [p.part_lo, p.part_hi)
+// (kmg_extract_parts); the tile counts kept keys instead of valid windows, order is unchanged.
+template <typename KeyT, int PPT, bool RC, int VAL_BYTES, bool HIST, int MODE, int EX_BLOCK, bool FILTER = false>
 __global__ void __launch_bounds__(EX_BLOCK) extract_narrow_kernel(const ExtractParams p) {
     static_assert(MODE != 1 || HIST, "the pre-pass exists for its histograms");
     static_assert(MODE != 2 || !HIST, "the fused pass takes its histograms from the pre-pass");
+    static_assert(!FILTER || (MODE == 0 && !HIST), "the range filter is a variant of the position-ordered extraction");
     constexpr int TILE = EX_BLOCK * PPT;
     constexpr int WORDS = TILE / 16 + EX_HALO_WORDS;
     constexpr int OUT_PER_WIN = RC ? 2 : 1;
@@ -231,11 +246,48 @@ __global__ void __launch_bounds__(EX_BLOCK) extract_narrow_kernel(const ExtractP
             if (in_range && im == 0 && bm != 0) ++nwide;
         }
     }
-    const uint32_t cnt = __popc(vf);
+    // key of my j-th window start
+    auto build_key = [&](int j) -> KeyT {
+        const int je = joff + j;
+        const int s2 = 2 * je;
+        const uint64_t hi = je == 0 ? X0 : ((X0 << s2) | (X1 >> (64 - s2)));
+        KeyT key;
+        if constexpr (sizeof(KeyT) == 8) {
+            key = hi >> (64 - 2 * k);
+        } else {
+            const uint64_t lo = je == 0 ? X1 : ((X1 << s2) | (X2 >> (64 - s2)));
+            const int s = 128 - 2 * k;
+            if (s == 0) {
+                key.lo = lo;
+                key.hi = hi;
+            } else {
+                key.lo = (lo >> s) | (hi << (64 - s));
+                key.hi = hi >> s;
+            }
+        }
+        return key;
+    };
+
+    // FILTER: bit OUT_PER_WIN*j (+1 for the '-' key) is set when that key of window j is kept
+    uint32_t kf = 0;
+    if constexpr (FILTER) {
+#pragma unroll
+        for (int j = 0; j < PPT; ++j) {
+            if (!(vf & (1u << j))) continue;
+            const KeyT key = build_key(j);
+            if (in_parts(key_digit(key, p.part_shift, p.part_mask), p)) kf |= 1u << (j * OUT_PER_WIN);
+            if constexpr (RC) {
+                if (in_parts(key_digit(rc_key(key, k), p.part_shift, p.part_mask), p)) kf |= 1u << (j * 2 + 1);
+            }
+        }
+    }
+    // keys per counted item: a valid window yields OUT_PER_WIN keys, a kept key one
+    constexpr uint32_t UNIT = FILTER ? 1 : OUT_PER_WIN;
+    const uint32_t cnt = FILTER ? __popc(kf) : __popc(vf);
     uint32_t total = 0, excl = 0;
     if constexpr (MODE != 2) excl = block_excl_scan<EX_BLOCK, uint32_t>(cnt, s_scan, total);
     if constexpr (MODE == 0) {
-        if (t == 0) tile_prefix_publish(p.tile_state, tile, (uint64_t)total * OUT_PER_WIN);
+        if (t == 0) tile_prefix_publish(p.tile_state, tile, (uint64_t)total * UNIT);
     }
     if (MODE != 2 && nwide) atomicAdd(&s_wide, nwide);
 
@@ -284,28 +336,6 @@ __global__ void __launch_bounds__(EX_BLOCK) extract_narrow_kernel(const ExtractP
         }
         return;
     }
-
-    // key of my j-th window start
-    auto build_key = [&](int j) -> KeyT {
-        const int je = joff + j;
-        const int s2 = 2 * je;
-        const uint64_t hi = je == 0 ? X0 : ((X0 << s2) | (X1 >> (64 - s2)));
-        KeyT key;
-        if constexpr (sizeof(KeyT) == 8) {
-            key = hi >> (64 - 2 * k);
-        } else {
-            const uint64_t lo = je == 0 ? X1 : ((X1 << s2) | (X2 >> (64 - s2)));
-            const int s = 128 - 2 * k;
-            if (s == 0) {
-                key.lo = lo;
-                key.hi = hi;
-            } else {
-                key.lo = (lo >> s) | (hi << (64 - s));
-                key.hi = hi >> s;
-            }
-        }
-        return key;
-    };
 
     if constexpr (MODE == 2) {
         // ---- fused first prefix pass: rank inside the tile = what the digit counter returned ----------
@@ -370,6 +400,21 @@ __global__ void __launch_bounds__(EX_BLOCK) extract_narrow_kernel(const ExtractP
         if (!(vf & (1u << j))) continue;
         const KeyT key = build_key(j);
         const uint64_t pos = tile_pos + (uint64_t)t * PPT + j + p.pos_offset;
+        if constexpr (FILTER) {
+            if ((kf >> (j * OUT_PER_WIN)) & 1u) {
+                s_keys[pad_idx<KB>(r)] = key;
+                if constexpr (VAL_BYTES != 0) s_vals[pad_idx<VB>(r)] = make_val<ValT>(pos, 0);
+                ++r;
+            }
+            if constexpr (RC) {
+                if ((kf >> (j * 2 + 1)) & 1u) {
+                    s_keys[pad_idx<KB>(r)] = rc_key(key, k);
+                    if constexpr (VAL_BYTES != 0) s_vals[pad_idx<VB>(r)] = make_val<ValT>(pos, 1);
+                    ++r;
+                }
+            }
+            continue;
+        }
         s_keys[pad_idx<KB>(r * OUT_PER_WIN)] = key;
         if constexpr (VAL_BYTES != 0) s_vals[pad_idx<VB>(r * OUT_PER_WIN)] = make_val<ValT>(pos, 0);
         if constexpr (RC) {
@@ -380,12 +425,12 @@ __global__ void __launch_bounds__(EX_BLOCK) extract_narrow_kernel(const ExtractP
     }
     __syncthreads();
     if (t < 32) {
-        const uint64_t e = tile_prefix_resolve_warp(p.tile_state, gridDim.x, tile, (uint64_t)total * OUT_PER_WIN, p.err);
+        const uint64_t e = tile_prefix_resolve_warp(p.tile_state, gridDim.x, tile, (uint64_t)total * UNIT, p.err);
         if (t == 0) s_base = e;
     }
     __syncthreads();
     const uint64_t base = s_base;
-    const uint32_t n_out = total * OUT_PER_WIN;
+    const uint32_t n_out = total * UNIT;
     KeyT* keys_out = reinterpret_cast<KeyT*>(p.keys_out) + base;
     for (uint32_t i = t; i < n_out; i += EX_BLOCK) keys_out[i] = s_keys[pad_idx<KB>(i)];
     if constexpr (VAL_BYTES != 0) {
@@ -424,7 +469,24 @@ struct WideKey {
     __device__ __forceinline__ void set_nibble(int q, uint32_t c) { w[q >> 4] |= (uint64_t)c << (4 * (q & 15)); }
 };
 
-template <bool RC, int VAL_BYTES, int LIMBS>
+// first 4 symbols of a wide key (its top 16 bits; k >= 4)
+template <int LIMBS>
+__device__ __forceinline__ uint32_t wide_top16(const WideKey<LIMBS>& key, int k) {
+    const int s = 4 * k - 16;
+    const int w = s >> 6, o = s & 63;
+    uint64_t v = 0;
+#pragma unroll
+    for (int i = 0; i < LIMBS; ++i) {
+        if (i == w) v |= key.w[i] >> o;
+        if (i == w + 1 && o > 48) v |= key.w[i] << (64 - o);
+    }
+    return (uint32_t)v & 0xFFFFu;
+}
+
+// FILTER 0: every wide key (kmg_extract).  1: only keys whose part lies in [p.part_lo, p.part_hi),
+// position order as in 0 (kmg_extract_parts).  2: count-only, keys per part into p.part_counts
+// (kmg_extract_wide_part_counts; p.part_hi = n_parts).
+template <bool RC, int VAL_BYTES, int LIMBS, int FILTER = 0>
 __global__ void __launch_bounds__(EXW_BLOCK) extract_wide_kernel(const ExtractParams p) {
     using ValT = typename std::conditional<VAL_BYTES == 4, uint32_t, uint64_t>::type;
     using KeyT = WideKey<LIMBS>;  // same layout as u128 / u256
@@ -435,11 +497,13 @@ __global__ void __launch_bounds__(EXW_BLOCK) extract_wide_kernel(const ExtractPa
     __shared__ uint32_t s_scan[EXW_BLOCK / 32 + 1];
     __shared__ uint32_t s_tile;
     __shared__ uint64_t s_base;
+    __shared__ uint32_t s_pc[FILTER == 2 ? 256 : 1];
 
     const int t = threadIdx.x;
-    if (t == 0) s_tile = atomicAdd(p.ticket, 1u);
+    if (t == 0) s_tile = FILTER == 2 ? blockIdx.x : atomicAdd(p.ticket, 1u);
     s_lut[t] = p.lut[t];
     if (t < 16) s_comp[t] = p.comp16[t];
+    if (FILTER == 2) s_pc[t] = 0;
     __syncthreads();
     const uint32_t tile = s_tile;
     const uint64_t tile_pos = (p.first_tile + tile) * (uint64_t)EXW_TILE;
@@ -469,6 +533,65 @@ __global__ void __launch_bounds__(EXW_BLOCK) extract_wide_kernel(const ExtractPa
         keys[j] = key;
         if (pos >= p.win_begin && pos < p.win_end && !any_inv && any_nonplain) vf |= 1u << j;
     }
+    // reverse complement: symbol q of the window (nibble k-1-q of the key) becomes nibble q
+    auto make_rc = [&](KeyT f) -> KeyT {
+        KeyT rcv;
+#pragma unroll
+        for (int i = 0; i < LIMBS; ++i) rcv.w[i] = 0;
+        for (int q = k - 1; q >= 0; --q) rcv.set_nibble(q, s_comp[f.pop()]);
+        return rcv;
+    };
+    if constexpr (FILTER != 0) {
+        // bit 2j: key of window j kept, bit 2j+1: its reverse complement kept
+        KeyT rcs[RC ? EXW_PPT : 1];
+        uint32_t kf = 0;
+#pragma unroll
+        for (int j = 0; j < EXW_PPT; ++j) {
+            if (!(vf & (1u << j))) continue;
+            const uint32_t pf = p.wide_parts[wide_top16(keys[j], k)];
+            if constexpr (FILTER == 2) atomicAdd(&s_pc[pf], 1u);
+            else if (in_parts(pf, p)) kf |= 1u << (2 * j);
+            if constexpr (RC) {
+                rcs[j] = make_rc(keys[j]);
+                const uint32_t pr = p.wide_parts[wide_top16(rcs[j], k)];
+                if constexpr (FILTER == 2) atomicAdd(&s_pc[pr], 1u);
+                else if (in_parts(pr, p)) kf |= 1u << (2 * j + 1);
+            }
+        }
+        if constexpr (FILTER == 2) {
+            __syncthreads();
+            if (t < (int)p.part_hi && s_pc[t]) atomicAdd(&p.part_counts[t], (unsigned long long)s_pc[t]);
+            return;
+        }
+        uint32_t total;
+        const uint32_t excl = block_excl_scan<EXW_BLOCK, uint32_t>(__popc(kf), s_scan, total);
+        if (t < 32) {
+            const uint64_t e = tile_prefix_exclusive_warp(p.tile_state, gridDim.x, tile, (uint64_t)total, p.err);
+            if (t == 0) s_base = e;
+        }
+        __syncthreads();
+        KeyT* keys_out = reinterpret_cast<KeyT*>(p.keys_out);
+        ValT* vals_out = reinterpret_cast<ValT*>(p.vals_out);
+        uint64_t r = s_base + excl;
+#pragma unroll
+        for (int j = 0; j < EXW_PPT; ++j) {
+            const uint64_t pos = tile_pos + t * EXW_PPT + j + p.pos_offset;
+            if ((kf >> (2 * j)) & 1u) {
+                keys_out[r] = keys[j];
+                if constexpr (VAL_BYTES != 0) vals_out[r] = make_val<ValT>(pos, 0);
+                ++r;
+            }
+            if constexpr (RC) {
+                if ((kf >> (2 * j + 1)) & 1u) {
+                    keys_out[r] = rcs[j];
+                    if constexpr (VAL_BYTES != 0) vals_out[r] = make_val<ValT>(pos, 1);
+                    ++r;
+                }
+            }
+        }
+        if (t == 0 && tile == gridDim.x - 1) p.counts[0] = s_base + (uint64_t)total;
+        return;
+    }
     const uint32_t cnt = __popc(vf);
     uint32_t total;
     const uint32_t excl = block_excl_scan<EXW_BLOCK, uint32_t>(cnt, s_scan, total);
@@ -489,12 +612,7 @@ __global__ void __launch_bounds__(EXW_BLOCK) extract_wide_kernel(const ExtractPa
         if constexpr (VAL_BYTES != 0) vals_out[r] = make_val<ValT>(pos, 0);
         ++r;
         if constexpr (RC) {
-            // reverse complement: symbol q of the window (nibble k-1-q of the key) becomes nibble q
-            KeyT f = keys[j], rcv;
-#pragma unroll
-            for (int i = 0; i < LIMBS; ++i) rcv.w[i] = 0;
-            for (int q = k - 1; q >= 0; --q) rcv.set_nibble(q, s_comp[f.pop()]);
-            keys_out[r] = rcv;
+            keys_out[r] = make_rc(keys[j]);
             if constexpr (VAL_BYTES != 0) vals_out[r] = make_val<ValT>(pos, 1);
             ++r;
         }
@@ -502,7 +620,7 @@ __global__ void __launch_bounds__(EXW_BLOCK) extract_wide_kernel(const ExtractPa
     if (t == 0 && tile == gridDim.x - 1) p.counts[0] = base + (uint64_t)total * OUT_PER_WIN;
 }
 
-template <typename KeyT, int PPT, bool RC, int VB, bool HIST, int MODE = 0, int BLOCK = EX_BLOCK_DEFAULT>
+template <typename KeyT, int PPT, bool RC, int VB, bool HIST, int MODE = 0, int BLOCK = EX_BLOCK_DEFAULT, bool FILTER = false>
 static int launch_narrow(const ExtractParams& p, uint32_t n_tiles, cudaStream_t st) {
     constexpr int TILE = BLOCK * PPT;
     constexpr uint32_t STAGE = TILE * (RC ? 2 : 1);
@@ -510,23 +628,24 @@ static int launch_narrow(const ExtractParams& p, uint32_t n_tiles, cudaStream_t 
     // (the pre-pass stages no keys: its dynamic shared memory only holds the correction tables)
     const size_t smem = MODE == 1 ? (size_t)8 * 256 * sizeof(uint32_t)
                                   : (sizeof(KeyT) + (VB == 4 ? 4 : (VB == 8 ? 8 : 0))) * (size_t)STAGE_PAD;
-    auto kern = extract_narrow_kernel<KeyT, PPT, RC, VB, HIST, MODE, BLOCK>;
+    auto kern = extract_narrow_kernel<KeyT, PPT, RC, VB, HIST, MODE, BLOCK, FILTER>;
     KMG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<n_tiles, BLOCK, smem, st>>>(p);
     KMG_LAUNCH_CHECK();
     return KMG_OK;
 }
 
-template <typename KeyT, int PPT, bool HIST>
+template <typename KeyT, int PPT, bool HIST, bool FILTER = false>
 static int dispatch_narrow2(const ExtractParams& p, uint32_t n_tiles, int rc, int vb, cudaStream_t st) {
+    constexpr int B = EX_BLOCK_DEFAULT;
     if (rc) {
-        if (vb == 0) return launch_narrow<KeyT, PPT, true, 0, HIST>(p, n_tiles, st);
-        if (vb == 4) return launch_narrow<KeyT, PPT, true, 4, HIST>(p, n_tiles, st);
-        return launch_narrow<KeyT, PPT, true, 8, HIST>(p, n_tiles, st);
+        if (vb == 0) return launch_narrow<KeyT, PPT, true, 0, HIST, 0, B, FILTER>(p, n_tiles, st);
+        if (vb == 4) return launch_narrow<KeyT, PPT, true, 4, HIST, 0, B, FILTER>(p, n_tiles, st);
+        return launch_narrow<KeyT, PPT, true, 8, HIST, 0, B, FILTER>(p, n_tiles, st);
     }
-    if (vb == 0) return launch_narrow<KeyT, PPT, false, 0, HIST>(p, n_tiles, st);
-    if (vb == 4) return launch_narrow<KeyT, PPT, false, 4, HIST>(p, n_tiles, st);
-    return launch_narrow<KeyT, PPT, false, 8, HIST>(p, n_tiles, st);
+    if (vb == 0) return launch_narrow<KeyT, PPT, false, 0, HIST, 0, B, FILTER>(p, n_tiles, st);
+    if (vb == 4) return launch_narrow<KeyT, PPT, false, 4, HIST, 0, B, FILTER>(p, n_tiles, st);
+    return launch_narrow<KeyT, PPT, false, 8, HIST, 0, B, FILTER>(p, n_tiles, st);
 }
 template <typename KeyT, int PPT>
 static int dispatch_narrow(const ExtractParams& p, uint32_t n_tiles, int rc, int vb, bool hist, cudaStream_t st) {
@@ -667,13 +786,19 @@ __global__ void hist_top_finalize_kernel(const unsigned long long* __restrict__ 
     }
 }
 
-template <bool RC, int LIMBS>
+template <bool RC, int LIMBS, int FILTER = 0>
 static int dispatch_wide(const ExtractParams& p, uint32_t n_tiles, int vb, cudaStream_t st) {
-    if (vb == 0) extract_wide_kernel<RC, 0, LIMBS><<<n_tiles, EXW_BLOCK, 0, st>>>(p);
-    else if (vb == 4) extract_wide_kernel<RC, 4, LIMBS><<<n_tiles, EXW_BLOCK, 0, st>>>(p);
-    else extract_wide_kernel<RC, 8, LIMBS><<<n_tiles, EXW_BLOCK, 0, st>>>(p);
+    if (vb == 0) extract_wide_kernel<RC, 0, LIMBS, FILTER><<<n_tiles, EXW_BLOCK, 0, st>>>(p);
+    else if (vb == 4) extract_wide_kernel<RC, 4, LIMBS, FILTER><<<n_tiles, EXW_BLOCK, 0, st>>>(p);
+    else extract_wide_kernel<RC, 8, LIMBS, FILTER><<<n_tiles, EXW_BLOCK, 0, st>>>(p);
     KMG_LAUNCH_CHECK();
     return KMG_OK;
+}
+// FILTER 2 stores nothing: the payload width does not matter
+template <int FILTER>
+static int dispatch_wide_any(const ExtractParams& p, uint32_t n_tiles, int k, int rc, int vb, cudaStream_t st) {
+    if (k <= 32) return rc ? dispatch_wide<true, 2, FILTER>(p, n_tiles, vb, st) : dispatch_wide<false, 2, FILTER>(p, n_tiles, vb, st);
+    return rc ? dispatch_wide<true, 4, FILTER>(p, n_tiles, vb, st) : dispatch_wide<false, 4, FILTER>(p, n_tiles, vb, st);
 }
 
 static void fill_common(ExtractParams& p, const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end,
@@ -765,11 +890,22 @@ extern "C" size_t kmg_extract_workspace_bytes(uint64_t n_windows) {
            (size_t)(EX_MAX_OFF + 1) * 256 * sizeof(uint64_t);
 }
 
-extern "C" int kmg_extract(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k,
-                           int rc, int wide, const uint8_t* d_lut256, const uint8_t* d_comp16, void* d_keys_out,
-                           int key_bytes, void* d_vals_out, int val_bytes, uint64_t pos_offset,
-                           uint64_t* d_counts, uint64_t* d_hist_out, void* d_ws, size_t ws_bytes, void* stream) {
-    cudaStream_t st = (cudaStream_t)stream;
+// range filter of kmg_extract_parts
+struct PartFilter {
+    int n_parts, part_lo, part_hi;
+    const uint8_t* wide_parts;
+};
+
+static int part_bits(int n_parts) {
+    int b = 0;
+    while ((1 << b) < n_parts) ++b;
+    return b;
+}
+
+static int extract_impl(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
+                        int wide, const uint8_t* d_lut256, const uint8_t* d_comp16, void* d_keys_out, int key_bytes,
+                        void* d_vals_out, int val_bytes, uint64_t pos_offset, uint64_t* d_counts, uint64_t* d_hist_out,
+                        void* d_ws, size_t ws_bytes, cudaStream_t st, const PartFilter* f) {
     KMG_REQUIRE(k >= 2, KMG_ERR_ARG, "k must be >= 2, got %d", k);  // batcher.py:477-478
     KMG_REQUIRE(k <= 64, KMG_ERR_RANGE, "k=%d: this build supports k <= 64 (no CPU fallback)", k);
     KMG_REQUIRE(win_begin <= win_end, KMG_ERR_ARG, "win_begin > win_end");
@@ -819,6 +955,17 @@ extern "C" int kmg_extract(const uint8_t* d_bases, uint64_t n_bases, uint64_t wi
     p.err = &hdr->err;
     p.hs = reinterpret_cast<unsigned long long*>((char*)d_ws + sizeof(WsHeader) + state_bytes);
     p.n_off = 0;
+    if (f) {
+        const int b = part_bits(f->n_parts);
+        p.part_shift = b ? 2 * k - b : 0;
+        p.part_mask = (1u << b) - 1u;
+        p.part_lo = (uint32_t)f->part_lo;
+        p.part_hi = (uint32_t)f->part_hi;
+        p.wide_parts = f->wide_parts;
+        if (wide) return dispatch_wide_any<1>(p, (uint32_t)n_tiles, k, rc, val_bytes, st);
+        if (key_bytes == 8) return dispatch_narrow2<uint64_t, 16, false, true>(p, (uint32_t)n_tiles, rc, val_bytes, st);
+        return dispatch_narrow2<u128, 8, false, true>(p, (uint32_t)n_tiles, rc, val_bytes, st);
+    }
     int top_idx = -1;
     if (d_hist_out) {
         const int P = (2 * k + 7) / 8;
@@ -854,4 +1001,59 @@ extern "C" int kmg_extract(const uint8_t* d_bases, uint64_t n_bases, uint64_t wi
     hist_finalize_kernel<<<1, 256, 0, st>>>(p.hs, p.n_off, k, rc, top_idx, reinterpret_cast<unsigned long long*>(d_hist_out));
     KMG_LAUNCH_CHECK();
     return KMG_OK;
+}
+
+extern "C" int kmg_extract(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k,
+                           int rc, int wide, const uint8_t* d_lut256, const uint8_t* d_comp16, void* d_keys_out,
+                           int key_bytes, void* d_vals_out, int val_bytes, uint64_t pos_offset,
+                           uint64_t* d_counts, uint64_t* d_hist_out, void* d_ws, size_t ws_bytes, void* stream) {
+    return extract_impl(d_bases, n_bases, win_begin, win_end, k, rc, wide, d_lut256, d_comp16, d_keys_out, key_bytes,
+                        d_vals_out, val_bytes, pos_offset, d_counts, d_hist_out, d_ws, ws_bytes, (cudaStream_t)stream, nullptr);
+}
+
+static int check_parts(int k, int n_parts, int part_lo, int part_hi, int wide, const uint8_t* d_wide_parts) {
+    KMG_REQUIRE(k >= 4, KMG_ERR_ARG, "the range filter needs k >= 4, got %d", k);
+    KMG_REQUIRE(n_parts >= 1 && n_parts <= 256 && (n_parts & (n_parts - 1)) == 0, KMG_ERR_ARG,
+                "n_parts must be a power of two <= 256, got %d", n_parts);
+    KMG_REQUIRE(0 <= part_lo && part_lo <= part_hi && part_hi <= n_parts, KMG_ERR_ARG,
+                "part range [%d, %d) outside [0, %d)", part_lo, part_hi, n_parts);
+    KMG_REQUIRE(!wide || d_wide_parts, KMG_ERR_ARG, "the wide stream needs d_wide_parts");
+    return KMG_OK;
+}
+
+extern "C" int kmg_extract_parts(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k,
+                                 int rc, int wide, const uint8_t* d_lut256, const uint8_t* d_comp16, int n_parts,
+                                 int part_lo, int part_hi, const uint8_t* d_wide_parts, void* d_keys_out, int key_bytes,
+                                 void* d_vals_out, int val_bytes, uint64_t pos_offset, uint64_t* d_counts,
+                                 uint64_t* d_hist_out, void* d_ws, size_t ws_bytes, void* stream) {
+    KMG_REQUIRE(!d_hist_out, KMG_ERR_ARG, "kmg_extract_parts computes no digit histograms (d_hist_out must be NULL)");
+    const int rcode = check_parts(k, n_parts, part_lo, part_hi, wide, d_wide_parts);
+    if (rcode != KMG_OK) return rcode;
+    const PartFilter f{n_parts, part_lo, part_hi, d_wide_parts};
+    return extract_impl(d_bases, n_bases, win_begin, win_end, k, rc, wide, d_lut256, d_comp16, d_keys_out, key_bytes,
+                        d_vals_out, val_bytes, pos_offset, d_counts, nullptr, d_ws, ws_bytes, (cudaStream_t)stream, &f);
+}
+
+extern "C" int kmg_extract_wide_part_counts(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end,
+                                            int k, int rc, const uint8_t* d_lut256, const uint8_t* d_comp16, int n_parts,
+                                            const uint8_t* d_wide_parts, uint64_t* d_counts, void* stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    const int rcode = check_parts(k, n_parts, 0, n_parts, 1, d_wide_parts);
+    if (rcode != KMG_OK) return rcode;
+    KMG_REQUIRE(k <= 64, KMG_ERR_RANGE, "k=%d: this build supports k <= 64 (no CPU fallback)", k);
+    KMG_REQUIRE(win_begin <= win_end, KMG_ERR_ARG, "win_begin > win_end");
+    KMG_REQUIRE(d_bases && d_lut256 && d_counts && (!rc || d_comp16), KMG_ERR_ARG, "null pointer argument");
+    KMG_CUDA(cudaMemsetAsync(d_counts, 0, sizeof(uint64_t) * n_parts, st));
+    if (win_end == win_begin) return KMG_OK;
+    const uint64_t first_tile = win_begin / EXW_TILE;
+    const uint64_t n_tiles = (win_end + EXW_TILE - 1) / EXW_TILE - first_tile;
+    KMG_REQUIRE(n_tiles < (1ull << 31), KMG_ERR_RANGE, "too many tiles");
+    ExtractParams p;
+    fill_common(p, d_bases, n_bases, win_begin, win_end, EXW_TILE, k, d_lut256);
+    p.comp16 = d_comp16;
+    p.part_lo = 0;
+    p.part_hi = (uint32_t)n_parts;
+    p.wide_parts = d_wide_parts;
+    p.part_counts = reinterpret_cast<unsigned long long*>(d_counts);
+    return dispatch_wide_any<2>(p, (uint32_t)n_tiles, k, rc, 0, st);
 }

@@ -14,8 +14,10 @@ Stage -> reference mapping (see DESIGN.md):
 from __future__ import annotations
 
 import ctypes as C
-from dataclasses import dataclass
-from typing import Dict, List, Optional, Tuple
+import os
+from concurrent.futures import ThreadPoolExecutor
+from dataclasses import dataclass, field
+from typing import BinaryIO, Callable, Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -112,6 +114,155 @@ class CountTable:
 
     def counts_host(self) -> np.ndarray:
         return self.counts[: self.n * 4].cpu().numpy().view(np.uint32)
+
+
+# ---- key-range passes (write_count / write_uniq) ------------------------------------------------------
+PASS_PARTS = 256  # parts of a multi-pass plan: the top 8 key bits (first 4 bases)
+DEVICE_HEADROOM = 2 << 30  # bytes of free device memory a default budget leaves alone (allocator, context)
+TEXT_CHUNK_BYTES = 256 << 20  # device text of one chunk (two of them on the device, two pinned on the host)
+
+
+def wide_part_table(rna: int, n_parts: int) -> np.ndarray:
+    """uint8[65536]: part of a wide-stream key from its top 16 bits (first 4 symbols), see
+    kmg_wide_part_table in include/kmg.h.  Host only."""
+    t = np.zeros(65536, np.uint8)
+    _lib.check(_lib.load().kmg_wide_part_table(int(rna), int(n_parts), t.ctypes.data_as(_lib.u8p)))
+    return t
+
+
+def plan_parts(narrow: Sequence[int], wide: Sequence[int], pass_bytes: Callable[[int, int], int],
+               budget: int) -> List[Tuple[int, int]]:
+    """Group contiguous parts [lo, hi) greedily into passes whose pass_bytes(narrow keys, wide keys) stays
+    within `budget` (pass_bytes grows with both, so greedy gives the fewest passes).  ValueError if one
+    part alone does not fit."""
+    out: List[Tuple[int, int]] = []
+    lo, n_parts = 0, len(narrow)
+    while lo < n_parts:
+        need = pass_bytes(int(narrow[lo]), int(wide[lo]))
+        if need > budget:
+            raise ValueError(f"part {lo} of {n_parts} needs {need} device bytes, more than the {budget} available")
+        hi, n, m = lo + 1, int(narrow[lo]), int(wide[lo])
+        while hi < n_parts and pass_bytes(n + int(narrow[hi]), m + int(wide[hi])) <= budget:
+            n, m = n + int(narrow[hi]), m + int(wide[hi])
+            hi += 1
+        out.append((lo, hi))
+        lo = hi
+    return out
+
+
+def pass_bytes(k: int, mode: str, n: int, m: int, val_bytes: int, text_bytes: int, n_win: int) -> int:
+    """Device bytes of one pass over n narrow and m wide keys: key (+ payload) buffers and their alternates,
+    counts, the sort workspace from the library's own *_workspace_bytes (one buffer the engine keeps and
+    grows, so the wide stage sees the larger of the two), the merge ranks, the extraction workspace and the
+    text chunk buffers (`text_bytes`)."""
+    lib = _lib.load()
+    kb, kw = (8, 16) if k <= 32 else (16, 32)
+    item = 4 if mode == "count" else val_bytes  # count / payload bytes per key
+    if mode == "count":
+        ws_n = lib.kmg_sort_count_workspace_bytes(n, kb, 2 * k)
+        ws_w = lib.kmg_sort_count_workspace_bytes(m, kw, 4 * k)
+    else:
+        ws_n = lib.kmg_sort_uniq_workspace_bytes(n, kb, val_bytes, 2 * k)
+        ws_w = lib.kmg_sort_uniq_workspace_bytes(m, kw, val_bytes, 4 * k)
+    if kw == 32:
+        ws_w = lib.kmg_sort256_workspace_bytes(m) + lib.kmg_rle_workspace_bytes(m)
+    stages = 2 * n * (kb + item) + ws_n
+    if m:  # the narrow table is held while the wide stream is extracted, sorted and ranked against it
+        merge = 8 * (n + m) + (16 * m if k > 32 else 0)
+        stages = max(stages, n * (kb + item) + 2 * m * (kw + item) + max(ws_n, ws_w) + merge)
+    return int(stages + lib.kmg_extract_workspace_bytes(n_win) + text_bytes)
+
+
+@dataclass
+class PassPlan:
+    """How write_count / write_uniq split the key space.  n_parts == 1: one pass on the whole-input path
+    (count() / uniq()); otherwise parts[i] = (lo, hi) of pass i over `n_parts` parts with `narrow[p]` /
+    `wide[p]` keys in part p, and pass_bytes[i] its modelled device bytes.  pass_ms[i]: time of pass i
+    between CUDA events (filled in by write_count / write_uniq)."""
+
+    n_parts: int
+    parts: List[Tuple[int, int]]
+    narrow: np.ndarray
+    wide: np.ndarray
+    pass_bytes: List[int] = field(default_factory=list)
+    pass_ms: List[float] = field(default_factory=list)
+
+    @property
+    def n_passes(self) -> int:
+        return len(self.parts)
+
+
+def make_plan(k: int, budget: int, one_pass_bytes: int, totals: Tuple[int, int],
+              part_counts: Callable[[], Tuple[np.ndarray, np.ndarray]], cost: Callable[[int, int], int]) -> PassPlan:
+    """One pass when the whole-input path fits `budget` (or there is nothing to do); otherwise group the
+    parts of part_counts() (narrow, wide keys per part) into passes by `cost` (plan_parts).  Key-range
+    passes need the per-part counts of the 4-mer histogram, so k < 12 that does not fit is a ValueError."""
+    n, m = totals
+    if one_pass_bytes <= budget or n + m == 0:
+        return PassPlan(1, [(0, 1)], np.array([n], np.int64), np.array([m], np.int64), [one_pass_bytes])
+    if k < 12:
+        raise ValueError(f"k={k}: the input needs {one_pass_bytes} device bytes, more than the {budget} available, "
+                         f"and key-range passes need k >= 12")
+    narrow, wide = part_counts()
+    parts = plan_parts(narrow, wide, cost, budget)
+    return PassPlan(len(narrow), parts, narrow, wide,
+                    [cost(int(narrow[lo:hi].sum()), int(wide[lo:hi].sum())) for lo, hi in parts])
+
+
+class _ChunkSink:
+    """Double-buffered device text -> pinned host buffer -> file: the copy of chunk i runs on a copy
+    stream and its file write on a worker thread while the GPU formats chunk i+1."""
+
+    def __init__(self, eng: "Engine", fh: BinaryIO, nbytes: int):
+        self.fh = fh
+        self.dev = [eng._new(nbytes), eng._new(nbytes)]
+        self.pinned = [torch.empty(max(nbytes, 16), dtype=torch.uint8, pin_memory=True) for _ in range(2)]
+        self.stream = torch.cuda.Stream(eng.device)
+        self.pool = ThreadPoolExecutor(1)
+        self.pending = [None, None]
+        self.slot = 0
+
+    def buffer(self) -> torch.Tensor:
+        """Device buffer of the next chunk (free once the write of the chunk before last is done)."""
+        s = self.slot
+        if self.pending[s] is not None:
+            self.pending[s].result()
+            self.pending[s] = None
+        return self.dev[s]
+
+    def submit(self, text: torch.Tensor, pieces: Optional[List[Tuple[Optional[np.ndarray], int, int]]]) -> None:
+        """Write `text` (a prefix of buffer()); pieces: (None, a, b) = text[a:b], (arr, a, b) = arr[a:b]
+        in this order, or None for the whole text."""
+        s, nb = self.slot, int(text.numel())
+        ready = torch.cuda.Event()
+        ready.record()
+        self.stream.wait_event(ready)
+        done = torch.cuda.Event()
+        with torch.cuda.stream(self.stream):
+            if nb:
+                self.pinned[s][:nb].copy_(text, non_blocking=True)
+            done.record()
+        host = self.pinned[s].numpy()
+        self.pending[s] = self.pool.submit(self._write, done, host, nb, pieces)
+        self.slot ^= 1
+
+    def _write(self, done, host: np.ndarray, nb: int, pieces) -> None:
+        done.synchronize()
+        if pieces is None:
+            self.fh.write(memoryview(host[:nb]))
+            return
+        for arr, a, b in pieces:
+            if b > a:
+                self.fh.write(memoryview((host if arr is None else arr)[a:b]))
+
+    def close(self) -> None:
+        try:
+            for f in self.pending:
+                if f is not None:
+                    f.result()
+        finally:
+            self.pool.shutdown(wait=True)
+            self.stream.synchronize()
 
 
 class Engine:
@@ -454,11 +605,12 @@ class Engine:
 
     # ---- K6 -----------------------------------------------------------------------------------
     @_on_device
-    def format_counts(self, t: CountTable, rna: int = 0) -> torch.Tensor:
-        """Device text "SEQ\\tCOUNT\\n" for one stream (uint8 tensor, exact length)."""
+    def format_counts(self, t: CountTable, rna: int = 0, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Device text "SEQ\\tCOUNT\\n" for one stream (uint8 tensor, exact length).  `out`: a buffer of at
+        least t.n * (t.k + 12) bytes to write it into."""
         if t.n == 0:
             return torch.empty(0, dtype=torch.uint8, device=self.device)
-        text = self._new(t.n * (t.k + 12))
+        text = self._new(t.n * (t.k + 12)) if out is None else out
         ws_bytes = self.lib.kmg_format_workspace_bytes(t.n)
         ws = self._buf("ws_fmt", ws_bytes)
         _lib.check(
@@ -471,14 +623,15 @@ class Engine:
         return text[:nbytes]
 
     @_on_device
-    def format_uniq(self, s: KeyArray, d: DeviceInput) -> torch.Tensor:
-        """Device text ">NAME:START-END:STRAND\\nSEQ\\n" for one stream."""
+    def format_uniq(self, s: KeyArray, d: DeviceInput, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Device text ">NAME:START-END:STRAND\\nSEQ\\n" for one stream.  `out`: a buffer of at least
+        s.n * (s.k + 48 + longest name) bytes to write it into."""
         if s.n == 0:
             return torch.empty(0, dtype=torch.uint8, device=self.device)
         if d.rec_starts is None:
             self._upload_names(d)
         max_name = max((len(nm) for nm in d.flat.names), default=0)
-        text = self._new(s.n * (s.k + 48 + max_name))
+        text = self._new(s.n * (s.k + 48 + max_name)) if out is None else out
         ws_bytes = self.lib.kmg_format_workspace_bytes(s.n)
         ws = self._buf("ws_fmt", ws_bytes)
         _lib.check(
@@ -584,6 +737,233 @@ class Engine:
         if n_other:
             out.append(self.sort_uniq(self.extract(d, k, rc, wide=True, val_bytes=vb)))
         return out
+
+    # ---- key-range passes: output larger than the device ---------------------------------------------
+    @_on_device
+    def part_counts(self, d: DeviceInput, k: int, rc: bool, n_parts: int) -> Tuple[np.ndarray, np.ndarray]:
+        """Keys per part of the narrow and of the wide stream (k >= 12): the narrow counts come from the
+        4-mer histogram of the bases (kmg_extract_dest_counts); a count-only wide extraction
+        (kmg_extract_wide_part_counts) runs only when the input has wide windows."""
+        n_win = max(0, d.n_bases - k + 1)
+        narrow, wide = np.zeros(n_parts, np.int64), np.zeros(n_parts, np.int64)
+        if n_win == 0:
+            return narrow, wide
+        counts = torch.zeros(n_parts + 1, dtype=torch.int64, device=self.device)
+        ws_bytes = self.lib.kmg_dest_counts_workspace_bytes()
+        ws = self._buf("ws_dest_counts", ws_bytes)
+        _lib.check(self.lib.kmg_extract_dest_counts(d.bases.data_ptr(), d.n_bases, 0, n_win, k, int(rc), d.lut.data_ptr(),
+                                                    n_parts, counts.data_ptr(), ws.data_ptr(), ws_bytes, self._stream()))
+        c = counts.cpu().numpy()
+        narrow[:] = c[:n_parts]
+        if c[n_parts]:
+            _lib.check(self.lib.kmg_extract_wide_part_counts(d.bases.data_ptr(), d.n_bases, 0, n_win, k, int(rc),
+                                                             d.lut.data_ptr(), d.comp16.data_ptr(), n_parts,
+                                                             self._wide_parts(d.rna, n_parts).data_ptr(),
+                                                             counts.data_ptr(), self._stream()))
+            wide[:] = counts[:n_parts].cpu().numpy()
+        return narrow, wide
+
+    def _wide_parts(self, rna: int, n_parts: int) -> torch.Tensor:
+        key = f"wide_parts_{rna}_{n_parts}"
+        if key not in self._scratch:
+            self._scratch[key] = torch.from_numpy(wide_part_table(rna, n_parts)).to(self.device)
+        return self._scratch[key]
+
+    @_on_device
+    def extract_parts(self, d: DeviceInput, k: int, rc: bool, wide: bool, val_bytes: int, n_parts: int, part_lo: int,
+                      part_hi: int, n_keys: int) -> KeyArray:
+        """extract() restricted to the keys of parts [part_lo, part_hi) (kmg_extract_parts), into buffers of
+        exactly `n_keys` keys (from part_counts)."""
+        n_win = max(0, d.n_bases - k + 1)
+        kb = (16 if k <= 32 else 32) if wide else (8 if k <= 32 else 16)
+        keys, keys_alt = self._new(n_keys * kb), self._new(n_keys * kb)
+        vals = self._new(n_keys * val_bytes) if val_bytes else None
+        vals_alt = self._new(n_keys * val_bytes) if val_bytes else None
+        ws_bytes = self.lib.kmg_extract_workspace_bytes(n_win)
+        ws = self._buf("ws_extract", ws_bytes)
+        _lib.check(self.lib.kmg_extract_parts(
+            d.bases.data_ptr(), d.n_bases, 0, n_win, k, int(rc), int(wide), d.lut.data_ptr(), d.comp16.data_ptr(), n_parts,
+            part_lo, part_hi, self._wide_parts(d.rna, n_parts).data_ptr(), keys.data_ptr(), kb, _ptr(vals), val_bytes,
+            d.pos_offset, self._small.data_ptr(), None, ws.data_ptr(), ws_bytes, self._stream()))
+        self._status(ws)
+        n = int(self._small[:1].cpu().numpy().view(np.uint64)[0])
+        if n != n_keys:
+            raise _lib.KmgError(f"parts [{part_lo}, {part_hi}) of {n_parts}: extracted {n} keys, counted {n_keys}")
+        return KeyArray(keys, keys_alt, vals, vals_alt, n, kb, val_bytes, k, wide)
+
+    def _line_bytes(self, d: DeviceInput, k: int, mode: str) -> int:
+        """Text capacity per row that format_counts / format_uniq require."""
+        return k + 12 if mode == "count" else k + 48 + max((len(nm) for nm in d.flat.names), default=0)
+
+    def _one_pass_bytes(self, d: DeviceInput, k: int, rc: bool, mode: str, n_other: int, val_bytes: int,
+                        text_bytes: int) -> int:
+        """Device bytes of the whole-input path (count() / uniq()): window-sized buffers of the fused
+        pipeline, then those of the wide stream while the narrow result is held."""
+        lib = self.lib
+        n_win = max(0, d.n_bases - k + 1)
+        cap = max(n_win * (2 if rc else 1), 1)
+        kb, kw = (8, 16) if k <= 32 else (16, 32)
+        item = kb + (4 if mode == "count" else val_bytes)
+        narrow = 2 * cap * item + lib.kmg_pipeline_workspace_bytes(n_win, k, int(rc), 0 if mode == "count" else val_bytes)
+        if n_other:
+            m = n_other * (2 if rc else 1)
+            witem = kw + (4 if mode == "count" else val_bytes)
+            wide = cap * item + 2 * cap * witem + pass_bytes(k, mode, 0, m, val_bytes, 0, n_win) + 8 * (cap + m)
+            narrow = max(narrow, wide)
+        return int(narrow + lib.kmg_extract_workspace_bytes(n_win) + text_bytes)
+
+    def _resident_bytes(self, d: DeviceInput) -> int:
+        return sum(int(t.numel()) * t.element_size() for t in (d.bases, d.rec_starts, d.names_buf, d.name_offs)
+                   if t is not None)
+
+    def device_budget(self, d: DeviceInput, budget_bytes: Optional[int] = None) -> int:
+        """Device bytes a pass may use.  `budget_bytes` (or the KMG_DEVICE_BUDGET environment variable) is the
+        whole job's budget, from which the resident bases, names and record starts are subtracted; by default
+        it is the device's free memory (plus what torch's allocator caches) minus DEVICE_HEADROOM."""
+        if budget_bytes is None and os.environ.get("KMG_DEVICE_BUDGET"):
+            budget_bytes = int(os.environ["KMG_DEVICE_BUDGET"])
+        if budget_bytes is not None:
+            return int(budget_bytes) - self._resident_bytes(d)
+        free, _ = torch.cuda.mem_get_info(self.device)
+        cached = torch.cuda.memory_reserved(self.device) - torch.cuda.memory_allocated(self.device)
+        return int(free + cached - DEVICE_HEADROOM)
+
+    def _text_plan(self, d: DeviceInput, k: int, mode: str, chunk_rows: Optional[int]) -> Tuple[int, int]:
+        """(rows per text chunk, device bytes of the text stage: two chunk buffers + the newline index)."""
+        line = self._line_bytes(d, k, mode)
+        rows = max(1, chunk_rows or TEXT_CHUNK_BYTES // line)
+        return rows, 2 * rows * line + rows * line + rows * (2 if mode == "uniq" else 1) * 8
+
+    @_on_device
+    def plan_passes(self, d: DeviceInput, k: int, rc: bool, mode: str, budget_bytes: Optional[int] = None,
+                    chunk_rows: Optional[int] = None) -> PassPlan:
+        """Split `kmer count` (mode "count") / `kmer uniq` ("uniq") into key-range passes that fit the device
+        budget (device_budget).  Everything fits: one pass on the whole-input path.  Otherwise contiguous
+        parts of PASS_PARTS are grouped (plan_parts; needs k >= 12, ValueError if not or if one part alone
+        does not fit)."""
+        if mode not in ("count", "uniq"):
+            raise AssertionError(f"unknown mode {mode!r}")
+        budget = self.device_budget(d, budget_bytes)
+        vb = 4 if ((d.pos_offset + d.n_bases) << 1) < (1 << 32) else 8
+        _, text_bytes = self._text_plan(d, k, mode, chunk_rows)
+        n, n_other = self.count_windows(d, k, rc)
+        one = self._one_pass_bytes(d, k, rc, mode, n_other, vb, text_bytes)
+        n_win = max(0, d.n_bases - k + 1)
+        return make_plan(k, budget, one, (n, n_other * (2 if rc else 1)), lambda: self.part_counts(d, k, rc, PASS_PARTS),
+                         lambda a, b: pass_bytes(k, mode, a, b, vb, text_bytes, n_win))
+
+    def write_count(self, d: DeviceInput, k: int, rc: bool, fh: BinaryIO, budget_bytes: Optional[int] = None,
+                    chunk_rows: Optional[int] = None) -> PassPlan:
+        """Write the bytes of count_text() to the binary file object `fh`, pass by pass and chunk by chunk, so
+        device memory is bounded by the budget and host memory by the text chunk.  Returns the plan."""
+        return self._write_passes(d, k, rc, fh, "count", budget_bytes, chunk_rows)
+
+    def write_uniq(self, d: DeviceInput, k: int, rc: bool, fh: BinaryIO, budget_bytes: Optional[int] = None,
+                   chunk_rows: Optional[int] = None) -> PassPlan:
+        """Write the bytes of uniq_text() to `fh` (see write_count)."""
+        return self._write_passes(d, k, rc, fh, "uniq", budget_bytes, chunk_rows)
+
+    @_on_device
+    def _write_passes(self, d: DeviceInput, k: int, rc: bool, fh: BinaryIO, mode: str, budget_bytes: Optional[int],
+                      chunk_rows: Optional[int]) -> PassPlan:
+        if d.rec_starts is None and mode == "uniq":
+            self._upload_names(d)
+        plan = self.plan_passes(d, k, rc, mode, budget_bytes, chunk_rows)
+        rows, _ = self._text_plan(d, k, mode, chunk_rows)
+        sink = _ChunkSink(self, fh, rows * self._line_bytes(d, k, mode))
+        passes = self.pass_tables(d, k, rc, mode, plan)
+        try:
+            while True:
+                t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                t0.record()
+                tabs = next(passes, None)
+                if tabs is None:
+                    break
+                self._emit_chunks(sink, d, k, mode, tabs, rows)
+                del tabs  # a pass's buffers are freed before the next pass allocates its own
+                t1.record()
+                t1.synchronize()
+                plan.pass_ms.append(t0.elapsed_time(t1))
+        finally:
+            sink.close()
+        return plan
+
+    def pass_tables(self, d: DeviceInput, k: int, rc: bool, mode: str, plan: PassPlan):
+        """Yield, pass by pass, the sorted tables of `plan`: [narrow] or [narrow, wide] CountTables (count) /
+        singleton KeyArrays (uniq).  Concatenated in pass order they are the tables of count() / uniq()."""
+        vb = 4 if ((d.pos_offset + d.n_bases) << 1) < (1 << 32) else 8
+        for lo, hi in plan.parts:
+            if plan.n_parts == 1:
+                yield self.count(d, k, rc) if mode == "count" else self.uniq(d, k, rc)
+                continue
+            tabs = []
+            for wide, n_keys in ((False, int(plan.narrow[lo:hi].sum())), (True, int(plan.wide[lo:hi].sum()))):
+                if wide and not n_keys:
+                    break
+                a = self.extract_parts(d, k, rc, wide, 0 if mode == "count" else vb, plan.n_parts, lo, hi, n_keys)
+                tabs.append(self.sort_count(a) if mode == "count" else self.sort_uniq(a))
+                del a
+            yield tabs
+            del tabs
+
+    def _emit_chunks(self, sink: _ChunkSink, d: DeviceInput, k: int, mode: str, tabs: list, rows: int) -> None:
+        """Text of one pass (narrow table + optional wide table) in chunks of `rows` narrow rows; the wide
+        lines go into the chunk whose rows they sort among (merge_ranks)."""
+        per = 1 if mode == "count" else 2  # lines per row
+        nar = tabs[0]
+        n = nar.n
+        rw = np.zeros(0, np.int64)
+        wid = tabs[1] if len(tabs) > 1 and tabs[1].n else None
+        if wid is not None:
+            if n:
+                rn, rw_d = self.merge_ranks(nar.keys, n, wid.keys, wid.n, k, d.rna)
+                del rn
+                rw = rw_d.cpu().numpy()
+            else:
+                rw = np.zeros(wid.n, np.int64)
+
+        def fmt(t, lo: int, cnt: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+            if mode == "count":
+                part = CountTable(t.keys[lo * t.key_bytes:], t.counts[lo * 4:], cnt, t.key_bytes, k, t.wide)
+                return self.format_counts(part, d.rna, out)
+            part = KeyArray(t.keys[lo * t.key_bytes:], None, t.vals[lo * t.val_bytes:], None, cnt, t.key_bytes,
+                            t.val_bytes, k, t.wide, is_sorted=True)
+            return self.format_uniq(part, d, out)
+
+        starts = list(range(0, n, rows)) or [0]
+        for ci, lo in enumerate(starts):
+            hi = min(lo + rows, n)
+            last = ci == len(starts) - 1
+            jlo = int(np.searchsorted(rw, lo, "left"))
+            jhi = len(rw) if last else int(np.searchsorted(rw, hi, "left"))
+            buf = sink.buffer()
+            text = fmt(nar, lo, hi - lo, buf)
+            if jhi == jlo:
+                sink.submit(text, None)
+                continue
+            # wide lines of this chunk: host text + line boundaries; byte offsets of the narrow rows they precede
+            tw = fmt(wid, jlo, jhi - jlo).cpu().numpy()
+            w_ends = np.concatenate(([0], np.flatnonzero(tw == 10)[per - 1::per] + 1))
+            q = rw[jlo:jhi] - lo  # insert before narrow row q of the chunk
+            inner = np.unique(q[(q > 0) & (q < hi - lo)])
+            offs = {0: 0, hi - lo: int(text.numel())}
+            if inner.size:
+                nl = torch.nonzero(text == 10).flatten()
+                at = torch.from_numpy(inner * per - 1).to(self.device)
+                for qq, e in zip(inner.tolist(), (nl[at] + 1).cpu().numpy().tolist()):
+                    offs[qq] = int(e)
+                del nl
+            pieces, prev, j = [], 0, 0
+            while j < len(q):
+                j2 = j
+                while j2 < len(q) and q[j2] == q[j]:
+                    j2 += 1
+                o = offs[int(q[j])]
+                pieces.append((None, prev, o))
+                pieces.append((tw, int(w_ends[j]), int(w_ends[j2])))
+                prev, j = o, j2
+            pieces.append((None, prev, int(text.numel())))
+            sink.submit(text, pieces)
 
     # ---- text (interleaves the narrow and the wide stream in ASCII order) -----------------------
     def _interleave(self, texts: List[torch.Tensor], keys: List[torch.Tensor], ns: List[int], k: int, rna: int,

@@ -4,7 +4,8 @@
 uniq` commands make.  In the reference it is an n-way `heapq.merge` over every batch file
 plus a grouping loop (join.py:63-130).  Here, for `DeviceBatch` inputs, it is the GPU path:
 extract -> radix sort -> run-length (count) or singleton selection (uniq) -> text emission,
-then one write of the output file.  The emitted bytes equal the reference's
+in key-range passes when the input does not fit the device at once, streamed to the output
+file in chunks.  The emitted bytes equal the reference's
 (join.py:262 ">%s\\n%s\\n", join.py:284 "%s\\t%d\\n"); an empty result leaves an empty file.
 """
 from __future__ import annotations
@@ -186,12 +187,13 @@ class KJoiner:
                 oh.write(text)
             return
         d = self._merged_device_input(batches)
-        if self.mode == self.MODE.SEQ_COUNT:
-            text = b0._eng.count_text(d, b0.k, b0.reverse)
-        else:
-            text = b0._eng.uniq_text(d, b0.k, b0.reverse)
+        # key-range passes and chunked text: device memory is bounded by the largest pass, host memory by a
+        # text chunk (KMG_DEVICE_BUDGET overrides the device budget)
         with open(outpath, "wb") as oh:  # join.py:351 opens "w+": the file exists even when empty
-            oh.write(text)
+            if self.mode == self.MODE.SEQ_COUNT:
+                b0._eng.write_count(d, b0.k, b0.reverse, oh)
+            else:
+                b0._eng.write_uniq(d, b0.k, b0.reverse, oh)
 
     def join(self, batches: List[Any], outpath: str) -> None:
         live = [b for b in batches if b is not None and not (isinstance(b, Batch) and b.current_size == 0)]
