@@ -319,8 +319,7 @@ class DeviceBatch:
         if not self._written or force:
             if doSort:
                 with open(self.tmp, "wb") as th:
-                    for chunk in self._eng.batch_text_chunks(self.device_input, self.k, self.reverse):
-                        th.write(chunk)
+                    self._eng.write_batch(self.device_input, self.k, self.reverse, th)
             else:
                 with open(self.tmp, "w+") as th:
                     for r in self._records(do_sort=False):
@@ -385,9 +384,6 @@ class LoadedKmerBatch(DeviceBatch):
         super().__init__(engine, d, k, False, natype, tmp_dir, size=max(2, n))
         self._n = n
         self.paths = list(paths)
-
-    def count_text(self) -> bytes:
-        return self._eng.count_text(self.device_input, self.k, False)
 
     def uniq_text(self) -> bytes:
         """">HEADER\nSEQ\n" of the k-mers that occur once, ascending by sequence (join.py:243-263), with the

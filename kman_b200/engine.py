@@ -9,15 +9,18 @@ Stage -> reference mapping (see DESIGN.md):
   sort()           batch.py:156-168 + join.py:63-93         K3
   rle_count()      join.py:95-130 + :265-285                K4
   singletons()     join.py:95-130 + :243-263                K4
-  count_text()/uniq_text()  join.py:262,284; seq.py:103-104 K6 (+ narrow/wide rank merge)
+  format_counts()/format_uniq()  join.py:262,284; seq.py:103-104  K6
+  _write_text()    join.py:262,284; batch.py:281-296        K6 in chunks (+ narrow/wide rank merge): the one text
+                   writer behind write_count()/write_uniq()/write_batch() and count_text()/uniq_text()
 """
 from __future__ import annotations
 
 import ctypes as C
+import io
 import os
 from concurrent.futures import ThreadPoolExecutor
 from dataclasses import dataclass, field
-from typing import BinaryIO, Callable, Dict, List, Optional, Sequence, Tuple
+from typing import BinaryIO, Callable, Dict, Iterable, List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -65,6 +68,28 @@ class DeviceInput:
     @property
     def rna(self) -> int:
         return 1 if self.natype == ab.NATYPES.RNA else 0
+
+    @property
+    def payload_bytes(self) -> int:
+        """Bytes of a (global position << 1 | strand) payload: 4 while every position of the input fits."""
+        return 4 if ((self.pos_offset + self.n_bases) << 1) < (1 << 32) else 8
+
+
+def key_bytes(k: int, wide: bool) -> int:
+    """Bytes of one key: narrow 2-bit codes take 8 / 16 bytes, wide 4-bit codes 16 / 32 (k <= 32 / k <= 64)."""
+    return (16 if k <= 32 else 32) if wide else (8 if k <= 32 else 16)
+
+
+def window_range(d: DeviceInput, k: int, win_begin: int = 0, win_end: Optional[int] = None) -> Tuple[int, int]:
+    """[win_begin, win_end) clamped to the windows of the input; AssertionError for k <= 1 and ValueError for
+    k > 64, the reference's check and this build's limit."""
+    if k <= 1:
+        raise AssertionError(f"k must be >= 1, got {k} instead.")  # batcher.py:477-478
+    if k > 64:
+        raise ValueError(f"k={k}: this build supports k <= 64 (no CPU fallback)")
+    n_win_total = max(0, d.n_bases - k + 1)
+    win_end = n_win_total if win_end is None else min(win_end, n_win_total)
+    return min(win_begin, win_end), win_end
 
 
 @dataclass
@@ -156,7 +181,7 @@ def pass_bytes(k: int, mode: str, n: int, m: int, val_bytes: int, text_bytes: in
     grows, so the wide stage sees the larger of the two), the merge ranks, the extraction workspace and the
     text chunk buffers (`text_bytes`)."""
     lib = _lib.load()
-    kb, kw = (8, 16) if k <= 32 else (16, 32)
+    kb, kw = key_bytes(k, False), key_bytes(k, True)
     item = 4 if mode == "count" else val_bytes  # count / payload bytes per key
     if mode == "count":
         ws_n = lib.kmg_sort_count_workspace_bytes(n, kb, 2 * k)
@@ -293,6 +318,10 @@ class Engine:
     def _new(self, nbytes: int) -> torch.Tensor:
         return torch.empty(max(int(nbytes), 16), dtype=torch.uint8, device=self.device)
 
+    def _out(self, reuse: Optional[str], name: str, nbytes: int) -> torch.Tensor:
+        """Output buffer: the engine scratch `reuse + name` when `reuse` is given (the benchmark loop), else fresh."""
+        return self._buf(reuse + name, nbytes) if reuse else self._new(nbytes)
+
     def _status(self, ws: torch.Tensor) -> None:
         _lib.check(self.lib.kmg_ws_status(ws.data_ptr(), self._stream()))
 
@@ -419,28 +448,18 @@ class Engine:
 
         `reuse`: name prefix of engine-owned scratch buffers to place the output in (the
         benchmark loop) instead of fresh allocations."""
-        if k <= 1:
-            raise AssertionError(f"k must be >= 1, got {k} instead.")  # batcher.py:477-478
-        if k > 64:
-            raise ValueError(f"k={k}: this build supports k <= 64 (no CPU fallback)")
-        n_win_total = max(0, d.n_bases - k + 1)
-        win_end = n_win_total if win_end is None else min(win_end, n_win_total)
-        win_begin = min(win_begin, win_end)
+        win_begin, win_end = window_range(d, k, win_begin, win_end)
         n_win = win_end - win_begin
-        # narrow: 2-bit codes, 8 / 16 bytes; wide: 4-bit codes, 16 bytes up to k = 32, 32 bytes up to k = 64
-        kb = (16 if k <= 32 else 32) if wide else (8 if k <= 32 else 16)
+        kb = key_bytes(k, wide)
         cap = max(n_win * (2 if rc else 1), 1)
-        mk = (lambda nm, nb: self._buf(reuse + nm, nb)) if reuse else (lambda nm, nb: self._new(nb))
-        keys = mk("keys", cap * kb)
-        keys_alt = mk("keys_alt", cap * kb)
-        vals = mk("vals", cap * val_bytes) if val_bytes else None
-        vals_alt = mk("vals_alt", cap * val_bytes) if val_bytes else None
+        keys = self._out(reuse, "keys", cap * kb)
+        keys_alt = self._out(reuse, "keys_alt", cap * kb)
+        vals = self._out(reuse, "vals", cap * val_bytes) if val_bytes else None
+        vals_alt = self._out(reuse, "vals_alt", cap * val_bytes) if val_bytes else None
         ws_bytes = self.lib.kmg_extract_workspace_bytes(n_win)
         ws = self._buf("ws_extract", ws_bytes)
         # fused digit histograms for the sort that follows (narrow stream only)
-        hist = None
-        if want_hist and not wide and k >= 4:
-            hist = self._buf((reuse or "") + "hist", 16 * 256 * 8) if reuse else self._new(16 * 256 * 8)
+        hist = self._out(reuse, "hist", 16 * 256 * 8) if want_hist and not wide and k >= 4 else None
         _lib.check(
             self.lib.kmg_extract(
                 d.bases.data_ptr(), d.n_bases, win_begin, win_end, k, int(rc), int(wide), d.lut.data_ptr(),
@@ -498,7 +517,7 @@ class Engine:
         assert a.val_bytes == 0
         if a.key_bytes == 32:
             return self.rle_count(self.sort(a, 0, end_bit), reuse=reuse)
-        counts = self._buf(reuse + "counts", a.n * 4) if reuse else self._new(a.n * 4)
+        counts = self._out(reuse, "counts", a.n * 4)
         if a.n == 0:
             return CountTable(a.keys_alt, counts, 0, a.key_bytes, a.k, a.wide)
         ws_bytes = self.lib.kmg_sort_count_workspace_bytes(a.n, a.key_bytes, end_bit)
@@ -530,7 +549,7 @@ class Engine:
     def rle_count(self, a: KeyArray, reuse: Optional[str] = None) -> CountTable:
         """Distinct keys + counts.  The distinct keys are written into `a.keys_alt`."""
         assert a.is_sorted
-        counts = self._buf(reuse + "counts", a.n * 4) if reuse else self._new(a.n * 4)
+        counts = self._out(reuse, "counts", a.n * 4)
         if a.n == 0:
             return CountTable(a.keys_alt, counts, 0, a.key_bytes, a.k, a.wide)
         ws_bytes = self.lib.kmg_rle_workspace_bytes(a.n)
@@ -673,19 +692,12 @@ class Engine:
 
     def _pipeline_buffers(self, d: DeviceInput, k: int, rc: bool, val_bytes: int, reuse: Optional[str],
                           win_begin: int, win_end: Optional[int]):
-        if k <= 1:
-            raise AssertionError(f"k must be >= 1, got {k} instead.")  # batcher.py:477-478
-        if k > 64:
-            raise ValueError(f"k={k}: this build supports k <= 64 (no CPU fallback)")
-        n_win_total = max(0, d.n_bases - k + 1)
-        win_end = n_win_total if win_end is None else min(win_end, n_win_total)
-        win_begin = min(win_begin, win_end)
-        kb = 16 if k > 32 else 8
+        win_begin, win_end = window_range(d, k, win_begin, win_end)
+        kb = key_bytes(k, False)
         cap = max((win_end - win_begin) * (2 if rc else 1), 1)
-        mk = (lambda nm, nb: self._buf(reuse + nm, nb)) if reuse else (lambda nm, nb: self._new(nb))
-        keys, keys_alt = mk("keys", cap * kb), mk("keys_alt", cap * kb)
-        vals = mk("vals", cap * val_bytes) if val_bytes else None
-        vals_alt = mk("vals_alt", cap * val_bytes) if val_bytes else None
+        keys, keys_alt = self._out(reuse, "keys", cap * kb), self._out(reuse, "keys_alt", cap * kb)
+        vals = self._out(reuse, "vals", cap * val_bytes) if val_bytes else None
+        vals_alt = self._out(reuse, "vals_alt", cap * val_bytes) if val_bytes else None
         ws_bytes = self.lib.kmg_pipeline_workspace_bytes(win_end - win_begin, k, int(rc), val_bytes)
         ws = self._buf("ws_pipeline", ws_bytes)
         return win_begin, win_end, kb, cap, keys, keys_alt, vals, vals_alt, ws, ws_bytes
@@ -698,7 +710,7 @@ class Engine:
         to the wide stream.  seq.py:284-328 + batch.py:156-168 + join.py:63-130,265-285."""
         win_begin, win_end, kb, cap, keys, keys_alt, _, _, ws, ws_bytes = self._pipeline_buffers(
             d, k, rc, 0, reuse, win_begin, win_end)
-        counts = self._buf(reuse + "counts", cap * 4) if reuse else self._new(cap * 4)
+        counts = self._out(reuse, "counts", cap * 4)
         res = (C.c_uint64 * 4)()
         _lib.check(self.lib.kmg_extract_sort_count(d.bases.data_ptr(), d.n_bases, win_begin, win_end, k, int(rc),
                                                    d.lut.data_ptr(), keys.data_ptr(), keys_alt.data_ptr(),
@@ -710,7 +722,7 @@ class Engine:
                     win_end: Optional[int] = None, val_bytes: Optional[int] = None) -> Tuple[KeyArray, int]:
         """Singleton keys with their (position << 1 | strand) payload of the narrow stream in ONE native
         call (kmg_extract_sort_uniq), and the number of wide-stream windows.  join.py:243-263."""
-        vb = val_bytes or (4 if ((d.pos_offset + d.n_bases) << 1) < (1 << 32) else 8)
+        vb = val_bytes or d.payload_bytes
         win_begin, win_end, kb, cap, keys, keys_alt, vals, vals_alt, ws, ws_bytes = self._pipeline_buffers(
             d, k, rc, vb, reuse, win_begin, win_end)
         res = (C.c_uint64 * 4)()
@@ -731,7 +743,7 @@ class Engine:
 
     def uniq(self, d: DeviceInput, k: int, rc: bool = False) -> List[KeyArray]:
         """`kmer uniq` on device: singleton keys with payload, one KeyArray per stream."""
-        vb = 4 if ((d.pos_offset + d.n_bases) << 1) < (1 << 32) else 8
+        vb = d.payload_bytes
         sing, n_other = self.uniq_narrow(d, k, rc, val_bytes=vb)
         out = [sing]
         if n_other:
@@ -775,7 +787,7 @@ class Engine:
         """extract() restricted to the keys of parts [part_lo, part_hi) (kmg_extract_parts), into buffers of
         exactly `n_keys` keys (from part_counts)."""
         n_win = max(0, d.n_bases - k + 1)
-        kb = (16 if k <= 32 else 32) if wide else (8 if k <= 32 else 16)
+        kb = key_bytes(k, wide)
         keys, keys_alt = self._new(n_keys * kb), self._new(n_keys * kb)
         vals = self._new(n_keys * val_bytes) if val_bytes else None
         vals_alt = self._new(n_keys * val_bytes) if val_bytes else None
@@ -802,8 +814,8 @@ class Engine:
         lib = self.lib
         n_win = max(0, d.n_bases - k + 1)
         cap = max(n_win * (2 if rc else 1), 1)
-        kb, kw = (8, 16) if k <= 32 else (16, 32)
-        item = kb + (4 if mode == "count" else val_bytes)
+        kb, kw = key_bytes(k, False), key_bytes(k, True)
+        item = kb +(4 if mode == "count" else val_bytes)
         narrow = 2 * cap * item + lib.kmg_pipeline_workspace_bytes(n_win, k, int(rc), 0 if mode == "count" else val_bytes)
         if n_other:
             m = n_other * (2 if rc else 1)
@@ -844,7 +856,7 @@ class Engine:
         if mode not in ("count", "uniq"):
             raise AssertionError(f"unknown mode {mode!r}")
         budget = self.device_budget(d, budget_bytes)
-        vb = 4 if ((d.pos_offset + d.n_bases) << 1) < (1 << 32) else 8
+        vb = d.payload_bytes
         _, text_bytes = self._text_plan(d, k, mode, chunk_rows)
         n, n_other = self.count_windows(d, k, rc)
         one = self._one_pass_bytes(d, k, rc, mode, n_other, vb, text_bytes)
@@ -863,15 +875,43 @@ class Engine:
         """Write the bytes of uniq_text() to `fh` (see write_count)."""
         return self._write_passes(d, k, rc, fh, "uniq", budget_bytes, chunk_rows)
 
+    def write_batch(self, d: DeviceInput, k: int, rc: bool, fh: BinaryIO, chunk_rows: Optional[int] = None) -> None:
+        """Write the text of the reference's batch files (batch.py:281-296: every k-mer as
+        ">ref:start-end:strand\\nSEQ\\n", stably sorted by sequence, batch.py:156-168) to `fh` as one sorted
+        batch; how the reference splits records over files is not part of its contract (SURVEY.md f-3).  The
+        payload sorts are stable, so equal sequences keep their emission order."""
+        self._write_text(d, k, "uniq", fh, [self.sorted_streams(d, k, rc, d.payload_bytes)], chunk_rows)
+
+    def count_text(self, d: DeviceInput, k: int, rc: bool = False) -> bytes:
+        """Bytes of the reference's `kmer count` output file (join.py:284), from the whole-input path."""
+        fh = io.BytesIO()
+        self._write_text(d, k, "count", fh, [self.count(d, k, rc)])
+        return fh.getvalue()
+
+    def uniq_text(self, d: DeviceInput, k: int, rc: bool = False) -> bytes:
+        """Bytes of the reference's `kmer uniq` output file (join.py:262), from the whole-input path."""
+        fh = io.BytesIO()
+        self._write_text(d, k, "uniq", fh, [self.uniq(d, k, rc)])
+        return fh.getvalue()
+
     @_on_device
     def _write_passes(self, d: DeviceInput, k: int, rc: bool, fh: BinaryIO, mode: str, budget_bytes: Optional[int],
                       chunk_rows: Optional[int]) -> PassPlan:
-        if d.rec_starts is None and mode == "uniq":
+        if d.rec_starts is None and mode == "uniq":  # resident before the budget is taken
             self._upload_names(d)
         plan = self.plan_passes(d, k, rc, mode, budget_bytes, chunk_rows)
+        plan.pass_ms = self._write_text(d, k, mode, fh, self.pass_tables(d, k, rc, mode, plan), chunk_rows)
+        return plan
+
+    @_on_device
+    def _write_text(self, d: DeviceInput, k: int, mode: str, fh: BinaryIO, passes: Iterable[list],
+                    chunk_rows: Optional[int] = None) -> List[float]:
+        """Write the text of every table list of `passes` ([narrow] or [narrow, wide] sorted tables, formatted
+        as `mode` "count" or "uniq" lines) to `fh`, in chunks of `chunk_rows` narrow rows (default: 256 MB of
+        text) through one _ChunkSink.  Returns each list's time between CUDA events, its production included."""
         rows, _ = self._text_plan(d, k, mode, chunk_rows)
         sink = _ChunkSink(self, fh, rows * self._line_bytes(d, k, mode))
-        passes = self.pass_tables(d, k, rc, mode, plan)
+        passes, pass_ms = iter(passes), []
         try:
             while True:
                 t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -883,15 +923,15 @@ class Engine:
                 del tabs  # a pass's buffers are freed before the next pass allocates its own
                 t1.record()
                 t1.synchronize()
-                plan.pass_ms.append(t0.elapsed_time(t1))
+                pass_ms.append(t0.elapsed_time(t1))
         finally:
             sink.close()
-        return plan
+        return pass_ms
 
     def pass_tables(self, d: DeviceInput, k: int, rc: bool, mode: str, plan: PassPlan):
         """Yield, pass by pass, the sorted tables of `plan`: [narrow] or [narrow, wide] CountTables (count) /
         singleton KeyArrays (uniq).  Concatenated in pass order they are the tables of count() / uniq()."""
-        vb = 4 if ((d.pos_offset + d.n_bases) << 1) < (1 << 32) else 8
+        vb = d.payload_bytes
         for lo, hi in plan.parts:
             if plan.n_parts == 1:
                 yield self.count(d, k, rc) if mode == "count" else self.uniq(d, k, rc)
@@ -965,62 +1005,18 @@ class Engine:
             pieces.append((None, prev, int(text.numel())))
             sink.submit(text, pieces)
 
-    # ---- text (interleaves the narrow and the wide stream in ASCII order) -----------------------
-    def _interleave(self, texts: List[torch.Tensor], keys: List[torch.Tensor], ns: List[int], k: int, rna: int,
-                    line_lens: Optional[List[torch.Tensor]]) -> bytes:
-        if len(texts) == 1 or ns[1] == 0:
-            return texts[0].cpu().numpy().tobytes()
-        if ns[0] == 0:
-            return texts[1].cpu().numpy().tobytes()
-        rn, rw = self.merge_ranks(keys[0], ns[0], keys[1], ns[1], k, rna)
-        # merged position of every line, then a stable host-side interleave of the two texts
-        pos_n = (torch.arange(ns[0], device=self.device) + rn).cpu().numpy()
-        pos_w = (torch.arange(ns[1], device=self.device) + rw).cpu().numpy()
-        tn, tw = texts[0].cpu().numpy(), texts[1].cpu().numpy()
-
-        def line_starts(t: np.ndarray, per_rec: int) -> np.ndarray:
-            nl = np.flatnonzero(t == 10)
-            ends = nl[per_rec - 1 :: per_rec] + 1
-            return np.concatenate(([0], ends))
-
-        per = 1 if line_lens is None else 2
-        sn, sw = line_starts(tn, per), line_starts(tw, per)
-        total = ns[0] + ns[1]
-        lens = np.empty(total, np.int64)
-        lens[pos_n] = np.diff(sn)
-        lens[pos_w] = np.diff(sw)
-        offs = np.concatenate(([0], np.cumsum(lens)))
-        out = np.empty(int(offs[-1]), np.uint8)
-        # wide lines are few: copy the narrow text in runs between them
-        src_is_wide = np.zeros(total, bool)
-        src_is_wide[pos_w] = True
-        # narrow runs
-        idx_n = 0
-        prev = 0
-        for j, pw in enumerate(pos_w):
-            run = pw - prev  # narrow lines before this wide line
-            if run:
-                out[offs[prev] : offs[pw]] = tn[sn[idx_n] : sn[idx_n + run]]
-                idx_n += run
-            out[offs[pw] : offs[pw + 1]] = tw[sw[j] : sw[j + 1]]
-            prev = pw + 1
-        if prev < total:
-            out[offs[prev] :] = tn[sn[idx_n] :]
-        return out.tobytes()
-
     @_on_device
     def abundance(self, d: DeviceInput, k: int, rc: bool = False, masked: bool = False) -> Tuple[np.ndarray, np.ndarray]:
         """VEC_COUNT / VEC_COUNT_MASKED (join.py:287-335): per flat position the number of occurrences of the
         k-mer that starts there ('+' vector) / of its reverse complement ('-' vector); masked: occurrences
         in other records only.  Both streams are sorted stably with their payload, then every element
         scatters its group's size (kmg_abundance_scatter).  Returns host uint32 arrays over the flat buffer."""
-        vb = 4 if ((d.pos_offset + d.n_bases) << 1) < (1 << 32) else 8
         if d.rec_starts is None:
             self._upload_names(d)
         out = torch.zeros(2 * (d.n_bases + 1), dtype=torch.int32, device=self.device)
         plus, minus = out[: d.n_bases + 1], out[d.n_bases + 1:]
         err = torch.zeros(1, dtype=torch.int32, device=self.device)
-        for s in self.sorted_streams(d, k, rc, vb):
+        for s in self.sorted_streams(d, k, rc, d.payload_bytes):
             if s.n == 0:
                 continue
             _lib.check(self.lib.kmg_abundance_scatter(s.keys.data_ptr(), s.vals.data_ptr(), s.n, s.key_bytes, s.val_bytes,
@@ -1030,36 +1026,6 @@ class Engine:
             raise ValueError("a k-mer occurs more than 2^32-1 times: count does not fit uint32")
         host = out.cpu().numpy().view(np.uint32)
         return host[: d.n_bases + 1], host[d.n_bases + 1:]
-
-    def batch_text_chunks(self, d: DeviceInput, k: int, rc: bool = False, chunk: int = 8_000_000):
-        """Text of the reference's batch files (batch.py:281-296: every k-mer as ">ref:start-end:strand\nSEQ\n",
-        stably sorted by sequence, batch.py:156-168), formatted on the GPU and yielded as bytes in chunks of
-        `chunk` records.  How the records are split over files is not a contract of the reference
-        (SURVEY.md f-3); concatenating the chunks gives one sorted batch."""
-        vb = 4 if ((d.pos_offset + d.n_bases) << 1) < (1 << 32) else 8
-        streams = self.sorted_streams(d, k, rc, vb)  # stable payload sorts: equal sequences keep emission order
-        if len(streams) == 2 and streams[1].n:
-            texts = [self.format_uniq(s, d) for s in streams]
-            yield self._interleave(texts, [s.keys for s in streams], [s.n for s in streams], k, d.rna, [])
-            return
-        s = streams[0]
-        for lo in range(0, s.n, chunk):
-            m = min(chunk, s.n - lo)
-            part = KeyArray(s.keys[lo * s.key_bytes:], None, s.vals[lo * s.val_bytes:], None, m, s.key_bytes, s.val_bytes,
-                            k, False, is_sorted=True)
-            yield self.format_uniq(part, d).cpu().numpy().tobytes()
-
-    def count_text(self, d: DeviceInput, k: int, rc: bool = False) -> bytes:
-        """Bytes of the reference's `kmer count` output file (join.py:284)."""
-        tabs = self.count(d, k, rc)
-        texts = [self.format_counts(t, d.rna) for t in tabs]
-        return self._interleave(texts, [t.keys for t in tabs], [t.n for t in tabs], k, d.rna, None)
-
-    def uniq_text(self, d: DeviceInput, k: int, rc: bool = False) -> bytes:
-        """Bytes of the reference's `kmer uniq` output file (join.py:262)."""
-        sing = self.uniq(d, k, rc)
-        texts = [self.format_uniq(s, d) for s in sing]
-        return self._interleave(texts, [s.keys for s in sing], [s.n for s in sing], k, d.rna, [])
 
 
 _engines: Dict[int, Engine] = {}

@@ -182,9 +182,11 @@ class KJoiner:
             # `-B`: re-imported batch files carry their own headers (one LoadedKmerBatch covers a folder)
             if len(batches) != 1:
                 raise AssertionError("re-imported batch files cannot be joined together with other batches")
-            text = b0.count_text() if self.mode == self.MODE.SEQ_COUNT else b0.uniq_text()
             with open(outpath, "wb") as oh:
-                oh.write(text)
+                if self.mode == self.MODE.SEQ_COUNT:
+                    b0._eng.write_count(b0.device_input, b0.k, False, oh)
+                else:
+                    oh.write(b0.uniq_text())
             return
         d = self._merged_device_input(batches)
         # key-range passes and chunked text: device memory is bounded by the largest pass, host memory by a

@@ -1,6 +1,7 @@
 """Key-range passes on the GPU: kmg_extract_parts against kmg_extract filtered in numpy, per-pass tables
-against the golden table hashes, and write_count / write_uniq (and the command line) byte for byte
-against count_text / uniq_text and the reference's golden outputs under a forced multi-pass budget."""
+against the golden table hashes, write_count / write_uniq (and the command line) byte for byte against the
+oracle and the reference's golden outputs under a forced multi-pass budget, and write_batch in chunks
+against the oracle's batch file."""
 import io
 import json
 import os
@@ -64,11 +65,14 @@ def parts_of(a, k: int, n_parts: int, rna: int) -> np.ndarray:
     return wide_part_table(rna, n_parts)[field(keys, 4 * k - 16, 16)].astype(np.int64)
 
 
+IUPAC_RECS = iupac_records(300_000, 77)
+
+
 @pytest.fixture(scope="module")
 def dev_iupac(eng):
     from kman_b200 import fasta
 
-    return eng.upload(fasta.from_records(iupac_records(300_000, 77)), alphabet="IUPAC")
+    return eng.upload(fasta.from_records(IUPAC_RECS), alphabet="IUPAC")
 
 
 @pytest.mark.parametrize("k", [12, 25, 31, 33, 45, 63])
@@ -128,10 +132,9 @@ def forced_budget(eng, d, k, rc, mode, passes=4, chunk_rows=None, slack=0):
     from kman_b200.engine import pass_bytes
 
     narrow, wide = eng.part_counts(d, k, rc, 256)
-    vb = 4 if ((d.pos_offset + d.n_bases) << 1) < (1 << 32) else 8
     _, text_bytes = eng._text_plan(d, k, mode, chunk_rows)
     n_win = max(0, d.n_bases - k + 1)
-    cost = lambda a, b: pass_bytes(k, mode, a, b, vb, text_bytes, n_win)  # noqa: E731
+    cost = lambda a, b: pass_bytes(k, mode, a, b, d.payload_bytes, text_bytes, n_win)  # noqa: E731
     target = cost(-(-int(narrow.sum()) // passes), -(-int(wide.sum()) // passes))
     biggest = max(cost(int(a), int(b)) for a, b in zip(narrow, wide))
     return max(target, biggest) + eng._resident_bytes(d) + slack
@@ -181,8 +184,10 @@ def _write(eng, d, k, rc, mode, **kw) -> bytes:
 @pytest.mark.parametrize("k,rc", [(12, True), (25, False), (31, True), (40, True), (63, False)])
 @pytest.mark.parametrize("mode", ["count", "uniq"])
 def test_write_multi_pass_equals_text(eng, dev_iupac, k, rc, mode):
+    import kmer_oracle as ko
+
     d = dev_iupac
-    want = eng.count_text(d, k, rc) if mode == "count" else eng.uniq_text(d, k, rc)
+    want = (ko.count_text_np if mode == "count" else ko.uniq_text_np)(IUPAC_RECS, k, rc, "IUPAC")
     got, plan = _write(eng, d, k, rc, mode, chunk_rows=5000,
                        budget_bytes=forced_budget(eng, d, k, rc, mode, passes=6, chunk_rows=5000))
     assert plan.n_passes >= 4 and len(plan.pass_ms) == plan.n_passes
@@ -227,6 +232,8 @@ def test_write_matches_reference_goldens(eng, golden):
 
 
 def test_cli_multi_pass_output_file(eng, tmp_path):
+    import kmer_oracle as ko
+
     from kman_b200 import fasta
 
     recs = iupac_records(200_000, 5)
@@ -234,7 +241,7 @@ def test_cli_multi_pass_output_file(eng, tmp_path):
     fa.write_bytes(b"".join(b">%s\n%s\n" % (n.encode(), s.encode()) for n, s in recs))
     d = eng.upload(fasta.from_records(recs), alphabet="IUPAC")
     for mode, args, k, rc in (("count", [], 31, False), ("uniq", ["-r"], 27, True)):
-        want = eng.count_text(d, k, rc) if mode == "count" else eng.uniq_text(d, k, rc)
+        want = (ko.count_text_np if mode == "count" else ko.uniq_text_np)(recs, k, rc, "IUPAC")
         budget = forced_budget(eng, d, k, rc, mode, passes=4, slack=4 * fa.stat().st_size)
         out = tmp_path / f"out_{mode}.txt"
         env = dict(os.environ, PYTHONPATH=ROOT, KMG_ALPHABET="IUPAC", KMG_DEVICE_BUDGET=str(budget))
@@ -243,6 +250,26 @@ def test_cli_multi_pass_output_file(eng, tmp_path):
         assert out.read_bytes() == want, mode
         plan = eng.plan_passes(d, k, rc, mode, budget_bytes=budget)
         assert plan.n_passes >= 2
+
+
+@pytest.mark.parametrize("k", [7, 25, 40])
+def test_write_batch_in_chunks_equals_oracle(eng, k):
+    """`kmer batch`'s sorted export with N / IUPAC windows: in chunks of 3 and 1000 rows and in one chunk, the wide
+    lines fall inside chunks, at chunk edges and after the last narrow row (windows starting with Y sort after T)."""
+    import kmer_oracle as ko
+
+    from kman_b200 import fasta
+
+    rng = np.random.default_rng(500 + k)
+    s1 = "".join(rng.choice(list("ACGT"), size=5000))
+    s2 = "".join(rng.choice(list("ACGT"), size=3000))
+    recs = [("chrA first", s1 + s1[:800].lower() + "NNNNNNNNNNRY" + s1[100:400]), ("chrB", s2 + "N" + s2[:500] + "ACGTN")]
+    d = eng.upload(fasta.from_records(recs), alphabet="IUPAC")
+    (want,) = ko.batch_text_py(recs, k, True, alphabet="IUPAC")
+    for chunk_rows in (3, 1000, None):
+        fh = io.BytesIO()
+        eng.write_batch(d, k, True, fh, chunk_rows=chunk_rows)
+        assert fh.getvalue() == want, chunk_rows
 
 
 def test_empty_result_leaves_empty_output(eng):

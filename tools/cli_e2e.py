@@ -1,8 +1,10 @@
 #!/usr/bin/env python
-"""Wall-clock of the drop-in command line on a synthetic FASTA (file in, file out), per mode.
+"""Wall-clock of the drop-in command line on a synthetic FASTA (file in, file out), per mode: `kmer count`,
+`kmer uniq` and `kmer batch` (sorted batch files in an output folder).
 usage: python tools/cli_e2e.py [--n 20000000] [--k 31]"""
 import argparse
 import os
+import shutil
 import subprocess
 import sys
 import tempfile
@@ -26,13 +28,17 @@ with open(fa, "wb") as fh:
         fh.write(np.concatenate([lines, np.full((lines.shape[0], 1), 10, np.uint8)], axis=1).tobytes())
     else:
         fh.write(seq.tobytes() + b"\n")
-env = dict(os.environ, PYTHONPATH=ROOT, KMG_ALPHABET="ACGT")
-for mode in ("count", "uniq"):
-    out = os.path.join(tmp, f"out_{mode}.txt")
-    t0 = time.perf_counter()
-    subprocess.run([sys.executable, "-m", "kman_b200.scripts.kmer", mode, fa, out, str(args.k)], check=True, env=env,
-                   stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
-    dt = time.perf_counter() - t0
-    sz = os.path.getsize(out)
-    print(f"kmer {mode}: {args.n} bp, k={args.k}: {dt:.2f} s wall (python start + CUDA init + FASTA load + GPU + {sz/1e6:.0f} MB of text written) "
-          f"= {(args.n - args.k + 1)/dt/1e6:.1f} M k-mers/s")
+env = dict(os.environ, PYTHONPATH=ROOT, KMG_ALPHABET="ACGT", TMPDIR=tmp)
+try:
+    for mode in ("count", "uniq", "batch"):
+        out = os.path.join(tmp, f"out_{mode}")
+        t0 = time.perf_counter()
+        subprocess.run([sys.executable, "-m", "kman_b200.scripts.kmer", mode, fa, out, str(args.k)], check=True, env=env,
+                       stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+        dt = time.perf_counter() - t0
+        files = [os.path.join(out, f) for f in os.listdir(out)] if os.path.isdir(out) else [out]
+        sz = sum(os.path.getsize(f) for f in files)
+        print(f"kmer {mode}: {args.n} bp, k={args.k}: {dt:.2f} s wall (python start + CUDA init + FASTA load + GPU + {sz/1e6:.0f} MB of text written) "
+              f"= {(args.n - args.k + 1)/dt/1e6:.1f} M k-mers/s")
+finally:
+    shutil.rmtree(tmp)
