@@ -291,6 +291,17 @@ int kmg_fasta_flatten(const uint8_t* d_raw, uint64_t n_raw, uint8_t* d_bases_out
 int kmg_abundance_scatter(const void* d_sorted_keys, const void* d_vals, uint64_t n, int key_bytes, int val_bytes,
                           const uint64_t* d_rec_starts, uint32_t n_rec, int masked, uint64_t pos_base,
                           uint32_t* d_out_plus, uint32_t* d_out_minus, uint32_t* d_err, void* stream);
+/* Length of every record's vector (abundance.py:137-146: a vector ends at its last written entry), computed where
+ * the vectors live.  d_plus / d_minus cover flat positions [0, n); record r covers [d_rec_starts[r],
+ * d_rec_starts[r+1] - 1).  d_lengths_out[2r + s] (s = 0 '+', 1 '-') = last non-zero position of the record's
+ * strand-s vector + 1 - d_rec_starts[r], or 0 if that vector is all zeros. */
+int kmg_vector_extents(const uint32_t* d_plus, const uint32_t* d_minus, uint64_t n, const uint64_t* d_rec_starts,
+                       uint32_t n_rec, uint64_t* d_lengths_out, void* stream);
+/* The text of n vector entries, "%d\n" per entry (abundance.py:168-172; the "# k=K" header line is the caller's),
+ * formatted with the tile prefix of kmg_format_counts.  *d_bytes_out = total bytes; d_text_out capacity must be
+ * 11*n.  Workspace: kmg_format_workspace_bytes(n). */
+int kmg_format_vector(const uint32_t* d_counts, uint64_t n, uint8_t* d_text_out, uint64_t* d_bytes_out, void* d_ws,
+                      size_t ws_bytes, void* stream);
 
 /* ---- merge ranks between the narrow and the wide stream -------------------------------
  * For two sorted, disjoint key lists, rank_of_wide[i] = number of narrow keys that sort

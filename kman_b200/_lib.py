@@ -45,6 +45,8 @@ SIGNATURES = {
     "kmg_extract_sort_count": (i32, [vp, u64, u64, u64, i32, i32, vp, vp, vp, vp, u64p, vp, sz, vp]),
     "kmg_extract_sort_uniq": (i32, [vp, u64, u64, u64, i32, i32, vp, vp, vp, vp, vp, i32, u64, u64p, vp, sz, vp]),
     "kmg_abundance_scatter": (i32, [vp, vp, u64, i32, i32, vp, C.c_uint32, i32, u64, vp, vp, vp, vp]),
+    "kmg_vector_extents": (i32, [vp, vp, u64, vp, C.c_uint32, vp, vp]),
+    "kmg_format_vector": (i32, [vp, u64, vp, vp, vp, sz, vp]),
     "kmg_sort256_workspace_bytes": (sz, [u64]),
     "kmg_sort256": (i32, [vp, vp, vp, vp, u64, i32, i32, vp, sz, vp]),
     "kmg_merge_ranks_wide": (i32, [vp, u64, vp, u64, i32, i32, vp, vp, vp, vp]),

@@ -10,14 +10,15 @@ reference with that one abstract method neutralised (tests/golden/golden_vec.jso
 
 Two producers fill the same files: the host classes below (records fed one by one through
 KJoiner.join_vector_count*, the reference's protocol for host batches) and the device path
-(`device_vectors`: run lengths scattered back through the window positions by kmg_abundance_scatter).
+(Engine.write_vectors: run lengths scattered back through the window positions by kmg_abundance_scatter in
+key-range passes, the text formatted on the device; `device_vectors` returns the same vectors as arrays).
 The reference's LOCAL memory mode keeps the vectors in HDF5 files while joining (abundance.py:175-303);
 here LOCAL and NORMAL differ in nothing: the vectors live in device memory either way."""
 from __future__ import annotations
 
 import gzip
 import os
-from typing import Dict, Set
+from typing import Dict, Iterable, List, Set, Tuple
 
 import numpy as np
 
@@ -44,17 +45,30 @@ def vector_text(counts: np.ndarray, k: int) -> bytes:
     return b"# k=%d\n" % k + out.tobytes()
 
 
-def write_vectors(vectors: Dict[str, Dict[str, np.ndarray]], k: int, dirpath: str) -> None:
-    """abundance.py:148-172: the extension is removed from `dirpath`; one gz file per (ref, strand)."""
+def vector_paths(dirpath: str, vectors: Iterable[Tuple[str, str]]) -> List[str]:
+    """abundance.py:148-172: the extension is removed from `dirpath`, which must not be a file and is created
+    (also when no vector follows); the path of the gz file of every (ref, strand) in `vectors`."""
     dirpath = os.path.splitext(dirpath)[0]
     if os.path.isfile(dirpath):
         raise AssertionError
     print('Writing output in "%s"' % dirpath)
     os.makedirs(dirpath, exist_ok=True)
-    for ref, per in vectors.items():
-        for strand, vec in per.items():
-            with gzip.open(os.path.join(dirpath, "%s___%s.gz" % (ref, strand)), "wb") as oh:
-                oh.write(vector_text(vec, k))
+    return [os.path.join(dirpath, "%s___%s.gz" % (ref, strand)) for ref, strand in vectors]
+
+
+def check_unique_names(names: List[str]) -> None:
+    if len(set(names)) != len(names):
+        # two records of one name write the same vector: the reference refuses the second write
+        raise AssertionError("can't update non-zero count w/o replace: records share a name")
+
+
+def write_vectors(vectors: Dict[str, Dict[str, np.ndarray]], k: int, dirpath: str) -> None:
+    """Host vectors to files: one gz file per (ref, strand) (see vector_paths; the device writer is
+    Engine.write_vectors)."""
+    keys = [(ref, strand) for ref, per in vectors.items() for strand in per]
+    for (ref, strand), path in zip(keys, vector_paths(dirpath, keys)):
+        with gzip.open(path, "wb") as oh:
+            oh.write(vector_text(vectors[ref][strand], k))
 
 
 class AbundanceVectorBase:
@@ -98,9 +112,7 @@ def device_vectors(engine, d, k: int, rc: bool, masked: bool) -> Dict[str, Dict[
     """{ref: {"+"/"-": counts}} of one DeviceInput, computed on the GPU.  A vector ends at its last
     non-zero entry (add_ref grows it only up to the positions that were written, abundance.py:137-146)."""
     names = d.flat.names
-    if len(set(names)) != len(names):
-        # two records of one name write the same vector: the reference refuses the second write
-        raise AssertionError("can't update non-zero count w/o replace: records share a name")
+    check_unique_names(names)
     plus, minus = engine.abundance(d, k, rc, masked)
     starts = d.flat.rec_starts.astype(np.int64)
     out: Dict[str, Dict[str, np.ndarray]] = {}

@@ -88,6 +88,65 @@ __global__ void __launch_bounds__(256) abundance_scatter_kernel(const KeyT* __re
     ((v & 1) ? out_minus : out_plus)[pos - pos_base] = (uint32_t)cnt;
 }
 
+// Length of every (record, strand) vector: its last non-zero position + 1 (abundance.py:137-146 grows a
+// vector only up to the positions that were written).  One tile of EXT_TILE positions per block and
+// strand; a tile inside one record (all but at most n_rec - 1 of them) reduces to one atomicMax.
+constexpr int EXT_BLOCK = 256;
+constexpr int EXT_ITEMS = 16;
+constexpr uint64_t EXT_TILE = (uint64_t)EXT_BLOCK * EXT_ITEMS;
+
+__device__ __forceinline__ uint32_t record_of(const uint64_t* __restrict__ rec_starts, uint32_t n_rec, uint64_t pos) {
+    uint32_t lo = 0, hi = n_rec;  // last r with rec_starts[r] <= pos
+    while (hi - lo > 1) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (rec_starts[mid] <= pos) lo = mid;
+        else hi = mid;
+    }
+    return lo;
+}
+
+__global__ void __launch_bounds__(EXT_BLOCK) vector_extents_kernel(const uint32_t* __restrict__ plus,
+                                                                   const uint32_t* __restrict__ minus, uint64_t n,
+                                                                   const uint64_t* __restrict__ rec_starts, uint32_t n_rec,
+                                                                   unsigned long long* __restrict__ lengths) {
+    __shared__ uint32_t s_rec[2];
+    __shared__ unsigned long long s_max[EXT_BLOCK / 32];
+    const uint32_t strand = blockIdx.y;
+    const uint32_t* __restrict__ v = strand ? minus : plus;
+    const uint64_t base = (uint64_t)blockIdx.x * EXT_TILE;
+    const uint64_t end = min(base + EXT_TILE, n);
+    if (threadIdx.x == 0) {
+        s_rec[0] = record_of(rec_starts, n_rec, base);
+        s_rec[1] = record_of(rec_starts, n_rec, end - 1);
+    }
+    __syncthreads();
+    const uint32_t r0 = s_rec[0];
+    const bool one_record = r0 == s_rec[1];
+    unsigned long long last = 0;  // one past the last non-zero position seen (0: none)
+#pragma unroll
+    for (int j = 0; j < EXT_ITEMS; ++j) {
+        const uint64_t i = base + (uint64_t)j * EXT_BLOCK + threadIdx.x;
+        if (i >= end || v[i] == 0) continue;
+        if (one_record) {
+            last = i + 1;
+        } else {
+            const uint32_t r = record_of(rec_starts, n_rec, i);
+            atomicMax(&lengths[2 * r + strand], (unsigned long long)(i + 1 - rec_starts[r]));
+        }
+    }
+    if (!one_record) return;  // (uniform across the block)
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) last = max(last, __shfl_xor_sync(0xffffffffu, last, o));
+    if ((threadIdx.x & 31) == 0) s_max[threadIdx.x >> 5] = last;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        unsigned long long m = 0;
+#pragma unroll
+        for (int w = 0; w < EXT_BLOCK / 32; ++w) m = max(m, s_max[w]);
+        if (m) atomicMax(&lengths[2 * r0 + strand], m - rec_starts[r0]);
+    }
+}
+
 }  // namespace kmg
 
 using namespace kmg;
@@ -117,6 +176,21 @@ extern "C" int kmg_abundance_scatter(const void* d_sorted_keys, const void* d_va
         else KMG_AB_LAUNCH(u256, uint64_t);
     }
 #undef KMG_AB_LAUNCH
+    KMG_LAUNCH_CHECK();
+    return KMG_OK;
+}
+
+extern "C" int kmg_vector_extents(const uint32_t* d_plus, const uint32_t* d_minus, uint64_t n, const uint64_t* d_rec_starts,
+                                  uint32_t n_rec, uint64_t* d_lengths_out, void* stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    KMG_REQUIRE(d_lengths_out && d_rec_starts && n_rec >= 1, KMG_ERR_ARG, "null pointer argument");
+    KMG_CUDA(cudaMemsetAsync(d_lengths_out, 0, 2 * (size_t)n_rec * sizeof(uint64_t), st));
+    if (n == 0) return KMG_OK;
+    KMG_REQUIRE(d_plus && d_minus, KMG_ERR_ARG, "null pointer argument");
+    const uint64_t tiles = (n + EXT_TILE - 1) / EXT_TILE;
+    KMG_REQUIRE(tiles < (1ull << 31), KMG_ERR_RANGE, "too many positions");
+    vector_extents_kernel<<<dim3((unsigned)tiles, 2), EXT_BLOCK, 0, st>>>(d_plus, d_minus, n, d_rec_starts, n_rec,
+                                                                         (unsigned long long*)d_lengths_out);
     KMG_LAUNCH_CHECK();
     return KMG_OK;
 }

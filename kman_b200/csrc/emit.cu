@@ -183,6 +183,59 @@ __global__ void __launch_bounds__(FMT_BLOCK) format_uniq_kernel(const FmtParams 
     }
 }
 
+// "COUNT\n" per entry of an abundance vector (abundance.py:168-172): the tile scheme of format_counts_kernel
+// with lines of 2..11 bytes.
+__global__ void __launch_bounds__(FMT_BLOCK) format_vector_kernel(const FmtParams p) {
+    __shared__ uint8_t s_text[FMT_TILE * 11];
+    __shared__ uint32_t s_scan[FMT_BLOCK / 32 + 1];
+    __shared__ uint32_t s_tile;
+    __shared__ uint64_t s_base;
+    const int t = threadIdx.x;
+    if (t == 0) s_tile = atomicAdd(p.ticket, 1u);
+    __syncthreads();
+    const uint32_t tile = s_tile;
+    const uint64_t first = (uint64_t)tile * FMT_TILE + (uint64_t)t * FMT_RPT;
+    const uint32_t* counts = reinterpret_cast<const uint32_t*>(p.second);
+
+    uint32_t cnt[FMT_RPT], nd[FMT_RPT], len = 0;
+#pragma unroll
+    for (int r = 0; r < FMT_RPT; ++r) {
+        const uint64_t i = first + r;
+        cnt[r] = i < p.n ? counts[i] : 0;
+        nd[r] = i < p.n ? ndigits_u64(cnt[r]) : 0;
+        if (i < p.n) len += nd[r] + 1;
+    }
+    uint32_t total;
+    uint32_t off = block_excl_scan<FMT_BLOCK, uint32_t>(len, s_scan, total);
+    if (t < 32) {
+        const uint64_t e = tile_prefix_exclusive_warp(p.state, gridDim.x, tile, total, p.err);
+        if (t == 0) {
+            s_base = e;
+            if (tile == gridDim.x - 1) *p.bytes_out = e + total;
+        }
+    }
+#pragma unroll
+    for (int r = 0; r < FMT_RPT; ++r) {
+        if (first + r >= p.n) break;
+        put_decimal(s_text + off, cnt[r], nd[r]);
+        s_text[off + nd[r]] = '\n';
+        off += nd[r] + 1;
+    }
+    __syncthreads();
+    uint8_t* out = p.text + s_base;
+    const uint32_t mis = (uint32_t)((4 - ((uintptr_t)out & 3)) & 3);
+    const uint32_t head = mis < total ? mis : total;
+    if ((uint32_t)t < head) out[t] = s_text[t];
+    const uint32_t words = (total - head) / 4;
+    uint32_t* out32 = reinterpret_cast<uint32_t*>(out + head);
+    for (uint32_t w = t; w < words; w += FMT_BLOCK) {
+        const uint8_t* s = s_text + head + 4 * w;
+        out32[w] = (uint32_t)s[0] | ((uint32_t)s[1] << 8) | ((uint32_t)s[2] << 16) | ((uint32_t)s[3] << 24);
+    }
+    const uint32_t done = head + 4 * words;
+    if (done + t < total) out[done + t] = s_text[done + t];
+}
+
 // ---- narrow/wide merge ranks ---------------------------------------------------------------------
 // For a wide key W (4-bit ASCII-rank symbols, at least one of them not a plain base) let j be
 // the first non-plain symbol and c the number of plain bases whose letter sorts before it.
@@ -364,6 +417,27 @@ extern "C" int kmg_format_uniq(const void* d_keys, const void* d_vals, uint64_t 
         if (val_bytes == 4) format_uniq_kernel<u256, 4><<<tiles, FMT_BLOCK, 0, st>>>(p);
         else format_uniq_kernel<u256, 8><<<tiles, FMT_BLOCK, 0, st>>>(p);
     }
+    KMG_LAUNCH_CHECK();
+    return KMG_OK;
+}
+
+extern "C" int kmg_format_vector(const uint32_t* d_counts, uint64_t n, uint8_t* d_text_out, uint64_t* d_bytes_out,
+                                 void* d_ws, size_t ws_bytes, void* stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    KMG_REQUIRE(d_bytes_out, KMG_ERR_ARG, "d_bytes_out is null");
+    KMG_CUDA(cudaMemsetAsync(d_bytes_out, 0, sizeof(uint64_t), st));
+    if (n == 0) return KMG_OK;
+    KMG_REQUIRE(d_counts && d_text_out, KMG_ERR_ARG, "null pointer argument");
+    FmtParams p;
+    memset(&p, 0, sizeof(p));
+    uint32_t tiles = 0;
+    int rcode = fmt_setup(p, n, FMT_TILE, d_ws, ws_bytes, tiles, st);
+    if (rcode != KMG_OK) return rcode;
+    p.second = d_counts;
+    p.n = n;
+    p.text = d_text_out;
+    p.bytes_out = reinterpret_cast<unsigned long long*>(d_bytes_out);
+    format_vector_kernel<<<tiles, FMT_BLOCK, 0, st>>>(p);
     KMG_LAUNCH_CHECK();
     return KMG_OK;
 }

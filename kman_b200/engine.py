@@ -12,6 +12,8 @@ Stage -> reference mapping (see DESIGN.md):
   format_counts()/format_uniq()  join.py:262,284; seq.py:103-104  K6
   _write_text()    join.py:262,284; batch.py:281-296        K6 in chunks (+ narrow/wide rank merge): the one text
                    writer behind write_count()/write_uniq()/write_batch() and count_text()/uniq_text()
+  write_vectors()  join.py:287-335 + abundance.py:104-172      vectors filled pass by pass, trimmed and formatted on
+                   the device, gzipped on host threads (abundance() returns the same vectors as host arrays)
 """
 from __future__ import annotations
 
@@ -145,6 +147,8 @@ class CountTable:
 PASS_PARTS = 256  # parts of a multi-pass plan: the top 8 key bits (first 4 bases)
 DEVICE_HEADROOM = 2 << 30  # bytes of free device memory a default budget leaves alone (allocator, context)
 TEXT_CHUNK_BYTES = 256 << 20  # device text of one chunk (two of them on the device, two pinned on the host)
+VEC_CHUNK_ROWS = 1 << 20  # vector entries per text chunk of write_vectors (at most 11 bytes each)
+VEC_GZIP_THREADS = min(16, os.cpu_count() or 1)  # write_vectors: files compressed at once (two chunk buffers each)
 
 
 def wide_part_table(rna: int, n_parts: int) -> np.ndarray:
@@ -179,9 +183,22 @@ def pass_bytes(k: int, mode: str, n: int, m: int, val_bytes: int, text_bytes: in
     """Device bytes of one pass over n narrow and m wide keys: key (+ payload) buffers and their alternates,
     counts, the sort workspace from the library's own *_workspace_bytes (one buffer the engine keeps and
     grows, so the wide stage sees the larger of the two), the merge ranks, the extraction workspace and the
-    text chunk buffers (`text_bytes`)."""
+    text chunk buffers (`text_bytes`).
+
+    mode "vec" (abundance vectors): keys + payload and their alternates and the stable payload sort's workspace
+    per stream.  The narrow buffers are freed before the wide stream is extracted, so a pass costs the larger
+    stage, not their sum, and there is no merge term; the text stage comes after the passes, with only the
+    (kept) sort workspaces beside it."""
     lib = _lib.load()
     kb, kw = key_bytes(k, False), key_bytes(k, True)
+    if mode == "vec":
+        ws_n = lib.kmg_radix_sort_workspace_bytes(n, kb, val_bytes, 0, 2 * k)
+        if kw == 32:  # kmg_sort256 has a workspace of its own, next to the narrow sort's
+            ws = ws_n + lib.kmg_sort256_workspace_bytes(m)
+        else:
+            ws = max(ws_n, lib.kmg_radix_sort_workspace_bytes(m, kw, val_bytes, 0, 4 * k))
+        stages = max(2 * n * (kb + val_bytes) + ws_n, 2 * m * (kw + val_bytes) + ws, ws + text_bytes)
+        return int(stages + lib.kmg_extract_workspace_bytes(n_win))
     item = 4 if mode == "count" else val_bytes  # count / payload bytes per key
     if mode == "count":
         ws_n = lib.kmg_sort_count_workspace_bytes(n, kb, 2 * k)
@@ -200,10 +217,11 @@ def pass_bytes(k: int, mode: str, n: int, m: int, val_bytes: int, text_bytes: in
 
 @dataclass
 class PassPlan:
-    """How write_count / write_uniq split the key space.  n_parts == 1: one pass on the whole-input path
-    (count() / uniq()); otherwise parts[i] = (lo, hi) of pass i over `n_parts` parts with `narrow[p]` /
-    `wide[p]` keys in part p, and pass_bytes[i] its modelled device bytes.  pass_ms[i]: time of pass i
-    between CUDA events (filled in by write_count / write_uniq)."""
+    """How write_count / write_uniq / write_vectors split the key space.  n_parts == 1: one pass on the
+    whole-input path (count() / uniq() / unfiltered extraction); otherwise parts[i] = (lo, hi) of pass i over
+    `n_parts` parts with `narrow[p]` / `wide[p]` keys in part p, and pass_bytes[i] its modelled device bytes.
+    pass_ms[i]: time of pass i between CUDA events (filled in by the writers).  text_ms: write_vectors' text
+    stage (device formatting and copies, waits for a free chunk buffer included)."""
 
     n_parts: int
     parts: List[Tuple[int, int]]
@@ -211,6 +229,7 @@ class PassPlan:
     wide: np.ndarray
     pass_bytes: List[int] = field(default_factory=list)
     pass_ms: List[float] = field(default_factory=list)
+    text_ms: float = 0.0
 
     @property
     def n_passes(self) -> int:
@@ -235,29 +254,34 @@ def make_plan(k: int, budget: int, one_pass_bytes: int, totals: Tuple[int, int],
 
 
 class _ChunkSink:
-    """Double-buffered device text -> pinned host buffer -> file: the copy of chunk i runs on a copy
-    stream and its file write on a worker thread while the GPU formats chunk i+1."""
+    """Device text -> pinned host buffer -> file through `slots` buffer pairs: the copy of a chunk runs on a
+    copy stream and its file write on one of `workers` threads while the GPU formats the next chunks.  Every
+    submit names its file (default `fh`); writes to one file keep their submission order, writes to different
+    files run in parallel.  With the defaults (two slots, one worker, one file) this is plain double buffering."""
 
-    def __init__(self, eng: "Engine", fh: BinaryIO, nbytes: int):
+    def __init__(self, eng: "Engine", fh: Optional[BinaryIO], nbytes: int, slots: int = 2, workers: int = 1):
         self.fh = fh
-        self.dev = [eng._new(nbytes), eng._new(nbytes)]
-        self.pinned = [torch.empty(max(nbytes, 16), dtype=torch.uint8, pin_memory=True) for _ in range(2)]
+        self.dev = [eng._new(nbytes) for _ in range(slots)]
+        self.pinned = [torch.empty(max(nbytes, 16), dtype=torch.uint8, pin_memory=True) for _ in range(slots)]
         self.stream = torch.cuda.Stream(eng.device)
-        self.pool = ThreadPoolExecutor(1)
-        self.pending = [None, None]
+        self.pool = ThreadPoolExecutor(workers)
+        self.pending = [None] * slots
+        self.last: dict = {}  # file -> future of the latest task submitted for it
         self.slot = 0
 
     def buffer(self) -> torch.Tensor:
-        """Device buffer of the next chunk (free once the write of the chunk before last is done)."""
+        """Device buffer of the next chunk (free once the write of the chunk `slots` submits back is done)."""
         s = self.slot
         if self.pending[s] is not None:
             self.pending[s].result()
             self.pending[s] = None
         return self.dev[s]
 
-    def submit(self, text: torch.Tensor, pieces: Optional[List[Tuple[Optional[np.ndarray], int, int]]]) -> None:
-        """Write `text` (a prefix of buffer()); pieces: (None, a, b) = text[a:b], (arr, a, b) = arr[a:b]
+    def submit(self, text: torch.Tensor, pieces: Optional[List[Tuple[Optional[np.ndarray], int, int]]],
+               fh: Optional[BinaryIO] = None) -> None:
+        """Write `text` (a prefix of buffer()) to `fh`; pieces: (None, a, b) = text[a:b], (arr, a, b) = arr[a:b]
         in this order, or None for the whole text."""
+        fh = self.fh if fh is None else fh
         s, nb = self.slot, int(text.numel())
         ready = torch.cuda.Event()
         ready.record()
@@ -268,21 +292,34 @@ class _ChunkSink:
                 self.pinned[s][:nb].copy_(text, non_blocking=True)
             done.record()
         host = self.pinned[s].numpy()
-        self.pending[s] = self.pool.submit(self._write, done, host, nb, pieces)
-        self.slot ^= 1
+        # FIFO workers: the task a write waits for was taken up before it, so the wait always ends
+        self.pending[s] = self.last[fh] = self.pool.submit(self._write, self.last.get(fh), done, host, nb, pieces, fh)
+        self.slot = (s + 1) % len(self.dev)
 
-    def _write(self, done, host: np.ndarray, nb: int, pieces) -> None:
+    def then(self, fh: BinaryIO, fn: Callable[[], None]) -> None:
+        """Run fn() on a worker once every write to `fh` submitted so far is done (e.g. close the file)."""
+        self.last[fh] = self.pool.submit(self._after, self.last.get(fh), fn)
+
+    @staticmethod
+    def _after(prev, fn) -> None:
+        if prev is not None:
+            prev.result()
+        fn()
+
+    def _write(self, prev, done, host: np.ndarray, nb: int, pieces, fh: BinaryIO) -> None:
+        if prev is not None:
+            prev.result()
         done.synchronize()
         if pieces is None:
-            self.fh.write(memoryview(host[:nb]))
+            fh.write(memoryview(host[:nb]))
             return
         for arr, a, b in pieces:
             if b > a:
-                self.fh.write(memoryview((host if arr is None else arr)[a:b]))
+                fh.write(memoryview((host if arr is None else arr)[a:b]))
 
     def close(self) -> None:
         try:
-            for f in self.pending:
+            for f in [*self.pending, *self.last.values()]:
                 if f is not None:
                     f.result()
         finally:
@@ -804,7 +841,9 @@ class Engine:
         return KeyArray(keys, keys_alt, vals, vals_alt, n, kb, val_bytes, k, wide)
 
     def _line_bytes(self, d: DeviceInput, k: int, mode: str) -> int:
-        """Text capacity per row that format_counts / format_uniq require."""
+        """Text capacity per row that format_counts / format_uniq / format_vector require."""
+        if mode == "vec":
+            return 11
         return k + 12 if mode == "count" else k + 48 + max((len(nm) for nm in d.flat.names), default=0)
 
     def _one_pass_bytes(self, d: DeviceInput, k: int, rc: bool, mode: str, n_other: int, val_bytes: int,
@@ -814,6 +853,8 @@ class Engine:
         lib = self.lib
         n_win = max(0, d.n_bases - k + 1)
         cap = max(n_win * (2 if rc else 1), 1)
+        if mode == "vec":  # extract() with window-sized buffers, one stream at a time
+            return pass_bytes(k, mode, cap, cap if n_other else 0, val_bytes, text_bytes, n_win)
         kb, kw = key_bytes(k, False), key_bytes(k, True)
         item = kb +(4 if mode == "count" else val_bytes)
         narrow = 2 * cap * item + lib.kmg_pipeline_workspace_bytes(n_win, k, int(rc), 0 if mode == "count" else val_bytes)
@@ -841,23 +882,33 @@ class Engine:
         return int(free + cached - DEVICE_HEADROOM)
 
     def _text_plan(self, d: DeviceInput, k: int, mode: str, chunk_rows: Optional[int]) -> Tuple[int, int]:
-        """(rows per text chunk, device bytes of the text stage: two chunk buffers + the newline index)."""
+        """(rows per text chunk, device bytes of the text stage: two chunk buffers + the newline index; for
+        "vec" two chunk buffers per gzip worker, chunks no longer than the longest record and by default no more
+        buffer rows than bases)."""
         line = self._line_bytes(d, k, mode)
+        if mode == "vec":
+            workers = self._vec_workers(d)
+            longest = int(np.diff(d.flat.rec_starts.astype(np.int64)).max(initial=1))
+            rows = max(1, min(chunk_rows or min(VEC_CHUNK_ROWS, -(-d.n_bases // (2 * workers))), longest))
+            return rows, 2 * workers * rows * line + self.lib.kmg_format_workspace_bytes(rows)
         rows = max(1, chunk_rows or TEXT_CHUNK_BYTES // line)
         return rows, 2 * rows * line + rows * line + rows * (2 if mode == "uniq" else 1) * 8
 
     @_on_device
     def plan_passes(self, d: DeviceInput, k: int, rc: bool, mode: str, budget_bytes: Optional[int] = None,
-                    chunk_rows: Optional[int] = None) -> PassPlan:
-        """Split `kmer count` (mode "count") / `kmer uniq` ("uniq") into key-range passes that fit the device
-        budget (device_budget).  Everything fits: one pass on the whole-input path.  Otherwise contiguous
+                    chunk_rows: Optional[int] = None, text: bool = True) -> PassPlan:
+        """Split `kmer count` (mode "count") / `kmer uniq` ("uniq") / `kmer count -m VEC_COUNT*` ("vec") into
+        key-range passes that fit the device budget (device_budget; for "vec" minus the resident vector pair,
+        8 * (n_bases + 1) bytes).  Everything fits: one pass on the whole-input path.  Otherwise contiguous
         parts of PASS_PARTS are grouped (plan_parts; needs k >= 12, ValueError if not or if one part alone
-        does not fit)."""
-        if mode not in ("count", "uniq"):
+        does not fit).  text=False: no text stage (Engine.abundance copies the vectors out instead)."""
+        if mode not in ("count", "uniq", "vec"):
             raise AssertionError(f"unknown mode {mode!r}")
         budget = self.device_budget(d, budget_bytes)
+        if mode == "vec":
+            budget -= 8 * (d.n_bases + 1)
         vb = d.payload_bytes
-        _, text_bytes = self._text_plan(d, k, mode, chunk_rows)
+        text_bytes = self._text_plan(d, k, mode, chunk_rows)[1] if text else 0
         n, n_other = self.count_windows(d, k, rc)
         one = self._one_pass_bytes(d, k, rc, mode, n_other, vb, text_bytes)
         n_win = max(0, d.n_bases - k + 1)
@@ -1005,27 +1056,147 @@ class Engine:
             pieces.append((None, prev, int(text.numel())))
             sink.submit(text, pieces)
 
+    # ---- abundance vectors: kmer count -m VEC_COUNT / VEC_COUNT_MASKED ----------------------------------
     @_on_device
-    def abundance(self, d: DeviceInput, k: int, rc: bool = False, masked: bool = False) -> Tuple[np.ndarray, np.ndarray]:
+    def abundance(self, d: DeviceInput, k: int, rc: bool = False, masked: bool = False,
+                  budget_bytes: Optional[int] = None) -> Tuple[np.ndarray, np.ndarray]:
         """VEC_COUNT / VEC_COUNT_MASKED (join.py:287-335): per flat position the number of occurrences of the
         k-mer that starts there ('+' vector) / of its reverse complement ('-' vector); masked: occurrences
-        in other records only.  Both streams are sorted stably with their payload, then every element
-        scatters its group's size (kmg_abundance_scatter).  Returns host uint32 arrays over the flat buffer."""
+        in other records only.  Computed by the pass loop of write_vectors (_fill_vectors) under
+        plan_passes(mode="vec").  Returns host uint32 arrays over the flat buffer."""
         if d.rec_starts is None:
             self._upload_names(d)
-        out = torch.zeros(2 * (d.n_bases + 1), dtype=torch.int32, device=self.device)
-        plus, minus = out[: d.n_bases + 1], out[d.n_bases + 1:]
-        err = torch.zeros(1, dtype=torch.int32, device=self.device)
-        for s in self.sorted_streams(d, k, rc, d.payload_bytes):
-            if s.n == 0:
-                continue
-            _lib.check(self.lib.kmg_abundance_scatter(s.keys.data_ptr(), s.vals.data_ptr(), s.n, s.key_bytes, s.val_bytes,
-                                                      d.rec_starts.data_ptr(), d.flat.n_rec, int(masked), d.pos_offset,
-                                                      plus.data_ptr(), minus.data_ptr(), err.data_ptr(), self._stream()))
-        if int(err.item()):
-            raise ValueError("a k-mer occurs more than 2^32-1 times: count does not fit uint32")
+        out, _ = self._fill_vectors(d, k, rc, masked, self.plan_passes(d, k, rc, "vec", budget_bytes, text=False))
         host = out.cpu().numpy().view(np.uint32)
         return host[: d.n_bases + 1], host[d.n_bases + 1:]
+
+    def _fill_vectors(self, d: DeviceInput, k: int, rc: bool, masked: bool, plan: PassPlan) -> Tuple[torch.Tensor, List[float]]:
+        """The device vector pair (int32 holding uint32, '+' over flat [0, n_bases], '-' after it) and the time of
+        each pass.  Every pass extracts the keys of its parts with their payload, one stream at a time, sorts
+        them stably (payloads ascend inside a run: position order in, stable sort) and scatters every element's
+        group size (kmg_abundance_scatter).  Equal k-mers share a part, so each group is whole inside one pass
+        and the scatter writes final values; the one-pass plan extracts without a part filter."""
+        n = d.n_bases
+        out = torch.zeros(2 * (n + 1), dtype=torch.int32, device=self.device)
+        plus, minus = out[: n + 1], out[n + 1:]
+        err = torch.zeros(1, dtype=torch.int32, device=self.device)
+        vb = d.payload_bytes
+        pass_ms = []
+        for lo, hi in plan.parts:
+            t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            t0.record()
+            for wide, per_part in ((False, plan.narrow), (True, plan.wide)):
+                n_keys = int(per_part[lo:hi].sum())
+                if plan.n_parts == 1 and (n_keys or not wide):
+                    a = self.extract(d, k, rc, wide=wide, val_bytes=vb, want_hist=not wide)
+                elif plan.n_parts > 1 and n_keys:
+                    a = self.extract_parts(d, k, rc, wide, vb, plan.n_parts, lo, hi, n_keys)
+                else:
+                    continue
+                a = self.sort(a)
+                if a.n:
+                    _lib.check(self.lib.kmg_abundance_scatter(
+                        a.keys.data_ptr(), a.vals.data_ptr(), a.n, a.key_bytes, a.val_bytes, d.rec_starts.data_ptr(),
+                        d.flat.n_rec, int(masked), d.pos_offset, plus.data_ptr(), minus.data_ptr(), err.data_ptr(),
+                        self._stream()))
+                del a  # the narrow buffers are freed before the wide stream is extracted
+            t1.record()
+            t1.synchronize()
+            pass_ms.append(t0.elapsed_time(t1))
+        if int(err.item()):
+            raise ValueError("a k-mer occurs more than 2^32-1 times: count does not fit uint32")
+        return out, pass_ms
+
+    @_on_device
+    def vector_extents(self, d: DeviceInput, plus: torch.Tensor, minus: torch.Tensor) -> np.ndarray:
+        """int64 [n_rec, 2]: length of every record's '+' / '-' vector, its last non-zero entry + 1 or 0
+        (kmg_vector_extents): one small copy instead of the vectors."""
+        n_rec = d.flat.n_rec
+        if n_rec == 0:
+            return np.zeros((0, 2), np.int64)
+        out = torch.empty(2 * n_rec, dtype=torch.int64, device=self.device)
+        _lib.check(self.lib.kmg_vector_extents(plus.data_ptr(), minus.data_ptr(), d.n_bases, d.rec_starts.data_ptr(), n_rec,
+                                               out.data_ptr(), self._stream()))
+        return out.cpu().numpy().reshape(n_rec, 2)
+
+    @_on_device
+    def format_vector(self, counts: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Device text "COUNT\\n" per entry of `counts` (a 32-bit vector slice, read as uint32), exact length.
+        `out`: a buffer of at least 11 * n bytes to write it into."""
+        n = int(counts.numel())
+        if n == 0:
+            return torch.empty(0, dtype=torch.uint8, device=self.device)
+        text = self._new(11 * n) if out is None else out
+        ws_bytes = self.lib.kmg_format_workspace_bytes(n)
+        ws = self._buf("ws_fmt", ws_bytes)
+        _lib.check(self.lib.kmg_format_vector(counts.data_ptr(), n, text.data_ptr(), self._small[4:].data_ptr(),
+                                              ws.data_ptr(), ws_bytes, self._stream()))
+        self._status(ws)
+        nbytes = int(self._small[4:5].cpu().numpy().view(np.uint64)[0])
+        return text[:nbytes]
+
+    def _vec_workers(self, d: DeviceInput) -> int:
+        return max(1, min(VEC_GZIP_THREADS, 2 * d.flat.n_rec))
+
+    @_on_device
+    def write_vectors(self, d: DeviceInput, k: int, rc: bool, masked: bool, dirpath: str,
+                      budget_bytes: Optional[int] = None, chunk_rows: Optional[int] = None) -> PassPlan:
+        """`kmer count -m VEC_COUNT` (masked: VEC_COUNT_MASKED): one `REF___STRAND.gz` per non-empty vector in
+        `dirpath` (extension stripped, abundance.vector_paths), the files abundance.write_vectors writes for
+        device_vectors().  The vector pair stays on the device: the passes of plan_passes(mode="vec") fill it,
+        kmg_vector_extents trims it, and each vector leaves as device text in chunks of `chunk_rows` entries
+        through pinned buffers.  Files are gzip-compressed (one stream each, level 9 as gzip.open) on a pool of
+        host threads while the GPU formats the next chunks: host memory is O(threads x chunk).  Returns the plan
+        with pass_ms and text_ms filled in."""
+        import gzip
+        from collections import deque
+
+        from kman_b200 import abundance
+
+        names = d.flat.names
+        abundance.check_unique_names(names)
+        if d.rec_starts is None:
+            self._upload_names(d)
+        plan = self.plan_passes(d, k, rc, "vec", budget_bytes, chunk_rows)
+        vec, plan.pass_ms = self._fill_vectors(d, k, rc, masked, plan)
+        n = d.n_bases
+        strands = (vec[: n + 1], vec[n + 1:])
+        lengths = self.vector_extents(d, *strands)
+        jobs = [(r, s, int(lengths[r, s])) for r in range(len(names)) for s in (0, 1) if lengths[r, s]]
+        paths = abundance.vector_paths(dirpath, [(names[r], "+-"[s]) for r, s, _ in jobs])
+        if not jobs:
+            return plan
+        rows, _ = self._text_plan(d, k, "vec", chunk_rows)
+        workers = min(self._vec_workers(d), len(jobs))
+        header = np.frombuffer(b"# k=%d\n" % k, np.uint8)
+        starts = d.flat.rec_starts.astype(np.int64)
+        t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        t0.record()
+        todo, active, opened = deque(zip(jobs, paths)), [], []
+        sink = _ChunkSink(self, None, rows * 11, slots=2 * workers, workers=workers)
+        try:
+            while todo or active:
+                while todo and len(active) < workers:  # one file per worker, chunks submitted round robin
+                    (r, s, length), path = todo.popleft()
+                    opened.append(gzip.open(path, "wb"))
+                    active.append([opened[-1], strands[s][int(starts[r]):int(starts[r]) + length], 0])
+                for lane in list(active):
+                    fh, v, off = lane
+                    cnt = min(rows, int(v.numel()) - off)
+                    text = self.format_vector(v[off:off + cnt], sink.buffer())
+                    sink.submit(text, [(header, 0, header.size), (None, 0, int(text.numel()))] if off == 0 else None, fh)
+                    lane[2] = off + cnt
+                    if lane[2] == v.numel():
+                        sink.then(fh, fh.close)
+                        active.remove(lane)
+            t1.record()
+        finally:
+            sink.close()
+            for fh in opened:
+                fh.close()
+        t1.synchronize()
+        plan.text_ms = t0.elapsed_time(t1)
+        return plan
 
 
 _engines: Dict[int, Engine] = {}

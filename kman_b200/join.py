@@ -167,14 +167,13 @@ class KJoiner:
     def _join_device(self, batches: List[DeviceBatch], outpath: str) -> None:
         b0 = batches[0]
         if self.mode.name.startswith("VEC_"):
-            from kman_b200 import abundance
             from kman_b200.batch import LoadedKmerBatch
 
             if any(isinstance(b, LoadedKmerBatch) for b in batches):
                 raise AssertionError("abundance vectors need the FASTA input, not re-imported batch files")
             d = self._merged_device_input(batches)
-            vecs = abundance.device_vectors(b0._eng, d, b0.k, b0.reverse, self.mode == self.MODE.VEC_COUNT_MASKED)
-            abundance.write_vectors(vecs, b0.k, outpath)  # join.py:370-372 -> abundance.py:148-172
+            # join.py:370-372 -> abundance.py:148-172, in key-range passes with device text (KMG_DEVICE_BUDGET applies)
+            b0._eng.write_vectors(d, b0.k, b0.reverse, self.mode == self.MODE.VEC_COUNT_MASKED, outpath)
             return
         from kman_b200.batch import LoadedKmerBatch
 

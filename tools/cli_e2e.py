@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """Wall-clock of the drop-in command line on a synthetic FASTA (file in, file out), per mode: `kmer count`,
-`kmer uniq` and `kmer batch` (sorted batch files in an output folder).
+`kmer uniq`, `kmer batch` (sorted batch files in an output folder) and `kmer count -m VEC_COUNT` (one gzipped
+abundance vector per record and strand in an output folder).
 usage: python tools/cli_e2e.py [--n 20000000] [--k 31]"""
 import argparse
 import os
@@ -30,15 +31,16 @@ with open(fa, "wb") as fh:
         fh.write(seq.tobytes() + b"\n")
 env = dict(os.environ, PYTHONPATH=ROOT, KMG_ALPHABET="ACGT", TMPDIR=tmp)
 try:
-    for mode in ("count", "uniq", "batch"):
-        out = os.path.join(tmp, f"out_{mode}")
+    for mode, opts in (("count", []), ("uniq", []), ("batch", []), ("count", ["-m", "VEC_COUNT"])):
+        name = " ".join([mode, *opts])
+        out = os.path.join(tmp, "out_" + "_".join([mode, *opts]))
         t0 = time.perf_counter()
-        subprocess.run([sys.executable, "-m", "kman_b200.scripts.kmer", mode, fa, out, str(args.k)], check=True, env=env,
-                       stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+        subprocess.run([sys.executable, "-m", "kman_b200.scripts.kmer", mode, *opts, fa, out, str(args.k)], check=True,
+                       env=env, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
         dt = time.perf_counter() - t0
         files = [os.path.join(out, f) for f in os.listdir(out)] if os.path.isdir(out) else [out]
         sz = sum(os.path.getsize(f) for f in files)
-        print(f"kmer {mode}: {args.n} bp, k={args.k}: {dt:.2f} s wall (python start + CUDA init + FASTA load + GPU + {sz/1e6:.0f} MB of text written) "
+        print(f"kmer {name}: {args.n} bp, k={args.k}: {dt:.2f} s wall (python start + CUDA init + FASTA load + GPU + {sz/1e6:.0f} MB written) "
               f"= {(args.n - args.k + 1)/dt/1e6:.1f} M k-mers/s")
 finally:
     shutil.rmtree(tmp)
