@@ -79,16 +79,40 @@ struct CountOut {
     unsigned long long* n_out;
     bool done;
 };
-// keys already grouped by the lowest prefix byte + the histograms of the three top key bytes
+// keys already grouped by the prefix: with bucket_starts == null by the lowest prefix byte only (the keys
+// are in d_keys; pb = 24), else by all 16 prefix bits (pb = 16; the keys are in d_keys_alt when in_alt)
+// -- plus the histograms of the three top key bytes
 struct PrePartitioned {
     int pb;                         // prefix width, 16 or 24
     const unsigned long long* top;  // device [3][256]: bits [2k-24,2k-16), [2k-16,2k-8), [2k-8,2k)
+    const unsigned long long* bucket_starts = nullptr;  // device [65537]: first key of every 16-bit bucket, then n
+    bool in_alt = false;
 };
 // extract.cu
 size_t top_hist_workspace_bytes();
 int extract_top_hist(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
                      const uint8_t* d_lut256, uint64_t* d_counts, unsigned long long* d_top, unsigned long long* d_plan,
                      void* d_ws, size_t ws_bytes, cudaStream_t st);
+// Pre-pass of the fused pipeline (histogram of the top 16 key bits over the valid narrow windows).
+// `zeroed` = spill [65536] | top [3][256] | plan [4], zeroed by the call; plan = keys, largest top-byte
+// count, valid narrow windows, wide-stream windows.
+constexpr size_t P16_ZEROED_WORDS = 65536 + 3 * 256 + 4;
+static inline unsigned long long* p16_top(unsigned long long* zeroed) { return zeroed + 65536; }
+static inline unsigned long long* p16_plan(unsigned long long* zeroed) { return zeroed + 65536 + 3 * 256; }
+struct Prefix16Out {
+    unsigned long long* zeroed;         // [P16_ZEROED_WORDS]
+    unsigned long long* region_starts;  // [256] exclusive scan of the top-byte row
+    unsigned long long* starts;         // [65537] first key of every 16-bit bucket, then the number of keys
+    unsigned long long* cursors;        // [65536] copy of starts[0 .. 65536) (region_partition's cursors)
+    uint32_t* rows;                     // prefix16_rows_bytes(): the per-CTA counts
+};
+size_t prefix16_rows_bytes();
+int extract_prefix16_hist(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
+                          const uint8_t* d_lut256, const Prefix16Out& o, cudaStream_t st);
+// keys (+ payload) grouped by their top byte -> grouped by their top 16 bits (cursors: Prefix16Out::cursors)
+int region_partition(const void* d_keys_in, void* d_keys_out, const void* d_vals_in, void* d_vals_out, uint64_t n,
+                     int key_bytes, int val_bytes, const unsigned long long* d_region_counts, unsigned long long* d_cursors,
+                     int digit_shift, cudaStream_t st);
 int extract_digit_scatter(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
                           const uint8_t* d_lut256, void* d_keys_out, int key_bytes, void* d_vals_out, int val_bytes,
                           uint64_t pos_offset, unsigned long long* d_cursors, int digit_shift, cudaStream_t st);

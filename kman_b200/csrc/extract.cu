@@ -97,11 +97,138 @@ __device__ __forceinline__ ValT make_val(uint64_t pos, uint32_t strand) {
     return (ValT)((pos << 1) | strand);
 }
 
+// K1 of extract_narrow_kernel for the pre-pass: the bases [tile_pos, tile_pos + 16 * WORDS) of p.bases as 16-base words of 2-bit
+// codes (first base in the top bits) plus the bad-for-narrow and invalid-for-any-stream bitmasks
+template <int BLOCK, int WORDS, typename Params>
+__device__ __forceinline__ void encode_tile_words(const Params& p, int t, uint64_t tile_pos, const uint8_t* s_lut,
+                                                  uint32_t* s_codes, uint16_t* s_bad, uint16_t* s_inv) {
+    for (int w = t; w < WORDS; w += BLOCK) {
+        const uint64_t pos = tile_pos + (uint64_t)w * 16;
+        uint32_t b[4];
+        if (pos + 16 <= p.n_bases) {
+            const uint4 v = __ldg(reinterpret_cast<const uint4*>(p.bases + pos));
+            b[0] = v.x; b[1] = v.y; b[2] = v.z; b[3] = v.w;
+        } else {
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                uint32_t x = 0;
+#pragma unroll
+                for (int r = 0; r < 4; ++r) {
+                    const uint64_t pp = pos + q * 4 + r;
+                    // 0xFF is never in an alphabet built by kmg_build_lut; the explicit
+                    // range test below does not rely on that.
+                    const uint32_t byte = (pp < p.n_bases) ? p.bases[pp] : 0xFFu;
+                    x |= byte << (8 * r);
+                }
+                b[q] = x;
+            }
+        }
+        const int nvalid = pos + 16 <= p.n_bases ? 16 : (pos < p.n_bases ? (int)(p.n_bases - pos) : 0);
+        uint32_t codes = 0, bad = 0, inv = 0;
+#pragma unroll
+        for (int j = 0; j < 16; ++j) {
+            const uint32_t byte = (b[j >> 2] >> (8 * (j & 3))) & 0xFFu;
+            uint32_t e = s_lut[byte];
+            if (j >= nvalid) e = KMG_LUT_INVALID;
+            codes |= (e & 3u) << (30 - 2 * j);
+            bad |= ((e >> 6) ? 1u : 0u) << (15 - j);
+            inv |= (e >> 7) << (15 - j);
+        }
+        s_codes[w] = codes;
+        s_bad[w] = (uint16_t)bad;
+        s_inv[w] = (uint16_t)inv;
+    }
+}
+
+// Validity of the PPT consecutive window starts first_pos .. first_pos + PPT - 1 (bit j: window j),
+// given the 128-base bad / invalid mask strings B0:B1, I0:I1 that start at the word of window 0
+// (joff = its base inside that word).  vf: the window lies in [win_begin, win_end) and all its k
+// bases are plain (the narrow stream); *nwide: windows of the range that belong to the wide stream.
+// *clean: no base of the PPT + k - 1 the windows span is bad (every window of the range is valid).
+template <int PPT>
+__device__ __forceinline__ uint32_t narrow_window_flags(uint64_t first_pos, uint64_t win_begin, uint64_t win_end, int k,
+                                                        int joff, uint64_t B0, uint64_t B1, uint64_t I0, uint64_t I1,
+                                                        uint32_t& in_range_mask, bool& span_clean, uint32_t& nwide) {
+    {   // window starts [win_begin, win_end) among my PPT positions
+        const uint64_t lo = win_begin > first_pos ? win_begin - first_pos : 0;
+        const uint64_t hi = win_end > first_pos ? win_end - first_pos : 0;
+        const uint32_t l = lo < PPT ? (uint32_t)lo : PPT, h = hi < PPT ? (uint32_t)hi : PPT;
+        in_range_mask = h > l ? (((1u << (h - l)) - 1u) << l) : 0u;
+    }
+    // fast path: no base that is bad for the narrow stream among the PPT+k-1 bases my windows span
+    {
+        const uint64_t W0 = joff == 0 ? B0 : ((B0 << joff) | (B1 >> (64 - joff)));
+        const int span = PPT + k - 1;  // 17 .. 79
+        if (span <= 64) span_clean = (W0 >> (64 - span)) == 0;
+        else span_clean = W0 == 0 && ((B1 << joff) >> (128 - span)) == 0;
+    }
+    uint32_t vf = 0;
+    nwide = 0;
+    if (span_clean) {
+        vf = in_range_mask;
+    } else {
+#pragma unroll
+        for (int j = 0; j < PPT; ++j) {
+            const int je = joff + j;  // 0..15
+            const uint64_t bm = (je == 0 ? B0 : ((B0 << je) | (B1 >> (64 - je)))) >> (64 - k);
+            const uint64_t im = (je == 0 ? I0 : ((I0 << je) | (I1 >> (64 - je)))) >> (64 - k);
+            const bool in_range = (in_range_mask >> j) & 1u;
+            if (in_range && bm == 0) vf |= 1u << j;
+            if (in_range && im == 0 && bm != 0) ++nwide;
+        }
+    }
+    return vf;
+}
+
+// The order-free prefix pass of one tile (extraction MODE 2 and region_partition_kernel): the keys of
+// a digit may land in any order inside the digit's region, because the local sort orders everything
+// below the prefix.  So a key's place in the tile's run of its digit is what a shared-memory counter
+// returns (rank), one thread per digit reserves the tile's run with one global atomic on the region's
+// cursor (reserve), the keys are staged in digit order (slot) and leave as runs (write_runs): no tile
+// waits for another one and no ranking needs to be stable.
+template <int BLOCK>
+struct DigitRuns {
+    uint32_t* s_cnt;            // [256] keys per digit in this tile (zeroed before the first rank)
+    uint32_t* s_off;            // [256] first staging slot of every digit
+    unsigned long long* s_gb;   // [256] global slot of staging slot i = s_gb[digit] + i
+    uint32_t* s_scan;           // [BLOCK / 32 + 1]
+
+    // digit | rank << 8
+    __device__ __forceinline__ uint32_t rank(uint32_t d) const { return d | (atomicAdd(&s_cnt[d], 1u) << 8); }
+    // after a __syncthreads() that follows the last rank(); returns the tile's number of keys
+    __device__ __forceinline__ uint32_t reserve(unsigned long long* cursors) const {
+        const int t = threadIdx.x;
+        const uint32_t c = t < 256 ? s_cnt[t] : 0u;
+        unsigned long long g = 0;
+        if (c) g = atomicAdd(&cursors[t], (unsigned long long)c);
+        uint32_t n_tile;
+        const uint32_t off = block_excl_scan<BLOCK, uint32_t>(c, s_scan, n_tile);
+        if (t < 256) {
+            s_off[t] = off;
+            s_gb[t] = g - off;
+        }
+        __syncthreads();
+        return n_tile;
+    }
+    __device__ __forceinline__ uint32_t slot(uint32_t wh) const { return s_off[wh & 255u] + (wh >> 8); }
+    // after a __syncthreads() that follows the staging
+    template <bool PAY, typename KeyT, typename ValT, typename DigitOf>
+    __device__ __forceinline__ void write_runs(const KeyT* s_keys, const ValT* s_vals, uint32_t n_tile, DigitOf digit_of,
+                                               KeyT* keys_out, ValT* vals_out) const {
+        for (uint32_t i = threadIdx.x; i < n_tile; i += BLOCK) {
+            const KeyT key = s_keys[i];
+            const unsigned long long at = s_gb[digit_of(key)] + i;
+            keys_out[at] = key;
+            if constexpr (PAY) vals_out[at] = s_vals[i];
+        }
+    }
+};
+
 // KeyT: uint64_t (k<=32) or u128 (33<=k<=64).  PPT: window starts per thread (8 or 16).
 // MODE 0: keys (and payload) of the valid windows in position order (kmg_extract).
 // MODE 1: nothing is emitted -- only the 4-mer histograms (HIST) and the window counts: the
-//         pre-pass of the fused pipeline (pipeline.cu), which needs every prefix pass' histogram
-//         before the first key is placed.
+//         top-byte histograms of kmg_extract_dest_counts (the fused pipeline has its own pre-pass,
+//         prefix16_hist_kernel).
 // MODE 2: extraction fused with the FIRST prefix pass of the hybrid sort: that pass may place the
 //         keys of one digit in any order (the local sort orders everything below the prefix), so
 //         a tile ranks its keys with the return values of shared-memory atomics, reserves its
@@ -340,56 +467,34 @@ __global__ void __launch_bounds__(EX_BLOCK) extract_narrow_kernel(const ExtractP
     if constexpr (MODE == 2) {
         // ---- fused first prefix pass: rank inside the tile = what the digit counter returned ----------
         const int dsh = p.digit_shift;
+        const DigitRuns<EX_BLOCK> runs{s_cnt, s_off, s_gb, s_scan};
         uint32_t wh[PPT * OUT_PER_WIN];  // digit | rank << 8
 #pragma unroll
         for (int j = 0; j < PPT; ++j) {
             if (!(vf & (1u << j))) continue;
             const KeyT key = build_key(j);
-            const uint32_t d0 = key_digit(key, dsh, 255u);
-            wh[j * OUT_PER_WIN] = d0 | (atomicAdd(&s_cnt[d0], 1u) << 8);
-            if constexpr (RC) {
-                const uint32_t d1 = key_digit(rc_key(key, k), dsh, 255u);
-                wh[j * 2 + 1] = d1 | (atomicAdd(&s_cnt[d1], 1u) << 8);
-            }
+            wh[j * OUT_PER_WIN] = runs.rank(key_digit(key, dsh, 255u));
+            if constexpr (RC) wh[j * 2 + 1] = runs.rank(key_digit(rc_key(key, k), dsh, 255u));
         }
         __syncthreads();
-        // one thread per digit: reserve the tile's slots in the digit's region (any order is fine,
-        // so a plain atomic cursor does it -- no tile waits for another one)
-        const uint32_t c = t < 256 ? s_cnt[t] : 0u;
-        unsigned long long g = 0;
-        if (c) g = atomicAdd(&p.cursors[t], (unsigned long long)c);
-        uint32_t n_tile;
-        const uint32_t off = block_excl_scan<EX_BLOCK, uint32_t>(c, s_scan, n_tile);
-        if (t < 256) {
-            s_off[t] = off;
-            s_gb[t] = g - off;
-        }
-        __syncthreads();
+        const uint32_t n_tile = runs.reserve(p.cursors);
 #pragma unroll
         for (int j = 0; j < PPT; ++j) {
             if (!(vf & (1u << j))) continue;
             const KeyT key = build_key(j);
             const uint64_t pos = tile_pos + (uint64_t)t * PPT + j + p.pos_offset;
-            const uint32_t w0 = wh[j * OUT_PER_WIN];
-            const uint32_t i0 = s_off[w0 & 255u] + (w0 >> 8);
+            const uint32_t i0 = runs.slot(wh[j * OUT_PER_WIN]);
             s_keys[i0] = key;
             if constexpr (VAL_BYTES != 0) s_vals[i0] = make_val<ValT>(pos, 0);
             if constexpr (RC) {
-                const uint32_t w1 = wh[j * 2 + 1];
-                const uint32_t i1 = s_off[w1 & 255u] + (w1 >> 8);
+                const uint32_t i1 = runs.slot(wh[j * 2 + 1]);
                 s_keys[i1] = rc_key(key, k);
                 if constexpr (VAL_BYTES != 0) s_vals[i1] = make_val<ValT>(pos, 1);
             }
         }
         __syncthreads();
-        KeyT* keys_out = reinterpret_cast<KeyT*>(p.keys_out);
-        ValT* vals_out = reinterpret_cast<ValT*>(p.vals_out);
-        for (uint32_t i = t; i < n_tile; i += EX_BLOCK) {
-            const KeyT key = s_keys[i];
-            const unsigned long long at = s_gb[key_digit(key, dsh, 255u)] + i;
-            keys_out[at] = key;
-            if constexpr (VAL_BYTES != 0) vals_out[at] = s_vals[i];
-        }
+        runs.template write_runs<VAL_BYTES != 0>(s_keys, s_vals, n_tile, [dsh](const KeyT& key) { return key_digit(key, dsh, 255u); },
+                                                 reinterpret_cast<KeyT*>(p.keys_out), reinterpret_cast<ValT*>(p.vals_out));
         return;
     }
 
@@ -746,7 +851,7 @@ __global__ void hist_finalize_kernel(const unsigned long long* __restrict__ hs, 
     }
 }
 
-// Pre-pass of the fused pipeline: histograms of the three TOP key bytes only (rows 0..2 = bits
+// Top-byte histograms of kmg_extract_dest_counts: histograms of the three TOP key bytes only (rows 0..2 = bits
 // [2k-24,2k-16), [2k-16,2k-8), [2k-8,2k)), i.e. of the 4-mers at window offsets 8, 4, 0 (rc keys:
 // rc4 of those at k-12, k-8, k-4) -- valid for 8- and 16-byte keys alike.  hs rows as laid out by
 // extract_top_hist: [0..2] forward offsets 8, 4, 0, then (rc) [3..5] offsets k-12, k-8, k-4.
@@ -784,6 +889,275 @@ __global__ void hist_top_finalize_kernel(const unsigned long long* __restrict__ 
         plan[0] = sum;
         plan[1] = mx;
     }
+}
+
+// ---- pre-pass of the fused pipeline: histogram of the top 16 key bits ------------------------------------
+// The top 16 bits of a forward key are the 8-mer at window offset 0, those of a reverse-complement key
+// the rc of the 8-mer at offset k-8.  Counting them over the exact valid windows gives the start of every
+// 16-bit prefix bucket before the first key is built, which is what lets the fused pass scatter by the
+// TOP byte and a second pass (region_partition_kernel) split every top-byte region by byte 2 with
+// order-free atomics -- no stable pass, no look-back.
+// A persistent grid of one CTA per SM keeps all 65536 counters in 128 KB of shared memory as 16-bit
+// halves of 32-bit words; a counter that reaches 2^15 hands 2^15 to a global spill row, so a half never
+// carries into its neighbour (poly-A and microsatellites stay exact).  Each CTA then writes its row of
+// packed counts; prefix16_reduce_kernel sums the rows.
+constexpr int P16_BLOCK = 1024;
+constexpr int P16_PPT = 16;  // window starts per thread: one 16-base word, so every window starts in word t
+constexpr uint64_t P16_TILE = (uint64_t)P16_BLOCK * P16_PPT;
+constexpr int P16_MAX_CTAS = 192;
+constexpr uint32_t P16_WORDS = 1u << 15;  // 32-bit words of one row (two counters each)
+constexpr uint32_t P16_SPILL = 1u << 15;
+
+struct Prefix16Params {
+    const uint8_t* bases;
+    uint64_t n_bases;
+    uint64_t win_begin, win_end;
+    uint64_t first_tile;
+    uint32_t n_tiles;
+    int k;
+    const uint8_t* lut;
+    uint32_t* rows;               // [gridDim.x][P16_WORDS] packed counts of every CTA
+    unsigned long long* spill;    // [65536] 2^15 for every time a CTA's counter reached 2^15
+    unsigned long long* byte3;    // [256] histogram of key bits [2k-24, 2k-16) (the 24-bit prefix)
+    unsigned long long* counts;   // [0] valid narrow windows, [1] wide-stream windows
+};
+
+// 8 consecutive bases starting at base e (0 <= e <= 88) of the 96-base big-endian string X0:X1:X2
+__device__ __forceinline__ uint32_t mer8_at(uint64_t X0, uint64_t X1, uint64_t X2, int e) {
+    const int w = e >> 5, off = 2 * (e & 31);
+    const uint64_t a = w == 0 ? X0 : (w == 1 ? X1 : X2);
+    const uint64_t b = w == 0 ? X1 : (w == 1 ? X2 : 0ull);
+    const uint64_t v = off == 0 ? a : ((a << off) | (b >> (64 - off)));
+    return (uint32_t)(v >> 48);
+}
+__device__ __forceinline__ uint32_t rc8(uint32_t x) { return (rc4(x & 0xFFu) << 8) | rc4(x >> 8); }
+
+__device__ __forceinline__ void count16(uint32_t* s_h, unsigned long long* spill, uint32_t b) {
+    const uint32_t sh = (b & 1u) << 4;
+    const uint32_t old = atomicAdd(&s_h[b >> 1], 1u << sh);
+    if (((old >> sh) & 0xFFFFu) == P16_SPILL - 1u) {  // this add took the counter to 2^15: exactly one thread sees it
+        atomicSub(&s_h[b >> 1], P16_SPILL << sh);
+        atomicAdd(&spill[b], (unsigned long long)P16_SPILL);
+    }
+}
+
+template <bool RC>
+__global__ void __launch_bounds__(P16_BLOCK, 1) prefix16_hist_kernel(const Prefix16Params p) {
+    constexpr int WORDS = (int)(P16_TILE / 16) + EX_HALO_WORDS;
+    extern __shared__ __align__(16) uint32_t s_h[];  // [P16_WORDS]: counter b is half (b & 1) of word b >> 1
+    __shared__ uint32_t s_codes[WORDS];
+    __shared__ uint16_t s_bad[WORDS];
+    __shared__ uint16_t s_inv[WORDS];
+    __shared__ uint8_t s_lut[256];
+    __shared__ uint32_t s_b3[256];
+    __shared__ unsigned long long s_n[2];
+    const int t = threadIdx.x;
+    for (uint32_t i = t; i < P16_WORDS / 4; i += P16_BLOCK) reinterpret_cast<uint4*>(s_h)[i] = make_uint4(0, 0, 0, 0);
+    if (t < 256) {
+        s_lut[t] = p.lut[t];
+        s_b3[t] = 0;
+    }
+    if (t < 2) s_n[t] = 0;
+    const int k = p.k;
+    uint32_t n_valid = 0, n_wide = 0;
+    for (uint32_t tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
+        __syncthreads();  // (the previous tile's words are consumed; first round: the tables are zeroed)
+        const uint64_t tile_pos = (p.first_tile + tile) * P16_TILE;
+        encode_tile_words<P16_BLOCK, WORDS>(p, t, tile_pos, s_lut, s_codes, s_bad, s_inv);
+        __syncthreads();
+        const uint64_t X0 = ((uint64_t)s_codes[t] << 32) | s_codes[t + 1];
+        const uint64_t X1 = ((uint64_t)s_codes[t + 2] << 32) | s_codes[t + 3];
+        const uint64_t X2 = ((uint64_t)s_codes[t + 4] << 32) | s_codes[t + 5];
+        const uint64_t B0 = ((uint64_t)s_bad[t] << 48) | ((uint64_t)s_bad[t + 1] << 32) | ((uint64_t)s_bad[t + 2] << 16) | s_bad[t + 3];
+        const uint64_t B1 = ((uint64_t)s_bad[t + 4] << 48) | ((uint64_t)s_bad[t + 5] << 32) | ((uint64_t)s_bad[t + 6] << 16) | s_bad[t + 7];
+        const uint64_t I0 = ((uint64_t)s_inv[t] << 48) | ((uint64_t)s_inv[t + 1] << 32) | ((uint64_t)s_inv[t + 2] << 16) | s_inv[t + 3];
+        const uint64_t I1 = ((uint64_t)s_inv[t + 4] << 48) | ((uint64_t)s_inv[t + 5] << 32) | ((uint64_t)s_inv[t + 6] << 16) | s_inv[t + 7];
+        uint32_t in_range_mask, nwide;
+        bool span_clean;
+        const uint32_t vf = narrow_window_flags<P16_PPT>(tile_pos + (uint64_t)t * P16_PPT, p.win_begin, p.win_end, k, 0, B0, B1,
+                                                         I0, I1, in_range_mask, span_clean, nwide);
+        n_valid += __popc(vf);
+        n_wide += nwide;
+#pragma unroll
+        for (int j = 0; j < P16_PPT; ++j) {
+            if (!(vf & (1u << j))) continue;
+            count16(s_h, p.spill, mer8_at(X0, X1, X2, j));
+            atomicAdd(&s_b3[mer4_at(X0, X1, X2, j + 8)], 1u);
+            if constexpr (RC) {
+                count16(s_h, p.spill, rc8(mer8_at(X0, X1, X2, j + k - 8)));
+                atomicAdd(&s_b3[rc4(mer4_at(X0, X1, X2, j + k - 12))], 1u);
+            }
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        n_valid += __shfl_xor_sync(0xffffffffu, n_valid, o);
+        n_wide += __shfl_xor_sync(0xffffffffu, n_wide, o);
+    }
+    if ((t & 31) == 0) {
+        if (n_valid) atomicAdd(&s_n[0], (unsigned long long)n_valid);
+        if (n_wide) atomicAdd(&s_n[1], (unsigned long long)n_wide);
+    }
+    __syncthreads();
+    uint4* row = reinterpret_cast<uint4*>(p.rows + (size_t)blockIdx.x * P16_WORDS);
+    for (uint32_t i = t; i < P16_WORDS / 4; i += P16_BLOCK) row[i] = reinterpret_cast<const uint4*>(s_h)[i];
+    if (t < 256 && s_b3[t]) atomicAdd(&p.byte3[t], (unsigned long long)s_b3[t]);
+    if (t < 2 && s_n[t]) atomicAdd(&p.counts[t], s_n[t]);
+}
+
+// Block r sums bucket r * 256 + t over the CTA rows: the top-byte row (top[2][r] = region total), the
+// byte-2 marginal (top[1]) and the bucket starts INSIDE region r.
+__global__ void __launch_bounds__(256) prefix16_reduce_kernel(const uint32_t* __restrict__ rows, int n_rows,
+                                                              const unsigned long long* __restrict__ spill,
+                                                              unsigned long long* __restrict__ top,
+                                                              unsigned long long* __restrict__ starts) {
+    __shared__ unsigned long long s_scan[256 / 32 + 1];
+    const uint32_t r = blockIdx.x, t = threadIdx.x, b = r * 256 + t;
+    const uint32_t* w = rows + (b >> 1);
+    const int sh = (int)(b & 1u) << 4;
+    uint32_t acc = 0;  // (at most P16_MAX_CTAS * (2^15 - 1))
+#pragma unroll 8
+    for (int c = 0; c < n_rows; ++c) acc += (w[(size_t)c * P16_WORDS] >> sh) & 0xFFFFu;
+    const unsigned long long v = spill[b] + acc;
+    unsigned long long tot;
+    const unsigned long long ex = block_excl_scan<256, unsigned long long>(v, s_scan, tot);
+    starts[b] = ex;
+    if (t == 0) top[2 * 256 + r] = tot;
+    if (v) atomicAdd(&top[256 + t], v);
+}
+
+// Makes the bucket starts absolute (starts[65536] = number of keys) and copies them into the cursors of
+// region_partition_kernel; region_starts = exclusive scan of the top-byte row (the cursors of the fused
+// top-byte scatter).  plan[0] = number of keys, plan[1] = largest top-byte count.
+__global__ void __launch_bounds__(256) prefix16_starts_kernel(const unsigned long long* __restrict__ top,
+                                                              unsigned long long* __restrict__ plan,
+                                                              unsigned long long* __restrict__ region_starts,
+                                                              unsigned long long* __restrict__ starts,
+                                                              unsigned long long* __restrict__ cursors) {
+    __shared__ unsigned long long s_scan[256 / 32 + 1], s_max[8], s_base;
+    const uint32_t r = blockIdx.x, t = threadIdx.x, b = r * 256 + t;
+    const unsigned long long c = top[2 * 256 + t];
+    unsigned long long total;
+    const unsigned long long ex = block_excl_scan<256, unsigned long long>(c, s_scan, total);
+    if (t == r) s_base = ex;
+    __syncthreads();
+    const unsigned long long s = starts[b] + s_base;
+    starts[b] = s;
+    cursors[b] = s;
+    if (t == 0) region_starts[r] = s_base;
+    if (r == 0) {
+        unsigned long long mx = c;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) mx = max(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+        if ((t & 31) == 0) s_max[t >> 5] = mx;
+        __syncthreads();
+        if (t == 0) {
+            for (int i = 1; i < 8; ++i) mx = max(mx, s_max[i]);
+            plan[0] = total;
+            plan[1] = mx;
+            starts[65536] = total;
+        }
+    }
+}
+
+// ---- second prefix pass of the pb = 16 pipeline: split every top-byte region by byte 2 --------------------
+// The keys arrive grouped by their top byte (region r = [R_r, R_r + count_r)).  Every 16-bit bucket's start
+// is known from the pre-pass, so each region is split on its own with the order-free DigitRuns pass:
+// tiles never straddle a region (region r owns ceil(count_r / TILE) consecutive tiles), a tile ranks its
+// keys with shared-memory atomics, reserves its runs with one global atomic per digit on the bucket
+// cursors and writes them through shared-memory staging.
+constexpr int RP_BLOCK = 512;
+// keys per thread: 48-80 KB of staging and at most 64 registers (two CTAs per SM) without spills
+template <typename KeyT, int VB>
+constexpr int rp_ipt() { return sizeof(KeyT) == 8 ? (VB == 0 ? 12 : 8) : (VB == 8 ? 6 : 8); }
+
+struct RegionPartParams {
+    const void* keys_in;
+    void* keys_out;
+    const void* vals_in;
+    void* vals_out;
+    const unsigned long long* counts;  // [256] keys per top-byte region
+    unsigned long long* cursors;       // [65536] next free slot of every 16-bit bucket
+    int digit_shift;                   // of byte 2
+};
+
+template <typename KeyT, int VB>
+__global__ void __launch_bounds__(RP_BLOCK, 2) region_partition_kernel(const RegionPartParams p) {
+    constexpr int IPT = rp_ipt<KeyT, VB>();
+    constexpr uint32_t TILE = RP_BLOCK * IPT;
+    using ValT = typename std::conditional<VB == 4, uint32_t, uint64_t>::type;
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    KeyT* s_keys = reinterpret_cast<KeyT*>(smem_raw);
+    ValT* s_vals = reinterpret_cast<ValT*>(smem_raw + sizeof(KeyT) * TILE);
+    __shared__ uint32_t s_cnt[256], s_off[256];
+    __shared__ unsigned long long s_gb[256];
+    __shared__ uint32_t s_scan[RP_BLOCK / 32 + 1];
+    __shared__ unsigned long long s_scan64[RP_BLOCK / 32 + 1];
+    __shared__ uint32_t s_region;
+    __shared__ unsigned long long s_lo, s_hi;
+
+    const int t = threadIdx.x;
+    const unsigned long long c = t < 256 ? p.counts[t] : 0ull;
+    const uint32_t nt = (uint32_t)((c + TILE - 1) / TILE);
+    uint32_t tiles_all;
+    unsigned long long keys_all;
+    const uint32_t t0 = block_excl_scan<RP_BLOCK, uint32_t>(nt, s_scan, tiles_all);
+    const unsigned long long k0 = block_excl_scan<RP_BLOCK, unsigned long long>(c, s_scan64, keys_all);
+    if (blockIdx.x >= tiles_all) return;  // surplus CTA (the grid is sized for the worst split)
+    if (t < 256) s_cnt[t] = 0;
+    if (blockIdx.x - t0 < nt) {  // the region this tile belongs to
+        s_region = t;
+        s_lo = k0 + (unsigned long long)(blockIdx.x - t0) * TILE;
+        s_hi = k0 + c;
+    }
+    __syncthreads();
+    const uint32_t r = s_region;
+    const unsigned long long lo = s_lo;
+    const uint32_t n_in = (uint32_t)min((unsigned long long)TILE, s_hi - lo);
+    const KeyT* keys_in = reinterpret_cast<const KeyT*>(p.keys_in) + lo;
+    const ValT* vals_in = reinterpret_cast<const ValT*>(p.vals_in) + lo;
+    const int dsh = p.digit_shift;
+    const DigitRuns<RP_BLOCK> runs{s_cnt, s_off, s_gb, s_scan};
+    KeyT key[IPT];
+    ValT val[VB ? IPT : 1];
+    uint32_t wh[IPT];
+#pragma unroll
+    for (int q = 0; q < IPT; ++q) {
+        const uint32_t i = q * RP_BLOCK + t;
+        if (i < n_in) {
+            key[q] = keys_in[i];
+            if constexpr (VB != 0) val[q] = vals_in[i];
+        }
+    }
+#pragma unroll
+    for (int q = 0; q < IPT; ++q)
+        if (q * RP_BLOCK + t < n_in) wh[q] = runs.rank(key_digit(key[q], dsh, 255u));
+    __syncthreads();
+    const uint32_t n_tile = runs.reserve(p.cursors + (size_t)r * 256);
+#pragma unroll
+    for (int q = 0; q < IPT; ++q) {
+        if (q * RP_BLOCK + t < n_in) {
+            const uint32_t i = runs.slot(wh[q]);
+            s_keys[i] = key[q];
+            if constexpr (VB != 0) s_vals[i] = val[q];
+        }
+    }
+    __syncthreads();
+    runs.template write_runs<VB != 0>(s_keys, s_vals, n_tile, [dsh](const KeyT& k_) { return key_digit(k_, dsh, 255u); },
+                                      reinterpret_cast<KeyT*>(p.keys_out), reinterpret_cast<ValT*>(p.vals_out));
+}
+
+template <typename KeyT, int VB>
+static int launch_region_partition(const RegionPartParams& p, uint64_t n, cudaStream_t st) {
+    constexpr uint64_t TILE = (uint64_t)RP_BLOCK * rp_ipt<KeyT, VB>();
+    const uint64_t grid = (n + TILE - 1) / TILE + 256;  // + one partial tile per region at most
+    KMG_REQUIRE(grid < (1ull << 31), KMG_ERR_RANGE, "too many tiles");
+    const size_t smem = TILE * (sizeof(KeyT) + VB);
+    auto kern = region_partition_kernel<KeyT, VB>;
+    KMG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<(uint32_t)grid, RP_BLOCK, smem, st>>>(p);
+    KMG_LAUNCH_CHECK();
+    return KMG_OK;
 }
 
 template <bool RC, int LIMBS, int FILTER = 0>
@@ -875,6 +1249,73 @@ int extract_digit_scatter(const uint8_t* d_bases, uint64_t n_bases, uint64_t win
     }
     if (key_bytes == 8) return dispatch_scatter_digit<uint64_t, 16>(p, n_tiles, rc, val_bytes, st);
     return dispatch_scatter_digit<u128, 8>(p, n_tiles, rc, val_bytes, st);
+}
+
+size_t prefix16_rows_bytes() { return (size_t)P16_MAX_CTAS * P16_WORDS * sizeof(uint32_t); }
+
+// see common.cuh
+int extract_prefix16_hist(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
+                          const uint8_t* d_lut256, const Prefix16Out& o, cudaStream_t st) {
+    KMG_REQUIRE(k >= 12 && k <= 64, KMG_ERR_ARG, "the prefix histograms need 12 <= k <= 64");
+    KMG_CUDA(cudaMemsetAsync(o.zeroed, 0, P16_ZEROED_WORDS * sizeof(uint64_t), st));
+    unsigned long long* spill = o.zeroed;
+    unsigned long long* top = p16_top(o.zeroed);
+    unsigned long long* plan = p16_plan(o.zeroed);
+    Prefix16Params p;
+    memset(&p, 0, sizeof(p));
+    p.bases = d_bases;
+    p.n_bases = n_bases;
+    p.win_begin = win_begin;
+    p.win_end = win_end;
+    p.k = k;
+    p.lut = d_lut256;
+    p.rows = o.rows;
+    p.spill = spill;
+    p.byte3 = top;
+    p.counts = plan + 2;
+    int n_rows = 0;
+    if (win_end > win_begin) {
+        p.first_tile = win_begin / P16_TILE;
+        const uint64_t n_tiles = (win_end + P16_TILE - 1) / P16_TILE - p.first_tile;
+        KMG_REQUIRE(n_tiles < (1ull << 31), KMG_ERR_RANGE, "too many tiles");
+        p.n_tiles = (uint32_t)n_tiles;
+        int dev = 0, sms = 148;
+        cudaGetDevice(&dev);
+        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+        n_rows = (int)std::min<uint64_t>(n_tiles, (uint64_t)std::min(sms, P16_MAX_CTAS));
+        const size_t smem = P16_WORDS * sizeof(uint32_t);
+        auto kern = rc ? prefix16_hist_kernel<true> : prefix16_hist_kernel<false>;
+        KMG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kern<<<n_rows, P16_BLOCK, smem, st>>>(p);
+        KMG_LAUNCH_CHECK();
+    }
+    prefix16_reduce_kernel<<<256, 256, 0, st>>>(o.rows, n_rows, spill, top, o.starts);
+    KMG_LAUNCH_CHECK();
+    prefix16_starts_kernel<<<256, 256, 0, st>>>(top, plan, o.region_starts, o.starts, o.cursors);
+    KMG_LAUNCH_CHECK();
+    return KMG_OK;
+}
+
+int region_partition(const void* d_keys_in, void* d_keys_out, const void* d_vals_in, void* d_vals_out, uint64_t n,
+                     int key_bytes, int val_bytes, const unsigned long long* d_region_counts, unsigned long long* d_cursors,
+                     int digit_shift, cudaStream_t st) {
+    if (n == 0) return KMG_OK;
+    RegionPartParams p;
+    p.keys_in = d_keys_in;
+    p.keys_out = d_keys_out;
+    p.vals_in = d_vals_in;
+    p.vals_out = d_vals_out;
+    p.counts = d_region_counts;
+    p.cursors = d_cursors;
+    p.digit_shift = digit_shift;
+    if (key_bytes == 8) {
+        if (val_bytes == 0) return launch_region_partition<uint64_t, 0>(p, n, st);
+        if (val_bytes == 4) return launch_region_partition<uint64_t, 4>(p, n, st);
+        return launch_region_partition<uint64_t, 8>(p, n, st);
+    }
+    if (val_bytes == 0) return launch_region_partition<u128, 0>(p, n, st);
+    if (val_bytes == 4) return launch_region_partition<u128, 4>(p, n, st);
+    return launch_region_partition<u128, 8>(p, n, st);
 }
 
 }  // namespace kmg

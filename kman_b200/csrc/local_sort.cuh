@@ -144,6 +144,23 @@ __global__ void __launch_bounds__(256) tile_bounds_kernel(const HybridParams p) 
     if (lane == 0) p.bounds[tile] = r;
 }
 
+// The same bounds for keys whose bucket starts are known (the fused pipeline's pre-pass):
+// starts[0 .. n_buckets] (starts[n_buckets] = n), so the first bucket start >= tile * tile_t is one
+// binary search -- an empty bucket starts where the next non-empty one does
+__global__ void __launch_bounds__(256) bounds_from_starts_kernel(const HybridParams p, const unsigned long long* __restrict__ starts,
+                                                                 uint32_t n_buckets) {
+    const uint32_t tile = blockIdx.x * blockDim.x + threadIdx.x;
+    if (tile > p.n_tiles) return;
+    const uint64_t pos = min((uint64_t)tile * p.tile_t, p.n);
+    uint32_t lo = 0, hi = n_buckets;
+    while (lo < hi) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (starts[mid] >= pos) hi = mid;
+        else lo = mid + 1;
+    }
+    p.bounds[tile] = min((uint64_t)starts[lo], p.n);
+}
+
 // Tiles that own more keys than the local sort holds are known from the bounds alone: count them
 // before the launch so that a fused count is not attempted in vain (repeats: real genomes always
 // have some).  The local sort flags them again, together with the rare crowded-cell tiles.

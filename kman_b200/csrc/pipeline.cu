@@ -6,14 +6,18 @@
 // Stage calls (kmg_extract -> kmg_sort_count) write every key to HBM in extraction order only to read
 // it straight back for the first prefix pass of the hybrid sort -- a pass that does not care about
 // the order inside a digit.  Here the extraction kernel IS that pass:
-//   1. pre-pass over the bases (extract_narrow_kernel MODE 1): 4-mer histogram -> histograms of the
-//      three top key bytes, number of keys, number of wide-stream windows.  100 MB instead of
-//      the 800 MB a histogram sweep over the keys would read.
+//   1. pre-pass over the bases (prefix16_hist_kernel + two small reduce kernels): histogram of the top
+//      16 key bits over the exact valid windows -> every 16-bit bucket start, the histograms of the
+//      three top key bytes, number of keys, number of wide-stream windows.  100 MB instead of the
+//      800 MB a histogram sweep over the keys would read.
 //   2. ONE host read-back (32 bytes): key count (grid sizes), skew of the top byte (prefix width).
-//   3. extract_narrow_kernel MODE 2: keys go straight into the 256 regions of the lowest prefix byte.
-//   4. the remaining 1-2 stable prefix passes (onesweep_kernel), tile bounds, local_sort_kernel with
-//      the fused count / singleton emission (radix_sort.cu: sort_impl with `pre`).
-//   5. ONE host read-back (the sort's status words, 56 bytes) carries the result count.
+//   3. pb = 16: extract_narrow_kernel MODE 2 puts the keys straight into the 256 regions of their TOP
+//      byte, region_partition_kernel splits every region by byte 2 (bucket starts known: no look-back,
+//      no stable ranking), tile bounds come from the bucket starts, local_sort_kernel with the fused
+//      count / singleton emission (radix_sort.cu: sort_impl with `pre`).
+//      pb = 24: MODE 2 scatters by byte 3, then the two stable prefix passes (onesweep_kernel), tile
+//      bounds and the local sort.
+//   4. ONE host read-back (the sort's status words, 56 bytes) carries the result count.
 // Inputs the hybrid finish does not take (fewer than 2^20 keys, k < 16)
 // run kmg_extract + kmg_sort_count / kmg_sort_uniq inside the same call: same result either way.
 #include <algorithm>
@@ -26,10 +30,13 @@ namespace kmg {
 
 namespace {
 struct PipeWs {
-    void* hist_ws;                // pre-pass workspace (header + hs rows)
+    unsigned long long* zeroed;   // pre-pass: spill [65536] | top [3][256] | plan [4] (see Prefix16Out)
     unsigned long long* top;      // [3][256]
-    unsigned long long* cursors;  // [256]
     unsigned long long* plan;     // [2] + counts [2]
+    unsigned long long* cursors;  // [256] region starts of the fused scatter
+    unsigned long long* starts;   // [65537] 16-bit bucket starts
+    unsigned long long* cursors16;  // [65536] bucket cursors of the region partition
+    uint32_t* rows;               // per-CTA rows of the pre-pass
     uint64_t* hist16;             // [16][256] digit histograms of the stage path
     uint64_t* n_out;              // device result count
     void* ex_ws;                  // kmg_extract workspace (stage path)
@@ -50,10 +57,13 @@ PipeWs carve_pipe(void* ws, uint64_t n_windows, int k, int rc, int val_bytes) {
     };
     const int kb = k <= 32 ? 8 : 16;
     const uint64_t cap = std::max<uint64_t>(n_windows * (rc ? 2 : 1), 1);
-    w.hist_ws = take(top_hist_workspace_bytes());
-    w.top = (unsigned long long*)take(3 * 256 * sizeof(uint64_t));
+    w.zeroed = (unsigned long long*)take(P16_ZEROED_WORDS * sizeof(uint64_t));
+    w.top = p16_top(w.zeroed);
+    w.plan = p16_plan(w.zeroed);
     w.cursors = (unsigned long long*)take(256 * sizeof(uint64_t));
-    w.plan = (unsigned long long*)take(4 * sizeof(uint64_t));
+    w.starts = (unsigned long long*)take(65537 * sizeof(uint64_t));
+    w.cursors16 = (unsigned long long*)take(65536 * sizeof(uint64_t));
+    w.rows = (uint32_t*)take(prefix16_rows_bytes());
     w.hist16 = (uint64_t*)take(16 * 256 * sizeof(uint64_t));
     w.n_out = (uint64_t*)take(sizeof(uint64_t));
     w.ex_ws_bytes = kmg_extract_workspace_bytes(n_windows);
@@ -118,8 +128,8 @@ int run_pipeline(int mode, const uint8_t* d_bases, uint64_t n_bases, uint64_t wi
     bool fused = k >= 16 && hybrid_sort_applies(cap, kb, val_bytes, 2 * k, true);
     if (fused) {
         timing_begin(st);
-        rcode = extract_top_hist(d_bases, n_bases, win_begin, win_end, k, rc, d_lut256, reinterpret_cast<uint64_t*>(w.plan + 2), w.top, w.plan, w.hist_ws,
-                                 top_hist_workspace_bytes(), st);
+        const Prefix16Out p16{w.zeroed, w.cursors, w.starts, w.cursors16, w.rows};
+        rcode = extract_prefix16_hist(d_bases, n_bases, win_begin, win_end, k, rc, d_lut256, p16, st);
         timing_end(st, 2);
         if (rcode != KMG_OK) return rcode;
         unsigned long long h_plan[4] = {0, 0, 0, 0};  // keys, largest top-byte count, windows counted, wide windows
@@ -129,7 +139,7 @@ int run_pipeline(int mode, const uint8_t* d_bases, uint64_t n_bases, uint64_t wi
         h_result[1] = n;
         h_result[2] = h_plan[3];
         KMG_REQUIRE(h_plan[2] * (rc ? 2 : 1) == n, KMG_ERR_STATE,
-                    "4-mer histograms (%llu keys) disagree with the window count (%llu)", h_plan[0],
+                    "prefix histogram (%llu keys) disagrees with the window count (%llu)", h_plan[0],
                     h_plan[2] * (rc ? 2 : 1));
         if (n == 0) return KMG_OK;
         fused = hybrid_sort_applies(n, kb, val_bytes, 2 * k, true);  // (most windows skipped: small after all)
@@ -137,12 +147,25 @@ int run_pipeline(int mode, const uint8_t* d_bases, uint64_t n_bases, uint64_t wi
             PrePartitioned pre;
             pre.pb = hybrid_choose_pb(n, h_plan[1], kb, val_bytes);
             pre.top = w.top;
-            exclusive_scan_256(w.top + (size_t)(3 - pre.pb / 8) * 256, w.cursors, st);
+            // pb = 16: the keys go to the regions of their TOP byte (cursors: the pre-pass' region starts),
+            // then every region is split by byte 2 on its own -- both passes order-free.
+            // pb = 24: byte 3 first, then the two stable passes of sort_impl.
+            const bool msd = pre.pb == 16;
+            if (!msd) exclusive_scan_256(w.top, w.cursors, st);
             timing_begin(st);
             rcode = extract_digit_scatter(d_bases, n_bases, win_begin, win_end, k, rc, d_lut256, d_keys, kb, d_vals, val_bytes,
-                                          pos_offset, w.cursors, 2 * k - pre.pb, st);
+                                          pos_offset, w.cursors, msd ? 2 * k - 8 : 2 * k - 24, st);
             timing_end(st, 3);
             if (rcode != KMG_OK) return rcode;
+            if (msd) {
+                timing_begin(st);
+                rcode = region_partition(d_keys, d_keys_alt, d_vals, d_vals_alt, n, kb, val_bytes, w.top + 2 * 256, w.cursors16,
+                                         2 * k - 16, st);
+                timing_end(st, 0);
+                if (rcode != KMG_OK) return rcode;
+                pre.bucket_starts = w.starts;
+                pre.in_alt = true;
+            }
             if (mode == 0)
                 rcode = sort_count_core(d_keys, d_keys_alt, n, kb, 2 * k, nullptr, d_counts_out, w.n_out, &sel, w.sort_ws,
                                         w.sort_ws_bytes, st, &pre);

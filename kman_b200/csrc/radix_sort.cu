@@ -497,7 +497,7 @@ thread_local int64_t g_stat_hybrid_irregular = -1;
 constexpr int MAX_TIMED = 64;
 thread_local cudaEvent_t g_ev[2 * MAX_TIMED];
 thread_local int g_ev_made = 0, g_ev_used = 0;
-thread_local int g_ev_kind[MAX_TIMED];          // 0: onesweep pass, 1: local sort, 2: histogram pre-pass, 3: fused extraction pass
+thread_local int g_ev_kind[MAX_TIMED];          // 0: prefix pass (onesweep / region partition), 1: local sort, 2: histogram pre-pass, 3: fused extraction pass
 thread_local double g_pass_ms_total[4] = {0, 0, 0, 0};
 thread_local int64_t g_pass_count_total[4] = {0, 0, 0, 0};
 
@@ -677,7 +677,9 @@ int hybrid_choose_pb(uint64_t n, unsigned long long max_top_byte_count, int key_
 
 // `pre` (fused pipeline): the keys in d_keys are ALREADY grouped by the lowest prefix byte (the first,
 // order-free prefix pass ran inside the extraction kernel); pre->top holds the histograms of the
-// three top key bytes and pre->pb the prefix width the caller chose.
+// three top key bytes and pre->pb the prefix width the caller chose.  With pre->bucket_starts the keys
+// are grouped by the whole 16-bit prefix (top byte in the extraction, byte 2 in region_partition_kernel):
+// no pass runs here at all.
 static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_alt, uint64_t n, int key_bytes,
                      int val_bytes, int begin_bit, int end_bit, const uint64_t* d_hist_in, int* h_selector_out,
                      void* d_ws, size_t ws_bytes, cudaStream_t st, bool hybrid, bool allow_hybrid,
@@ -686,6 +688,9 @@ static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_
     KMG_REQUIRE(ws_bytes >= w.total, KMG_ERR_WS, "sort workspace too small: %zu < %zu", ws_bytes, w.total);
     hybrid = hybrid && allow_hybrid;
     KMG_REQUIRE(!pre || hybrid, KMG_ERR_ARG, "pre-partitioned keys need the hybrid finish");
+    // (all prefix bits done: no pass runs here, the local sort takes its tile bounds from the bucket starts)
+    const bool prefix_done = pre && pre->bucket_starts;
+    KMG_REQUIRE(!prefix_done || pre->pb == 16, KMG_ERR_ARG, "bucket starts come with the 16-bit prefix");
 
     PassPlan plan = make_plan(begin_bit, end_bit);
     int np = plan.num_passes;
@@ -712,7 +717,8 @@ static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_
             plan.bits[i] = 8;
         }
         if (pre) {
-            KMG_CUDA(cudaMemcpyAsync(w.hist, pre->top, (size_t)3 * SORT_RADIX * sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
+            if (!prefix_done)  // (only the passes below read the rows)
+                KMG_CUDA(cudaMemcpyAsync(w.hist, pre->top, (size_t)3 * SORT_RADIX * sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
         } else if (d_hist_in && key_bytes == 8 && (end_bit & 1) == 0) {
             KMG_CUDA(cudaMemcpyAsync(w.hist, d_hist_in + (size_t)13 * SORT_RADIX, (size_t)3 * SORT_RADIX * sizeof(uint64_t),
                                      cudaMemcpyDeviceToDevice, st));
@@ -756,15 +762,24 @@ static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_
             radix_hist_kernel<u128, SORT_RADIX_BITS><<<grid, 512, smem, st>>>((const u128*)d_keys, n, plan, w.hist);
         KMG_LAUNCH_CHECK();
     }
-    radix_scan_kernel<<<np, 32, 0, st>>>(hist, w.bins, SORT_RADIX, 2 * SORT_RADIX, nullptr);
-    KMG_LAUNCH_CHECK();
+    if (!prefix_done) {
+        radix_scan_kernel<<<np, 32, 0, st>>>(hist, w.bins, SORT_RADIX, 2 * SORT_RADIX, nullptr);
+        KMG_LAUNCH_CHECK();
+    }
 
     char* kin = (char*)d_keys;
     char* kout = (char*)d_keys_alt;
     char* vin = (char*)d_vals;
     char* vout = (char*)d_vals_alt;
+    if (prefix_done) {
+        if (pre->in_alt) {
+            std::swap(kin, kout);
+            std::swap(vin, vout);
+        }
+        ++g_stat_sort_passes;  // the caller's region partition: the one prefix pass after the fused extraction
+    }
     uint32_t launch = 0;
-    for (int pass = pre ? 1 : 0; pass < np; ++pass) {
+    for (int pass = prefix_done ? np : (pre ? 1 : 0); pass < np; ++pass) {
         const ShiftDigit op{plan.shift[pass], (1u << plan.bits[pass]) - 1u};
         for (uint64_t part = 0; part < n_parts; ++part) {
             const uint64_t off = part * PART_MAX;
@@ -869,7 +884,8 @@ static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_
     auto launch_bounds = [&](uint32_t T) -> int {
         hp.tile_t = T;
         hp.n_tiles = (uint32_t)((n + T - 1) / T);
-        if (wide_key) tile_bounds_kernel<u128><<<(hp.n_tiles + 1 + 7) / 8, 256, 0, st>>>(hp);
+        if (prefix_done) bounds_from_starts_kernel<<<(hp.n_tiles + 1 + 255) / 256, 256, 0, st>>>(hp, pre->bucket_starts, 1u << pb);
+        else if (wide_key) tile_bounds_kernel<u128><<<(hp.n_tiles + 1 + 7) / 8, 256, 0, st>>>(hp);
         else tile_bounds_kernel<uint64_t><<<(hp.n_tiles + 1 + 7) / 8, 256, 0, st>>>(hp);
         KMG_LAUNCH_CHECK();
         // tiles that own more keys than the local sort holds (huge prefix buckets: repeats) are known
