@@ -181,9 +181,10 @@ int kmg_select_singletons(const void* d_sorted_keys, const void* d_vals, uint64_
  * (FastaBatcher.do batcher.py:454-487 + KJoiner.join join.py:337-391 on one flat base buffer.)
  * Same results as kmg_extract followed by kmg_sort_count / kmg_sort_uniq, but when the hybrid sort
  * applies (>= 2^20 keys, k >= 16) the extraction kernel itself is the sort's
- * first prefix pass: a pre-pass over the BASES yields the histograms of the top key bytes (4-mer
- * histogram), then every key is written once, straight into the region of its digit -- the keys are
- * never stored in extraction order.  Two host synchronisations per call (32 + 56 bytes read back).
+ * first prefix pass: a pre-pass over the BASES (the 16-bit prefix histogram of the valid windows)
+ * yields the histograms of the top key bytes, then every key is written once, straight into the region
+ * of its digit -- the keys are never stored in extraction order.  Two host synchronisations per call
+ * (32 + 56 bytes read back).
  * d_keys / d_keys_alt (and d_vals / d_vals_alt): capacity (win_end-win_begin)*(1+rc) items each.
  * h_result[4] (host): [0] rows of the result ((k-mer, count) pairs / singletons), [1] keys that were
  * sorted, [2] windows that belong to the WIDE stream (the caller runs those through the stage

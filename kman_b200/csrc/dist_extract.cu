@@ -1,7 +1,7 @@
 // Fused extraction + range partition + peer-memory exchange for the multi-GPU path.
 //
 // There is no counterpart in the reference (it merges batch files on one host,
-// kmermaid/join.py:63-93).  The extraction itself is the same K1+K2 as extract.cu
+// kmermaid/join.py:63-93).  The extraction itself is the K1+K2 front end of extract_tile.cuh
 // (kmermaid/seq.py:284-328, rc :245-282); what differs is where the keys go: every key is
 // written straight into the receive buffer of the GPU that owns its key range
 //     part = ((key >> (2k-16)) * n_parts) >> 16
@@ -15,13 +15,12 @@
 // slots with an atomic cursor); the full radix sort that follows makes the result deterministic.
 #include <type_traits>
 
-#include "common.cuh"
+#include "extract_tile.cuh"
 
 namespace kmg {
 
 int g_dx_align = 1;  // kmg_set_option("dx_align", 0/1): peer stores assigned from 128-byte line boundaries
 constexpr int DX_BLOCK = 256;
-constexpr int DX_HALO_WORDS = 8;
 constexpr int DX_MAX_PARTS = 64;
 
 struct ScatterParams {
@@ -45,25 +44,6 @@ struct ScatterParams {
     int align_stores;                        // peer stores assigned from 128-byte line boundaries (kmg_set_option "dx_align")
 };
 constexpr unsigned long long DX_NO_STORE = ~0ull;
-
-__device__ __forceinline__ uint64_t dx_rev2_64(uint64_t x) {
-    x = __brevll(x);
-    return ((x >> 1) & 0x5555555555555555ull) | ((x & 0x5555555555555555ull) << 1);
-}
-__device__ __forceinline__ uint64_t dx_rc_key(uint64_t key, int k) { return dx_rev2_64(~key) >> (64 - 2 * k); }
-__device__ __forceinline__ u128 dx_rc_key(const u128& key, int k) {
-    uint64_t hi = dx_rev2_64(~key.lo), lo = dx_rev2_64(~key.hi);
-    const int s = 128 - 2 * k;
-    u128 r;
-    if (s == 0) {
-        r.lo = lo;
-        r.hi = hi;
-    } else {
-        r.lo = (lo >> s) | (hi << (64 - s));
-        r.hi = hi >> s;
-    }
-    return r;
-}
 
 template <typename KeyT>
 __device__ __forceinline__ uint32_t part_of(const KeyT& key, int key_bits, uint32_t n_parts) {
@@ -90,7 +70,7 @@ __device__ __forceinline__ uint32_t part_rank(uint32_t part, bool active, int pa
 template <typename KeyT, int PPT, bool RC, int VAL_BYTES, bool COUNT_ONLY>
 __global__ void __launch_bounds__(DX_BLOCK) extract_scatter_kernel(const ScatterParams p) {
     constexpr int TILE = DX_BLOCK * PPT;
-    constexpr int WORDS = TILE / 16 + DX_HALO_WORDS;
+    constexpr int WORDS = TILE / 16 + EX_HALO_WORDS;
     constexpr int OUT_PER_WIN = RC ? 2 : 1;
     using ValT = typename std::conditional<VAL_BYTES == 4, uint32_t, uint64_t>::type;
 
@@ -113,62 +93,20 @@ __global__ void __launch_bounds__(DX_BLOCK) extract_scatter_kernel(const Scatter
     __syncthreads();
     const uint64_t tile_pos = (p.first_tile + tile) * (uint64_t)TILE;
 
-    // ---- K1: encode 16 bases per word (as extract.cu) -------------------------------------------
-    for (int w = t; w < WORDS; w += DX_BLOCK) {
-        const uint64_t pos = tile_pos + (uint64_t)w * 16;
-        uint32_t b[4];
-        if (pos + 16 <= p.n_bases) {
-            const uint4 v = __ldg(reinterpret_cast<const uint4*>(p.bases + pos));
-            b[0] = v.x; b[1] = v.y; b[2] = v.z; b[3] = v.w;
-        } else {
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                uint32_t x = 0;
-#pragma unroll
-                for (int r = 0; r < 4; ++r) {
-                    const uint64_t pp = pos + q * 4 + r;
-                    const uint32_t byte = (pp < p.n_bases) ? p.bases[pp] : 0xFFu;
-                    x |= byte << (8 * r);
-                }
-                b[q] = x;
-            }
-        }
-        const int nvalid = pos + 16 <= p.n_bases ? 16 : (pos < p.n_bases ? (int)(p.n_bases - pos) : 0);
-        uint32_t codes = 0, bad = 0, inv = 0;
-#pragma unroll
-        for (int j = 0; j < 16; ++j) {
-            const uint32_t byte = (b[j >> 2] >> (8 * (j & 3))) & 0xFFu;
-            uint32_t e = s_lut[byte];
-            if (j >= nvalid) e = KMG_LUT_INVALID;
-            codes |= (e & 3u) << (30 - 2 * j);
-            bad |= ((e >> 6) ? 1u : 0u) << (15 - j);
-            inv |= (e >> 7) << (15 - j);
-        }
-        s_codes[w] = codes;
-        s_bad[w] = (uint16_t)bad;
-        s_inv[w] = (uint16_t)inv;
-    }
+    encode_tile_words<DX_BLOCK, WORDS>(p.bases, p.n_bases, t, tile_pos, s_lut, s_codes, s_bad, s_inv);
     __syncthreads();
 
     // ---- K2: rolling windows ---------------------------------------------------------------------
     const int k = p.k;
     const int key_bits = 2 * k;
-    const int wbase = (t * PPT) >> 4;
     const int joff = (t * PPT) & 15;
-    const uint64_t X0 = ((uint64_t)s_codes[wbase] << 32) | s_codes[wbase + 1];
-    const uint64_t X1 = ((uint64_t)s_codes[wbase + 2] << 32) | s_codes[wbase + 3];
-    const uint64_t X2 = ((uint64_t)s_codes[wbase + 4] << 32) | s_codes[wbase + 5];
-    const uint64_t B0 = ((uint64_t)s_bad[wbase] << 48) | ((uint64_t)s_bad[wbase + 1] << 32) |
-                        ((uint64_t)s_bad[wbase + 2] << 16) | s_bad[wbase + 3];
-    const uint64_t B1 = ((uint64_t)s_bad[wbase + 4] << 48) | ((uint64_t)s_bad[wbase + 5] << 32) |
-                        ((uint64_t)s_bad[wbase + 6] << 16) | s_bad[wbase + 7];
-    const uint64_t I0 = ((uint64_t)s_inv[wbase] << 48) | ((uint64_t)s_inv[wbase + 1] << 32) |
-                        ((uint64_t)s_inv[wbase + 2] << 16) | s_inv[wbase + 3];
-    const uint64_t I1 = ((uint64_t)s_inv[wbase + 4] << 48) | ((uint64_t)s_inv[wbase + 5] << 32) |
-                        ((uint64_t)s_inv[wbase + 6] << 16) | s_inv[wbase + 7];
+    const auto [X0, X1, X2, B0, B1, I0, I1] = load_tile_words(s_codes, s_bad, s_inv, (t * PPT) >> 4);
     int part_bits = 0;
     while ((1 << part_bits) < p.n_parts) ++part_bits;
 
+    // Window validity as narrow_window_flags (extract_tile.cuh) decides it, but taken one window at a time
+    // next to that window's ranks: computed for all PPT windows up front, the same rule costs this kernel
+    // up to 10 registers (rc) and an 8-byte spill (u128 keys, 8-byte payload).
     // fast path: no base that is bad for the narrow stream among the PPT+k-1 bases my windows span
     bool span_clean;
     {
@@ -177,12 +115,13 @@ __global__ void __launch_bounds__(DX_BLOCK) extract_scatter_kernel(const Scatter
         if (span <= 64) span_clean = (W0 >> (64 - span)) == 0;
         else span_clean = W0 == 0 && ((B1 << joff) >> (128 - span)) == 0;
     }
+    uint32_t vf = 0, nwide = 0;
     // slot of every emitted key inside its destination group of the tile: (part << 20) | rank
     uint32_t where[PPT * OUT_PER_WIN];
     KeyT keys[PPT];
-    uint32_t vf = 0, nwide = 0;
 #pragma unroll
     for (int j = 0; j < PPT; ++j) {
+        // (every lane ranks every window: part_rank's ballots are warp-collective)
         const int je = joff + j;
         const uint64_t pos = tile_pos + (uint64_t)t * PPT + j;
         const bool in_range = pos >= p.win_begin && pos < p.win_end;
@@ -194,28 +133,13 @@ __global__ void __launch_bounds__(DX_BLOCK) extract_scatter_kernel(const Scatter
             if (in_range && im == 0 && bm != 0) ++nwide;
         }
         if (valid) vf |= 1u << j;
-        const int s2 = 2 * je;
-        const uint64_t hi = je == 0 ? X0 : ((X0 << s2) | (X1 >> (64 - s2)));
-        KeyT key;
-        if constexpr (sizeof(KeyT) == 8) {
-            key = hi >> (64 - 2 * k);
-        } else {
-            const uint64_t lo = je == 0 ? X1 : ((X1 << s2) | (X2 >> (64 - s2)));
-            const int s = 128 - 2 * k;
-            if (s == 0) {
-                key.lo = lo;
-                key.hi = hi;
-            } else {
-                key.lo = (lo >> s) | (hi << (64 - s));
-                key.hi = hi >> s;
-            }
-        }
+        const KeyT key = build_key<KeyT>(X0, X1, X2, joff + j, k);
         keys[j] = key;
         const uint32_t part = valid ? part_of(key, key_bits, (uint32_t)p.n_parts) : 0u;
         const uint32_t rank = part_rank(part, valid, part_bits, s_cnt);
         where[j * OUT_PER_WIN] = (part << 20) | rank;
         if constexpr (RC) {
-            const KeyT rk = dx_rc_key(key, k);
+            const KeyT rk = rc_key(key, k);
             const uint32_t part2 = valid ? part_of(rk, key_bits, (uint32_t)p.n_parts) : 0u;
             const uint32_t rank2 = part_rank(part2, valid, part_bits, s_cnt);
             where[j * 2 + 1] = (part2 << 20) | rank2;
@@ -268,12 +192,12 @@ __global__ void __launch_bounds__(DX_BLOCK) extract_scatter_kernel(const Scatter
             const uint32_t w0 = where[j * OUT_PER_WIN];
             const uint32_t i0 = s_off[w0 >> 20] + (w0 & 0xFFFFFu);
             s_keys[i0] = keys[j];
-            if constexpr (VAL_BYTES != 0) s_vals[i0] = (ValT)((pos << 1) | 0u);
+            if constexpr (VAL_BYTES != 0) s_vals[i0] = make_val<ValT>(pos, 0);
             if constexpr (RC) {
                 const uint32_t w1 = where[j * 2 + 1];
                 const uint32_t i1 = s_off[w1 >> 20] + (w1 & 0xFFFFFu);
-                s_keys[i1] = dx_rc_key(keys[j], k);
-                if constexpr (VAL_BYTES != 0) s_vals[i1] = (ValT)((pos << 1) | 1u);
+                s_keys[i1] = rc_key(keys[j], k);
+                if constexpr (VAL_BYTES != 0) s_vals[i1] = make_val<ValT>(pos, 1);
             }
         }
         __syncthreads();

@@ -3,18 +3,15 @@
 // Replaces Sequence.yield_kmers (kmermaid/seq.py:284-328), its reverse-complement variant
 // (seq.py:245-282) and the second alphabet filter (seq.py:500-509 via batcher.py:559-561).
 //
-// Narrow stream: a tile of 16-base words is staged in shared memory as 2-bit codes plus two
-// bitmasks (bad-for-narrow, invalid-for-any-stream); every thread then produces the keys of
-// its consecutive window starts with funnel shifts out of 64-bit big-endian code words, so a
-// base is looked up in the LUT exactly once.  Valid keys are compacted in position order
+// Narrow stream: the tile front end of extract_tile.cuh (LUT encode once per base, keys by funnel
+// shifts out of 64-bit big-endian code words).  Valid keys are compacted in position order
 // (block scan + decoupled look-back across tiles), staged in shared memory and written with
 // fully coalesced stores.
-#include "common.cuh"
+#include "extract_tile.cuh"
 
 namespace kmg {
 
 constexpr int EX_BLOCK_DEFAULT = 256;  // threads of the position-ordered extraction (MODE 0)
-constexpr int EX_HALO_WORDS = 8;  // 16-base words past the tile that masks/codes may touch
 
 struct ExtractParams {
     const uint8_t* bases;
@@ -71,113 +68,6 @@ __device__ __forceinline__ bool plain4_at(uint64_t B0, uint64_t B1, int e) {
     else if (e < 64) v = (B0 << e) | (B1 >> (64 - e));
     else v = B1 << (e - 64);
     return (v >> 60) == 0;
-}
-
-__device__ __forceinline__ uint64_t rev2_64(uint64_t x) {
-    x = __brevll(x);
-    return ((x >> 1) & 0x5555555555555555ull) | ((x & 0x5555555555555555ull) << 1);
-}
-__device__ __forceinline__ uint64_t rc_key(uint64_t key, int k) { return rev2_64(~key) >> (64 - 2 * k); }
-__device__ __forceinline__ u128 rc_key(const u128& key, int k) {
-    uint64_t hi = rev2_64(~key.lo), lo = rev2_64(~key.hi);
-    int s = 128 - 2 * k;  // 0 <= s <= 62 because k >= 33
-    u128 r;
-    if (s == 0) {
-        r.lo = lo;
-        r.hi = hi;
-    } else {
-        r.lo = (lo >> s) | (hi << (64 - s));
-        r.hi = hi >> s;
-    }
-    return r;
-}
-
-template <typename ValT>
-__device__ __forceinline__ ValT make_val(uint64_t pos, uint32_t strand) {
-    return (ValT)((pos << 1) | strand);
-}
-
-// K1 of extract_narrow_kernel for the pre-pass: the bases [tile_pos, tile_pos + 16 * WORDS) of p.bases as 16-base words of 2-bit
-// codes (first base in the top bits) plus the bad-for-narrow and invalid-for-any-stream bitmasks
-template <int BLOCK, int WORDS, typename Params>
-__device__ __forceinline__ void encode_tile_words(const Params& p, int t, uint64_t tile_pos, const uint8_t* s_lut,
-                                                  uint32_t* s_codes, uint16_t* s_bad, uint16_t* s_inv) {
-    for (int w = t; w < WORDS; w += BLOCK) {
-        const uint64_t pos = tile_pos + (uint64_t)w * 16;
-        uint32_t b[4];
-        if (pos + 16 <= p.n_bases) {
-            const uint4 v = __ldg(reinterpret_cast<const uint4*>(p.bases + pos));
-            b[0] = v.x; b[1] = v.y; b[2] = v.z; b[3] = v.w;
-        } else {
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                uint32_t x = 0;
-#pragma unroll
-                for (int r = 0; r < 4; ++r) {
-                    const uint64_t pp = pos + q * 4 + r;
-                    // 0xFF is never in an alphabet built by kmg_build_lut; the explicit
-                    // range test below does not rely on that.
-                    const uint32_t byte = (pp < p.n_bases) ? p.bases[pp] : 0xFFu;
-                    x |= byte << (8 * r);
-                }
-                b[q] = x;
-            }
-        }
-        const int nvalid = pos + 16 <= p.n_bases ? 16 : (pos < p.n_bases ? (int)(p.n_bases - pos) : 0);
-        uint32_t codes = 0, bad = 0, inv = 0;
-#pragma unroll
-        for (int j = 0; j < 16; ++j) {
-            const uint32_t byte = (b[j >> 2] >> (8 * (j & 3))) & 0xFFu;
-            uint32_t e = s_lut[byte];
-            if (j >= nvalid) e = KMG_LUT_INVALID;
-            codes |= (e & 3u) << (30 - 2 * j);
-            bad |= ((e >> 6) ? 1u : 0u) << (15 - j);
-            inv |= (e >> 7) << (15 - j);
-        }
-        s_codes[w] = codes;
-        s_bad[w] = (uint16_t)bad;
-        s_inv[w] = (uint16_t)inv;
-    }
-}
-
-// Validity of the PPT consecutive window starts first_pos .. first_pos + PPT - 1 (bit j: window j),
-// given the 128-base bad / invalid mask strings B0:B1, I0:I1 that start at the word of window 0
-// (joff = its base inside that word).  vf: the window lies in [win_begin, win_end) and all its k
-// bases are plain (the narrow stream); *nwide: windows of the range that belong to the wide stream.
-// *clean: no base of the PPT + k - 1 the windows span is bad (every window of the range is valid).
-template <int PPT>
-__device__ __forceinline__ uint32_t narrow_window_flags(uint64_t first_pos, uint64_t win_begin, uint64_t win_end, int k,
-                                                        int joff, uint64_t B0, uint64_t B1, uint64_t I0, uint64_t I1,
-                                                        uint32_t& in_range_mask, bool& span_clean, uint32_t& nwide) {
-    {   // window starts [win_begin, win_end) among my PPT positions
-        const uint64_t lo = win_begin > first_pos ? win_begin - first_pos : 0;
-        const uint64_t hi = win_end > first_pos ? win_end - first_pos : 0;
-        const uint32_t l = lo < PPT ? (uint32_t)lo : PPT, h = hi < PPT ? (uint32_t)hi : PPT;
-        in_range_mask = h > l ? (((1u << (h - l)) - 1u) << l) : 0u;
-    }
-    // fast path: no base that is bad for the narrow stream among the PPT+k-1 bases my windows span
-    {
-        const uint64_t W0 = joff == 0 ? B0 : ((B0 << joff) | (B1 >> (64 - joff)));
-        const int span = PPT + k - 1;  // 17 .. 79
-        if (span <= 64) span_clean = (W0 >> (64 - span)) == 0;
-        else span_clean = W0 == 0 && ((B1 << joff) >> (128 - span)) == 0;
-    }
-    uint32_t vf = 0;
-    nwide = 0;
-    if (span_clean) {
-        vf = in_range_mask;
-    } else {
-#pragma unroll
-        for (int j = 0; j < PPT; ++j) {
-            const int je = joff + j;  // 0..15
-            const uint64_t bm = (je == 0 ? B0 : ((B0 << je) | (B1 >> (64 - je)))) >> (64 - k);
-            const uint64_t im = (je == 0 ? I0 : ((I0 << je) | (I1 >> (64 - je)))) >> (64 - k);
-            const bool in_range = (in_range_mask >> j) & 1u;
-            if (in_range && bm == 0) vf |= 1u << j;
-            if (in_range && im == 0 && bm != 0) ++nwide;
-        }
-    }
-    return vf;
 }
 
 // The order-free prefix pass of one tile (extraction MODE 2 and region_partition_kernel): the keys of
@@ -286,114 +176,22 @@ __global__ void __launch_bounds__(EX_BLOCK) extract_narrow_kernel(const ExtractP
     const uint32_t tile = s_tile;
     const uint64_t tile_pos = (p.first_tile + tile) * (uint64_t)TILE;
 
-    // ---- K1: encode 16 bases per word ----------------------------------------------------
-    for (int w = t; w < WORDS; w += EX_BLOCK) {
-        const uint64_t pos = tile_pos + (uint64_t)w * 16;
-        uint32_t b[4];
-        if (pos + 16 <= p.n_bases) {
-            const uint4 v = __ldg(reinterpret_cast<const uint4*>(p.bases + pos));
-            b[0] = v.x; b[1] = v.y; b[2] = v.z; b[3] = v.w;
-        } else {
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                uint32_t x = 0;
-#pragma unroll
-                for (int r = 0; r < 4; ++r) {
-                    const uint64_t pp = pos + q * 4 + r;
-                    // 0xFF is never in an alphabet built by kmg_build_lut; the explicit
-                    // range test below does not rely on that.
-                    const uint32_t byte = (pp < p.n_bases) ? p.bases[pp] : 0xFFu;
-                    x |= byte << (8 * r);
-                }
-                b[q] = x;
-            }
-        }
-        const int nvalid = pos + 16 <= p.n_bases ? 16 : (pos < p.n_bases ? (int)(p.n_bases - pos) : 0);
-        uint32_t codes = 0, bad = 0, inv = 0;
-#pragma unroll
-        for (int j = 0; j < 16; ++j) {
-            const uint32_t byte = (b[j >> 2] >> (8 * (j & 3))) & 0xFFu;
-            uint32_t e = s_lut[byte];
-            if (j >= nvalid) e = KMG_LUT_INVALID;
-            codes |= (e & 3u) << (30 - 2 * j);
-            bad |= ((e >> 6) ? 1u : 0u) << (15 - j);
-            inv |= (e >> 7) << (15 - j);
-        }
-        s_codes[w] = codes;
-        s_bad[w] = (uint16_t)bad;
-        s_inv[w] = (uint16_t)inv;
-    }
+    encode_tile_words<EX_BLOCK, WORDS>(p.bases, p.n_bases, t, tile_pos, s_lut, s_codes, s_bad, s_inv);
     __syncthreads();
 
     // ---- K2: rolling windows ---------------------------------------------------------------
     const int k = p.k;
-    const int wbase = (t * PPT) >> 4;
     const int joff = (t * PPT) & 15;
-    const uint64_t X0 = ((uint64_t)s_codes[wbase] << 32) | s_codes[wbase + 1];
-    const uint64_t X1 = ((uint64_t)s_codes[wbase + 2] << 32) | s_codes[wbase + 3];
-    const uint64_t X2 = ((uint64_t)s_codes[wbase + 4] << 32) | s_codes[wbase + 5];
-    const uint64_t B0 = ((uint64_t)s_bad[wbase] << 48) | ((uint64_t)s_bad[wbase + 1] << 32) |
-                        ((uint64_t)s_bad[wbase + 2] << 16) | s_bad[wbase + 3];
-    const uint64_t B1 = ((uint64_t)s_bad[wbase + 4] << 48) | ((uint64_t)s_bad[wbase + 5] << 32) |
-                        ((uint64_t)s_bad[wbase + 6] << 16) | s_bad[wbase + 7];
-    const uint64_t I0 = ((uint64_t)s_inv[wbase] << 48) | ((uint64_t)s_inv[wbase + 1] << 32) |
-                        ((uint64_t)s_inv[wbase + 2] << 16) | s_inv[wbase + 3];
-    const uint64_t I1 = ((uint64_t)s_inv[wbase + 4] << 48) | ((uint64_t)s_inv[wbase + 5] << 32) |
-                        ((uint64_t)s_inv[wbase + 6] << 16) | s_inv[wbase + 7];
+    const auto [X0, X1, X2, B0, B1, I0, I1] = load_tile_words(s_codes, s_bad, s_inv, (t * PPT) >> 4);
 
     // validity of my PPT windows first: the tile's count is published as early as possible and
-    // the prefix over the earlier tiles is resolved only after the keys have been built
-    const uint64_t first_pos = tile_pos + (uint64_t)t * PPT;
-    uint32_t in_range_mask;
-    {   // window starts [win_begin, win_end) among my PPT positions
-        const uint64_t lo = p.win_begin > first_pos ? p.win_begin - first_pos : 0;
-        const uint64_t hi = p.win_end > first_pos ? p.win_end - first_pos : 0;
-        const uint32_t l = lo < PPT ? (uint32_t)lo : PPT, h = hi < PPT ? (uint32_t)hi : PPT;
-        in_range_mask = h > l ? (((1u << (h - l)) - 1u) << l) : 0u;
-    }
-    // fast path: no base that is bad for the narrow stream among the PPT+k-1 bases my windows span
+    // the prefix over the earlier tiles is resolved only after the keys have been built.  MODE 2 counts
+    // no wide windows (the pre-pass does): all-invalid masks let the compiler drop s_inv altogether.
+    uint32_t in_range_mask, nwide;
     bool span_clean;
-    {
-        const uint64_t W0 = joff == 0 ? B0 : ((B0 << joff) | (B1 >> (64 - joff)));
-        const int span = PPT + k - 1;  // 17 .. 79
-        if (span <= 64) span_clean = (W0 >> (64 - span)) == 0;
-        else span_clean = W0 == 0 && ((B1 << joff) >> (128 - span)) == 0;
-    }
-    uint32_t vf = 0, nwide = 0;
-    if (span_clean) {
-        vf = in_range_mask;
-    } else {
-#pragma unroll
-        for (int j = 0; j < PPT; ++j) {
-            const int je = joff + j;  // 0..15
-            const uint64_t bm = (je == 0 ? B0 : ((B0 << je) | (B1 >> (64 - je)))) >> (64 - k);
-            const uint64_t im = (je == 0 ? I0 : ((I0 << je) | (I1 >> (64 - je)))) >> (64 - k);
-            const bool in_range = (in_range_mask >> j) & 1u;
-            if (in_range && bm == 0) vf |= 1u << j;
-            if (in_range && im == 0 && bm != 0) ++nwide;
-        }
-    }
-    // key of my j-th window start
-    auto build_key = [&](int j) -> KeyT {
-        const int je = joff + j;
-        const int s2 = 2 * je;
-        const uint64_t hi = je == 0 ? X0 : ((X0 << s2) | (X1 >> (64 - s2)));
-        KeyT key;
-        if constexpr (sizeof(KeyT) == 8) {
-            key = hi >> (64 - 2 * k);
-        } else {
-            const uint64_t lo = je == 0 ? X1 : ((X1 << s2) | (X2 >> (64 - s2)));
-            const int s = 128 - 2 * k;
-            if (s == 0) {
-                key.lo = lo;
-                key.hi = hi;
-            } else {
-                key.lo = (lo >> s) | (hi << (64 - s));
-                key.hi = hi >> s;
-            }
-        }
-        return key;
-    };
+    const uint32_t vf = narrow_window_flags<PPT>(tile_pos + (uint64_t)t * PPT, p.win_begin, p.win_end, k, joff, B0, B1,
+                                                 MODE == 2 ? ~0ull : I0, MODE == 2 ? ~0ull : I1, in_range_mask,
+                                                 span_clean, nwide);
 
     // FILTER: bit OUT_PER_WIN*j (+1 for the '-' key) is set when that key of window j is kept
     uint32_t kf = 0;
@@ -401,7 +199,7 @@ __global__ void __launch_bounds__(EX_BLOCK) extract_narrow_kernel(const ExtractP
 #pragma unroll
         for (int j = 0; j < PPT; ++j) {
             if (!(vf & (1u << j))) continue;
-            const KeyT key = build_key(j);
+            const KeyT key = build_key<KeyT>(X0, X1, X2, joff + j, k);
             if (in_parts(key_digit(key, p.part_shift, p.part_mask), p)) kf |= 1u << (j * OUT_PER_WIN);
             if constexpr (RC) {
                 if (in_parts(key_digit(rc_key(key, k), p.part_shift, p.part_mask), p)) kf |= 1u << (j * 2 + 1);
@@ -472,7 +270,7 @@ __global__ void __launch_bounds__(EX_BLOCK) extract_narrow_kernel(const ExtractP
 #pragma unroll
         for (int j = 0; j < PPT; ++j) {
             if (!(vf & (1u << j))) continue;
-            const KeyT key = build_key(j);
+            const KeyT key = build_key<KeyT>(X0, X1, X2, joff + j, k);
             wh[j * OUT_PER_WIN] = runs.rank(key_digit(key, dsh, 255u));
             if constexpr (RC) wh[j * 2 + 1] = runs.rank(key_digit(rc_key(key, k), dsh, 255u));
         }
@@ -481,7 +279,7 @@ __global__ void __launch_bounds__(EX_BLOCK) extract_narrow_kernel(const ExtractP
 #pragma unroll
         for (int j = 0; j < PPT; ++j) {
             if (!(vf & (1u << j))) continue;
-            const KeyT key = build_key(j);
+            const KeyT key = build_key<KeyT>(X0, X1, X2, joff + j, k);
             const uint64_t pos = tile_pos + (uint64_t)t * PPT + j + p.pos_offset;
             const uint32_t i0 = runs.slot(wh[j * OUT_PER_WIN]);
             s_keys[i0] = key;
@@ -503,7 +301,7 @@ __global__ void __launch_bounds__(EX_BLOCK) extract_narrow_kernel(const ExtractP
 #pragma unroll
     for (int j = 0; j < PPT; ++j) {
         if (!(vf & (1u << j))) continue;
-        const KeyT key = build_key(j);
+        const KeyT key = build_key<KeyT>(X0, X1, X2, joff + j, k);
         const uint64_t pos = tile_pos + (uint64_t)t * PPT + j + p.pos_offset;
         if constexpr (FILTER) {
             if ((kf >> (j * OUT_PER_WIN)) & 1u) {
@@ -963,15 +761,9 @@ __global__ void __launch_bounds__(P16_BLOCK, 1) prefix16_hist_kernel(const Prefi
     for (uint32_t tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
         __syncthreads();  // (the previous tile's words are consumed; first round: the tables are zeroed)
         const uint64_t tile_pos = (p.first_tile + tile) * P16_TILE;
-        encode_tile_words<P16_BLOCK, WORDS>(p, t, tile_pos, s_lut, s_codes, s_bad, s_inv);
+        encode_tile_words<P16_BLOCK, WORDS>(p.bases, p.n_bases, t, tile_pos, s_lut, s_codes, s_bad, s_inv);
         __syncthreads();
-        const uint64_t X0 = ((uint64_t)s_codes[t] << 32) | s_codes[t + 1];
-        const uint64_t X1 = ((uint64_t)s_codes[t + 2] << 32) | s_codes[t + 3];
-        const uint64_t X2 = ((uint64_t)s_codes[t + 4] << 32) | s_codes[t + 5];
-        const uint64_t B0 = ((uint64_t)s_bad[t] << 48) | ((uint64_t)s_bad[t + 1] << 32) | ((uint64_t)s_bad[t + 2] << 16) | s_bad[t + 3];
-        const uint64_t B1 = ((uint64_t)s_bad[t + 4] << 48) | ((uint64_t)s_bad[t + 5] << 32) | ((uint64_t)s_bad[t + 6] << 16) | s_bad[t + 7];
-        const uint64_t I0 = ((uint64_t)s_inv[t] << 48) | ((uint64_t)s_inv[t + 1] << 32) | ((uint64_t)s_inv[t + 2] << 16) | s_inv[t + 3];
-        const uint64_t I1 = ((uint64_t)s_inv[t + 4] << 48) | ((uint64_t)s_inv[t + 5] << 32) | ((uint64_t)s_inv[t + 6] << 16) | s_inv[t + 7];
+        const auto [X0, X1, X2, B0, B1, I0, I1] = load_tile_words(s_codes, s_bad, s_inv, t);
         uint32_t in_range_mask, nwide;
         bool span_clean;
         const uint32_t vf = narrow_window_flags<P16_PPT>(tile_pos + (uint64_t)t * P16_PPT, p.win_begin, p.win_end, k, 0, B0, B1,
@@ -1379,13 +1171,7 @@ static int extract_impl(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_b
     WsHeader* hdr = reinterpret_cast<WsHeader*>(d_ws);
 
     ExtractParams p;
-    p.bases = d_bases;
-    p.n_bases = n_bases;
-    p.win_begin = win_begin;
-    p.win_end = win_end;
-    p.first_tile = first_tile;
-    p.k = k;
-    p.lut = d_lut256;
+    fill_common(p, d_bases, n_bases, win_begin, win_end, tile, k, d_lut256);
     p.comp16 = d_comp16;
     p.keys_out = d_keys_out;
     p.vals_out = d_vals_out;
@@ -1395,7 +1181,6 @@ static int extract_impl(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_b
     p.ticket = &hdr->ticket;
     p.err = &hdr->err;
     p.hs = reinterpret_cast<unsigned long long*>((char*)d_ws + sizeof(WsHeader) + state_bytes);
-    p.n_off = 0;
     if (f) {
         const int b = part_bits(f->n_parts);
         p.part_shift = b ? 2 * k - b : 0;
