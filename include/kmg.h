@@ -344,18 +344,8 @@ int kmg_uniq_host(kmg_ctx* ctx, const uint8_t* h_bases, uint64_t n_bases, int k,
  * Options (process-wide; defaults in brackets):
  *   "hybrid" [1]           hybrid finish of key-only 8-byte sorts (0: plain LSD passes only)
  *   "hybrid_pb" [0]        force its prefix width to 16 or 24 bits (0: by n and key skew)
- *   "hybrid_unstable" [1]  first prefix pass ranks with the histogram atomics' return values
- *   "unstable_config" [10] tile shape of that pass (10: 256x24, 11: 256x16, 12: 384x16)
  *   "count_fused" [1]      kmg_sort_count: the local sort emits the (k-mer, count) table itself
  *   "local_tile" [7936]    target tile width of the local sort (positions)
- *   "dx_align" [1]         kmg_extract_scatter*: assign the threads of a peer store from the 128-byte line the
- *                          destination run starts in (whole-line NVLink writes) instead of from the run's start
- *   "local_v" [2]          local sort kernel: 1 = one cell per key + per-thread walks, 2 = fine cells
- *                          (only colliding keys are ever compared; local_sort_fine.cuh) wherever a tile holds
- *                          several prefix buckets and kernel 1 for one-bucket tiles, 3 = fine cells always
- *   "sort_config" [3]      tile configuration of the onesweep kernel (radix_sort.cu: dispatch_tile)
- *   "lb_group" [32]        tiles per look-back group of the onesweep kernel
- *   "prefetch_tiles" [192] L2 prefetch distance of the onesweep kernel, in tiles (0: off)
  *   "time_passes" [0]      bracket every onesweep / local sort launch with CUDA events
  *   "count_limit" [0]      test hook: run lengths above it raise KMG_ERR_RANGE in the run-length stage
  *                          (0 = the real limit 2^32-1)

@@ -12,21 +12,14 @@ namespace kmg {
 
 static thread_local char g_err[512] = "";
 static thread_local int64_t g_launches = 0;
-extern int g_sort_config;
 extern int g_time_passes;
-extern int g_lb_group;
 extern int g_hybrid;
 extern int g_hybrid_pb;
 extern int g_count_fused;
-extern int g_dx_align;
-extern int g_local_v;
-extern int g_hybrid_unstable;
-extern int g_unstable_config;
 extern int g_local_tile;
 extern thread_local int64_t g_stat_hybrid_irregular;
 extern thread_local int64_t g_stat_hybrid_path;
 extern thread_local int64_t g_stat_hybrid_big_runs;
-extern int g_prefetch_tiles;
 extern int64_t g_count_limit;
 extern thread_local int64_t g_stat_sort_passes;
 void timing_collect();
@@ -62,31 +55,9 @@ extern "C" int kmg_device_count(void) {
 
 extern "C" int kmg_set_option(const char* name, int64_t value) {
     KMG_REQUIRE(name, KMG_ERR_ARG, "option name is null");
-    if (!strcmp(name, "sort_config")) {
-        g_sort_config = (int)value;
-        return KMG_OK;
-    }
     if (!strcmp(name, "local_tile")) {
         KMG_REQUIRE(value >= 2048 && value <= 7936, KMG_ERR_ARG, "local_tile must be in [2048,7936]");
         g_local_tile = (int)value;
-        return KMG_OK;
-    }
-    if (!strcmp(name, "dx_align")) {
-        g_dx_align = value != 0;
-        return KMG_OK;
-    }
-    if (!strcmp(name, "local_v")) {
-        KMG_REQUIRE(value >= 1 && value <= 3, KMG_ERR_ARG, "local_v must be 1, 2 or 3");
-        g_local_v = (int)value;
-        return KMG_OK;
-    }
-    if (!strcmp(name, "unstable_config")) {
-        KMG_REQUIRE(value >= 10 && value <= 12, KMG_ERR_ARG, "unstable_config must be 10, 11 or 12");
-        g_unstable_config = (int)value;
-        return KMG_OK;
-    }
-    if (!strcmp(name, "hybrid_unstable")) {
-        g_hybrid_unstable = value != 0;
         return KMG_OK;
     }
     if (!strcmp(name, "count_fused")) {
@@ -99,16 +70,6 @@ extern "C" int kmg_set_option(const char* name, int64_t value) {
     }
     if (!strcmp(name, "hybrid")) {
         g_hybrid = value != 0;
-        return KMG_OK;
-    }
-    if (!strcmp(name, "prefetch_tiles")) {
-        KMG_REQUIRE(value >= 0 && value <= 65536, KMG_ERR_ARG, "prefetch_tiles must be in [0,65536]");
-        g_prefetch_tiles = (int)value;
-        return KMG_OK;
-    }
-    if (!strcmp(name, "lb_group")) {
-        KMG_REQUIRE(value >= 8 && value <= 4096, KMG_ERR_ARG, "lb_group must be in [8,4096]");
-        g_lb_group = (int)value;
         return KMG_OK;
     }
     if (!strcmp(name, "count_limit")) {

@@ -19,7 +19,6 @@
 
 namespace kmg {
 
-int g_dx_align = 1;  // kmg_set_option("dx_align", 0/1): peer stores assigned from 128-byte line boundaries
 constexpr int DX_BLOCK = 256;
 constexpr int DX_MAX_PARTS = 64;
 
@@ -41,7 +40,6 @@ struct ScatterParams {
     unsigned long long* const* cursor_ptrs;  // device array [n_parts] or null
     unsigned long long capacity;             // elements every receive buffer holds
     uint32_t* status;                        // [0] = 1: a reservation passed `capacity`; [1] = 1: wide windows seen
-    int align_stores;                        // peer stores assigned from 128-byte line boundaries (kmg_set_option "dx_align")
 };
 constexpr unsigned long long DX_NO_STORE = ~0ull;
 
@@ -201,34 +199,22 @@ __global__ void __launch_bounds__(DX_BLOCK) extract_scatter_kernel(const Scatter
             }
         }
         __syncthreads();
-        // peer stores: every destination group is a contiguous run -> coalesced NVLink writes
-        if (p.align_stores) {
-            // ... and 128-byte aligned ones: a run starts anywhere in its destination, so the threads are
-            // assigned from the 128-byte line the run starts in (the first lanes of the first round sit idle)
-            // and every warp store covers whole lines instead of straddling them
-            constexpr uint32_t LINE = 128 / sizeof(KeyT);
-            for (int d = 0; d < p.n_parts; ++d) {
-                const unsigned long long b = s_base[d];
-                if (b == DX_NO_STORE) continue;
-                const uint32_t cnt = s_off[d + 1] - s_off[d];
-                const uint32_t shift = (uint32_t)((reinterpret_cast<uintptr_t>(p.dest_keys[d]) / sizeof(KeyT) + b) & (LINE - 1));
-                KeyT* dk = reinterpret_cast<KeyT*>(p.dest_keys[d]) + b;
-                for (uint32_t j = t; j < cnt + shift; j += DX_BLOCK) {
-                    if (j < shift) continue;
-                    const uint32_t o = j - shift;
-                    dk[o] = s_keys[s_off[d] + o];
-                    if constexpr (VAL_BYTES != 0) (reinterpret_cast<ValT*>(p.dest_vals[d]) + b)[o] = s_vals[s_off[d] + o];
-                }
-            }
-        } else {
-            const uint32_t total = s_off[p.n_parts];
-            for (uint32_t i = t; i < total; i += DX_BLOCK) {
-                const KeyT key = s_keys[i];
-                const uint32_t d = part_of(key, key_bits, (uint32_t)p.n_parts);
-                if (s_base[d] == DX_NO_STORE) continue;
-                const unsigned long long at = s_base[d] + (i - s_off[d]);
-                reinterpret_cast<KeyT*>(p.dest_keys[d])[at] = key;
-                if constexpr (VAL_BYTES != 0) reinterpret_cast<ValT*>(p.dest_vals[d])[at] = s_vals[i];
+        // peer stores: every destination group is a contiguous run -> coalesced NVLink writes, and 128-byte
+        // aligned ones: a run starts anywhere in its destination, so the threads are assigned from the
+        // 128-byte line the run starts in (the first lanes of the first round sit idle) and every warp store
+        // covers whole lines instead of straddling them
+        constexpr uint32_t LINE = 128 / sizeof(KeyT);
+        for (int d = 0; d < p.n_parts; ++d) {
+            const unsigned long long b = s_base[d];
+            if (b == DX_NO_STORE) continue;
+            const uint32_t cnt = s_off[d + 1] - s_off[d];
+            const uint32_t shift = (uint32_t)((reinterpret_cast<uintptr_t>(p.dest_keys[d]) / sizeof(KeyT) + b) & (LINE - 1));
+            KeyT* dk = reinterpret_cast<KeyT*>(p.dest_keys[d]) + b;
+            for (uint32_t j = t; j < cnt + shift; j += DX_BLOCK) {
+                if (j < shift) continue;
+                const uint32_t o = j - shift;
+                dk[o] = s_keys[s_off[d] + o];
+                if constexpr (VAL_BYTES != 0) (reinterpret_cast<ValT*>(p.dest_vals[d]) + b)[o] = s_vals[s_off[d] + o];
             }
         }
     }
@@ -301,7 +287,6 @@ static int scatter_impl(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_b
     p.dest_vals = d_dest_vals;
     p.cursors = reinterpret_cast<unsigned long long*>(d_cursors);
     p.counts = reinterpret_cast<unsigned long long*>(d_counts);
-    p.align_stores = g_dx_align;
     p.pos_offset = pos_offset;
     p.cursor_ptrs = reinterpret_cast<unsigned long long* const*>(d_cursor_ptrs);
     p.capacity = capacity;

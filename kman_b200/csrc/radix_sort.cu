@@ -115,8 +115,6 @@ struct OnesweepParams {
     uint32_t* lb_ginc;        // [groups][RADIX]  tag | digit count of all tiles up to the END of the group
     uint32_t* ticket;
     uint32_t* err;
-    uint32_t prefetch_tiles;  // L2 prefetch distance in tiles (0 = off)
-    uint32_t lb_group;  // tiles per look-back group
     uint32_t tag;  // (epoch 1..3) << 30: words carrying another tag are "not written yet", so the
                    // arrays need no re-zeroing between the passes of one sort
 };
@@ -136,14 +134,16 @@ struct ValType<4> {
 // only dependency chain runs over the groups' last tiles, which resolve their prefix EARLY
 // (right after publishing their counts): one link per LB_GROUP tiles instead of one per tile.
 // Every word carries the launch's 2-bit tag; a word with another tag has not been written yet.
-constexpr uint32_t LB_GROUP_MIN = 8;   // workspace sizing
+// (group sizes 16 to 48 and prefetch distances 96 to 400 measured within 5 %: profiles/r01_stage_sweep_v15.log)
+constexpr uint32_t LB_GROUP = 32;
 constexpr int LB_BATCH = 16;           // loads a thread keeps in flight
+constexpr uint32_t PREFETCH_TILES = 192;  // L2 prefetch distance in tiles
 
 __device__ __forceinline__ uint32_t lookback_two_level(const uint32_t* __restrict__ lb_agg,
                                                        const uint32_t* __restrict__ lb_ginc, uint32_t tile,
-                                                       uint32_t lb_group, int d, int radix, uint32_t tag,
+                                                       int d, int radix, uint32_t tag,
                                                        uint32_t* err) {
-    const uint32_t g = tile / lb_group, r = tile % lb_group;
+    const uint32_t g = tile / LB_GROUP, r = tile % LB_GROUP;
     uint32_t excl = 0, spins = 0;
     const uint32_t* gsrc = lb_ginc + (size_t)(g ? g - 1 : 0) * radix + d;
     uint32_t gw = g ? ld_relaxed_u32(gsrc) : tag;  // issued first: it is the one that may lag
@@ -176,26 +176,25 @@ __device__ __forceinline__ uint32_t lookback_two_level(const uint32_t* __restric
     return excl + (gw & LB_VALUE_MASK);
 }
 
-// MIX: how a warp finds the lanes that hold the same digit
-//   0 = 8 ballots per key (ALU), 1 = shared-memory lane-mask table (LSU), 2 = alternate per item,
-//   3 = table for every 4th item, 4 = table for 3 items out of 4
-//   5 = UNSTABLE: the rank among equal digits is the value the histogram atomic returned -- no
-//       matching at all.  Only for a pass whose order inside a digit does not matter: the first
-//       prefix pass of the hybrid finish (the local sort orders everything below the prefix).
-__host__ __device__ constexpr bool mix_uses_table(int mix, int i) {
-    return mix == 1 || (mix == 2 && (i & 1)) || (mix == 3 && (i & 3) == 3) || (mix == 4 && (i & 3) != 0);
-}
-__host__ __device__ constexpr int mix_tables(int mix) { return (mix == 0 || mix == 5) ? 0 : ((mix == 1 || mix == 4) ? 2 : 1); }
-template <typename KeyT, int VAL_BYTES, int RADIX_BITS, int BLOCK, int IPT, int MIX, typename DigitOp, bool FULL>
+constexpr int OS_BLOCK = 256;  // threads of an onesweep CTA
+
+// How a warp finds the lanes that hold the same digit (phase 3).  The stable ranking alternates per
+// item between 8 ballots (ALU) and a shared-memory table of lane masks (LSU).  UNSTABLE: the rank among
+// equal digits is the value the histogram atomic returned -- no matching at all.  Only for a pass whose
+// order inside a digit does not matter: the first prefix pass of the hybrid finish (the local sort
+// orders everything below the prefix).
+template <typename KeyT, int VAL_BYTES, int IPT, bool UNSTABLE, typename DigitOp, bool FULL>
 __device__ __forceinline__ void onesweep_tile(const OnesweepParams& p, const DigitOp& digit_of, unsigned char* smem_raw,
                                               uint32_t* s_scan, uint64_t* s_bar, const uint32_t tile,
                                               const uint32_t n_valid) {
-    constexpr int RADIX = 1 << RADIX_BITS;
+    constexpr int RADIX_BITS = SORT_RADIX_BITS;
+    constexpr int RADIX = SORT_RADIX;
+    constexpr int BLOCK = OS_BLOCK;
     constexpr int WARPS = BLOCK / 32;
     constexpr int TILE = BLOCK * IPT;
-    constexpr int NTBL = mix_tables(MIX);
-    // (a partial tile pads with digit RADIX-1 slots that must rank AFTER the real keys: stable path)
-    constexpr bool UNSTABLE = MIX == 5 && FULL;
+    // (a partial tile pads with digit RADIX-1 slots that must rank AFTER the real keys: stable path,
+    // ballots only -- the unstable kernel has no lane-mask table)
+    constexpr bool ATOMIC_RANK = UNSTABLE && FULL;
     static_assert(RADIX <= BLOCK, "one thread per digit in the prefix / look-back phases");
     using ValT = typename ValType<VAL_BYTES>::type;
     constexpr int ITEM_BYTES = sizeof(KeyT) > sizeof(ValT) ? sizeof(KeyT) : sizeof(ValT);
@@ -203,8 +202,8 @@ __device__ __forceinline__ void onesweep_tile(const OnesweepParams& p, const Dig
     KeyT* s_keys = reinterpret_cast<KeyT*>(smem_raw);
     ValT* s_vals = reinterpret_cast<ValT*>(smem_raw);
     uint32_t* s_whist = reinterpret_cast<uint32_t*>(smem_raw + (size_t)ITEM_BYTES * TILE);  // [WARPS][RADIX]
-    uint32_t* s_tbl = s_whist + WARPS * RADIX;                                               // [NTBL][WARPS][RADIX]
-    uint64_t* s_goff = reinterpret_cast<uint64_t*>(s_tbl + NTBL * WARPS * RADIX);            // [RADIX]
+    uint32_t* s_tbl = s_whist + WARPS * RADIX;                                               // [WARPS][RADIX] (stable)
+    uint64_t* s_goff = reinterpret_cast<uint64_t*>(s_tbl + (UNSTABLE ? 0 : WARPS * RADIX));  // [RADIX]
 
     const int t = threadIdx.x;
     const uint32_t lane = t & 31, warp = t >> 5;
@@ -238,7 +237,7 @@ __device__ __forceinline__ void onesweep_tile(const OnesweepParams& p, const Dig
         const uint32_t idx = wbase + i * 32;
         // slots past the end of a partial tile rank into the last digit, after every real key
         dg[i] = (FULL || idx < n_valid) ? digit_of(keys[i]) : (uint32_t)(RADIX - 1);
-        if constexpr (UNSTABLE) dg[i] |= atomicAdd(&my_hist[dg[i]], 1u) << RADIX_BITS;  // digit | rank in the warp
+        if constexpr (ATOMIC_RANK) dg[i] |= atomicAdd(&my_hist[dg[i]], 1u) << RADIX_BITS;  // digit | rank in the warp
         else atomicAdd(&my_hist[dg[i]], 1u);
     }
     __syncthreads();
@@ -262,8 +261,7 @@ __device__ __forceinline__ void onesweep_tile(const OnesweepParams& p, const Dig
     }
     uint32_t total;
     const uint32_t bin_excl = block_excl_scan<BLOCK, uint32_t>(cnt, s_scan, total);
-    const uint32_t lb_group = p.lb_group;
-    const bool group_end = tile % lb_group == lb_group - 1;
+    const bool group_end = tile % LB_GROUP == LB_GROUP - 1;
     uint32_t excl = 0;
     if (d < RADIX) {
         // fold the digit's tile-local base into every warp's running offset
@@ -272,8 +270,8 @@ __device__ __forceinline__ void onesweep_tile(const OnesweepParams& p, const Dig
         if (group_end) {  // the chain link: resolve and publish the group's inclusive prefix now
             uint32_t c = cnt;
             if (!FULL && d == RADIX - 1) c -= padding;
-            excl = lookback_two_level(p.lb_agg, p.lb_ginc, tile, lb_group, d, RADIX, tag, p.err);
-            st_relaxed_u32(p.lb_ginc + (size_t)(tile / lb_group) * RADIX + d, tag | (excl + c));
+            excl = lookback_two_level(p.lb_agg, p.lb_ginc, tile, d, RADIX, tag, p.err);
+            st_relaxed_u32(p.lb_ginc + (size_t)(tile / LB_GROUP) * RADIX + d, tag | (excl + c));
         }
     }
     __syncthreads();
@@ -281,22 +279,21 @@ __device__ __forceinline__ void onesweep_tile(const OnesweepParams& p, const Dig
     // ---- 3. rank inside the warp; my_hist[] already holds final tile-local offsets, so
     //         slot = offset + rank among the same-digit lanes.  The lanes holding the same digit
     //         are found either with 8 ballots (ALU) or through a shared-memory table of lane
-    //         masks (one atomicOr + one load per key, LSU); mixing both keeps either pipe off
-    //         its limit (profiles/r01_ncu_summary.md). ------------------------------------------
+    //         masks (one atomicOr + one load per key, LSU); alternating both keeps either pipe
+    //         off its limit (profiles/r01_ncu_summary.md). ----------------------------------------
     uint32_t slot[IPT];
     const uint32_t lt = lanemask_lt();
     const uint32_t my_bit = 1u << lane;
 #pragma unroll
     for (int i = 0; i < IPT; ++i) {
-        if constexpr (UNSTABLE) {
+        if constexpr (ATOMIC_RANK) {
             slot[i] = my_hist[dg[i] & (RADIX - 1)] + (dg[i] >> RADIX_BITS);
             continue;
         }
         const uint32_t dd = dg[i];
-        const bool use_table = mix_uses_table(MIX, i);
         uint32_t m, cur;
-        if (use_table) {
-            uint32_t* tbl = s_tbl + ((NTBL == 2 ? (i & 1) : 0) * WARPS + warp) * RADIX;
+        if (!UNSTABLE && (i & 1)) {
+            uint32_t* tbl = s_tbl + warp * RADIX;
             atomicOr(&tbl[dd], my_bit);
             __syncwarp();
             m = tbl[dd];
@@ -327,7 +324,7 @@ __device__ __forceinline__ void onesweep_tile(const OnesweepParams& p, const Dig
     if (d < RADIX) {
         uint32_t c = cnt;
         if (!FULL && d == RADIX - 1) c -= padding;
-        if (!group_end && tile != 0) excl = lookback_two_level(p.lb_agg, p.lb_ginc, tile, lb_group, d, RADIX, tag, p.err);
+        if (!group_end && tile != 0) excl = lookback_two_level(p.lb_agg, p.lb_ginc, tile, d, RADIX, tag, p.err);
         const uint64_t gbase = p.bins_in[d];
         // destination of local sorted slot s holding digit d:  s_goff[d] + s
         s_goff[d] = gbase + excl - bin_excl;
@@ -369,14 +366,15 @@ __device__ __forceinline__ void onesweep_tile(const OnesweepParams& p, const Dig
 }
 
 // resident CTAs per SM the register allocation aims for
-constexpr int min_ctas(int block, int ipt) { return block == 256 ? (ipt <= 16 ? 3 : 2) : 2; }
+constexpr int min_ctas(int ipt) { return ipt <= 16 ? 3 : 2; }
 
-template <typename KeyT, int VAL_BYTES, int RADIX_BITS, int BLOCK, int IPT, int MIX, typename DigitOp>
-__global__ void __launch_bounds__(BLOCK, min_ctas(BLOCK, IPT)) onesweep_kernel(const OnesweepParams p, const DigitOp digit_of) {
-    constexpr int RADIX = 1 << RADIX_BITS;
+template <typename KeyT, int VAL_BYTES, int IPT, bool UNSTABLE, typename DigitOp>
+__global__ void __launch_bounds__(OS_BLOCK, min_ctas(IPT)) onesweep_kernel(const OnesweepParams p, const DigitOp digit_of) {
+    constexpr int RADIX = SORT_RADIX;
+    constexpr int BLOCK = OS_BLOCK;
     constexpr int WARPS = BLOCK / 32;
     constexpr int TILE = BLOCK * IPT;
-    constexpr int NTBL = mix_tables(MIX);
+    constexpr int NTBL = UNSTABLE ? 0 : 1;
     using ValT = typename ValType<VAL_BYTES>::type;
     constexpr int ITEM_BYTES = sizeof(KeyT) > sizeof(ValT) ? sizeof(KeyT) : sizeof(ValT);
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -399,8 +397,8 @@ __global__ void __launch_bounds__(BLOCK, min_ctas(BLOCK, IPT)) onesweep_kernel(c
             for (uint32_t o = 0; o < BYTES; o += CHUNK)
                 tma_load_1d(smem_raw + o, src + o, BYTES - o < CHUNK ? BYTES - o : CHUNK, &s_bar);
             // pull the tile a later CTA will work on into L2 (DRAM has headroom, latency does not)
-            const uint64_t ahead = (uint64_t)my_tile + p.prefetch_tiles;
-            if (p.prefetch_tiles && (ahead + 1) * TILE <= p.n) {
+            const uint64_t ahead = (uint64_t)my_tile + PREFETCH_TILES;
+            if ((ahead + 1) * TILE <= p.n) {
                 const char* nxt = reinterpret_cast<const char*>(p.keys_in) + (size_t)ahead * BYTES;
                 for (uint32_t o = 0; o < BYTES; o += CHUNK) tma_prefetch_l2(nxt + o, BYTES - o < CHUNK ? BYTES - o : CHUNK);
             }
@@ -415,79 +413,57 @@ __global__ void __launch_bounds__(BLOCK, min_ctas(BLOCK, IPT)) onesweep_kernel(c
     if (t == 0 && tile == gridDim.x - 1) *p.ticket = 0;  // every ticket of this launch is taken
     const uint32_t n_valid = min((uint32_t)TILE, p.n - tile * (uint32_t)TILE);
     if (n_valid == (uint32_t)TILE)
-        onesweep_tile<KeyT, VAL_BYTES, RADIX_BITS, BLOCK, IPT, MIX, DigitOp, true>(p, digit_of, smem_raw, s_scan, &s_bar, tile, n_valid);
+        onesweep_tile<KeyT, VAL_BYTES, IPT, UNSTABLE, DigitOp, true>(p, digit_of, smem_raw, s_scan, &s_bar, tile, n_valid);
     else
-        onesweep_tile<KeyT, VAL_BYTES, RADIX_BITS, BLOCK, IPT, MIX, DigitOp, false>(p, digit_of, smem_raw, s_scan, &s_bar, tile, n_valid);
+        onesweep_tile<KeyT, VAL_BYTES, IPT, UNSTABLE, DigitOp, false>(p, digit_of, smem_raw, s_scan, &s_bar, tile, n_valid);
 }
 
 #include "local_sort.cuh"
 #include "local_sort_fine.cuh"
 
-// kmg_set_option("sort_config", i) -> (threads, keys per thread, ranking mix), see dispatch_tile():
-//   0: 256x16 mix2   1: 256x16 mix0   2: 256x16 mix1   3: 256x24 mix2 (default)   4: 512x16 mix2
-//   5: 256x16 mix3   6: 384x16 mix2   7: 256x16 mix4   8: 256x24 mix3   9: 256x20 mix2
-//  10: 256x24 mix5 (unstable ranking; the hybrid finish uses it for its first prefix pass)   11: 256x16 mix5   12: 384x16 mix5
-
-template <typename KeyT, int VB, int RB, int BLOCK, int IPT, int MIX>
+template <typename KeyT, int VB, int IPT, bool UNSTABLE>
 static size_t onesweep_smem() {
     using ValT = typename ValType<VB>::type;
     const size_t item = sizeof(KeyT) > (VB ? sizeof(ValT) : 0) ? sizeof(KeyT) : sizeof(ValT);
-    const int ntbl = mix_tables(MIX);
-    return item * BLOCK * IPT + (size_t)(1 + ntbl) * (BLOCK / 32) * (1 << RB) * 4 + (size_t)(1 << RB) * 8;
+    return item * OS_BLOCK * IPT + (size_t)(UNSTABLE ? 1 : 2) * (OS_BLOCK / 32) * SORT_RADIX * 4 + (size_t)SORT_RADIX * 8;
 }
 
-template <typename KeyT, int VB, int RB, int BLOCK, int IPT, int MIX, typename DigitOp>
+template <typename KeyT, int VB, int IPT, bool UNSTABLE, typename DigitOp>
 static int launch_onesweep(const OnesweepParams& p, const DigitOp& op, cudaStream_t st) {
-    auto kern = onesweep_kernel<KeyT, VB, RB, BLOCK, IPT, MIX, DigitOp>;
-    const size_t smem = onesweep_smem<KeyT, VB, RB, BLOCK, IPT, MIX>();
+    auto kern = onesweep_kernel<KeyT, VB, IPT, UNSTABLE, DigitOp>;
+    const size_t smem = onesweep_smem<KeyT, VB, IPT, UNSTABLE>();
     KMG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const uint32_t tiles = (p.n + BLOCK * IPT - 1) / (BLOCK * IPT);
-    kern<<<tiles, BLOCK, smem, st>>>(p, op);
+    const uint32_t tiles = (p.n + OS_BLOCK * IPT - 1) / (OS_BLOCK * IPT);
+    kern<<<tiles, OS_BLOCK, smem, st>>>(p, op);
     KMG_LAUNCH_CHECK();
     return KMG_OK;
 }
 
+// 8-byte keys: 24 keys per thread (best measured on B200)
 template <typename KeyT, int VB>
-static int dispatch_tile(int cfg, const OnesweepParams& p, const ShiftDigit& op, cudaStream_t st) {
-    switch (cfg) {
-        case 1: return launch_onesweep<KeyT, VB, 8, 256, 16, 0>(p, op, st);
-        case 2: return launch_onesweep<KeyT, VB, 8, 256, 16, 1>(p, op, st);
-        case 3: return launch_onesweep<KeyT, VB, 8, 256, 24, 2>(p, op, st);
-        case 4: return launch_onesweep<KeyT, VB, 8, 512, 16, 2>(p, op, st);
-        case 5: return launch_onesweep<KeyT, VB, 8, 256, 16, 3>(p, op, st);
-        case 6: return launch_onesweep<KeyT, VB, 8, 384, 16, 2>(p, op, st);
-        case 7: return launch_onesweep<KeyT, VB, 8, 256, 16, 4>(p, op, st);
-        case 8: return launch_onesweep<KeyT, VB, 8, 256, 24, 3>(p, op, st);
-        case 9: return launch_onesweep<KeyT, VB, 8, 256, 20, 2>(p, op, st);
-        case 10: return launch_onesweep<KeyT, VB, 8, 256, 24, 5>(p, op, st);
-        case 11: return launch_onesweep<KeyT, VB, 8, 256, 16, 5>(p, op, st);
-        case 12: return launch_onesweep<KeyT, VB, 8, 384, 16, 5>(p, op, st);
-        default: return launch_onesweep<KeyT, VB, 8, 256, 16, 2>(p, op, st);
-    }
+static int dispatch_tile(bool unstable, const OnesweepParams& p, const ShiftDigit& op, cudaStream_t st) {
+    return unstable ? launch_onesweep<KeyT, VB, 24, true>(p, op, st) : launch_onesweep<KeyT, VB, 24, false>(p, op, st);
 }
 // the partition pass runs once per exchange: one configuration is enough
 template <typename KeyT, int VB>
-static int dispatch_tile(int, const OnesweepParams& p, const RangeDigit& op, cudaStream_t st) {
-    return launch_onesweep<KeyT, VB, 8, 256, 16, 2>(p, op, st);
+static int dispatch_tile(bool, const OnesweepParams& p, const RangeDigit& op, cudaStream_t st) {
+    return launch_onesweep<KeyT, VB, 16, false>(p, op, st);
 }
 
 template <typename DigitOp>
-static int dispatch_onesweep(int cfg, int key_bytes, int val_bytes, const OnesweepParams& p, const DigitOp& op,
+static int dispatch_onesweep(bool unstable, int key_bytes, int val_bytes, const OnesweepParams& p, const DigitOp& op,
                              cudaStream_t st) {
     if (key_bytes == 8) {
-        if (val_bytes == 0) return dispatch_tile<uint64_t, 0>(cfg, p, op, st);
-        if (val_bytes == 4) return dispatch_tile<uint64_t, 4>(cfg, p, op, st);
-        return dispatch_tile<uint64_t, 8>(cfg, p, op, st);
+        if (val_bytes == 0) return dispatch_tile<uint64_t, 0>(unstable, p, op, st);
+        if (val_bytes == 4) return dispatch_tile<uint64_t, 4>(unstable, p, op, st);
+        return dispatch_tile<uint64_t, 8>(unstable, p, op, st);
     }
-    // 16-byte keys: half the items per thread
-    if (val_bytes == 0) return launch_onesweep<u128, 0, 8, 256, 8, 2>(p, op, st);
-    if (val_bytes == 4) return launch_onesweep<u128, 4, 8, 256, 8, 2>(p, op, st);
-    return launch_onesweep<u128, 8, 8, 256, 8, 2>(p, op, st);
+    // 16-byte keys: half the items per thread, stable ranking
+    if (val_bytes == 0) return launch_onesweep<u128, 0, 8, false>(p, op, st);
+    if (val_bytes == 4) return launch_onesweep<u128, 4, 8, false>(p, op, st);
+    return launch_onesweep<u128, 8, 8, false>(p, op, st);
 }
 
-int g_sort_config = 3;  // 256 threads x 24 keys, alternating ballot / lane-mask ranking: best measured on B200
-int g_lb_group = 32;   // tiles per look-back group (kmg_set_option("lb_group", n), n >= 32)
-int g_prefetch_tiles = 192;  // L2 prefetch distance in tiles (kmg_set_option("prefetch_tiles", n)); 148-296 measured best
 int g_time_passes = 0;  // kmg_set_option("time_passes", 1): bracket every pass launch with events
 thread_local int64_t g_stat_sort_passes = 0;
 thread_local int64_t g_stat_hybrid_irregular = -1;
@@ -561,10 +537,7 @@ struct SortWs {
 };
 
 int g_hybrid = 1;     // kmg_set_option("hybrid", 0/1)
-int g_unstable_config = 10;  // kmg_set_option("unstable_config", 10 | 11 | 12): tile shape of that pass
-int g_hybrid_unstable = 1;  // kmg_set_option("hybrid_unstable", 0/1): first prefix pass without stable ranking
 int g_local_tile = 7936;  // kmg_set_option("local_tile", positions): target tile width of the local sort
-int g_local_v = 2;     // kmg_set_option("local_v", 1 | 2 | 3): 2 = the fine-cell local sort (local_sort_fine.cuh) where it wins, 3 = always
 int g_count_fused = 1;  // kmg_set_option("count_fused", 0/1): let the hybrid finish emit the count table itself
 int g_hybrid_pb = 0;  // kmg_set_option("hybrid_pb", 0 | 16 | 24): force the prefix width (0 = by n and skew)
 constexpr uint64_t HYBRID_MIN_N = 1ull << 20;
@@ -588,7 +561,7 @@ static SortWs carve_sort_ws(void* ws, uint64_t n, int key_bytes, bool hybrid, in
     const uint64_t min_tile = key_bytes == 16 ? 2048 : 4096;  // smallest tile of any configuration
     const uint64_t tiles = (part + min_tile - 1) / min_tile + 1;
     w.lb_words = align_up(tiles * SORT_RADIX * sizeof(uint32_t), 256) / sizeof(uint32_t);
-    p += w.lb_words * sizeof(uint32_t) + align_up((tiles / LB_GROUP_MIN + 2) * SORT_RADIX * sizeof(uint32_t), 256);
+    p += w.lb_words * sizeof(uint32_t) + align_up((tiles / LB_GROUP + 2) * SORT_RADIX * sizeof(uint32_t), 256);
     w.hybrid = hybrid;
     if (hybrid) {
         const uint64_t lt = n / LS_T_MIN + 2;
@@ -694,7 +667,6 @@ static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_
 
     PassPlan plan = make_plan(begin_bit, end_bit);
     int np = plan.num_passes;
-    const int cfg = g_sort_config;
     const uint64_t n_parts = (n + PART_MAX - 1) / PART_MAX;
 
     // header + hist zero; look-back words zero once per sort -- see OnesweepParams::tag
@@ -794,8 +766,6 @@ static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_
             p.bins_out = (part + 1 < n_parts) ? bins + ((part + 1) & 1) * SORT_RADIX : nullptr;
             p.lb_agg = w.lookback;
             p.lb_ginc = w.lookback + w.lb_words;
-            p.lb_group = (uint32_t)g_lb_group;
-            p.prefetch_tiles = (uint32_t)g_prefetch_tiles;
             p.ticket = &w.hdr->ticket;
             p.err = &w.hdr->err;
             if (n_parts > 1) {
@@ -811,8 +781,7 @@ static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_
             if (g_ev_used >= MAX_TIMED) timing_collect();
             timing_begin(st);
             // the hybrid finish does not care about the order inside the first pass' digits
-            const int pass_cfg = (hybrid && pass == 0 && g_hybrid_unstable && cfg == 3) ? g_unstable_config : cfg;
-            int rcode = dispatch_onesweep(pass_cfg, key_bytes, val_bytes, p, op, st);
+            int rcode = dispatch_onesweep(hybrid && pass == 0, key_bytes, val_bytes, p, op, st);
             timing_end(st, 0);
             if (rcode != KMG_OK) return rcode;
             ++launch;
@@ -867,12 +836,12 @@ static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_
     // per tile (a 16-bit prefix under more than ~160 M evenly spread keys: config 3 on 8 GPUs, 387.5 M keys per
     // rank) its tile prefix jams -- 70 % of the warp samples sit behind warp 0's look-back polls, 28 ms against
     // the first kernel's 4.3 ms (profiles/r02_local_sort_one_bucket_tiles.md) -- so tiles narrower than two
-    // average buckets keep the first kernel (local_v 3 forces the fine cells there too).
+    // average buckets keep the first kernel.
     const double avg_bucket = (double)n / (double)(1ull << pb);
     const bool few_bucket_tiles =
         avg_bucket > cap / 2.4 ||
         (avg_bucket >= 64 && std::min<double>(g_local_tile, cap - std::max(256.0, 1.35 * avg_bucket)) < 2.0 * avg_bucket);
-    const bool fine = g_local_v == 3 || (g_local_v == 2 && !few_bucket_tiles);
+    const bool fine = !few_bucket_tiles;
     const size_t smem = fine ? (wide_key ? (pairs ? lsf_smem_bytes<u128, true>() : lsf_smem_bytes<u128, false>())
                                          : (pairs ? lsf_smem_bytes<uint64_t, true>() : lsf_smem_bytes<uint64_t, false>()))
                              : (wide_key ? (pairs ? ls_smem_bytes<u128, true>() : ls_smem_bytes<u128, false>())
@@ -1240,13 +1209,11 @@ extern "C" int kmg_range_partition(const void* d_keys, const void* d_vals, uint6
         p.bins_out = (part + 1 < n_lb_parts) ? w.bins + ((part + 1) & 1) * SORT_RADIX : nullptr;
         p.lb_agg = w.lookback;
         p.lb_ginc = w.lookback + w.lb_words;
-        p.lb_group = (uint32_t)g_lb_group;
-        p.prefetch_tiles = (uint32_t)g_prefetch_tiles;
         p.ticket = &w.hdr->ticket;
         p.err = &w.hdr->err;
         p.tag = 1u << 30;
         if (part > 0) KMG_CUDA(cudaMemsetAsync(w.lookback, 0, (char*)d_ws + w.total - (char*)w.lookback, st));
-        int rcode = dispatch_onesweep(g_sort_config, key_bytes, val_bytes, p, op, st);
+        int rcode = dispatch_onesweep(false, key_bytes, val_bytes, p, op, st);
         if (rcode != KMG_OK) return rcode;
     }
     return KMG_OK;

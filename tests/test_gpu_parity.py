@@ -115,7 +115,7 @@ def test_extract_window_ranges_partition_the_input(eng):
 
 
 # ---- K3 ---------------------------------------------------------------------------------------
-def _sort_case(eng, n, kb, vb, bits, seed, cfg=0, dup=False):
+def _sort_case(eng, n, kb, vb, bits, seed, dup=False):
     import torch
 
     from kman_b200.engine import KeyArray
@@ -136,24 +136,21 @@ def _sort_case(eng, n, kb, vb, bits, seed, cfg=0, dup=False):
     t = lambda x: torch.from_numpy(x.view(np.uint8).reshape(-1).copy()).to(dev)  # noqa: E731
     a = KeyArray(t(raw), t(np.zeros_like(raw)), t(vals) if vb else None, t(np.zeros_like(vals)) if vb else None,
                  n, kb, vb, bits // 2, False)
-    eng.lib.kmg_set_option(b"sort_config", cfg)
-    try:
-        a = eng.sort(a, 0, bits)
-        eng._status(eng._last_sort_ws) if n > 1 else None
-    finally:
-        eng.lib.kmg_set_option(b"sort_config", 3)
+    a = eng.sort(a, 0, bits)
+    eng._status(eng._last_sort_ws) if n > 1 else None
     if limbs == 1:
         order = np.argsort(raw[:, 0], kind="stable")
         want = raw[order, 0]
     else:
         order = np.lexsort((raw[:, 0], raw[:, 1]))
         want = raw[order]
-    assert first_diff(a.keys_host(), want) == "equal", (n, kb, vb, bits, cfg)
+    assert first_diff(a.keys_host(), want) == "equal", (n, kb, vb, bits)
     if vb:
         assert first_diff(a.vals_host().astype(np.uint64), vals[order].astype(np.uint64)) == "equal", "payload/stability"
 
 
-@pytest.mark.parametrize("n", [0, 1, 2, 31, 4095, 4096, 4097, 70001, 1_000_003])
+# (8-byte keys sort in tiles of 6144 keys; the range partition and 16-byte keys in tiles of 4096)
+@pytest.mark.parametrize("n", [0, 1, 2, 31, 4095, 4096, 4097, 6143, 6144, 6145, 12_289, 70001, 1_000_003])
 def test_radix_sort_u64_sizes(eng, n):
     _sort_case(eng, n, 8, 0, 62, seed=n)
     _sort_case(eng, n, 8, 8, 62, seed=n + 1, dup=True)
@@ -164,10 +161,9 @@ def test_radix_sort_u64_bit_ranges(eng, bits):
     _sort_case(eng, 300_000, 8, 4, bits, seed=bits, dup=True)
 
 
-@pytest.mark.parametrize("cfg", [0, 1, 2, 3, 4, 5, 6, 7, 8, 9])
 @pytest.mark.parametrize("vb", [0, 4, 8])
-def test_radix_sort_u64_tile_configs(eng, cfg, vb):
-    _sort_case(eng, 500_009, 8, vb, 62, seed=cfg * 10 + vb, cfg=cfg, dup=True)
+def test_radix_sort_u64_payload_widths(eng, vb):
+    _sort_case(eng, 500_009, 8, vb, 62, seed=30 + vb, dup=True)
 
 
 @pytest.mark.parametrize("bits", [66, 100, 126, 128])
@@ -1028,6 +1024,42 @@ def test_hybrid_tiles_without_output_keep_the_tile_prefix_moving(eng, mode):
         eng.lib.kmg_set_option(b"local_tile", 7936)
     assert eng.lib.kmg_get_stat(b"hybrid_path") == 1
     assert eng.lib.kmg_get_stat(b"hybrid_irregular") == 0
+
+
+@pytest.mark.parametrize("mode", ["sort", "count", "uniq"])
+def test_hybrid_one_bucket_tiles_take_the_first_local_sort_kernel(eng, mode):
+    """Tiles narrower than two average prefix buckets are finished by local_sort_kernel: the persistent
+    fine-cell kernel's tile prefix jams there.  72 M random 62-bit keys under a 16-bit prefix make buckets
+    of n / 2^16 = 1099 keys on average.  With local_tile 2048 the target width min(2048, cap - 1.35 * 1099)
+    is 2048 < 2 * 1099 for both the key-only tile (cap 8192: sort, count) and the tile with a u32 payload
+    (cap 6144: uniq), so few_bucket_tiles holds and sort_impl picks the first kernel.  A third of the keys
+    repeat another one: counts of 2 and dropped pairs."""
+    n, bits = 72_000_000, 62
+    rng = np.random.default_rng(1099)
+    raw = rng.integers(0, 1 << 62, size=n, dtype=np.uint64)
+    raw[1::3] = raw[::3]
+    eng.lib.kmg_set_option(b"hybrid_pb", 16)
+    eng.lib.kmg_set_option(b"local_tile", 2048)
+    try:
+        if mode == "sort":
+            a = _keyonly_sort(eng, raw, bits)
+            assert first_diff(a.keys_host(), np.sort(raw)) == "equal"
+        elif mode == "count":
+            keys, counts = _sort_count(eng, raw, bits)
+            wk, wc = np.unique(raw, return_counts=True)
+            assert first_diff(keys, wk) == "equal"
+            assert first_diff(counts.astype(np.uint64), wc.astype(np.uint64)) == "equal"
+        else:
+            vals = np.arange(n, dtype=np.uint32)
+            keys, got_v = _sort_uniq(eng, raw, vals, bits)
+            wk, wv = _want_singletons(raw, vals)
+            assert first_diff(keys, wk) == "equal"
+            assert first_diff(got_v.astype(np.uint64), wv.astype(np.uint64)) == "equal"
+    finally:
+        eng.lib.kmg_set_option(b"hybrid_pb", 0)
+        eng.lib.kmg_set_option(b"local_tile", 7936)
+    assert eng.lib.kmg_get_stat(b"hybrid_path") == 1
+    assert eng.lib.kmg_get_stat(b"sort_passes") == 2
 
 
 def test_hybrid_tiles_without_output_u128(eng):

@@ -20,8 +20,6 @@ torch.cuda.set_device(lr)
 dist.init_process_group("nccl", device_id=torch.device("cuda", lr))
 eng = get_engine(lr)
 dc = DistributedCounter(eng)
-if "KMG_DX_ALIGN" in os.environ:
-    eng.lib.kmg_set_option(b"dx_align", int(os.environ["KMG_DX_ALIGN"]))
 n, k = int(os.environ.get("KMG_STAGE_N", "100000000")), 31  # bases per rank (config 3 on 8 GPUs: 387500000)
 rng = np.random.default_rng(1234 + rank)
 chunk = np.frombuffer(b"ACGT", np.uint8)[rng.integers(0, 4, size=n, dtype=np.uint8)]

@@ -79,12 +79,6 @@ def main():
         print(f"{name}: {med:8.3f} ms (min {mn:.3f})  {N / med / 1e6:8.2f} G k-mers/s  rows {r.n}  passes "
               f"{lib.kmg_get_stat(b'sort_passes')} path {lib.kmg_get_stat(b'hybrid_path')}")
         print("    kernels per call:", kernel_split(lib, fn))
-    for v in (1, 2):
-        lib.kmg_set_option(b"local_v", v)
-        for name, fn in (("count", pipe_count), ("uniq ", pipe_uniq)):
-            med, mn = timed(fn)
-            print(f"local_v {v} {name}, fused path: {med:8.3f} ms (min {mn:.3f})  {N / med / 1e6:8.2f} G k-mers/s")
-            print("    kernels per call:", kernel_split(lib, fn))
     for pb in (16, 24):
         lib.kmg_set_option(b"hybrid_pb", pb)
         med, mn = timed(pipe_count)

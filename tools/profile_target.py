@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Minimal profiling target: two passes of the config-2 count path on cuda:0 -- the fused device path
 (kmg_extract_sort_count; KMG_PROF_STAGE=1: the stage calls extract -> sort -> rle).  Run plain first,
-then under ncu (B200_PROFILING.md).  KMG_PROF_N / _K / _VB / KMG_SORT_CONFIG."""
+then under ncu (B200_PROFILING.md).  KMG_PROF_N / _K / _VB."""
 import os
 import sys
 
@@ -17,8 +17,6 @@ n = int(os.environ.get("KMG_PROF_N", "100000000"))
 k = int(os.environ.get("KMG_PROF_K", "31"))
 vb = int(os.environ.get("KMG_PROF_VB", "0"))
 eng = get_engine(0)
-if "KMG_SORT_CONFIG" in os.environ:
-    eng.lib.kmg_set_option(b"sort_config", int(os.environ["KMG_SORT_CONFIG"]))
 rng = np.random.default_rng(1234)
 bases = np.frombuffer(b"ACGT", np.uint8)[rng.integers(0, 4, size=n, dtype=np.uint8)]
 flat = fasta.FlatInput(np.concatenate([bases, np.array([10], np.uint8)]), np.array([0, n + 1], np.uint64), ["chr1"], ["chr1"])

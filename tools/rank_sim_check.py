@@ -19,11 +19,9 @@ ap.add_argument("--n", type=int, default=387_500_000)
 ap.add_argument("--rank", type=int, default=5)
 ap.add_argument("--world", type=int, default=8)
 ap.add_argument("--reps", type=int, default=3)
-ap.add_argument("--local-v", type=int, default=2)
 ap.add_argument("--pb", type=int, default=0)
 args = ap.parse_args()
 eng = get_engine(0)
-eng.lib.kmg_set_option(b"local_v", args.local_v)
 eng.lib.kmg_set_option(b"time_passes", 1)
 eng.lib.kmg_set_option(b"hybrid_pb", args.pb)
 n, key_bits = args.n, 62
@@ -49,7 +47,7 @@ for rep in range(args.reps):
     got_sum = int((k * c).sum().item()) & (2**64 - 1)
     assert got_sum == want_sum, (got_sum, want_sum)
     kt = {nm: (eng.lib.kmg_get_stat((nm + "_ns").encode()), eng.lib.kmg_get_stat((nm + "_count").encode())) for nm in ("sort_pass", "local_sort")}
-    print(f"rep {rep}: local_v {args.local_v} kernels (cumulative ns, launches) {kt}")
+    print(f"rep {rep}: kernels (cumulative ns, launches) {kt}")
     print(f"rep {rep}: n {n} distinct {tab.n} sort_count {e0.elapsed_time(e1):.3f} ms  passes {eng.lib.kmg_get_stat(b'sort_passes')} "
           f"path {eng.lib.kmg_get_stat(b'hybrid_path')} irregular {eng.lib.kmg_get_stat(b'hybrid_irregular')}", flush=True)
     del a, tab, k, c

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Per-stage device timings (CUDA events) of the hot path on one GPU; a development tool.
-usage: python tools/stage_bench.py [--n 100000000] [--k 31] [--configs 0,1,2,3,4] [--yardstick]"""
+usage: python tools/stage_bench.py [--n 100000000] [--k 31] [--local-tiles 4096,7936] [--yardstick]"""
 import argparse
 import json
 import os
@@ -36,11 +36,8 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--n", type=int, default=100_000_000)
     ap.add_argument("--k", type=int, default=31)
-    ap.add_argument("--configs", default="0,1,2,3,4,5,6,7,8,9")
     ap.add_argument("--vb", type=int, default=0)
     ap.add_argument("--yardstick", action="store_true")
-    ap.add_argument("--lb-groups", default="")
-    ap.add_argument("--prefetch", default="")
     ap.add_argument("--local-tiles", default="")
     args = ap.parse_args()
     eng = get_engine(0)
@@ -62,75 +59,24 @@ def main():
     print(f"extract        : {med:8.3f} ms (min {mn:.3f})  {N/med/1e6:8.2f} G kmers/s   alg {(1+W+args.vb)*N/med/1e6:8.1f} GB/s")
     res["extract_ms"] = med
     P8 = (2 * k + 7) // 8
-    for cfg in [int(c) for c in args.configs.split(",")]:
-        eng.lib.kmg_set_option(b"sort_config", cfg)
 
-        def run():
-            a = eng.extract(d, k, False, val_bytes=args.vb, reuse="b_", want_hist=True)
-            return eng.sort(a)
+    def run():
+        a = eng.extract(d, k, False, val_bytes=args.vb, reuse="b_", want_hist=True)
+        return eng.sort(a)
 
-        med_all, _ = timed(run, flush=flush)
-        srt = med_all - res["extract_ms"]
-        alg = N * (W * (2 * P8 + 1) + 2 * P8 * args.vb)
-        print(f"sort cfg {cfg}     : {srt:8.3f} ms  {N/srt/1e6:8.2f} G keys/s  model {alg/srt/1e6:8.1f} GB/s = {alg/srt/1e6/peak:5.3f} of measured peak")
-        res[f"sort_cfg{cfg}_ms"] = srt
-    eng.lib.kmg_set_option(b"sort_config", 3)
-    for un in (0, 1):
-        eng.lib.kmg_set_option(b"hybrid_unstable", un)
-
-        def run_u():
-            a = eng.extract(d, k, False, val_bytes=args.vb, reuse="b_", want_hist=True)
-            return eng.sort(a)
-
-        med_all, _ = timed(run_u, flush=flush)
-        print(f"hybrid, unstable first pass {un}: sort {med_all - res['extract_ms']:8.3f} ms")
-    for uc in (10, 11, 12):
-        eng.lib.kmg_set_option(b"unstable_config", uc)
-
-        def run_uc():
-            a = eng.extract(d, k, False, val_bytes=args.vb, reuse="b_", want_hist=True)
-            return eng.sort(a)
-
-        med_all, _ = timed(run_uc, flush=flush)
-        print(f"unstable_config {uc}: sort {med_all - res['extract_ms']:8.3f} ms")
-    eng.lib.kmg_set_option(b"unstable_config", 10)
+    med_all, _ = timed(run, flush=flush)
+    srt = med_all - res["extract_ms"]
+    alg = N * (W * (2 * P8 + 1) + 2 * P8 * args.vb)
+    print(f"sort           : {srt:8.3f} ms  {N/srt/1e6:8.2f} G keys/s  model {alg/srt/1e6:8.1f} GB/s = {alg/srt/1e6/peak:5.3f} of measured peak")
+    res["sort_ms"] = srt
     for hy, pb in ((0, 0), (1, 16), (1, 24), (1, 0)):
         eng.lib.kmg_set_option(b"hybrid", hy)
         eng.lib.kmg_set_option(b"hybrid_pb", pb)
-
-        def run_h():
-            a = eng.extract(d, k, False, val_bytes=args.vb, reuse="b_", want_hist=True)
-            return eng.sort(a)
-
-        med_all, _ = timed(run_h, flush=flush)
+        med_all, _ = timed(run, flush=flush)
         srt = med_all - res["extract_ms"]
         print(f"hybrid {hy} pb {pb:2d}: sort {srt:8.3f} ms  {N/srt/1e6:8.2f} G keys/s  passes {eng.lib.kmg_get_stat(b'sort_passes')} irregular {eng.lib.kmg_get_stat(b'hybrid_irregular')}")
         res[f"sort_hy{hy}_pb{pb}_ms"] = srt
     eng.lib.kmg_set_option(b"hybrid_pb", 0)
-    for g in [int(x) for x in args.lb_groups.split(",") if x]:
-        eng.lib.kmg_set_option(b"lb_group", g)
-
-        def run_g():
-            a = eng.extract(d, k, False, val_bytes=args.vb, reuse="b_", want_hist=True)
-            return eng.sort(a)
-
-        med_all, _ = timed(run_g, flush=flush)
-        srt = med_all - res["extract_ms"]
-        print(f"lb_group {g:4d} (cfg 3): sort {srt:8.3f} ms  {N/srt/1e6:8.2f} G keys/s")
-        res[f"sort_lbg{g}_ms"] = srt
-    eng.lib.kmg_set_option(b"lb_group", 32)
-    for g in [int(x) for x in args.prefetch.split(",") if x]:
-        eng.lib.kmg_set_option(b"prefetch_tiles", g)
-
-        def run_p():
-            a = eng.extract(d, k, False, val_bytes=args.vb, reuse="b_", want_hist=True)
-            return eng.sort(a)
-
-        med_all, _ = timed(run_p, flush=flush)
-        srt = med_all - res["extract_ms"]
-        print(f"prefetch {g:5d} tiles (cfg 3): sort {srt:8.3f} ms  {N/srt/1e6:8.2f} G keys/s")
-        res[f"sort_pf{g}_ms"] = srt
-    eng.lib.kmg_set_option(b"prefetch_tiles", 192)
 
     def full():
         return eng.sort_count(eng.extract(d, k, False, val_bytes=0, reuse="b_", want_hist=True), reuse="b_")
