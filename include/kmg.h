@@ -57,6 +57,10 @@ extern "C" {
 #define KMG_LUT_INVALID 0x80u
 #define KMG_LUT_NONPLAIN 0x40u
 
+/* Bins of a multiplicity histogram (kmg_sort_histo and friends): d_hist[m] for m < KMG_HISTO_BINS,
+ * larger multiplicities go to a list. */
+#define KMG_HISTO_BINS 4096
+
 int kmg_version(void);
 const char* kmg_last_error(void);
 /* number of CUDA devices visible, or <0 */
@@ -176,6 +180,24 @@ int kmg_sort_uniq(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_alt
 int kmg_select_singletons(const void* d_sorted_keys, const void* d_vals, uint64_t n, int key_bytes, int val_bytes,
                           void* d_keys_out, void* d_vals_out, uint64_t* d_n_out, void* d_ws, size_t ws_bytes,
                           void* stream);
+/* The multiplicity spectrum of the keys (`kmer histo`: what a histogram of kmg_sort_count's counts
+ * gives) without the table.  Output, ADDED to the caller's arrays (zero them once, then sum streams and
+ * passes on the device):
+ *   d_hist[KMG_HISTO_BINS]: d_hist[m] = distinct keys that occur exactly m times (m >= 1);
+ *   d_big[] / *d_n_big: one entry per distinct key that occurs >= KMG_HISTO_BINS times, its multiplicity,
+ *   in no particular order, appended at *d_n_big.  Capacity (total keys) / KMG_HISTO_BINS + 1 always holds.
+ * kmg_sort_histo consumes both key buffers (sorts n 8- or 16-byte keys on bits [0, end_bit)).  When the
+ * hybrid finish applies, its local sort adds every tile's run lengths to the histogram and writes no key
+ * (no output order, no compaction); tiles it cannot hold (huge prefix buckets: repeats) are gathered,
+ * sorted with the plain passes and histogrammed on the side ("hybrid_path" 2), above n/8 such keys all
+ * keys are sorted and histogrammed ("hybrid_path" 3).  The status word (kmg_ws_status(d_ws)) becomes
+ * KMG_ERR_RANGE for a multiplicity beyond uint32, as in the count path.
+ * kmg_count_histogram: the same histogram of an existing count table (d_counts[0..n)); no workspace. */
+size_t kmg_sort_histo_workspace_bytes(uint64_t n, int key_bytes, int end_bit);
+int kmg_sort_histo(void* d_keys, void* d_keys_alt, uint64_t n, int key_bytes, int end_bit, const uint64_t* d_hist_in,
+                   uint64_t* d_hist, uint32_t* d_big, uint64_t* d_n_big, void* d_ws, size_t ws_bytes, void* stream);
+int kmg_count_histogram(const uint32_t* d_counts, uint64_t n, uint64_t* d_hist, uint32_t* d_big, uint64_t* d_n_big,
+                        void* stream);
 
 /* ---- K1-K4 in one call: the device path of `kmer count` / `kmer uniq` for the narrow stream -------
  * (FastaBatcher.do batcher.py:454-487 + KJoiner.join join.py:337-391 on one flat base buffer.)
@@ -198,6 +220,13 @@ int kmg_extract_sort_uniq(const uint8_t* d_bases, uint64_t n_bases, uint64_t win
                           const uint8_t* d_lut256, void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_alt,
                           int val_bytes, uint64_t pos_offset, uint64_t* h_result, void* d_ws, size_t ws_bytes,
                           void* stream);
+/* The same front end with kmg_sort_histo's finish: the narrow stream's multiplicity histogram added to
+ * d_hist / d_big / d_n_big (see kmg_sort_histo).  h_result as above, except that there is no table:
+ * [0] and [3] are 0.  Three host synchronisations (the last one reads the status word). */
+size_t kmg_pipeline_histo_workspace_bytes(uint64_t n_windows, int k, int rc);
+int kmg_extract_sort_histo(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
+                           const uint8_t* d_lut256, void* d_keys, void* d_keys_alt, uint64_t* d_hist, uint32_t* d_big,
+                           uint64_t* d_n_big, uint64_t* h_result, void* d_ws, size_t ws_bytes, void* stream);
 
 /* ---- K5: range partition for the multi-GPU exchange (no reference counterpart) --------
  * Stable split of keys into n_parts contiguous regions of the output by
@@ -351,7 +380,7 @@ int kmg_uniq_host(kmg_ctx* ctx, const uint8_t* h_bases, uint64_t n_bases, int k,
  *                          (0 = the real limit 2^32-1)
  * Stats of the calling thread's last call: "launches" (kernel launches since "reset_launches"),
  * "sort_passes", "hybrid_path" (0 plain passes, 1 hybrid, 2 hybrid + re-sorted ranges, 3 fell
- * back), "hybrid_irregular" (tiles), "hybrid_big_runs" (runs a whole block had to sort),
+ * back; kmg_sort_histo: 2 = fused histogram plus re-sorted ranges), "hybrid_irregular" (tiles), "hybrid_big_runs" (runs a whole block had to sort),
  * "n_out" / "ws_err" (result rows and status word the last kmg_sort_count / kmg_sort_uniq already
  * read back when its hybrid finish synchronised, -1 otherwise: a caller can then skip its own
  * read-back of *d_n_out and kmg_ws_status), and with time_passes: "sort_pass_ns" /

@@ -11,6 +11,7 @@ LIB_PATH = os.path.join(_HERE, "libkmg.so")
 
 KMG_OK = 0
 KMG_ERR_ARG, KMG_ERR_CUDA, KMG_ERR_WS, KMG_ERR_RANGE, KMG_ERR_STATE = -1, -2, -3, -4, -5
+KMG_HISTO_BINS = 4096  # include/kmg.h
 
 u8p = C.POINTER(C.c_uint8)
 u32p = C.POINTER(C.c_uint32)
@@ -44,6 +45,11 @@ SIGNATURES = {
     "kmg_pipeline_workspace_bytes": (sz, [u64, i32, i32, i32]),
     "kmg_extract_sort_count": (i32, [vp, u64, u64, u64, i32, i32, vp, vp, vp, vp, u64p, vp, sz, vp]),
     "kmg_extract_sort_uniq": (i32, [vp, u64, u64, u64, i32, i32, vp, vp, vp, vp, vp, i32, u64, u64p, vp, sz, vp]),
+    "kmg_sort_histo_workspace_bytes": (sz, [u64, i32, i32]),
+    "kmg_sort_histo": (i32, [vp, vp, u64, i32, i32, vp, vp, vp, vp, vp, sz, vp]),
+    "kmg_count_histogram": (i32, [vp, u64, vp, vp, vp, vp]),
+    "kmg_pipeline_histo_workspace_bytes": (sz, [u64, i32, i32]),
+    "kmg_extract_sort_histo": (i32, [vp, u64, u64, u64, i32, i32, vp, vp, vp, vp, vp, vp, u64p, vp, sz, vp]),
     "kmg_abundance_scatter": (i32, [vp, vp, u64, i32, i32, vp, C.c_uint32, i32, u64, vp, vp, vp, vp]),
     "kmg_vector_extents": (i32, [vp, vp, u64, vp, C.c_uint32, vp, vp]),
     "kmg_format_vector": (i32, [vp, u64, vp, vp, vp, sz, vp]),

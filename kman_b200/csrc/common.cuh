@@ -79,6 +79,21 @@ struct CountOut {
     unsigned long long* n_out;
     bool done;
 };
+// multiplicity histogram (kmg_sort_histo): hist[m] = distinct keys seen m times for m < KMG_HISTO_BINS;
+// larger multiplicities are appended to big[] (*n_big entries, in no order); *err becomes 2 for a
+// multiplicity beyond uint32
+struct HistoOut {
+    unsigned long long* hist;
+    uint32_t* big;
+    unsigned long long* n_big;
+    uint32_t* err;
+};
+// histogram request of a hybrid sort: `done` = the finish (fused local sort + re-sorted ranges) produced
+// all of it; otherwise the caller histograms the sorted keys after resetting `out`
+struct HistoReq {
+    HistoOut out;
+    bool done;
+};
 // keys already grouped by the prefix: with bucket_starts == null by the lowest prefix byte only (the keys
 // are in d_keys; pb = 24), else by all 16 prefix bits (pb = 16; the keys are in d_keys_alt when in_alt)
 // -- plus the histograms of the three top key bytes
@@ -125,6 +140,8 @@ int sort_count_core(void* d_keys, void* d_keys_alt, uint64_t n, int key_bytes, i
 int sort_uniq_core(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_alt, uint64_t n, int key_bytes, int val_bytes,
                    int end_bit, const uint64_t* d_hist_in, uint64_t* d_n_out, int* h_selector_out, void* d_ws,
                    size_t ws_bytes, void* stream, const PrePartitioned* pre);
+int sort_histo_core(void* d_keys, void* d_keys_alt, uint64_t n, int key_bytes, int end_bit, const uint64_t* d_hist_in,
+                    const HistoOut& out, void* d_ws, size_t ws_bytes, cudaStream_t st, const PrePartitioned* pre);
 void exclusive_scan_256(const unsigned long long* d_hist_row, unsigned long long* d_out, cudaStream_t st);
 extern thread_local int64_t g_stat_last_n_out, g_stat_last_err;
 // kmg_set_option("time_passes", 1): event pairs around a launch (kind 0 onesweep pass, 1 local sort,

@@ -92,7 +92,27 @@ struct HybridParams {
     uint64_t* tile_state;           // tile prefix over the tiles' distinct-key counts
     uint32_t* ticket;
     uint32_t* err;
+    HistoOut histo;                 // multiplicity histogram (EMIT 3)
 };
+
+// ---- multiplicity histogram (EMIT 3, kmg_sort_histo, kmg_count_histogram) ---------------------------
+// The small multiplicities (nearly all of them) go to per-CTA shared bins that are flushed with one
+// global atomic per non-empty bin; larger ones take a global atomic, and those >= KMG_HISTO_BINS an entry
+// of the `big` list.
+constexpr int HISTO_SMEM_BINS = 64;
+__device__ __forceinline__ void histo_add_global(const HistoOut& h, uint64_t m) {
+    if (m < (uint64_t)KMG_HISTO_BINS) atomicAdd(&h.hist[m], 1ull);
+    else if (m <= 0xFFFFFFFFull) h.big[atomicAdd(h.n_big, 1ull)] = (uint32_t)m;
+    else atomicMax(h.err, 2u);  // (the count path's limit: a multiplicity must fit uint32)
+}
+__device__ __forceinline__ void histo_add(uint32_t* s_h, const HistoOut& h, uint64_t m) {
+    if (m < (uint64_t)HISTO_SMEM_BINS) atomicAdd(&s_h[m], 1u);
+    else histo_add_global(h, m);
+}
+__device__ __forceinline__ void histo_flush(const uint32_t* s_h, const HistoOut& h) {
+    for (uint32_t i = threadIdx.x; i < (uint32_t)HISTO_SMEM_BINS; i += blockDim.x)
+        if (s_h[i]) atomicAdd(&h.hist[i], (unsigned long long)s_h[i]);
+}
 
 // First i in [lo, hi) whose prefix differs from `ref`, or hi; the prefixes are non-decreasing.
 // Whole-warp 32-ary search: the common case (buckets of a few keys) ends after one probe round.
@@ -195,12 +215,15 @@ struct CellMap {
 // staged keys and the payload is gathered from the tile's (L2-resident) input range at the end.
 // Equal keys come out in no particular order (kmg_sort_uniq only keeps keys that occur once).
 // EMIT: 0 = the sorted keys (and payload), 1 = the count table (COUNT above), 2 = the keys that
-// occur exactly once with their payload, compacted across tiles like the count table (kmg_sort_uniq).
+// occur exactly once with their payload, compacted across tiles like the count table (kmg_sort_uniq),
+// 3 = nothing but the run lengths, added to the multiplicity histogram p.histo (kmg_sort_histo): no
+// output order, so no ticket and no tile prefix, and a tile the scheme cannot hold adds nothing (the
+// host re-sorts its range and histograms it on the side).
 template <typename KeyT, int EMIT, int VB>
 __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_kernel(const HybridParams p) {
     constexpr bool PAIRS = VB != 0;
-    constexpr bool COUNT = EMIT == 1, UNIQ = EMIT == 2, FUSED = EMIT != 0;
-    static_assert(!(PAIRS && COUNT), "the fused count is key-only");
+    constexpr bool COUNT = EMIT == 1, UNIQ = EMIT == 2, FUSED = EMIT == 1 || EMIT == 2, HISTO = EMIT == 3;
+    static_assert(!(PAIRS && (COUNT || HISTO)), "the fused count and histogram are key-only");
     static_assert(!UNIQ || PAIRS, "singletons carry their payload");
     constexpr int IPT = LS<KeyT, PAIRS>::IPT, CPT = LS<KeyT, PAIRS>::CPT;
     constexpr int CAP = ls_cap<KeyT, PAIRS>(), CELLS = ls_cells<KeyT, PAIRS>(), CELL_WORDS = ls_cell_words<KeyT, PAIRS>();
@@ -478,7 +501,25 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_kernel(const HybridPar
         finish_without_output();
         return;
     }
-    if constexpr (!FUSED) {
+    if constexpr (HISTO) {
+        // a run of equal keys lies inside one thread's run of cells: every thread measures its own runs
+        uint32_t* s_h = s_cell;  // [HISTO_SMEM_BINS] (the cell array is dead by now)
+        if (t < HISTO_SMEM_BINS) s_h[t] = 0;
+        __syncthreads();
+        uint32_t start = lo;
+        KeyT prev{};
+        for (uint32_t i = lo; i < hi; ++i) {
+            const KeyT key = s_stage[i];
+            if (i != lo && key != prev) {
+                histo_add(s_h, p.histo, i - start);
+                start = i;
+            }
+            prev = key;
+        }
+        if (hi > lo) histo_add(s_h, p.histo, hi - start);
+        __syncthreads();
+        histo_flush(s_h, p.histo);
+    } else if constexpr (!FUSED) {
         KeyT* kout = reinterpret_cast<KeyT*>(p.keys_out) + s;
 #pragma unroll
         for (int j = 0; j < IPT; ++j) {

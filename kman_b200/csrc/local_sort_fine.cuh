@@ -47,8 +47,9 @@ __host__ __device__ constexpr size_t lsf_smem_bytes() {
 template <typename KeyT, int EMIT, int VB>
 __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const HybridParams p) {
     constexpr bool PAIRS = VB != 0;
-    constexpr bool COUNT = EMIT == 1, UNIQ = EMIT == 2, FUSED = EMIT != 0;
-    static_assert(!(PAIRS && COUNT), "the fused count is key-only");
+    // (EMIT 3, the histogram: tiles by stride as in the plain sort, no tile prefix; see local_sort_kernel)
+    constexpr bool COUNT = EMIT == 1, UNIQ = EMIT == 2, FUSED = EMIT == 1 || EMIT == 2, HISTO = EMIT == 3;
+    static_assert(!(PAIRS && (COUNT || HISTO)), "the fused count and histogram are key-only");
     static_assert(!UNIQ || PAIRS, "singletons carry their payload");
     constexpr int IPT = LS<KeyT, PAIRS>::IPT;
     constexpr int CAP = ls_cap<KeyT, PAIRS>();  // keys = counter words; cells = 2 * CAP
@@ -68,7 +69,7 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
     __shared__ uint32_t s_scan[LS_BLOCK / 32 + 1];
     __shared__ uint32_t s_dup[NW + 1];   // bit p: position p holds the same key as position p - 1
     __shared__ uint32_t s_emit[NW];      // bit p: position p is emitted (run head / singleton)
-    __shared__ uint32_t s_epre[NW];      // emitted positions before word w
+    __shared__ uint32_t s_epre[NW];      // emitted positions before word w (HISTO: the CTA's shared bins)
     __shared__ int s_bad;
     __shared__ uint32_t s_has_mid, s_big_n, s_ndup;
     __shared__ uint32_t s_nfix[2];       // list lengths: the tile in flight / the next one
@@ -423,6 +424,10 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
         s_ndup = 0;
     }
     if (t <= NW) s_dup[t] = 0;
+    if constexpr (HISTO) {
+        static_assert(NW >= HISTO_SMEM_BINS, "shared bins");
+        if (t < HISTO_SMEM_BINS) s_epre[t] = 0;  // kept across the CTA's tiles, flushed once at its end
+    }
     zero_cells();
     Tile A = fetch_sortable();  // (its barriers also cover the zeroing above)
     if (A.kind == 0) return;
@@ -480,7 +485,36 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
             front(N, keys, meta_n, 1);
         }
         // ---- emission of A ----
-        if constexpr (!FUSED) {
+        if constexpr (HISTO) {
+            // run lengths from the duplicate bitmask: a run head is a position without a mark, a singleton a
+            // head whose successor carries none either (one ballot per word), a longer run the head's mark count
+            uint32_t* s_h = s_epre;
+            const uint32_t m = A.m;
+            if (ok && ndup == 0) {
+                if (t == 0) atomicAdd(&s_h[1], m);
+            } else if (ok) {
+                uint32_t singles = 0;
+#pragma unroll
+                for (int j = 0; j < IPT; ++j) {
+                    const uint32_t pos = t + j * LS_BLOCK;
+                    const uint32_t w = pos >> 5;
+                    const uint64_t window = ((uint64_t)s_dup[w] | ((uint64_t)s_dup[w + 1] << 32)) >> lane;
+                    const bool head = pos < m && !(window & 1u);
+                    const bool single = head && !(window & 2u);  // (marks stop at m: none beyond the tile)
+                    singles += (uint32_t)__popc(__ballot_sync(0xffffffffu, single));
+                    if (head && !single) {
+                        uint32_t extra = (uint32_t)__ffsll((long long)~(window >> 1)) - 1u;  // marks right after the head
+                        if (extra >= 63u - lane) {  // the run leaves the 64-bit window: walk the words (long runs only)
+                            uint32_t q = pos + 1u + extra;
+                            while (q < m && ((s_dup[q >> 5] >> (q & 31u)) & 1u)) ++q;
+                            extra = q - pos - 1u;
+                        }
+                        histo_add(s_h, p.histo, 1u + extra);
+                    }
+                }
+                if (lane == 0 && singles) atomicAdd(&s_h[1], singles);
+            }
+        } else if constexpr (!FUSED) {
             if (ok) {
                 KeyT* kout = reinterpret_cast<KeyT*>(p.keys_out) + A.s;
 #pragma unroll
@@ -608,7 +642,10 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
                 front(N, keys, meta_n, 0);
             }
         }
-        if (N.kind == 0) return;
+        if (N.kind == 0) {
+            if constexpr (HISTO) histo_flush(s_epre, p.histo);  // (the barrier above covers the last tile's adds)
+            return;
+        }
         __syncthreads();
         placement(N, meta_n);
         A = N;

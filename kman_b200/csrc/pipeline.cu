@@ -25,6 +25,7 @@
 #include "common.cuh"
 
 extern "C" size_t kmg_rle_workspace_bytes(uint64_t n);
+extern "C" size_t kmg_sort_histo_workspace_bytes(uint64_t n, int key_bytes, int end_bit);
 
 namespace kmg {
 
@@ -46,7 +47,8 @@ struct PipeWs {
     size_t total;
 };
 
-PipeWs carve_pipe(void* ws, uint64_t n_windows, int k, int rc, int val_bytes) {
+// mode as in run_pipeline: 0 count, 1 uniq (val_bytes 4 / 8), 2 histogram
+PipeWs carve_pipe(void* ws, uint64_t n_windows, int k, int rc, int val_bytes, int mode) {
     PipeWs w;
     memset(&w, 0, sizeof(w));
     char* p = (char*)ws;
@@ -72,8 +74,9 @@ PipeWs carve_pipe(void* ws, uint64_t n_windows, int k, int rc, int val_bytes) {
     const uint64_t caps[2] = {cap, std::min<uint64_t>(cap, 1ull << 33)};
     size_t sw = 0;
     for (uint64_t c : caps) {
-        const size_t a = val_bytes ? kmg_sort_uniq_workspace_bytes(c, kb, val_bytes, 2 * k)
-                                   : kmg_sort_count_workspace_bytes(c, kb, 2 * k);
+        const size_t a = mode == 2 ? kmg_sort_histo_workspace_bytes(c, kb, 2 * k)
+                         : val_bytes ? kmg_sort_uniq_workspace_bytes(c, kb, val_bytes, 2 * k)
+                                     : kmg_sort_count_workspace_bytes(c, kb, 2 * k);
         sw = std::max(sw, a);
     }
     w.sort_ws_bytes = sw;
@@ -94,31 +97,33 @@ int status_from_err(int64_t err) {
     return KMG_OK;
 }
 
-// mode 0: (k-mer, count) table; mode 1: singletons with payload.  h_result: [0] rows of the result,
-// [1] keys sorted (valid narrow windows, x2 with rc), [2] windows that belong to the wide stream,
-// [3] selector (0: result in d_keys / d_vals, 1: in the alt buffers)
+// mode 0: (k-mer, count) table; mode 1: singletons with payload; mode 2: the multiplicity histogram, added
+// to *histo.  h_result: [0] rows of the result, [1] keys sorted (valid narrow windows, x2 with rc),
+// [2] windows that belong to the wide stream, [3] selector (0: result in d_keys / d_vals, 1: in the alt
+// buffers); mode 2 has no table: [0] and [3] stay 0
 int run_pipeline(int mode, const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
                  const uint8_t* d_lut256, void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_alt, int val_bytes,
                  uint64_t pos_offset, uint32_t* d_counts_out, uint64_t* h_result, void* d_ws, size_t ws_bytes,
-                 cudaStream_t st) {
+                 cudaStream_t st, const HistoOut* histo = nullptr) {
     KMG_REQUIRE(h_result, KMG_ERR_ARG, "h_result is null");
     h_result[0] = h_result[1] = h_result[2] = h_result[3] = 0;
     KMG_REQUIRE(k >= 2, KMG_ERR_ARG, "k must be >= 2, got %d", k);  // batcher.py:477-478
     KMG_REQUIRE(k <= 64, KMG_ERR_RANGE, "k=%d: this build supports k <= 64 (no CPU fallback)", k);
     KMG_REQUIRE(win_begin <= win_end, KMG_ERR_ARG, "win_begin > win_end");
-    KMG_REQUIRE(mode == 0 ? val_bytes == 0 : (val_bytes == 4 || val_bytes == 8), KMG_ERR_ARG,
+    KMG_REQUIRE(mode != 1 ? val_bytes == 0 : (val_bytes == 4 || val_bytes == 8), KMG_ERR_ARG,
                 "val_bytes must be 0 (count) or 4 / 8 (uniq)");
+    KMG_REQUIRE(mode != 2 || (histo && histo->hist && histo->big && histo->n_big), KMG_ERR_ARG, "null histogram argument");
     KMG_REQUIRE(d_bases && d_lut256 && d_ws, KMG_ERR_ARG, "null pointer argument");
     KMG_REQUIRE(((uintptr_t)d_bases & 15) == 0, KMG_ERR_ARG, "d_bases must be 16-byte aligned");
     const uint64_t n_win = win_end - win_begin;
     if (n_win == 0) return KMG_OK;
     const int kb = k <= 32 ? 8 : 16;
-    KMG_REQUIRE(d_keys && d_keys_alt && (mode == 1 || d_counts_out) && (mode == 0 || (d_vals && d_vals_alt)), KMG_ERR_ARG,
+    KMG_REQUIRE(d_keys && d_keys_alt && (mode != 0 || d_counts_out) && (mode != 1 || (d_vals && d_vals_alt)), KMG_ERR_ARG,
                 "null pointer argument");
     KMG_REQUIRE(((uintptr_t)d_keys % kb) == 0 && ((uintptr_t)d_keys_alt % kb) == 0, KMG_ERR_ARG, "key buffers misaligned");
     if (val_bytes == 4)
         KMG_REQUIRE(((pos_offset + n_bases) << 1) < (1ull << 32), KMG_ERR_RANGE, "val_bytes=4 needs < 2^31 positions");
-    const PipeWs w = carve_pipe(d_ws, n_win, k, rc, val_bytes);
+    const PipeWs w = carve_pipe(d_ws, n_win, k, rc, val_bytes, mode);
     KMG_REQUIRE(ws_bytes >= w.total, KMG_ERR_WS, "pipeline workspace too small: %zu < %zu", ws_bytes, w.total);
     const uint64_t cap = n_win * (rc ? 2 : 1);
     int sel = 0;
@@ -166,7 +171,9 @@ int run_pipeline(int mode, const uint8_t* d_bases, uint64_t n_bases, uint64_t wi
                 pre.bucket_starts = w.starts;
                 pre.in_alt = true;
             }
-            if (mode == 0)
+            if (mode == 2)
+                rcode = sort_histo_core(d_keys, d_keys_alt, n, kb, 2 * k, nullptr, *histo, w.sort_ws, w.sort_ws_bytes, st, &pre);
+            else if (mode == 0)
                 rcode = sort_count_core(d_keys, d_keys_alt, n, kb, 2 * k, nullptr, d_counts_out, w.n_out, &sel, w.sort_ws,
                                         w.sort_ws_bytes, st, &pre);
             else
@@ -189,7 +196,9 @@ int run_pipeline(int mode, const uint8_t* d_bases, uint64_t n_bases, uint64_t wi
         h_result[1] = n;
         h_result[2] = h_cnt[1];
         if (n == 0) return KMG_OK;
-        if (mode == 0)
+        if (mode == 2)
+            rcode = sort_histo_core(d_keys, d_keys_alt, n, kb, 2 * k, hist, *histo, w.sort_ws, w.sort_ws_bytes, st, nullptr);
+        else if (mode == 0)
             rcode = sort_count_core(d_keys, d_keys_alt, n, kb, 2 * k, hist, d_counts_out, w.n_out, &sel, w.sort_ws,
                                     w.sort_ws_bytes, st, nullptr);
         else
@@ -197,6 +206,7 @@ int run_pipeline(int mode, const uint8_t* d_bases, uint64_t n_bases, uint64_t wi
                                    w.sort_ws, w.sort_ws_bytes, st, nullptr);
         if (rcode != KMG_OK) return rcode;
     }
+    if (mode == 2) return kmg_ws_status(w.sort_ws, st);  // (synchronises)
     h_result[3] = (uint64_t)sel;
     if (g_stat_last_n_out >= 0 && g_stat_last_err >= 0) {  // the sort's own read-back already has it all
         h_result[0] = (uint64_t)g_stat_last_n_out;
@@ -258,7 +268,12 @@ extern "C" int kmg_extract_dest_counts(const uint8_t* d_bases, uint64_t n_bases,
 
 extern "C" size_t kmg_pipeline_workspace_bytes(uint64_t n_windows, int k, int rc, int val_bytes) {
     if (k < 2 || k > 64) return 0;
-    return carve_pipe(nullptr, n_windows, k, rc, val_bytes).total;
+    return carve_pipe(nullptr, n_windows, k, rc, val_bytes, val_bytes ? 1 : 0).total;
+}
+
+extern "C" size_t kmg_pipeline_histo_workspace_bytes(uint64_t n_windows, int k, int rc) {
+    if (k < 2 || k > 64) return 0;
+    return carve_pipe(nullptr, n_windows, k, rc, 0, 2).total;
 }
 
 extern "C" int kmg_extract_sort_count(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k,
@@ -275,4 +290,14 @@ extern "C" int kmg_extract_sort_uniq(const uint8_t* d_bases, uint64_t n_bases, u
                                      size_t ws_bytes, void* stream) {
     return run_pipeline(1, d_bases, n_bases, win_begin, win_end, k, rc, d_lut256, d_keys, d_keys_alt, d_vals, d_vals_alt,
                         val_bytes, pos_offset, nullptr, h_result, d_ws, ws_bytes, (cudaStream_t)stream);
+}
+
+extern "C" int kmg_extract_sort_histo(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k,
+                                      int rc, const uint8_t* d_lut256, void* d_keys, void* d_keys_alt, uint64_t* d_hist,
+                                      uint32_t* d_big, uint64_t* d_n_big, uint64_t* h_result, void* d_ws, size_t ws_bytes,
+                                      void* stream) {
+    const HistoOut histo{reinterpret_cast<unsigned long long*>(d_hist), d_big, reinterpret_cast<unsigned long long*>(d_n_big),
+                         nullptr};
+    return run_pipeline(2, d_bases, n_bases, win_begin, win_end, k, rc, d_lut256, d_keys, d_keys_alt, nullptr, nullptr, 0, 0,
+                        nullptr, h_result, d_ws, ws_bytes, (cudaStream_t)stream, &histo);
 }

@@ -648,15 +648,89 @@ int hybrid_choose_pb(uint64_t n, unsigned long long max_top_byte_count, int key_
     return hybrid_pb16_ok(n, max_top_byte_count, key_bytes, val_bytes) ? 16 : 24;
 }
 
+// Run lengths of SORTED keys into the histogram (the re-sorted irregular ranges of EMIT 3, and whole
+// sorts that did not take the fused finish).  The thread at a run's first key finds the run's end: the
+// neighbour first (singletons), then a galloping search -- the keys are sorted, so a run of a million
+// copies costs ~40 probes instead of a million.
+template <typename KeyT>
+__global__ void __launch_bounds__(256) runs_histogram_kernel(const KeyT* __restrict__ keys, uint64_t n, const HistoOut h) {
+    __shared__ uint32_t s_h[HISTO_SMEM_BINS];
+    if (threadIdx.x < HISTO_SMEM_BINS) s_h[threadIdx.x] = 0;
+    __syncthreads();
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const KeyT key = keys[i];
+        if (i > 0 && keys[i - 1] == key) continue;
+        uint64_t a = i, b = n, step = 1;  // keys[a] == key; the run ends at b or before
+        for (;;) {
+            const uint64_t c = a + step;
+            if (c >= n) break;
+            if (keys[c] != key) {
+                b = c;
+                break;
+            }
+            a = c;
+            step <<= 1;
+        }
+        while (b - a > 1) {
+            const uint64_t mid = a + (b - a) / 2;
+            if (keys[mid] == key) a = mid;
+            else b = mid;
+        }
+        histo_add(s_h, h, b - i);
+    }
+    __syncthreads();
+    histo_flush(s_h, h);
+}
+
+// the histogram of a count table's multiplicities (kmg_count_histogram)
+__global__ void __launch_bounds__(256) count_histogram_kernel(const uint32_t* __restrict__ counts, uint64_t n, const HistoOut h) {
+    __shared__ uint32_t s_h[HISTO_SMEM_BINS];
+    if (threadIdx.x < HISTO_SMEM_BINS) s_h[threadIdx.x] = 0;
+    __syncthreads();
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) histo_add(s_h, h, counts[i]);
+    __syncthreads();
+    histo_flush(s_h, h);
+}
+
+// dst += src: bins added, src's list appended to dst's
+__global__ void __launch_bounds__(256) histo_merge_kernel(const HistoOut dst, const HistoOut src) {
+    const uint64_t nb = *src.n_big;
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < KMG_HISTO_BINS || i < nb; i += stride) {
+        if (i < KMG_HISTO_BINS && src.hist[i]) atomicAdd(&dst.hist[i], src.hist[i]);
+        if (i < nb) dst.big[atomicAdd(dst.n_big, 1ull)] = src.big[i];
+    }
+}
+
+static int histo_grid(uint64_t n) {
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    return (int)std::max<uint64_t>(1, std::min<uint64_t>((n + 255) / 256, (uint64_t)sms * 8));
+}
+
+static int runs_histogram(const void* d_sorted, uint64_t n, int key_bytes, const HistoOut& h, cudaStream_t st) {
+    if (n == 0) return KMG_OK;
+    if (key_bytes == 8) runs_histogram_kernel<uint64_t><<<histo_grid(n), 256, 0, st>>>((const uint64_t*)d_sorted, n, h);
+    else runs_histogram_kernel<u128><<<histo_grid(n), 256, 0, st>>>((const u128*)d_sorted, n, h);
+    KMG_LAUNCH_CHECK();
+    return KMG_OK;
+}
+
 // `pre` (fused pipeline): the keys in d_keys are ALREADY grouped by the lowest prefix byte (the first,
 // order-free prefix pass ran inside the extraction kernel); pre->top holds the histograms of the
 // three top key bytes and pre->pb the prefix width the caller chose.  With pre->bucket_starts the keys
 // are grouped by the whole 16-bit prefix (top byte in the extraction, byte 2 in region_partition_kernel):
 // no pass runs here at all.
+// `hr` (kmg_sort_histo): the local sort adds the run lengths to the histogram instead of writing keys
+// (EMIT 3); the ranges of the tiles it cannot hold are gathered, sorted and histogrammed on the side.
+// Only above irr_cap such keys are the keys sorted in full and hr->done left false.
 static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_alt, uint64_t n, int key_bytes,
                      int val_bytes, int begin_bit, int end_bit, const uint64_t* d_hist_in, int* h_selector_out,
                      void* d_ws, size_t ws_bytes, cudaStream_t st, bool hybrid, bool allow_hybrid,
-                     CountOut* co = nullptr, const PrePartitioned* pre = nullptr) {
+                     CountOut* co = nullptr, const PrePartitioned* pre = nullptr, HistoReq* hr = nullptr) {
     SortWs w = carve_sort_ws(d_ws, n, key_bytes, hybrid, val_bytes);
     KMG_REQUIRE(ws_bytes >= w.total, KMG_ERR_WS, "sort workspace too small: %zu < %zu", ws_bytes, w.total);
     hybrid = hybrid && allow_hybrid;
@@ -849,6 +923,8 @@ static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_
     const int sel_in = kin == (char*)d_keys ? 0 : 1;  // where the prefix-ordered keys are
     const int sel_done = sel_in ^ 1;                   // ... and where the finish puts its result
     const bool want_fused = co != nullptr && g_count_fused;
+    const bool want_histo = hr != nullptr;
+    if (want_histo) hp.histo = hr->out;
 
     auto launch_bounds = [&](uint32_t T) -> int {
         hp.tile_t = T;
@@ -866,8 +942,8 @@ static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_
         return KMG_OK;
     };
     auto launch_local = [&](bool fused) -> int {
-        hp.counts_out = fused ? co->counts : nullptr;
-        hp.n_out = fused ? co->n_out : nullptr;
+        hp.counts_out = fused && co ? co->counts : nullptr;  // (the histogram has neither)
+        hp.n_out = fused && co ? co->n_out : nullptr;
         if (g_ev_used >= MAX_TIMED) timing_collect();
         timing_begin(st);
 #define KMG_LS_LAUNCH(K, E, V)                                                                                   \
@@ -883,6 +959,9 @@ static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_
         } else if (fused && pairs) {
             if (val_bytes == 4) KMG_LS_LAUNCH(uint64_t, 2, 4);
             else KMG_LS_LAUNCH(uint64_t, 2, 8);
+        } else if (fused && want_histo) {
+            if (wide_key) KMG_LS_LAUNCH(u128, 3, 0);
+            else KMG_LS_LAUNCH(uint64_t, 3, 0);
         } else if (fused) {
             if (wide_key) KMG_LS_LAUNCH(u128, 1, 0);
             else KMG_LS_LAUNCH(uint64_t, 1, 0);
@@ -915,7 +994,7 @@ static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_
     // First attempt at the widest tiles: the fused emission when the caller asked for one, else the sort.
     int rcode = launch_bounds(tile_width(g_local_tile));
     if (rcode != KMG_OK) return rcode;
-    rcode = launch_local(want_fused);
+    rcode = launch_local(want_fused || want_histo);
     if (rcode != KMG_OK) return rcode;
     rcode = read_header();
     if (rcode != KMG_OK) return rcode;
@@ -925,14 +1004,16 @@ static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_
             co->done = true;
             g_stat_last_n_out = (int64_t)hh.n_out;
         }
+        if (want_histo) hr->done = true;
         *h_selector_out = sel_done;
         return KMG_OK;
     }
     // Some tiles own more keys than the local scheme holds (a huge prefix bucket: repeats) or crowd
     // too many distinct keys into one cell.  The keys get sorted (no fused emission: the caller
     // follows up with kmg_rle_count / kmg_select_singletons), the irregular tiles' ranges are
-    // gathered, sorted with the plain passes and put back.
-    if (want_fused || hh.over_keys > n / 32) {
+    // gathered, sorted with the plain passes and put back.  The histogram keeps what the fused launch
+    // added for the regular tiles: only the flagged ranges are gathered, sorted and histogrammed.
+    if (!want_histo && (want_fused || hh.over_keys > n / 32)) {
         // The widest tiles are the fastest, but a tile owns WHOLE buckets: with big buckets around
         // (repeat families: thousands of keys per 12-mer prefix) wide tiles overflow.  Take the widest
         // candidate width that leaves at most n/32 keys in oversize tiles.
@@ -976,6 +1057,13 @@ static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_
                           false);
         g_stat_sort_passes = passes;
         if (rcode != KMG_OK) return rcode;
+        if (want_histo) {  // (a bucket never straddles tiles: every run of the gathered keys is whole)
+            rcode = runs_histogram(w.irr_buf[sel2], m_irr, key_bytes, hr->out, st);
+            if (rcode != KMG_OK) return rcode;
+            hr->done = true;
+            *h_selector_out = sel_in;
+            return KMG_OK;
+        }
         rc2 = irregular_copy<false>(hp, key_bytes, nullptr, kout, w.irr_buf[sel2], grid, st);
         if (rc2 == KMG_OK && pairs) rc2 = irregular_copy<false>(hp, val_bytes, nullptr, vout, w.irr_vbuf[sel2], grid, st);
         if (rc2 != KMG_OK) return rc2;
@@ -1097,6 +1185,90 @@ extern "C" int kmg_sort_count(void* d_keys, void* d_keys_alt, uint64_t n, int ke
                               void* d_ws, size_t ws_bytes, void* stream) {
     return sort_count_core(d_keys, d_keys_alt, n, key_bytes, end_bit, d_hist_in, d_counts_out, d_n_out, h_selector_out, d_ws,
                            ws_bytes, stream, nullptr);
+}
+
+// The histogram of a sort is built in the workspace and added to the caller's arrays at the end: should
+// the irregular ranges exceed the gather buffer, what the fused launch added for the regular tiles is
+// dropped and the fully sorted keys are histogrammed instead.  Layout after the sort's own workspace:
+// bins [KMG_HISTO_BINS] | list length | list [n / KMG_HISTO_BINS + 1].
+static size_t sort_histo_sort_ws(uint64_t n, int key_bytes, int end_bit) {
+    return align_up(kmg_radix_sort_workspace_bytes(n, key_bytes, 0, 0, end_bit), 256);
+}
+static size_t histo_ws_bytes(uint64_t n) {
+    return align_up((KMG_HISTO_BINS + 1) * sizeof(uint64_t), 256) + align_up((n / KMG_HISTO_BINS + 1) * sizeof(uint32_t), 256);
+}
+
+extern "C" size_t kmg_sort_histo_workspace_bytes(uint64_t n, int key_bytes, int end_bit) {
+    return sort_histo_sort_ws(n, key_bytes, end_bit) + histo_ws_bytes(n);
+}
+
+static int check_histo_out(const uint64_t* d_hist, const uint32_t* d_big, const uint64_t* d_n_big) {
+    KMG_REQUIRE(d_hist && d_big && d_n_big, KMG_ERR_ARG, "null histogram argument");
+    return KMG_OK;
+}
+
+int kmg::sort_histo_core(void* d_keys, void* d_keys_alt, uint64_t n, int key_bytes, int end_bit, const uint64_t* d_hist_in,
+                         const HistoOut& out, void* d_ws, size_t ws_bytes, cudaStream_t st, const PrePartitioned* pre) {
+    KMG_REQUIRE(key_bytes == 8 || key_bytes == 16, KMG_ERR_ARG, "key_bytes must be 8 or 16");
+    KMG_REQUIRE(end_bit >= 0 && end_bit <= key_bytes * 8, KMG_ERR_ARG, "bad end_bit %d", end_bit);
+    g_stat_sort_passes = 0;
+    g_stat_hybrid_path = 0;
+    g_stat_hybrid_irregular = -1;
+    g_stat_last_n_out = g_stat_last_err = -1;
+    if (n == 0) return KMG_OK;
+    KMG_REQUIRE(d_keys && d_keys_alt && d_ws, KMG_ERR_ARG, "null pointer argument");
+    KMG_REQUIRE(((uintptr_t)d_keys % key_bytes) == 0 && ((uintptr_t)d_keys_alt % key_bytes) == 0, KMG_ERR_ARG,
+                "key buffers misaligned");
+    const size_t sort_ws = sort_histo_sort_ws(n, key_bytes, end_bit);
+    KMG_REQUIRE(ws_bytes >= sort_ws + histo_ws_bytes(n), KMG_ERR_WS, "sort_histo workspace too small");
+    char* hw = (char*)d_ws + sort_ws;
+    HistoReq hr;
+    hr.out.hist = reinterpret_cast<unsigned long long*>(hw);
+    hr.out.n_big = hr.out.hist + KMG_HISTO_BINS;
+    hr.out.big = reinterpret_cast<uint32_t*>(hw + align_up((KMG_HISTO_BINS + 1) * sizeof(uint64_t), 256));
+    hr.out.err = &reinterpret_cast<WsHeader*>(d_ws)->err;
+    hr.done = false;
+    const size_t bins_bytes = (KMG_HISTO_BINS + 1) * sizeof(uint64_t);
+    KMG_CUDA(cudaMemsetAsync(d_ws, 0, sizeof(WsHeader), st));  // (the status word, also when no sort runs)
+    KMG_CUDA(cudaMemsetAsync(hw, 0, bins_bytes, st));
+    int sel = 0;
+    if (n > 1 && end_bit > 0) {
+        const bool hybrid = hybrid_applies(n, key_bytes, 0, 0, end_bit);
+        const int rcode = sort_impl(d_keys, d_keys_alt, nullptr, nullptr, n, key_bytes, 0, 0, end_bit, d_hist_in, &sel, d_ws,
+                                    sort_ws, st, hybrid, true, nullptr, pre, &hr);
+        if (rcode != KMG_OK) return rcode;
+    }
+    if (!hr.done) {  // plain passes, or the fallback after a partial fused histogram: start from the sorted keys
+        KMG_CUDA(cudaMemsetAsync(hw, 0, bins_bytes, st));
+        const int rcode = runs_histogram(sel ? d_keys_alt : d_keys, n, key_bytes, hr.out, st);
+        if (rcode != KMG_OK) return rcode;
+    }
+    histo_merge_kernel<<<histo_grid(KMG_HISTO_BINS), 256, 0, st>>>(out, hr.out);
+    KMG_LAUNCH_CHECK();
+    return KMG_OK;
+}
+
+extern "C" int kmg_sort_histo(void* d_keys, void* d_keys_alt, uint64_t n, int key_bytes, int end_bit, const uint64_t* d_hist_in,
+                              uint64_t* d_hist, uint32_t* d_big, uint64_t* d_n_big, void* d_ws, size_t ws_bytes, void* stream) {
+    const int rcode = check_histo_out(d_hist, d_big, d_n_big);
+    if (rcode != KMG_OK) return rcode;
+    HistoOut out{reinterpret_cast<unsigned long long*>(d_hist), d_big, reinterpret_cast<unsigned long long*>(d_n_big), nullptr};
+    return sort_histo_core(d_keys, d_keys_alt, n, key_bytes, end_bit, d_hist_in, out, d_ws, ws_bytes, (cudaStream_t)stream,
+                           nullptr);
+}
+
+extern "C" int kmg_count_histogram(const uint32_t* d_counts, uint64_t n, uint64_t* d_hist, uint32_t* d_big, uint64_t* d_n_big,
+                                   void* stream) {
+    const int rcode = check_histo_out(d_hist, d_big, d_n_big);
+    if (rcode != KMG_OK) return rcode;
+    if (n == 0) return KMG_OK;
+    KMG_REQUIRE(d_counts, KMG_ERR_ARG, "null pointer argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    // (counts are uint32: every multiplicity has a place, err is never written)
+    HistoOut out{reinterpret_cast<unsigned long long*>(d_hist), d_big, reinterpret_cast<unsigned long long*>(d_n_big), nullptr};
+    count_histogram_kernel<<<histo_grid(n), 256, 0, st>>>(d_counts, n, out);
+    KMG_LAUNCH_CHECK();
+    return KMG_OK;
 }
 
 extern "C" int kmg_select_singletons(const void* d_sorted_keys, const void* d_vals, uint64_t n, int key_bytes, int val_bytes,

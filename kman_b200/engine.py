@@ -14,6 +14,8 @@ Stage -> reference mapping (see DESIGN.md):
                    writer behind write_count()/write_uniq()/write_batch() and count_text()/uniq_text()
   write_vectors()  join.py:287-335 + abundance.py:104-172      vectors filled pass by pass, trimmed and formatted on
                    the device, gzipped on host threads (abundance() returns the same vectors as host arrays)
+  histogram()      `kmer histo`: the spectrum of count()'s count column, summed on the device pass by pass
+                   (write_histogram() writes it as text)
 """
 from __future__ import annotations
 
@@ -188,9 +190,20 @@ def pass_bytes(k: int, mode: str, n: int, m: int, val_bytes: int, text_bytes: in
     mode "vec" (abundance vectors): keys + payload and their alternates and the stable payload sort's workspace
     per stream.  The narrow buffers are freed before the wide stream is extracted, so a pass costs the larger
     stage, not their sum, and there is no merge term; the text stage comes after the passes, with only the
-    (kept) sort workspaces beside it."""
+    (kept) sort workspaces beside it.
+
+    mode "histo" (multiplicity spectrum): keys and their alternates and kmg_sort_histo's workspace per stream
+    (32-byte wide keys: kmg_sort256 + kmg_rle_count and the counts), the larger stage as in "vec"; no counts,
+    merge ranks or text.  The histogram arrays themselves (a few MB) are not counted."""
     lib = _lib.load()
     kb, kw = key_bytes(k, False), key_bytes(k, True)
+    if mode == "histo":
+        ws_n = lib.kmg_sort_histo_workspace_bytes(n, kb, 2 * k)
+        if kw == 32:
+            ws = ws_n + lib.kmg_sort256_workspace_bytes(m) + lib.kmg_rle_workspace_bytes(m) + 4 * m
+        else:
+            ws = max(ws_n, lib.kmg_sort_histo_workspace_bytes(m, kw, 4 * k))
+        return int(max(2 * n * kb + ws_n, 2 * m * kw + ws) + lib.kmg_extract_workspace_bytes(n_win))
     if mode == "vec":
         ws_n = lib.kmg_radix_sort_workspace_bytes(n, kb, val_bytes, 0, 2 * k)
         if kw == 32:  # kmg_sort256 has a workspace of its own, next to the narrow sort's
@@ -855,6 +868,12 @@ class Engine:
         cap = max(n_win * (2 if rc else 1), 1)
         if mode == "vec":  # extract() with window-sized buffers, one stream at a time
             return pass_bytes(k, mode, cap, cap if n_other else 0, val_bytes, text_bytes, n_win)
+        if mode == "histo":  # the fused pipeline, then the wide stream beside the (kept) pipeline workspace
+            ws_pipe = lib.kmg_pipeline_histo_workspace_bytes(n_win, k, int(rc))
+            need = 2 * cap * key_bytes(k, False) + ws_pipe + lib.kmg_extract_workspace_bytes(n_win)
+            if n_other:
+                need = max(need, ws_pipe + pass_bytes(k, mode, 0, n_other * (2 if rc else 1), 0, 0, n_win))
+            return int(need)
         kb, kw = key_bytes(k, False), key_bytes(k, True)
         item = kb +(4 if mode == "count" else val_bytes)
         narrow = 2 * cap * item + lib.kmg_pipeline_workspace_bytes(n_win, k, int(rc), 0 if mode == "count" else val_bytes)
@@ -897,18 +916,19 @@ class Engine:
     @_on_device
     def plan_passes(self, d: DeviceInput, k: int, rc: bool, mode: str, budget_bytes: Optional[int] = None,
                     chunk_rows: Optional[int] = None, text: bool = True) -> PassPlan:
-        """Split `kmer count` (mode "count") / `kmer uniq` ("uniq") / `kmer count -m VEC_COUNT*` ("vec") into
+        """Split `kmer count` (mode "count") / `kmer uniq` ("uniq") / `kmer count -m VEC_COUNT*` ("vec") / `kmer histo`
+        ("histo", never a text stage) into
         key-range passes that fit the device budget (device_budget; for "vec" minus the resident vector pair,
         8 * (n_bases + 1) bytes).  Everything fits: one pass on the whole-input path.  Otherwise contiguous
         parts of PASS_PARTS are grouped (plan_parts; needs k >= 12, ValueError if not or if one part alone
         does not fit).  text=False: no text stage (Engine.abundance copies the vectors out instead)."""
-        if mode not in ("count", "uniq", "vec"):
+        if mode not in ("count", "uniq", "vec", "histo"):
             raise AssertionError(f"unknown mode {mode!r}")
         budget = self.device_budget(d, budget_bytes)
         if mode == "vec":
             budget -= 8 * (d.n_bases + 1)
         vb = d.payload_bytes
-        text_bytes = self._text_plan(d, k, mode, chunk_rows)[1] if text else 0
+        text_bytes = self._text_plan(d, k, mode, chunk_rows)[1] if text and mode != "histo" else 0
         n, n_other = self.count_windows(d, k, rc)
         one = self._one_pass_bytes(d, k, rc, mode, n_other, vb, text_bytes)
         n_win = max(0, d.n_bases - k + 1)
@@ -1196,6 +1216,94 @@ class Engine:
                 fh.close()
         t1.synchronize()
         plan.text_ms = t0.elapsed_time(t1)
+        return plan
+
+    # ---- multiplicity spectrum: kmer histo ---------------------------------------------------------------
+    @_on_device
+    def histo_narrow(self, d: DeviceInput, k: int, rc: bool, out: Tuple[int, int, int], reuse: Optional[str] = None) -> int:
+        """Add the narrow stream's multiplicity histogram to `out` = (d_hist, d_big, d_n_big) device addresses in ONE
+        native call (kmg_extract_sort_histo: count_narrow()'s front end, no table); returns the number of windows
+        that belong to the wide stream."""
+        win_begin, win_end = window_range(d, k)
+        kb = key_bytes(k, False)
+        cap = max((win_end - win_begin) * (2 if rc else 1), 1)
+        keys, keys_alt = self._out(reuse, "keys", cap * kb), self._out(reuse, "keys_alt", cap * kb)
+        ws_bytes = self.lib.kmg_pipeline_histo_workspace_bytes(win_end - win_begin, k, int(rc))
+        ws = self._buf("ws_pipeline", ws_bytes)
+        res = (C.c_uint64 * 4)()
+        _lib.check(self.lib.kmg_extract_sort_histo(d.bases.data_ptr(), d.n_bases, win_begin, win_end, k, int(rc),
+                                                   d.lut.data_ptr(), keys.data_ptr(), keys_alt.data_ptr(), *out, res,
+                                                   ws.data_ptr(), ws_bytes, self._stream()))
+        return int(res[2])
+
+    @_on_device
+    def sort_histo(self, a: KeyArray, out: Tuple[int, int, int]) -> None:
+        """Add the multiplicity histogram of the keys of `a` to `out` (see histo_narrow).  8- and 16-byte keys:
+        kmg_sort_histo (consumes both key buffers); 32-byte wide keys: kmg_sort256 + kmg_rle_count +
+        kmg_count_histogram."""
+        assert a.val_bytes == 0
+        if a.n == 0:
+            return
+        if a.key_bytes == 32:
+            t = self.rle_count(self.sort(a))
+            _lib.check(self.lib.kmg_count_histogram(t.counts.data_ptr(), t.n, *out, self._stream()))
+            return
+        ws_bytes = self.lib.kmg_sort_histo_workspace_bytes(a.n, a.key_bytes, a.key_bits)
+        ws = self._buf("ws_sort", ws_bytes)
+        _lib.check(self.lib.kmg_sort_histo(a.keys.data_ptr(), a.keys_alt.data_ptr(), a.n, a.key_bytes, a.key_bits,
+                                           _ptr(a.hist), *out, ws.data_ptr(), ws_bytes, self._stream()))
+        a.hist = None
+        self._status(ws)
+
+    def _histogram(self, d: DeviceInput, k: int, rc: bool, budget_bytes: Optional[int]) -> Tuple[np.ndarray, np.ndarray, PassPlan]:
+        window_range(d, k)  # (the k checks, before any work)
+        plan = self.plan_passes(d, k, rc, "histo", budget_bytes, text=False)
+        total = int(plan.narrow.sum() + plan.wide.sum())
+        nbins = _lib.KMG_HISTO_BINS
+        # one device buffer, read back once: bins [nbins] | list length | list of multiplicities >= nbins
+        acc = torch.zeros(8 * (nbins + 1) + 4 * (total // nbins + 1), dtype=torch.uint8, device=self.device)
+        out = (acc.data_ptr(), acc.data_ptr() + 8 * (nbins + 1), acc.data_ptr() + 8 * nbins)
+        for lo, hi in plan.parts:
+            t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            t0.record()
+            if plan.n_parts == 1:
+                if self.histo_narrow(d, k, rc, out):
+                    self.sort_histo(self.extract(d, k, rc, wide=True, val_bytes=0), out)
+            else:
+                for wide, per_part in ((False, plan.narrow), (True, plan.wide)):
+                    n_keys = int(per_part[lo:hi].sum())
+                    if n_keys:
+                        self.sort_histo(self.extract_parts(d, k, rc, wide, 0, plan.n_parts, lo, hi, n_keys), out)
+            t1.record()
+            t1.synchronize()
+            plan.pass_ms.append(t0.elapsed_time(t1))
+        raw = acc.cpu().numpy()
+        bins = raw[: 8 * (nbins + 1)].view(np.uint64)
+        big = raw[8 * (nbins + 1):].view(np.uint32)[: int(bins[nbins])]
+        mult = np.flatnonzero(bins[:nbins]).astype(np.uint64)
+        n_kmers = bins[:nbins][mult.astype(np.int64)]
+        if big.size:
+            bm, bc = np.unique(big, return_counts=True)
+            mult = np.concatenate([mult, bm.astype(np.uint64)])
+            n_kmers = np.concatenate([n_kmers, bc.astype(np.uint64)])
+        return mult, n_kmers.astype(np.uint64), plan
+
+    @_on_device
+    def histogram(self, d: DeviceInput, k: int, rc: bool = False,
+                  budget_bytes: Optional[int] = None) -> Tuple[np.ndarray, np.ndarray]:
+        """`kmer histo`: the multiplicity spectrum of the (k-mer, count) table count() would build, without the
+        table.  Returns uint64 arrays (mult, n_kmers): every multiplicity that occurs, ascending, and the number
+        of distinct k-mers seen exactly that often.  Narrow and wide stream, and the key-range passes of
+        plan_passes(mode="histo") when the input does not fit `budget_bytes`, add into one device histogram."""
+        mult, n_kmers, _ = self._histogram(d, k, rc, budget_bytes)
+        return mult, n_kmers
+
+    def write_histogram(self, d: DeviceInput, k: int, rc: bool, fh: BinaryIO,
+                        budget_bytes: Optional[int] = None) -> PassPlan:
+        """Write histogram() to the binary file `fh`, one "M\tN\n" line per multiplicity M (nothing for an empty
+        result).  Returns the plan with pass_ms filled in."""
+        mult, n_kmers, plan = self._histogram(d, k, rc, budget_bytes)
+        fh.write("".join("%d\t%d\n" % mn for mn in zip(mult.tolist(), n_kmers.tolist())).encode("ascii"))
         return plan
 
 
