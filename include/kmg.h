@@ -155,6 +155,13 @@ int kmg_radix_sort(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_al
 size_t kmg_rle_workspace_bytes(uint64_t n);
 int kmg_rle_count(const void* d_sorted_keys, uint64_t n, int key_bytes, void* d_uniq_keys_out,
                   uint32_t* d_counts_out, uint64_t* d_n_out, void* d_ws, size_t ws_bytes, void* stream);
+/* Keeps the rows of a count table (n 8-, 16- or 32-byte keys and their counts) with
+ * min_count <= count <= max_count, in their order; *d_n_out (device) = their number.  May run in place
+ * (d_keys_out == d_keys and d_counts_out == d_counts); other overlaps are undefined.  KMG_ERR_ARG unless
+ * 1 <= min_count <= max_count.  Workspace: kmg_rle_workspace_bytes(n). */
+int kmg_filter_counts(const void* d_keys, const uint32_t* d_counts, uint64_t n, int key_bytes, uint32_t min_count,
+                      uint32_t max_count, void* d_keys_out, uint32_t* d_counts_out, uint64_t* d_n_out, void* d_ws,
+                      size_t ws_bytes, void* stream);
 
 /* sort + rle_count in one call (the count path: join.py:63-130 after batch.py:156-168).  Sorts
  * the n keys on bits [0, end_bit) and leaves the distinct keys ascending in d_keys
@@ -166,6 +173,14 @@ size_t kmg_sort_count_workspace_bytes(uint64_t n, int key_bytes, int end_bit);
 int kmg_sort_count(void* d_keys, void* d_keys_alt, uint64_t n, int key_bytes, int end_bit, const uint64_t* d_hist_in,
                    uint32_t* d_counts_out, uint64_t* d_n_out, int* h_selector_out, void* d_ws, size_t ws_bytes,
                    void* stream);
+/* kmg_sort_count's table restricted to the rows with min_count <= count <= max_count (KMG_ERR_ARG unless
+ * 1 <= min_count <= max_count), in the same order.  The full range [1, 2^32-1] is kmg_sort_count.  Otherwise
+ * the hybrid finish's local sort writes only the kept rows; where it does not finish the table (plain
+ * passes, tiles it cannot hold) kmg_sort_count's table is compacted in place with kmg_filter_counts.  A run
+ * beyond uint32 is KMG_ERR_RANGE whatever the range.  Workspace: kmg_sort_count_workspace_bytes. */
+int kmg_sort_count_range(void* d_keys, void* d_keys_alt, uint64_t n, int key_bytes, int end_bit, const uint64_t* d_hist_in,
+                         uint32_t min_count, uint32_t max_count, uint32_t* d_counts_out, uint64_t* d_n_out,
+                         int* h_selector_out, void* d_ws, size_t ws_bytes, void* stream);
 /* sort + select_singletons in one call (the uniq path: join.py:63-130 + join_unique :243-263).
  * Leaves the keys that occur exactly once, ascending, with their payload in (d_keys, d_vals)
  * (*h_selector_out = 0) or (d_keys_alt, d_vals_alt) (1); *d_n_out (device) = their number.  Because
@@ -216,6 +231,12 @@ size_t kmg_pipeline_workspace_bytes(uint64_t n_windows, int k, int rc, int val_b
 int kmg_extract_sort_count(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
                            const uint8_t* d_lut256, void* d_keys, void* d_keys_alt, uint32_t* d_counts_out,
                            uint64_t* h_result, void* d_ws, size_t ws_bytes, void* stream);
+/* kmg_extract_sort_count with kmg_sort_count_range's finish: only the rows with
+ * min_count <= count <= max_count; h_result[0] counts them.  Workspace: kmg_pipeline_workspace_bytes(n, k, rc, 0). */
+int kmg_extract_sort_count_range(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k,
+                                 int rc, const uint8_t* d_lut256, void* d_keys, void* d_keys_alt, uint32_t min_count,
+                                 uint32_t max_count, uint32_t* d_counts_out, uint64_t* h_result, void* d_ws,
+                                 size_t ws_bytes, void* stream);
 int kmg_extract_sort_uniq(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
                           const uint8_t* d_lut256, void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_alt,
                           int val_bytes, uint64_t pos_offset, uint64_t* h_result, void* d_ws, size_t ws_bytes,

@@ -18,6 +18,7 @@ u32p = C.POINTER(C.c_uint32)
 u64p = C.POINTER(C.c_uint64)
 vp = C.c_void_p
 u64 = C.c_uint64
+u32 = C.c_uint32
 sz = C.c_size_t
 i32 = C.c_int
 
@@ -44,6 +45,9 @@ SIGNATURES = {
     "kmg_sort_count": (i32, [vp, vp, u64, i32, i32, vp, vp, vp, C.POINTER(C.c_int), vp, sz, vp]),
     "kmg_pipeline_workspace_bytes": (sz, [u64, i32, i32, i32]),
     "kmg_extract_sort_count": (i32, [vp, u64, u64, u64, i32, i32, vp, vp, vp, vp, u64p, vp, sz, vp]),
+    "kmg_sort_count_range": (i32, [vp, vp, u64, i32, i32, vp, u32, u32, vp, vp, C.POINTER(C.c_int), vp, sz, vp]),
+    "kmg_extract_sort_count_range": (i32, [vp, u64, u64, u64, i32, i32, vp, vp, vp, u32, u32, vp, u64p, vp, sz, vp]),
+    "kmg_filter_counts": (i32, [vp, vp, u64, i32, u32, u32, vp, vp, vp, vp, sz, vp]),
     "kmg_extract_sort_uniq": (i32, [vp, u64, u64, u64, i32, i32, vp, vp, vp, vp, vp, i32, u64, u64p, vp, sz, vp]),
     "kmg_sort_histo_workspace_bytes": (sz, [u64, i32, i32]),
     "kmg_sort_histo": (i32, [vp, vp, u64, i32, i32, vp, vp, vp, vp, vp, sz, vp]),

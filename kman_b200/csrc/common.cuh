@@ -72,12 +72,19 @@ static inline PassPlan make_plan(int begin_bit, int end_bit) {
 }
 
 // ---- cross-file plumbing of the fused pipeline (pipeline.cu) -----------------------------------------
+// the rows a count table keeps (kmg_sort_count_range): min_count <= count <= max_count; the full range is
+// the plain count table
+struct CountRange {
+    uint32_t min_count = 1, max_count = 0xFFFFFFFFu;
+    bool full() const { return min_count == 1 && max_count == 0xFFFFFFFFu; }
+};
 // fused run-length count / singleton request of a hybrid sort: `done` = the local sort produced the
 // result itself (counts == null: singletons with payload, kmg_sort_uniq)
 struct CountOut {
     uint32_t* counts;
     unsigned long long* n_out;
     bool done;
+    CountRange range = {};
 };
 // multiplicity histogram (kmg_sort_histo): hist[m] = distinct keys seen m times for m < KMG_HISTO_BINS;
 // larger multiplicities are appended to big[] (*n_big entries, in no order); *err becomes 2 for a
@@ -136,7 +143,10 @@ bool hybrid_sort_applies(uint64_t n, int key_bytes, int val_bytes, int end_bit, 
 int hybrid_choose_pb(uint64_t n, unsigned long long max_top_byte_count, int key_bytes, int val_bytes);
 int sort_count_core(void* d_keys, void* d_keys_alt, uint64_t n, int key_bytes, int end_bit, const uint64_t* d_hist_in,
                     uint32_t* d_counts_out, uint64_t* d_n_out, int* h_selector_out, void* d_ws, size_t ws_bytes, void* stream,
-                    const PrePartitioned* pre);
+                    const PrePartitioned* pre, CountRange range = {});
+// order-preserving compaction of a count table to the rows in range (kmg_filter_counts); may run in place
+int filter_counts(const void* d_keys, const uint32_t* d_counts, uint64_t n, int key_bytes, CountRange range, void* d_keys_out,
+                  uint32_t* d_counts_out, uint64_t* d_n_out, void* d_ws, size_t ws_bytes, cudaStream_t st);
 int sort_uniq_core(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_alt, uint64_t n, int key_bytes, int val_bytes,
                    int end_bit, const uint64_t* d_hist_in, uint64_t* d_n_out, int* h_selector_out, void* d_ws,
                    size_t ws_bytes, void* stream, const PrePartitioned* pre);

@@ -93,6 +93,8 @@ struct HybridParams {
     uint32_t* ticket;
     uint32_t* err;
     HistoOut histo;                 // multiplicity histogram (EMIT 3)
+    uint32_t min_count, max_count;  // EMIT 4: the rows of the count table that are kept
+    uint32_t pad[2];                // (keeps the parameters that follow HybridParams 16-byte aligned as before)
 };
 
 // ---- multiplicity histogram (EMIT 3, kmg_sort_histo, kmg_count_histogram) ---------------------------
@@ -218,12 +220,14 @@ struct CellMap {
 // occur exactly once with their payload, compacted across tiles like the count table (kmg_sort_uniq),
 // 3 = nothing but the run lengths, added to the multiplicity histogram p.histo (kmg_sort_histo): no
 // output order, so no ticket and no tile prefix, and a tile the scheme cannot hold adds nothing (the
-// host re-sorts its range and histograms it on the side).
+// host re-sorts its range and histograms it on the side), 4 = the count table restricted to the rows with
+// p.min_count <= count <= p.max_count, compacted across tiles like the full table.
 template <typename KeyT, int EMIT, int VB>
 __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_kernel(const HybridParams p) {
     constexpr bool PAIRS = VB != 0;
-    constexpr bool COUNT = EMIT == 1, UNIQ = EMIT == 2, FUSED = EMIT == 1 || EMIT == 2, HISTO = EMIT == 3;
-    static_assert(!(PAIRS && (COUNT || HISTO)), "the fused count and histogram are key-only");
+    constexpr bool COUNT = EMIT == 1, UNIQ = EMIT == 2, HISTO = EMIT == 3, RANGE = EMIT == 4;
+    constexpr bool FUSED = EMIT == 1 || EMIT == 2 || EMIT == 4;
+    static_assert(!(PAIRS && (COUNT || HISTO || RANGE)), "the fused count and histogram are key-only");
     static_assert(!UNIQ || PAIRS, "singletons carry their payload");
     constexpr int IPT = LS<KeyT, PAIRS>::IPT, CPT = LS<KeyT, PAIRS>::CPT;
     constexpr int CAP = ls_cap<KeyT, PAIRS>(), CELLS = ls_cells<KeyT, PAIRS>(), CELL_WORDS = ls_cell_words<KeyT, PAIRS>();
@@ -535,6 +539,42 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_kernel(const HybridPar
                 if (idx < m) vout[idx] = vin[s_idx[idx]];
             }
         }
+    } else if constexpr (RANGE) {
+        // the runs whose length is in range: every thread measures its own runs (as the histogram does),
+        // a block scan ranks the kept ones, and every thread writes its own after the tile prefix
+        auto walk = [&](auto&& emit) {
+            uint32_t start = lo;
+            KeyT prev{};
+            for (uint32_t i = lo; i < hi; ++i) {
+                const KeyT key = s_stage[i];
+                if (i != lo && key != prev) {
+                    if (i - start >= p.min_count && i - start <= p.max_count) emit(start, i - start);
+                    start = i;
+                }
+                prev = key;
+            }
+            if (hi > lo && hi - start >= p.min_count && hi - start <= p.max_count) emit(start, hi - start);
+        };
+        uint32_t hk = 0;
+        walk([&](uint32_t, uint32_t) { ++hk; });
+        uint32_t H;
+        uint32_t hoff = block_excl_scan<LS_BLOCK, uint32_t>(hk, s_scan, H);
+        if (t == 0) tile_prefix_publish(p.tile_state, tile, H);
+        if (t < 32) {
+            const uint64_t base = tile_prefix_resolve_warp(p.tile_state, p.n_tiles, tile, H, p.err);
+            if (t == 0) {
+                s_base = base;
+                if (tile == p.n_tiles - 1) *p.n_out = *p.n_out_copy = base + H;
+            }
+        }
+        __syncthreads();
+        const uint64_t base = s_base;
+        KeyT* kout = reinterpret_cast<KeyT*>(p.keys_out);
+        walk([&](uint32_t i, uint32_t len) {
+            kout[base + hoff] = s_stage[i];
+            p.counts_out[base + hoff] = len;
+            ++hoff;
+        });
     } else if constexpr (UNIQ) {
         // keys that occur once: a run of equal keys lies inside one thread's run, so every thread
         // finds the singletons of its own run; a block scan ranks them, the tile prefix places them

@@ -48,8 +48,9 @@ template <typename KeyT, int EMIT, int VB>
 __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const HybridParams p) {
     constexpr bool PAIRS = VB != 0;
     // (EMIT 3, the histogram: tiles by stride as in the plain sort, no tile prefix; see local_sort_kernel)
-    constexpr bool COUNT = EMIT == 1, UNIQ = EMIT == 2, FUSED = EMIT == 1 || EMIT == 2, HISTO = EMIT == 3;
-    static_assert(!(PAIRS && (COUNT || HISTO)), "the fused count and histogram are key-only");
+    constexpr bool COUNT = EMIT == 1, UNIQ = EMIT == 2, HISTO = EMIT == 3, RANGE = EMIT == 4;
+    constexpr bool FUSED = EMIT == 1 || EMIT == 2 || EMIT == 4;
+    static_assert(!(PAIRS && (COUNT || HISTO || RANGE)), "the fused count and histogram are key-only");
     static_assert(!UNIQ || PAIRS, "singletons carry their payload");
     constexpr int IPT = LS<KeyT, PAIRS>::IPT;
     constexpr int CAP = ls_cap<KeyT, PAIRS>();  // keys = counter words; cells = 2 * CAP
@@ -463,7 +464,8 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
         if (N.kind == 2) publish_nothing(N.tile);  // (more of them in a row than the list holds)
         const bool ok = fixup(A, s_nfix[0]);
         const uint32_t ndup = s_ndup;
-        // A's aggregate: distinct keys (count), singletons (uniq; known here only without duplicates)
+        // A's aggregate: distinct keys (count), singletons (uniq; known here only without duplicates), kept
+        // rows (count in range: without duplicates all of them or none)
         if (!ok && t == 0) {
             atomicAdd(p.irregular, 1ull);
             p.flag[A.tile] = 1;
@@ -472,7 +474,7 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
             if (!ok) {
                 publish_nothing(A.tile);
             } else if (COUNT || ndup == 0) {
-                if (t == 0) tile_prefix_publish(p.tile_state, A.tile, A.m - ndup);
+                if (t == 0) tile_prefix_publish(p.tile_state, A.tile, RANGE && p.min_count != 1u ? 0u : A.m - ndup);
             }
         }
         // the next tile's front, between A's publish and A's resolve
@@ -535,7 +537,7 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
         } else {
             const uint32_t m = A.m;
             KeyT* kout_all = reinterpret_cast<KeyT*>(p.keys_out);
-            if (!ok) {
+            if (!ok || (RANGE && ndup == 0 && p.min_count != 1u)) {
                 resolve_nothing(A.tile);
             } else if (ndup == 0) {
                 // every key of the tile is distinct (the rule on non-repetitive sequence): positions ARE
@@ -554,13 +556,33 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
                     const uint32_t pos = t + j * LS_BLOCK;
                     if (pos < m) {
                         kout_all[base + pos] = s_stage[pos];
-                        if constexpr (COUNT) p.counts_out[base + pos] = 1u;
+                        if constexpr (COUNT || RANGE) p.counts_out[base + pos] = 1u;
                         else reinterpret_cast<ValT*>(p.vals_out)[base + pos] = (reinterpret_cast<const ValT*>(p.vals_in) + A.s)[s_idx[pos]];
                     }
                 }
             } else {
                 // what is emitted, as a bitmask over the positions: COUNT the run heads (not a duplicate of the
-                // key before), UNIQ the singletons (a head whose successor is not its duplicate); one warp ranks them
+                // key before), UNIQ the singletons (a head whose successor is not its duplicate), RANGE the heads
+                // whose run length is in range (every warp classifies its word of each round: one ballot, no
+                // atomics); one warp ranks them
+                if constexpr (RANGE) {
+#pragma unroll
+                    for (int j = 0; j < IPT; ++j) {
+                        const uint32_t pos = t + j * LS_BLOCK;
+                        const uint32_t w = pos >> 5;
+                        const uint64_t window = ((uint64_t)s_dup[w] | ((uint64_t)s_dup[w + 1] << 32)) >> lane;
+                        const bool head = pos < m && !(window & 1u);
+                        uint32_t extra = (uint32_t)__ffsll((long long)~(window >> 1)) - 1u;
+                        if (head && extra >= 63u - lane) {  // the run leaves the 64-bit window: walk the words
+                            uint32_t q = pos + 1u + extra;
+                            while (q < m && ((s_dup[q >> 5] >> (q & 31u)) & 1u)) ++q;
+                            extra = q - pos - 1u;
+                        }
+                        const uint32_t keep = __ballot_sync(0xffffffffu, head && 1u + extra >= p.min_count && 1u + extra <= p.max_count);
+                        if (lane == 0) s_emit[w] = keep;
+                    }
+                    __syncthreads();
+                }
                 if (warp == 0) {
                     constexpr int PER = NW / 32;
                     uint32_t em[PER], sum = 0;
@@ -571,6 +593,7 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
                         const uint32_t d0 = s_dup[w];
                         uint32_t x = ~d0 & valid;
                         if constexpr (UNIQ) x &= ~((d0 >> 1) | (s_dup[w + 1] << 31));
+                        if constexpr (RANGE) x = s_emit[w];
                         em[i] = x;
                         sum += __popc(x);
                     }
@@ -583,7 +606,7 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
                         run += __popc(em[i]);
                     }
                     const uint32_t H = __shfl_sync(0xffffffffu, incl, 31);
-                    if (UNIQ && lane == 0) tile_prefix_publish(p.tile_state, A.tile, H);
+                    if ((UNIQ || RANGE) && lane == 0) tile_prefix_publish(p.tile_state, A.tile, H);
                     const uint64_t base = tile_prefix_resolve_warp(p.tile_state, p.n_tiles, A.tile, H, p.err);
                     if (lane == 0) {
                         s_base = base;
@@ -601,7 +624,7 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
                     if (!((em >> lane) & 1u)) continue;
                     const uint32_t h = s_epre[w] + __popc(em & lanemask_lt());
                     kout[h] = s_stage[pos];
-                    if constexpr (COUNT) {
+                    if constexpr (COUNT || RANGE) {
                         // run length = 1 + the duplicate marks that follow without a gap
                         const uint64_t window = ((uint64_t)s_dup[w] | ((uint64_t)s_dup[w + 1] << 32)) >> lane >> 1;
                         uint32_t extra = (uint32_t)__ffsll((long long)~window) - 1u;  // marks right after me inside the window

@@ -97,14 +97,14 @@ int status_from_err(int64_t err) {
     return KMG_OK;
 }
 
-// mode 0: (k-mer, count) table; mode 1: singletons with payload; mode 2: the multiplicity histogram, added
-// to *histo.  h_result: [0] rows of the result, [1] keys sorted (valid narrow windows, x2 with rc),
+// mode 0: (k-mer, count) table, restricted to `range`; mode 1: singletons with payload; mode 2: the multiplicity
+// histogram, added to *histo.  h_result: [0] rows of the result, [1] keys sorted (valid narrow windows, x2 with rc),
 // [2] windows that belong to the wide stream, [3] selector (0: result in d_keys / d_vals, 1: in the alt
 // buffers); mode 2 has no table: [0] and [3] stay 0
 int run_pipeline(int mode, const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
                  const uint8_t* d_lut256, void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_alt, int val_bytes,
                  uint64_t pos_offset, uint32_t* d_counts_out, uint64_t* h_result, void* d_ws, size_t ws_bytes,
-                 cudaStream_t st, const HistoOut* histo = nullptr) {
+                 cudaStream_t st, const HistoOut* histo = nullptr, CountRange range = {}) {
     KMG_REQUIRE(h_result, KMG_ERR_ARG, "h_result is null");
     h_result[0] = h_result[1] = h_result[2] = h_result[3] = 0;
     KMG_REQUIRE(k >= 2, KMG_ERR_ARG, "k must be >= 2, got %d", k);  // batcher.py:477-478
@@ -175,7 +175,7 @@ int run_pipeline(int mode, const uint8_t* d_bases, uint64_t n_bases, uint64_t wi
                 rcode = sort_histo_core(d_keys, d_keys_alt, n, kb, 2 * k, nullptr, *histo, w.sort_ws, w.sort_ws_bytes, st, &pre);
             else if (mode == 0)
                 rcode = sort_count_core(d_keys, d_keys_alt, n, kb, 2 * k, nullptr, d_counts_out, w.n_out, &sel, w.sort_ws,
-                                        w.sort_ws_bytes, st, &pre);
+                                        w.sort_ws_bytes, st, &pre, range);
             else
                 rcode = sort_uniq_core(d_keys, d_keys_alt, d_vals, d_vals_alt, n, kb, val_bytes, 2 * k, nullptr, w.n_out, &sel,
                                        w.sort_ws, w.sort_ws_bytes, st, &pre);
@@ -200,7 +200,7 @@ int run_pipeline(int mode, const uint8_t* d_bases, uint64_t n_bases, uint64_t wi
             rcode = sort_histo_core(d_keys, d_keys_alt, n, kb, 2 * k, hist, *histo, w.sort_ws, w.sort_ws_bytes, st, nullptr);
         else if (mode == 0)
             rcode = sort_count_core(d_keys, d_keys_alt, n, kb, 2 * k, hist, d_counts_out, w.n_out, &sel, w.sort_ws,
-                                    w.sort_ws_bytes, st, nullptr);
+                                    w.sort_ws_bytes, st, nullptr, range);
         else
             rcode = sort_uniq_core(d_keys, d_keys_alt, d_vals, d_vals_alt, n, kb, val_bytes, 2 * k, hist, w.n_out, &sel,
                                    w.sort_ws, w.sort_ws_bytes, st, nullptr);
@@ -282,6 +282,17 @@ extern "C" int kmg_extract_sort_count(const uint8_t* d_bases, uint64_t n_bases, 
                                       void* stream) {
     return run_pipeline(0, d_bases, n_bases, win_begin, win_end, k, rc, d_lut256, d_keys, d_keys_alt, nullptr, nullptr, 0, 0,
                         d_counts_out, h_result, d_ws, ws_bytes, (cudaStream_t)stream);
+}
+
+extern "C" int kmg_extract_sort_count_range(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end,
+                                            int k, int rc, const uint8_t* d_lut256, void* d_keys, void* d_keys_alt,
+                                            uint32_t min_count, uint32_t max_count, uint32_t* d_counts_out, uint64_t* h_result,
+                                            void* d_ws, size_t ws_bytes, void* stream) {
+    KMG_REQUIRE(h_result, KMG_ERR_ARG, "h_result is null");
+    h_result[0] = h_result[1] = h_result[2] = h_result[3] = 0;
+    KMG_REQUIRE(min_count >= 1 && min_count <= max_count, KMG_ERR_ARG, "bad count range [%u, %u]", min_count, max_count);
+    return run_pipeline(0, d_bases, n_bases, win_begin, win_end, k, rc, d_lut256, d_keys, d_keys_alt, nullptr, nullptr, 0, 0,
+                        d_counts_out, h_result, d_ws, ws_bytes, (cudaStream_t)stream, nullptr, CountRange{min_count, max_count});
 }
 
 extern "C" int kmg_extract_sort_uniq(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k,

@@ -924,7 +924,12 @@ static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_
     const int sel_done = sel_in ^ 1;                   // ... and where the finish puts its result
     const bool want_fused = co != nullptr && g_count_fused;
     const bool want_histo = hr != nullptr;
+    const bool want_range = co != nullptr && !co->range.full();
     if (want_histo) hp.histo = hr->out;
+    if (want_range) {
+        hp.min_count = co->range.min_count;
+        hp.max_count = co->range.max_count;
+    }
 
     auto launch_bounds = [&](uint32_t T) -> int {
         hp.tile_t = T;
@@ -962,6 +967,9 @@ static int sort_impl(void* d_keys, void* d_keys_alt, void* d_vals, void* d_vals_
         } else if (fused && want_histo) {
             if (wide_key) KMG_LS_LAUNCH(u128, 3, 0);
             else KMG_LS_LAUNCH(uint64_t, 3, 0);
+        } else if (fused && want_range) {
+            if (wide_key) KMG_LS_LAUNCH(u128, 4, 0);
+            else KMG_LS_LAUNCH(uint64_t, 4, 0);
         } else if (fused) {
             if (wide_key) KMG_LS_LAUNCH(u128, 1, 0);
             else KMG_LS_LAUNCH(uint64_t, 1, 0);
@@ -1138,9 +1146,11 @@ __global__ void merge_err_kernel(uint32_t* dst, const uint32_t* src) {
 
 int kmg::sort_count_core(void* d_keys, void* d_keys_alt, uint64_t n, int key_bytes, int end_bit, const uint64_t* d_hist_in,
                          uint32_t* d_counts_out, uint64_t* d_n_out, int* h_selector_out, void* d_ws, size_t ws_bytes,
-                         void* stream, const PrePartitioned* pre) {
+                         void* stream, const PrePartitioned* pre, CountRange range) {
     cudaStream_t st = (cudaStream_t)stream;
     KMG_REQUIRE(key_bytes == 8 || key_bytes == 16, KMG_ERR_ARG, "key_bytes must be 8 or 16");
+    KMG_REQUIRE(range.min_count >= 1 && range.min_count <= range.max_count, KMG_ERR_ARG, "bad count range [%u, %u]",
+                range.min_count, range.max_count);
     KMG_REQUIRE(end_bit >= 0 && end_bit <= key_bytes * 8, KMG_ERR_ARG, "bad end_bit %d", end_bit);
     KMG_REQUIRE(h_selector_out && d_n_out, KMG_ERR_ARG, "null pointer argument");
     *h_selector_out = 0;
@@ -1156,7 +1166,7 @@ int kmg::sort_count_core(void* d_keys, void* d_keys_alt, uint64_t n, int key_byt
     const size_t sort_ws = align_up(kmg_radix_sort_workspace_bytes(n, key_bytes, 0, 0, end_bit), 256);
     KMG_REQUIRE(ws_bytes >= sort_ws + kmg_rle_workspace_bytes(n), KMG_ERR_WS, "sort_count workspace too small");
     int sel = 0;
-    CountOut co{d_counts_out, reinterpret_cast<unsigned long long*>(d_n_out), false};
+    CountOut co{d_counts_out, reinterpret_cast<unsigned long long*>(d_n_out), false, range};
     if (n > 1 && end_bit > 0) {
         const bool hybrid = hybrid_applies(n, key_bytes, 0, 0, end_bit);
         const int rcode = sort_impl(d_keys, d_keys_alt, nullptr, nullptr, n, key_bytes, 0, 0, end_bit, d_hist_in, &sel, d_ws,
@@ -1171,8 +1181,20 @@ int kmg::sort_count_core(void* d_keys, void* d_keys_alt, uint64_t n, int key_byt
     void* sorted = sel ? d_keys_alt : d_keys;
     void* other = sel ? d_keys : d_keys_alt;
     *h_selector_out = sel ^ 1;
-    const int rcode = kmg_rle_count(sorted, n, key_bytes, other, d_counts_out, d_n_out, (char*)d_ws + sort_ws,
-                                    ws_bytes - sort_ws, stream);
+    int rcode = kmg_rle_count(sorted, n, key_bytes, other, d_counts_out, d_n_out, (char*)d_ws + sort_ws,
+                              ws_bytes - sort_ws, stream);
+    if (rcode != KMG_OK) return rcode;
+    merge_err_kernel<<<1, 1, 0, st>>>(&reinterpret_cast<WsHeader*>(d_ws)->err,
+                                      &reinterpret_cast<WsHeader*>((char*)d_ws + sort_ws)->err);
+    KMG_LAUNCH_CHECK();
+    if (range.full()) return KMG_OK;
+    // a narrower range on a path the local sort did not finish (plain passes, oversize or crowded tiles):
+    // the table is compacted in place, in the run-length stage's workspace (its status word is merged above)
+    unsigned long long n_rows = 0;
+    KMG_CUDA(cudaMemcpyAsync(&n_rows, d_n_out, sizeof(n_rows), cudaMemcpyDeviceToHost, st));
+    KMG_CUDA(cudaStreamSynchronize(st));
+    rcode = filter_counts(other, d_counts_out, n_rows, key_bytes, range, other, d_counts_out, d_n_out, (char*)d_ws + sort_ws,
+                          ws_bytes - sort_ws, st);
     if (rcode != KMG_OK) return rcode;
     merge_err_kernel<<<1, 1, 0, st>>>(&reinterpret_cast<WsHeader*>(d_ws)->err,
                                       &reinterpret_cast<WsHeader*>((char*)d_ws + sort_ws)->err);
@@ -1185,6 +1207,13 @@ extern "C" int kmg_sort_count(void* d_keys, void* d_keys_alt, uint64_t n, int ke
                               void* d_ws, size_t ws_bytes, void* stream) {
     return sort_count_core(d_keys, d_keys_alt, n, key_bytes, end_bit, d_hist_in, d_counts_out, d_n_out, h_selector_out, d_ws,
                            ws_bytes, stream, nullptr);
+}
+
+extern "C" int kmg_sort_count_range(void* d_keys, void* d_keys_alt, uint64_t n, int key_bytes, int end_bit,
+                                    const uint64_t* d_hist_in, uint32_t min_count, uint32_t max_count, uint32_t* d_counts_out,
+                                    uint64_t* d_n_out, int* h_selector_out, void* d_ws, size_t ws_bytes, void* stream) {
+    return sort_count_core(d_keys, d_keys_alt, n, key_bytes, end_bit, d_hist_in, d_counts_out, d_n_out, h_selector_out, d_ws,
+                           ws_bytes, stream, nullptr, CountRange{min_count, max_count});
 }
 
 // The histogram of a sort is built in the workspace and added to the caller's arrays at the end: should

@@ -368,6 +368,94 @@ __global__ void __launch_bounds__(RLE_BLOCK, 3) select_singletons_kernel(const R
 constexpr int RLE_IPT8 = 16;   // 8-byte keys: 4096-key tiles
 constexpr int RLE_IPT16 = 8;   // 16-byte keys: 2048-key tiles
 
+// ---- 4. order-preserving compaction of a count table to the rows in range (kmg_filter_counts) ---------
+// One pass with a ticketed tile prefix.  A tile loads its rows into registers before it publishes its
+// aggregate, and its rows go to [prefix, prefix + kept) <= its own input's end; a later tile writes only
+// once every earlier one has published (it needs their aggregates), so the table can be compacted in place.
+struct FilterParams {
+    const void* keys_in;
+    const uint32_t* counts_in;
+    void* keys_out;
+    uint32_t* counts_out;
+    uint64_t n;
+    uint32_t n_tiles;
+    uint32_t min_count, max_count;
+    unsigned long long* n_out;
+    uint64_t* tile_state;
+    uint32_t* ticket;
+    uint32_t* err;
+};
+
+template <typename KeyT, int IPT>
+__global__ void __launch_bounds__(RLE_BLOCK) filter_counts_kernel(const FilterParams p) {
+    constexpr int TILE = RLE_BLOCK * IPT;
+    __shared__ uint32_t s_off[IPT][RLE_WARPS];  // kept rows of warp w in round j, then their exclusive prefix
+    __shared__ uint32_t s_tile;
+    __shared__ uint64_t s_base;
+    const uint32_t t = threadIdx.x, lane = t & 31u, warp = t >> 5;
+    if (t == 0) s_tile = atomicAdd(p.ticket, 1u);
+    __syncthreads();
+    const uint32_t tile = s_tile;
+    const uint64_t tile_base = (uint64_t)tile * TILE;
+    const KeyT* kin = reinterpret_cast<const KeyT*>(p.keys_in) + tile_base;
+    const uint32_t* cin = p.counts_in + tile_base;
+    const uint64_t left = p.n - tile_base;
+    KeyT keys[IPT];
+    uint32_t counts[IPT], keep[IPT];
+#pragma unroll
+    for (int j = 0; j < IPT; ++j) {
+        const uint32_t i = j * RLE_BLOCK + t;
+        keys[j] = i < left ? kin[i] : KeyT{};
+        counts[j] = i < left ? cin[i] : 0u;
+    }
+#pragma unroll
+    for (int j = 0; j < IPT; ++j) {
+        keep[j] = __ballot_sync(0xffffffffu, counts[j] >= p.min_count && counts[j] <= p.max_count);
+        if (lane == 0) s_off[j][warp] = __popc(keep[j]);
+    }
+    __syncthreads();  // (every row of the tile is in registers: the tile may publish)
+    if (warp == 0) {
+        constexpr int PER = IPT * RLE_WARPS / 32;
+        uint32_t* flat = &s_off[0][0];
+        uint32_t v[PER], sum = 0;
+#pragma unroll
+        for (int i = 0; i < PER; ++i) {
+            v[i] = flat[lane * PER + i];
+            sum += v[i];
+        }
+        const uint32_t incl = warp_incl_scan(sum);
+        uint32_t run = incl - sum;
+#pragma unroll
+        for (int i = 0; i < PER; ++i) {
+            flat[lane * PER + i] = run;
+            run += v[i];
+        }
+        const uint32_t agg = __shfl_sync(0xffffffffu, incl, 31);
+        if (lane == 0) {
+            __threadfence();
+            tile_prefix_publish(p.tile_state, tile, agg);
+        }
+        const uint64_t base = tile_prefix_resolve_warp(p.tile_state, p.n_tiles, tile, agg, p.err);
+        if (lane == 0) {
+            s_base = base;
+            if (tile == p.n_tiles - 1) *p.n_out = base + agg;
+        }
+    }
+    __syncthreads();
+    const uint64_t base = s_base;
+    KeyT* kout = reinterpret_cast<KeyT*>(p.keys_out) + base;
+    uint32_t* cout = p.counts_out + base;
+    const uint32_t lt = lanemask_lt();
+#pragma unroll
+    for (int j = 0; j < IPT; ++j) {
+        if ((keep[j] >> lane) & 1u) {
+            const uint32_t o = s_off[j][warp] + __popc(keep[j] & lt);
+            kout[o] = keys[j];
+            cout[o] = counts[j];
+        }
+    }
+}
+
 }  // namespace kmg
 
 using namespace kmg;
@@ -478,4 +566,48 @@ extern "C" int kmg_select_singletons(const void* d_sorted_keys, const void* d_va
     }
     KMG_LAUNCH_CHECK();
     return KMG_OK;
+}
+
+int kmg::filter_counts(const void* d_keys, const uint32_t* d_counts, uint64_t n, int key_bytes, CountRange range, void* d_keys_out,
+                       uint32_t* d_counts_out, uint64_t* d_n_out, void* d_ws, size_t ws_bytes, cudaStream_t st) {
+    KMG_REQUIRE(key_bytes == 8 || key_bytes == 16 || key_bytes == 32, KMG_ERR_ARG, "key_bytes must be 8, 16 or 32");
+    KMG_REQUIRE(range.min_count >= 1 && range.min_count <= range.max_count, KMG_ERR_ARG, "bad count range [%u, %u]",
+                range.min_count, range.max_count);
+    KMG_REQUIRE(d_n_out, KMG_ERR_ARG, "d_n_out is null");
+    KMG_CUDA(cudaMemsetAsync(d_n_out, 0, sizeof(uint64_t), st));
+    if (n == 0) return KMG_OK;
+    KMG_REQUIRE(d_keys && d_counts && d_keys_out && d_counts_out && d_ws, KMG_ERR_ARG, "null pointer argument");
+    KMG_REQUIRE(ws_bytes >= kmg_rle_workspace_bytes(n), KMG_ERR_WS, "filter workspace too small");
+    const uint64_t tile = key_bytes == 8 ? RLE_BLOCK * RLE_IPT8 : RLE_BLOCK * RLE_IPT16;
+    const uint64_t nt = (n + tile - 1) / tile;
+    KMG_REQUIRE(nt < (1ull << 31), KMG_ERR_RANGE, "too many tiles");
+    // header (ticket, status word) | tile prefix state: inside kmg_rle_workspace_bytes(n) for tiles of >= 2048 rows
+    const size_t state_bytes = sc_state_words(nt) * sizeof(uint64_t);
+    KMG_CUDA(cudaMemsetAsync(d_ws, 0, sizeof(WsHeader) + state_bytes, st));
+    WsHeader* hdr = reinterpret_cast<WsHeader*>(d_ws);
+    FilterParams p;
+    p.keys_in = d_keys;
+    p.counts_in = d_counts;
+    p.keys_out = d_keys_out;
+    p.counts_out = d_counts_out;
+    p.n = n;
+    p.n_tiles = (uint32_t)nt;
+    p.min_count = range.min_count;
+    p.max_count = range.max_count;
+    p.n_out = reinterpret_cast<unsigned long long*>(d_n_out);
+    p.tile_state = reinterpret_cast<uint64_t*>((char*)d_ws + sizeof(WsHeader));
+    p.ticket = &hdr->ticket;
+    p.err = &hdr->err;
+    if (key_bytes == 8) filter_counts_kernel<uint64_t, RLE_IPT8><<<p.n_tiles, RLE_BLOCK, 0, st>>>(p);
+    else if (key_bytes == 16) filter_counts_kernel<u128, RLE_IPT16><<<p.n_tiles, RLE_BLOCK, 0, st>>>(p);
+    else filter_counts_kernel<u256, RLE_IPT16><<<p.n_tiles, RLE_BLOCK, 0, st>>>(p);
+    KMG_LAUNCH_CHECK();
+    return KMG_OK;
+}
+
+extern "C" int kmg_filter_counts(const void* d_keys, const uint32_t* d_counts, uint64_t n, int key_bytes, uint32_t min_count,
+                                 uint32_t max_count, void* d_keys_out, uint32_t* d_counts_out, uint64_t* d_n_out, void* d_ws,
+                                 size_t ws_bytes, void* stream) {
+    return filter_counts(d_keys, d_counts, n, key_bytes, CountRange{min_count, max_count}, d_keys_out, d_counts_out, d_n_out,
+                         d_ws, ws_bytes, (cudaStream_t)stream);
 }

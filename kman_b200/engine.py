@@ -181,6 +181,18 @@ def plan_parts(narrow: Sequence[int], wide: Sequence[int], pass_bytes: Callable[
     return out
 
 
+COUNT_MAX = 2**32 - 1  # the largest count a table holds (uint32)
+
+
+def count_range(min_count: int = 1, max_count: Optional[int] = None) -> Optional[Tuple[int, int]]:
+    """(min_count, max_count) of a count restricted to min_count <= count <= max_count (max_count None: no upper
+    limit), or None for the full range [1, 2^32-1]: the plain count table.  A bad range raises AssertionError."""
+    hi = COUNT_MAX if max_count is None else int(max_count)
+    lo = int(min_count)
+    assert 1 <= lo <= hi <= COUNT_MAX, f"bad count range: need 1 <= min_count <= max_count <= {COUNT_MAX}, got [{lo}, {hi}]"
+    return None if (lo, hi) == (1, COUNT_MAX) else (lo, hi)
+
+
 def pass_bytes(k: int, mode: str, n: int, m: int, val_bytes: int, text_bytes: int, n_win: int) -> int:
     """Device bytes of one pass over n narrow and m wide keys: key (+ payload) buffers and their alternates,
     counts, the sort workspace from the library's own *_workspace_bytes (one buffer the engine keeps and
@@ -194,7 +206,11 @@ def pass_bytes(k: int, mode: str, n: int, m: int, val_bytes: int, text_bytes: in
 
     mode "histo" (multiplicity spectrum): keys and their alternates and kmg_sort_histo's workspace per stream
     (32-byte wide keys: kmg_sort256 + kmg_rle_count and the counts), the larger stage as in "vec"; no counts,
-    merge ranks or text.  The histogram arrays themselves (a few MB) are not counted."""
+    merge ranks or text.  The histogram arrays themselves (a few MB) are not counted.
+
+    A count restricted to a multiplicity range (write_count(min_count=, max_count=)) takes the "count" plan:
+    its tables, counts and workspaces (kmg_sort_count_range, kmg_filter_counts in place) are never larger than
+    the unfiltered ones, so the count plan is an upper bound for it."""
     lib = _lib.load()
     kb, kw = key_bytes(k, False), key_bytes(k, True)
     if mode == "histo":
@@ -560,13 +576,18 @@ class Engine:
         return a
 
     @_on_device
-    def sort_count(self, a: KeyArray, end_bit: Optional[int] = None, reuse: Optional[str] = None) -> CountTable:
+    def sort_count(self, a: KeyArray, end_bit: Optional[int] = None, reuse: Optional[str] = None, min_count: int = 1,
+                   max_count: Optional[int] = None) -> CountTable:
         """sort() + rle_count() in one native call (kmg_sort_count): when the hybrid finish applies,
-        its local sort emits the (k-mer, count) table directly.  Consumes `a` (both key buffers)."""
+        its local sort emits the (k-mer, count) table directly.  Consumes `a` (both key buffers).
+        min_count / max_count: keep only the rows with min_count <= count <= max_count (kmg_sort_count_range;
+        32-byte keys: kmg_filter_counts on the table)."""
         end_bit = a.key_bits if end_bit is None else end_bit
         assert a.val_bytes == 0
+        rng = count_range(min_count, max_count)
         if a.key_bytes == 32:
-            return self.rle_count(self.sort(a, 0, end_bit), reuse=reuse)
+            t = self.rle_count(self.sort(a, 0, end_bit), reuse=reuse)
+            return t if rng is None else self.filter_counts(t, *rng)
         counts = self._out(reuse, "counts", a.n * 4)
         if a.n == 0:
             return CountTable(a.keys_alt, counts, 0, a.key_bytes, a.k, a.wide)
@@ -574,11 +595,18 @@ class Engine:
         ws = self._buf("ws_sort", ws_bytes)
         sel = C.c_int(0)
         hist = a.hist if end_bit == a.key_bits else None
-        _lib.check(
-            self.lib.kmg_sort_count(a.keys.data_ptr(), a.keys_alt.data_ptr(), a.n, a.key_bytes, end_bit, _ptr(hist),
-                                    counts.data_ptr(), self._small[2:].data_ptr(), C.byref(sel), ws.data_ptr(), ws_bytes,
-                                    self._stream())
-        )
+        if rng is None:
+            _lib.check(
+                self.lib.kmg_sort_count(a.keys.data_ptr(), a.keys_alt.data_ptr(), a.n, a.key_bytes, end_bit, _ptr(hist),
+                                        counts.data_ptr(), self._small[2:].data_ptr(), C.byref(sel), ws.data_ptr(),
+                                        ws_bytes, self._stream())
+            )
+        else:
+            _lib.check(
+                self.lib.kmg_sort_count_range(a.keys.data_ptr(), a.keys_alt.data_ptr(), a.n, a.key_bytes, end_bit,
+                                              _ptr(hist), rng[0], rng[1], counts.data_ptr(), self._small[2:].data_ptr(),
+                                              C.byref(sel), ws.data_ptr(), ws_bytes, self._stream())
+            )
         a.hist = None
         self._last_sort_ws = ws
         n_out = self._sort_result_rows(ws)
@@ -611,6 +639,22 @@ class Engine:
         self._status(ws)
         n_out = int(self._small[2:3].cpu().numpy().view(np.uint64)[0])
         return CountTable(a.keys_alt, counts, n_out, a.key_bytes, a.k, a.wide)
+
+    @_on_device
+    def filter_counts(self, t: CountTable, min_count: int, max_count: int) -> CountTable:
+        """The rows of `t` with min_count <= count <= max_count, in order, compacted in place (kmg_filter_counts)."""
+        if t.n == 0:
+            return t
+        ws_bytes = self.lib.kmg_rle_workspace_bytes(t.n)
+        ws = self._buf("ws_rle", ws_bytes)
+        _lib.check(
+            self.lib.kmg_filter_counts(t.keys.data_ptr(), t.counts.data_ptr(), t.n, t.key_bytes, min_count, max_count,
+                                       t.keys.data_ptr(), t.counts.data_ptr(), self._small[2:].data_ptr(), ws.data_ptr(),
+                                       ws_bytes, self._stream())
+        )
+        self._status(ws)
+        n_out = int(self._small[2:3].cpu().numpy().view(np.uint64)[0])
+        return CountTable(t.keys, t.counts, n_out, t.key_bytes, t.k, t.wide)
 
     @_on_device
     def sort_uniq(self, a: KeyArray, end_bit: Optional[int] = None) -> KeyArray:
@@ -754,17 +798,26 @@ class Engine:
 
     @_on_device
     def count_narrow(self, d: DeviceInput, k: int, rc: bool = False, reuse: Optional[str] = None, win_begin: int = 0,
-                     win_end: Optional[int] = None) -> Tuple[CountTable, int]:
+                     win_end: Optional[int] = None, min_count: int = 1,
+                     max_count: Optional[int] = None) -> Tuple[CountTable, int]:
         """(k-mer, count) table of the narrow stream in ONE native call (kmg_extract_sort_count: the
         extraction kernel is the sort's first prefix pass), and the number of windows that belong
-        to the wide stream.  seq.py:284-328 + batch.py:156-168 + join.py:63-130,265-285."""
+        to the wide stream.  seq.py:284-328 + batch.py:156-168 + join.py:63-130,265-285.
+        min_count / max_count: only the rows with min_count <= count <= max_count (kmg_extract_sort_count_range)."""
+        rng = count_range(min_count, max_count)
         win_begin, win_end, kb, cap, keys, keys_alt, _, _, ws, ws_bytes = self._pipeline_buffers(
             d, k, rc, 0, reuse, win_begin, win_end)
         counts = self._out(reuse, "counts", cap * 4)
         res = (C.c_uint64 * 4)()
-        _lib.check(self.lib.kmg_extract_sort_count(d.bases.data_ptr(), d.n_bases, win_begin, win_end, k, int(rc),
-                                                   d.lut.data_ptr(), keys.data_ptr(), keys_alt.data_ptr(),
-                                                   counts.data_ptr(), res, ws.data_ptr(), ws_bytes, self._stream()))
+        if rng is None:
+            _lib.check(self.lib.kmg_extract_sort_count(d.bases.data_ptr(), d.n_bases, win_begin, win_end, k, int(rc),
+                                                       d.lut.data_ptr(), keys.data_ptr(), keys_alt.data_ptr(),
+                                                       counts.data_ptr(), res, ws.data_ptr(), ws_bytes, self._stream()))
+        else:
+            _lib.check(self.lib.kmg_extract_sort_count_range(d.bases.data_ptr(), d.n_bases, win_begin, win_end, k, int(rc),
+                                                             d.lut.data_ptr(), keys.data_ptr(), keys_alt.data_ptr(), rng[0],
+                                                             rng[1], counts.data_ptr(), res, ws.data_ptr(), ws_bytes,
+                                                             self._stream()))
         return CountTable(keys_alt if res[3] else keys, counts, int(res[0]), kb, k, False), int(res[2])
 
     @_on_device
@@ -783,12 +836,15 @@ class Engine:
         k_, v_ = (keys_alt, vals_alt) if res[3] else (keys, vals)
         return KeyArray(k_, None, v_, None, int(res[0]), kb, vb, k, False, is_sorted=True), int(res[2])
 
-    def count(self, d: DeviceInput, k: int, rc: bool = False) -> List[CountTable]:
-        """`kmer count` (SEQ_COUNT) on device: one CountTable per stream."""
-        tab, n_other = self.count_narrow(d, k, rc)
+    def count(self, d: DeviceInput, k: int, rc: bool = False, min_count: int = 1,
+              max_count: Optional[int] = None) -> List[CountTable]:
+        """`kmer count` (SEQ_COUNT) on device: one CountTable per stream, restricted to the rows with
+        min_count <= count <= max_count."""
+        tab, n_other = self.count_narrow(d, k, rc, min_count=min_count, max_count=max_count)
         out = [tab]
         if n_other:
-            out.append(self.sort_count(self.extract(d, k, rc, wide=True, val_bytes=0)))
+            out.append(self.sort_count(self.extract(d, k, rc, wide=True, val_bytes=0), min_count=min_count,
+                                       max_count=max_count))
         return out
 
     def uniq(self, d: DeviceInput, k: int, rc: bool = False) -> List[KeyArray]:
@@ -936,10 +992,11 @@ class Engine:
                          lambda a, b: pass_bytes(k, mode, a, b, vb, text_bytes, n_win))
 
     def write_count(self, d: DeviceInput, k: int, rc: bool, fh: BinaryIO, budget_bytes: Optional[int] = None,
-                    chunk_rows: Optional[int] = None) -> PassPlan:
+                    chunk_rows: Optional[int] = None, min_count: int = 1, max_count: Optional[int] = None) -> PassPlan:
         """Write the bytes of count_text() to the binary file object `fh`, pass by pass and chunk by chunk, so
-        device memory is bounded by the budget and host memory by the text chunk.  Returns the plan."""
-        return self._write_passes(d, k, rc, fh, "count", budget_bytes, chunk_rows)
+        device memory is bounded by the budget and host memory by the text chunk.  Returns the plan.
+        min_count / max_count: only the lines whose count is in [min_count, max_count] (the count plan)."""
+        return self._write_passes(d, k, rc, fh, "count", budget_bytes, chunk_rows, count_range(min_count, max_count))
 
     def write_uniq(self, d: DeviceInput, k: int, rc: bool, fh: BinaryIO, budget_bytes: Optional[int] = None,
                    chunk_rows: Optional[int] = None) -> PassPlan:
@@ -953,10 +1010,12 @@ class Engine:
         payload sorts are stable, so equal sequences keep their emission order."""
         self._write_text(d, k, "uniq", fh, [self.sorted_streams(d, k, rc, d.payload_bytes)], chunk_rows)
 
-    def count_text(self, d: DeviceInput, k: int, rc: bool = False) -> bytes:
-        """Bytes of the reference's `kmer count` output file (join.py:284), from the whole-input path."""
+    def count_text(self, d: DeviceInput, k: int, rc: bool = False, min_count: int = 1,
+                   max_count: Optional[int] = None) -> bytes:
+        """Bytes of the reference's `kmer count` output file (join.py:284), from the whole-input path; with a
+        range, only the lines whose count is in [min_count, max_count]."""
         fh = io.BytesIO()
-        self._write_text(d, k, "count", fh, [self.count(d, k, rc)])
+        self._write_text(d, k, "count", fh, [self.count(d, k, rc, min_count, max_count)])
         return fh.getvalue()
 
     def uniq_text(self, d: DeviceInput, k: int, rc: bool = False) -> bytes:
@@ -967,11 +1026,11 @@ class Engine:
 
     @_on_device
     def _write_passes(self, d: DeviceInput, k: int, rc: bool, fh: BinaryIO, mode: str, budget_bytes: Optional[int],
-                      chunk_rows: Optional[int]) -> PassPlan:
+                      chunk_rows: Optional[int], rng: Optional[Tuple[int, int]] = None) -> PassPlan:
         if d.rec_starts is None and mode == "uniq":  # resident before the budget is taken
             self._upload_names(d)
         plan = self.plan_passes(d, k, rc, mode, budget_bytes, chunk_rows)
-        plan.pass_ms = self._write_text(d, k, mode, fh, self.pass_tables(d, k, rc, mode, plan), chunk_rows)
+        plan.pass_ms = self._write_text(d, k, mode, fh, self.pass_tables(d, k, rc, mode, plan, rng), chunk_rows)
         return plan
 
     @_on_device
@@ -999,20 +1058,23 @@ class Engine:
             sink.close()
         return pass_ms
 
-    def pass_tables(self, d: DeviceInput, k: int, rc: bool, mode: str, plan: PassPlan):
+    def pass_tables(self, d: DeviceInput, k: int, rc: bool, mode: str, plan: PassPlan,
+                    rng: Optional[Tuple[int, int]] = None):
         """Yield, pass by pass, the sorted tables of `plan`: [narrow] or [narrow, wide] CountTables (count) /
-        singleton KeyArrays (uniq).  Concatenated in pass order they are the tables of count() / uniq()."""
+        singleton KeyArrays (uniq).  Concatenated in pass order they are the tables of count() / uniq().
+        rng (count): (min_count, max_count) of the rows kept, None for all."""
         vb = d.payload_bytes
+        lo_c, hi_c = rng if rng is not None else (1, None)
         for lo, hi in plan.parts:
             if plan.n_parts == 1:
-                yield self.count(d, k, rc) if mode == "count" else self.uniq(d, k, rc)
+                yield self.count(d, k, rc, lo_c, hi_c) if mode == "count" else self.uniq(d, k, rc)
                 continue
             tabs = []
             for wide, n_keys in ((False, int(plan.narrow[lo:hi].sum())), (True, int(plan.wide[lo:hi].sum()))):
                 if wide and not n_keys:
                     break
                 a = self.extract_parts(d, k, rc, wide, 0 if mode == "count" else vb, plan.n_parts, lo, hi, n_keys)
-                tabs.append(self.sort_count(a) if mode == "count" else self.sort_uniq(a))
+                tabs.append(self.sort_count(a, min_count=lo_c, max_count=hi_c) if mode == "count" else self.sort_uniq(a))
                 del a
             yield tabs
             del tabs

@@ -7,6 +7,8 @@ extract -> radix sort -> run-length (count) or singleton selection (uniq) -> tex
 in key-range passes when the input does not fit the device at once, streamed to the output
 file in chunks.  The emitted bytes equal the reference's
 (join.py:262 ">%s\\n%s\\n", join.py:284 "%s\\t%d\\n"); an empty result leaves an empty file.
+A SEQ_COUNT join can keep only the lines whose count is in `count_range` (`kmer count --min-count /
+--max-count`): the same file with the other lines removed, on every path.
 """
 from __future__ import annotations
 
@@ -79,6 +81,7 @@ class KJoiner:
     def __init__(self, mode: Optional["KJoiner.MODE"] = None, memory: Optional["KJoiner.MEMORY"] = None):
         self.__mode = self.DEFAULT_MODE
         self.__memory = self.DEFAULT_MEMORY
+        self.__count_range: Tuple[int, Optional[int]] = (1, None)
         if mode is not None:
             self.mode = mode
         if memory is not None:
@@ -103,6 +106,29 @@ class KJoiner:
         if memory not in self.MEMORY:
             raise AssertionError
         self.__memory = memory
+
+    @property
+    def count_range(self) -> Tuple[int, Optional[int]]:
+        """(min_count, max_count) of the SEQ_COUNT lines written; max_count None: no upper limit."""
+        return self.__count_range
+
+    @count_range.setter
+    def count_range(self, r: Tuple[int, Optional[int]]) -> None:
+        lo, hi = int(r[0]), None if r[1] is None else int(r[1])
+        self._check_range(lo, hi)
+        self.__count_range = (lo, hi)
+
+    def _check_range(self, lo: int, hi: Optional[int]) -> Optional[Tuple[int, int]]:
+        """(min_count, max_count) for the native calls, None for every line; AssertionError for a bad range or a
+        range outside SEQ_COUNT."""
+        if (lo, hi) == (1, None):  # (the default: no engine import on the host path)
+            return None
+        from kman_b200.engine import count_range
+
+        rng = count_range(lo, hi)
+        if rng is not None and self.mode != self.MODE.SEQ_COUNT:
+            raise AssertionError(f"--min-count / --max-count apply to SEQ_COUNT only, not to {self.mode.name}")
+        return rng
 
     @property
     def join_function(self):
@@ -177,13 +203,14 @@ class KJoiner:
             return
         from kman_b200.batch import LoadedKmerBatch
 
+        lo, hi = self._check_range(*self.count_range) or (1, None)
         if any(isinstance(b, LoadedKmerBatch) for b in batches):
             # `-B`: re-imported batch files carry their own headers (one LoadedKmerBatch covers a folder)
             if len(batches) != 1:
                 raise AssertionError("re-imported batch files cannot be joined together with other batches")
             with open(outpath, "wb") as oh:
                 if self.mode == self.MODE.SEQ_COUNT:
-                    b0._eng.write_count(b0.device_input, b0.k, False, oh)
+                    b0._eng.write_count(b0.device_input, b0.k, False, oh, min_count=lo, max_count=hi)
                 else:
                     oh.write(b0.uniq_text())
             return
@@ -192,11 +219,12 @@ class KJoiner:
         # text chunk (KMG_DEVICE_BUDGET overrides the device budget)
         with open(outpath, "wb") as oh:  # join.py:351 opens "w+": the file exists even when empty
             if self.mode == self.MODE.SEQ_COUNT:
-                b0._eng.write_count(d, b0.k, b0.reverse, oh)
+                b0._eng.write_count(d, b0.k, b0.reverse, oh, min_count=lo, max_count=hi)
             else:
                 b0._eng.write_uniq(d, b0.k, b0.reverse, oh)
 
     def join(self, batches: List[Any], outpath: str) -> None:
+        rng = self._check_range(*self.count_range)
         live = [b for b in batches if b is not None and not (isinstance(b, Batch) and b.current_size == 0)]
         if live and all(isinstance(b, DeviceBatch) for b in live):
             print("Joining...")
@@ -215,7 +243,8 @@ class KJoiner:
             return
         with open(outpath, "w+") as oh:
             for headers, seq in Crawler().do_batch(live):
-                self.join_function(headers, seq, OH=oh)
+                if rng is None or rng[0] <= len(headers) <= rng[1]:
+                    self.join_function(headers, seq, OH=oh)
 
 
 class KJoinerThreading(KJoiner):

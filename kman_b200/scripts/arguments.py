@@ -73,3 +73,13 @@ def compress():
 
 def re_sort():
     return click.option("--re-sort", "-R", is_flag=True, help="Force batch re-sorting, when loaded with -B.")
+
+
+def min_count():
+    return click.option("--min-count", type=click.INT, default=1,
+                        help="Write only the k-mers that occur at least this many times. Default: 1")
+
+
+def max_count():
+    return click.option("--max-count", type=click.INT, default=None,
+                        help="Write only the k-mers that occur at most this many times (at most 4294967295). Default: no limit")

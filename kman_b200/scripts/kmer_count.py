@@ -26,20 +26,23 @@ from kman_b200.scripts import arguments as args
 @args.threads()
 @args.tmp()
 @args.re_sort()
+@args.min_count()
+@args.max_count()
 def run(input_path: str, output_path: str, k: int, reverse: bool = False, scan_mode: str = FastaBatcher.MODE.KMERS.name,
         batch_size: int = 1000000, batch_mode: str = BatcherThreading.FEED_MODE.APPEND.name,
         previous_batches: Optional[str] = None, count_mode: str = KJoiner.MODE.SEQ_COUNT.name,
         memory_mode: str = KJoiner.MEMORY.NORMAL.name, threads: int = 1, tmp: str = tempfile.gettempdir(),
-        re_sort: bool = False) -> None:
+        re_sort: bool = False, min_count: int = 1, max_count: Optional[int] = None) -> None:
     input_file_exists(input_path)
     set_tempdir(tmp)
+    joiner = KJoinerThreading(KJoiner.MODE[count_mode], KJoiner.MEMORY[memory_mode])
+    joiner.count_range = (min_count, max_count)  # (a bad range or a VEC mode fails before any work)
     if previous_batches is not None:
         batches = load_batches(previous_batches, threads, re_sort)
     else:
         batches = (FastaBatcher(scan_mode=FastaBatcher.MODE[scan_mode], reverse=reverse, size=batch_size, threads=threads)
                    .do(input_path, k, BatcherThreading.FEED_MODE[batch_mode]).collection)
-    prep_joiner(KJoinerThreading(KJoiner.MODE[count_mode], KJoiner.MEMORY[memory_mode]), len(batches), threads).join(
-        batches, output_path)
+    prep_joiner(joiner, len(batches), threads).join(batches, output_path)
     logging.info("That's all! :smiley:")
 
 
