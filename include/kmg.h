@@ -266,7 +266,9 @@ int kmg_range_partition(const void* d_keys, const void* d_vals, uint64_t n, int 
  * pointers (peer-mapped, e.g. from kmg_ipc_open), d_cursors[n_parts] holds, per destination,
  * the first free element of THIS source's region and is advanced atomically.  With
  * count_only != 0 nothing is written: d_counts[0..n_parts) receives the number of keys per
- * destination and d_counts[n_parts] the number of windows that belong to the wide stream. */
+ * destination and d_counts[n_parts] the number of windows that belong to the wide stream.
+ * As in kmg_extract, val_bytes = 4 with ((pos_offset + n_bases) << 1) >= 2^32 is KMG_ERR_RANGE (the
+ * payload would not hold the position); this holds for all three kmg_extract_scatter* calls. */
 int kmg_extract_scatter(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
                         const uint8_t* d_lut256, int n_parts, void* const* d_dest_keys, void* const* d_dest_vals,
                         int key_bytes, int val_bytes, uint64_t pos_offset, uint64_t* d_cursors, uint64_t* d_counts,

@@ -259,6 +259,8 @@ static int scatter_impl(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_b
     KMG_REQUIRE(n_parts >= 1 && n_parts <= DX_MAX_PARTS, KMG_ERR_ARG, "n_parts must be in [1,%d]", DX_MAX_PARTS);
     KMG_REQUIRE(win_begin <= win_end, KMG_ERR_ARG, "win_begin > win_end");
     KMG_REQUIRE(val_bytes == 0 || val_bytes == 4 || val_bytes == 8, KMG_ERR_ARG, "val_bytes must be 0, 4 or 8");
+    if (val_bytes == 4)
+        KMG_REQUIRE(((pos_offset + n_bases) << 1) < (1ull << 32), KMG_ERR_RANGE, "val_bytes=4 needs < 2^31 positions");
     KMG_REQUIRE(key_bytes == (k <= 32 ? 8 : 16), KMG_ERR_ARG, "key_bytes must be %d for k=%d", k <= 32 ? 8 : 16, k);
     KMG_REQUIRE(((uintptr_t)d_bases & 15) == 0, KMG_ERR_ARG, "d_bases must be 16-byte aligned");
     KMG_REQUIRE(d_lut256, KMG_ERR_ARG, "null pointer argument");

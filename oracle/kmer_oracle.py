@@ -560,6 +560,11 @@ def _put_decimal(buf: np.ndarray, at: np.ndarray, v: np.ndarray, nd: np.ndarray)
 
 def count_text_np(records, k, rc=False, alphabet=DEFAULT_ALPHABET, natype="DNA") -> bytes:
     txt, counts, _ = count_np(records, k, rc, alphabet, natype)
+    return count_text_from(txt, counts, k)
+
+
+def count_text_from(txt: np.ndarray, counts: np.ndarray, k: int) -> bytes:
+    """"SEQ\tCOUNT\n" lines of count_np's (txt, counts)."""
     n = counts.shape[0]
     if n == 0:
         return b""
@@ -577,6 +582,11 @@ def count_text_np(records, k, rc=False, alphabet=DEFAULT_ALPHABET, natype="DNA")
 
 def uniq_text_np(records, k, rc=False, alphabet=DEFAULT_ALPHABET, natype="DNA") -> bytes:
     txt, rec, start, strand, names, _ = uniq_np(records, k, rc, alphabet, natype)
+    return uniq_text_from(txt, rec, start, strand, names, k)
+
+
+def uniq_text_from(txt: np.ndarray, rec: np.ndarray, start: np.ndarray, strand: np.ndarray, names, k: int) -> bytes:
+    """">NAME:START-END:STRAND\nSEQ\n" lines of uniq_np's (txt, rec, start, strand, names)."""
     n = rec.shape[0]
     if n == 0:
         return b""

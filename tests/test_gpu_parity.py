@@ -47,6 +47,27 @@ def _rand_records(rng, n_rec, max_len, alphabet="ACGT", p_other=0.0):
     return recs
 
 
+# Global position of bases[0] (DeviceInput.pos_offset): 0, one that makes the payloads straddle 2^32,
+# and two past it.  Payloads are (global position << 1) | strand in 8 bytes; 4-byte payloads are refused.
+POS_OFFSETS = [0, "straddle", 2**32 + 3, 2**47 + 5]
+
+
+def _pos_offset(p, n_bases: int) -> int:
+    return (1 << 31) - n_bases // 2 if p == "straddle" else p
+
+
+def _want_vals(st, offset: int) -> np.ndarray:
+    """Payloads the device stores for the oracle stream `st` of an input whose bases[0] is at `offset`."""
+    return ((st["pos"].astype(np.uint64) + np.uint64(offset)) << np.uint64(1)) | st["strand"].astype(np.uint64)
+
+
+def _payload64(rng, lo: np.ndarray) -> np.ndarray:
+    """8-byte payloads whose upper word is non-zero (bit 63 set) and unrelated to the lower word `lo`: a
+    kernel that moves only the low 32 bits of a payload fails on them."""
+    hi = rng.permutation(len(lo)).astype(np.uint64) + np.uint64(0x8000_0001)
+    return (hi << np.uint64(32)) | lo.astype(np.uint64)
+
+
 # ---- K1+K2 ---------------------------------------------------------------------------------
 @pytest.mark.parametrize("k", [2, 3, 15, 16, 17, 21, 31, 32, 33, 47, 63, 64])
 @pytest.mark.parametrize("rc", [False, True])
@@ -55,15 +76,20 @@ def test_extract_narrow_matches_oracle(eng, k, rc):
     recs = _rand_records(rng, 4, 9000, p_other=0.01)
     ex = ko.extract_np(recs, k, rc)
     d = eng.upload(_flat(recs))
-    for vb in (0, 4, 8):
-        a = eng.extract(d, k, rc, wide=False, val_bytes=vb)
-        want = limbs_to_rows(ex["narrow"]["keys"])
-        assert a.n == want.shape[0], (a.n, want.shape[0])
-        assert first_diff(a.keys_host(), want) == "equal"
-        assert a.n_other == ex["wide"]["pos"].shape[0] // (2 if rc else 1)
-        if vb:
-            wv = (ex["narrow"]["pos"].astype(np.uint64) << np.uint64(1)) | ex["narrow"]["strand"].astype(np.uint64)
-            assert first_diff(a.vals_host().astype(np.uint64), wv) == "equal"
+    want = limbs_to_rows(ex["narrow"]["keys"])
+    for p in POS_OFFSETS:
+        d.pos_offset = _pos_offset(p, d.n_bases)
+        for vb in (0, 4, 8):
+            if vb == 4 and d.payload_bytes == 8:
+                with pytest.raises(ValueError, match="val_bytes=4"):
+                    eng.extract(d, k, rc, wide=False, val_bytes=vb)
+                continue
+            a = eng.extract(d, k, rc, wide=False, val_bytes=vb)
+            assert a.n == want.shape[0], (a.n, want.shape[0])
+            assert first_diff(a.keys_host(), want) == "equal"
+            assert a.n_other == ex["wide"]["pos"].shape[0] // (2 if rc else 1)
+            if vb:
+                assert first_diff(a.vals_host().astype(np.uint64), _want_vals(ex["narrow"], d.pos_offset)) == "equal", (p, vb)
 
 
 @pytest.mark.parametrize("k", [2, 5, 16, 17, 25, 32, 33, 45, 48, 49, 63, 64])
@@ -73,12 +99,13 @@ def test_extract_wide_matches_oracle(eng, k, rc):
     recs = _rand_records(rng, 3, 6000, p_other=0.03)
     ex = ko.extract_np(recs, k, rc)
     d = eng.upload(_flat(recs))
-    a = eng.extract(d, k, rc, wide=True, val_bytes=8)
     want = limbs_to_rows(widen(ex["wide"]["keys"]))
-    assert a.n == want.shape[0]
-    assert first_diff(a.keys_host(), want) == "equal"
-    wv = (ex["wide"]["pos"].astype(np.uint64) << np.uint64(1)) | ex["wide"]["strand"].astype(np.uint64)
-    assert first_diff(a.vals_host(), wv) == "equal"
+    for p in POS_OFFSETS:
+        d.pos_offset = _pos_offset(p, d.n_bases)
+        a = eng.extract(d, k, rc, wide=True, val_bytes=8)
+        assert a.n == want.shape[0]
+        assert first_diff(a.keys_host(), want) == "equal"
+        assert first_diff(a.vals_host(), _want_vals(ex["wide"], d.pos_offset)) == "equal", p
 
 
 @pytest.mark.parametrize("k", [33, 40, 47, 48, 57, 64])
@@ -131,7 +158,7 @@ def _sort_case(eng, n, kb, vb, bits, seed, dup=False):
     else:
         hb = bits - 64
         raw[:, 1] &= np.uint64((1 << hb) - 1) if hb < 64 else np.uint64(2**64 - 1)
-    vals = np.arange(n, dtype=np.uint32 if vb == 4 else np.uint64)
+    vals = np.arange(n, dtype=np.uint32) if vb == 4 else _payload64(rng, np.arange(n))
     dev = eng.device
     t = lambda x: torch.from_numpy(x.view(np.uint8).reshape(-1).copy()).to(dev)  # noqa: E731
     a = KeyArray(t(raw), t(np.zeros_like(raw)), t(vals) if vb else None, t(np.zeros_like(vals)) if vb else None,
@@ -192,7 +219,7 @@ def test_rle_and_singletons(eng, kb, n):
     if limbs == 2:
         raw[:, 1] = base // np.uint64(7)
         raw = raw[np.lexsort((raw[:, 0], raw[:, 1]))]
-    vals = rng.permutation(n).astype(np.uint64)
+    vals = _payload64(rng, rng.permutation(n))
     dev = eng.device
     t = lambda x: torch.from_numpy(x.view(np.uint8).reshape(-1).copy()).to(dev)  # noqa: E731
     a = KeyArray(t(raw), t(np.zeros_like(raw)), t(vals), t(np.zeros_like(vals)), n, kb, 8, 31, False, is_sorted=True)
@@ -503,26 +530,29 @@ def test_extract_scatter_partitions_like_extract_plus_range_partition(eng, k, rc
     want_counts = np.bincount(part, minlength=n_parts)
     assert list(cnt[:n_parts]) == list(want_counts)
     assert cnt[n_parts] == 0
-    bufs = [torch.zeros(max(int(c), 1) * kb, dtype=torch.uint8, device=eng.device) for c in want_counts]
-    vbufs = [torch.zeros(max(int(c), 1) * 8, dtype=torch.uint8, device=eng.device) for c in want_counts]
-    ptrs = torch.tensor([b.data_ptr() for b in bufs], dtype=torch.int64, device=eng.device)
-    vptrs = torch.tensor([b.data_ptr() for b in vbufs], dtype=torch.int64, device=eng.device)
-    cursors = torch.zeros(n_parts, dtype=torch.int64, device=eng.device)
-    _lib.check(lib.kmg_extract_scatter(d.bases.data_ptr(), d.n_bases, 0, n_win, k, int(rc), d.lut.data_ptr(), n_parts,
-                                       ptrs.data_ptr(), vptrs.data_ptr(), kb, 8, 0, cursors.data_ptr(), None, 0, eng._stream()))
-    torch.cuda.synchronize()
-    assert list(cursors.cpu().numpy()) == list(want_counts)
     rows = limbs_to_rows(limbs)
-    wv = (ex["narrow"]["pos"].astype(np.uint64) << np.uint64(1)) | ex["narrow"]["strand"].astype(np.uint64)
-    for p in range(n_parts):
-        c = int(want_counts[p])
-        got_k = bufs[p][: c * kb].cpu().numpy().view(np.uint64)
-        got_k = got_k if kb == 8 else got_k.reshape(-1, 2)
-        got_v = vbufs[p][: c * 8].cpu().numpy().view(np.uint64)
-        sel = part == p
-        o_got, o_want = np.argsort(got_v), np.argsort(wv[sel])  # payloads are unique: align by them
-        assert first_diff(got_v[o_got], wv[sel][o_want]) == "equal", p
-        assert first_diff(got_k[o_got], rows[sel][o_want]) == "equal", p
+    for po in POS_OFFSETS:
+        off = _pos_offset(po, d.n_bases)
+        bufs = [torch.zeros(max(int(c), 1) * kb, dtype=torch.uint8, device=eng.device) for c in want_counts]
+        vbufs = [torch.zeros(max(int(c), 1) * 8, dtype=torch.uint8, device=eng.device) for c in want_counts]
+        ptrs = torch.tensor([b.data_ptr() for b in bufs], dtype=torch.int64, device=eng.device)
+        vptrs = torch.tensor([b.data_ptr() for b in vbufs], dtype=torch.int64, device=eng.device)
+        cursors = torch.zeros(n_parts, dtype=torch.int64, device=eng.device)
+        _lib.check(lib.kmg_extract_scatter(d.bases.data_ptr(), d.n_bases, 0, n_win, k, int(rc), d.lut.data_ptr(), n_parts,
+                                           ptrs.data_ptr(), vptrs.data_ptr(), kb, 8, off, cursors.data_ptr(), None, 0,
+                                           eng._stream()))
+        torch.cuda.synchronize()
+        assert list(cursors.cpu().numpy()) == list(want_counts)
+        wv = _want_vals(ex["narrow"], off)
+        for p in range(n_parts):
+            c = int(want_counts[p])
+            got_k = bufs[p][: c * kb].cpu().numpy().view(np.uint64)
+            got_k = got_k if kb == 8 else got_k.reshape(-1, 2)
+            got_v = vbufs[p][: c * 8].cpu().numpy().view(np.uint64)
+            sel = part == p
+            o_got, o_want = np.argsort(got_v), np.argsort(wv[sel])  # payloads are unique: align by them
+            assert first_diff(got_v[o_got], wv[sel][o_want]) == "equal", (po, p)
+            assert first_diff(got_k[o_got], rows[sel][o_want]) == "equal", (po, p)
 
 
 # ---- hybrid finish of key-only sorts (top-prefix passes + one shared-memory local sort) ---------------
@@ -753,8 +783,10 @@ def test_extract_scatter_shared_cursors(eng, k, rc, n_parts):
     want_counts = np.bincount(part, minlength=n_parts)
     cap = int(want_counts.max())
     rows = limbs_to_rows(limbs)
-    wv = (ex["narrow"]["pos"].astype(np.uint64) << np.uint64(1)) | ex["narrow"]["strand"].astype(np.uint64)
-    for capacity, expect_overflow in ((cap, False), (cap - 1, True)):
+    runs = [(po, cap, False) for po in POS_OFFSETS] + [(POS_OFFSETS[-1], cap - 1, True)]
+    for po, capacity, expect_overflow in runs:
+        off = _pos_offset(po, d.n_bases)
+        wv = _want_vals(ex["narrow"], off)
         bufs = [torch.zeros(cap * kb, dtype=torch.uint8, device=eng.device) for _ in range(n_parts)]
         vbufs = [torch.zeros(cap * 8, dtype=torch.uint8, device=eng.device) for _ in range(n_parts)]
         cursors = torch.zeros(n_parts * 32, dtype=torch.int64, device=eng.device)  # one cursor per 256-byte line
@@ -763,7 +795,7 @@ def test_extract_scatter_shared_cursors(eng, k, rc, n_parts):
         cptrs = torch.tensor([cursors.data_ptr() + 256 * i for i in range(n_parts)], dtype=torch.int64, device=eng.device)
         status = torch.zeros(2, dtype=torch.int32, device=eng.device)
         _lib.check(lib.kmg_extract_scatter_shared(d.bases.data_ptr(), d.n_bases, 0, n_win, k, int(rc), d.lut.data_ptr(),
-                                                  n_parts, ptrs.data_ptr(), vptrs.data_ptr(), kb, 8, 0, cptrs.data_ptr(),
+                                                  n_parts, ptrs.data_ptr(), vptrs.data_ptr(), kb, 8, off, cptrs.data_ptr(),
                                                   capacity, status.data_ptr(), eng._stream()))
         torch.cuda.synchronize()
         st = status.cpu().numpy()
@@ -883,6 +915,8 @@ def test_sort_uniq_u64_matches_numpy(eng, n, vdt, dup):
     pool = rng.integers(0, 1 << 62, size=max(1, n // dup), dtype=np.uint64)
     raw = pool[rng.integers(0, len(pool), size=n)] if dup > 1 else pool[:n]
     vals = np.arange(n, dtype=vdt) * vdt(3) + vdt(1)
+    if vdt == np.uint64:
+        vals = _payload64(rng, vals)
     keys, got_v = _sort_uniq(eng, raw, vals, 62)
     wk, wv = _want_singletons(raw, vals)
     assert first_diff(keys, wk) == "equal", (n, dup)
@@ -908,7 +942,7 @@ def test_sort_uniq_skewed_inputs(eng, pattern):
     else:
         bits = 59
         raw = (rnd & np.uint64((1 << 59) - 1)) | np.uint64(0b101 << 59)
-    vals = np.arange(n, dtype=np.uint64)
+    vals = _payload64(rng, np.arange(n))
     keys, got_v = _sort_uniq(eng, raw, vals, bits)
     wk, wv = _want_singletons(raw, vals)
     assert first_diff(keys, wk) == "equal", pattern

@@ -49,9 +49,10 @@ def _want_table(ex):
     return srt[idx], np.diff(np.append(idx, len(srt)))
 
 
-def _want_singletons(ex):
+def _want_singletons(ex, pos_offset=0):
     rows = limbs_to_rows(ex["narrow"]["keys"])
-    vals = (ex["narrow"]["pos"].astype(np.uint64) << np.uint64(1)) | ex["narrow"]["strand"].astype(np.uint64)
+    vals = ((ex["narrow"]["pos"].astype(np.uint64) + np.uint64(pos_offset)) << np.uint64(1)) | \
+        ex["narrow"]["strand"].astype(np.uint64)
     if rows.ndim == 1:
         order = np.argsort(rows, kind="stable")
     else:
@@ -125,13 +126,18 @@ def test_uniq_narrow_matches_oracle(eng, k, rc, n, kw):
     recs = _genome(2000 + k, n, **kw)
     ex = ko.extract_np(recs, k, rc)
     d = eng.upload(_flat(recs))
-    for vb in (4, 8):
+    # global position of bases[0]: 0, payloads straddling 2^32, and past it (8-byte payloads only)
+    for off, vb in ((0, 4), (0, 8), ((1 << 31) - n // 2, 8), (2**32 + 3, 8), (2**47 + 5, 8)):
+        d.pos_offset = off
         s, n_other = eng.uniq_narrow(d, k, rc, val_bytes=vb)
-        wk, wv = _want_singletons(ex)
+        wk, wv = _want_singletons(ex, off)
         assert s.n == len(wk), (s.n, len(wk))
         assert first_diff(s.keys_host(), wk) == "equal"
-        assert first_diff(s.vals_host().astype(np.uint64), wv) == "equal"
+        assert first_diff(s.vals_host().astype(np.uint64), wv) == "equal", (off, vb)
         assert n_other == ex["wide"]["pos"].shape[0] // (2 if rc else 1)
+    d.pos_offset = 2**32 + 3
+    with pytest.raises(ValueError, match="val_bytes=4"):
+        eng.uniq_narrow(d, k, rc, val_bytes=4)
 
 
 @pytest.mark.parametrize("pb", [16, 24])
