@@ -28,6 +28,16 @@
  *   k <= 32 : 128-bit {lo, hi}; k <= 64 : 256-bit, four little-endian 64-bit limbs (key_bytes = 32).
  * Payload ("val") format: (global window start in the flat base buffer << 1) | strand
  *   (0 '+', 1 '-'), as uint32 (val_bytes 4) or uint64 (val_bytes 8).
+ * Strand rule (the `rc` argument of the extraction and whole-path calls):
+ *   0             : one key per valid window, the window itself (strand '+');
+ *   1             : two keys per valid window, the window ('+') and then its reverse complement ('-'),
+ *                   both with the window's coordinates (seq.py:245-282, `kmer ... -r`);
+ *   KMG_CANONICAL : one key per valid window, the smaller (in the key order above, which is the
+ *                   reference's string order) of the window and its reverse complement, with the
+ *                   window's coordinates and strand '-' exactly when the reverse complement is strictly
+ *                   smaller (a palindrome keeps '+' and counts once per occurrence, as jellyfish -C).
+ *                   A wide window's reverse complement (through d_comp16) is wide, so both stay in one stream.
+ *   Output capacities and workspaces are per key: (win_end - win_begin) * (rc == 1 ? 2 : 1).
  */
 #ifndef KMG_H_
 #define KMG_H_
@@ -47,6 +57,9 @@ extern "C" {
 #define KMG_ERR_WS (-3)     /* workspace too small */
 #define KMG_ERR_RANGE (-4)  /* size beyond what this build supports */
 #define KMG_ERR_STATE (-5)  /* device-side consistency check failed */
+
+/* `rc` value of the canonical strand rule (see "Strand rule" above) */
+#define KMG_CANONICAL 2
 
 /* LUT byte layout (one entry per input byte value, see kmg_build_lut):
  *   bit 7    : symbol not in the alphabet -> every window touching it is skipped
@@ -85,12 +98,15 @@ int kmg_ws_status(void* d_ws, void* stream);
  * d_vals_out may be NULL (val_bytes 0).  `pos_offset` is added to the window start before
  * it is stored in the payload (multi-GPU chunks).
  * d_counts[0] = number of keys emitted, d_counts[1] (narrow only) = number of windows
- * that belong to the wide stream.  Output capacity must be (win_end-win_begin)*(1+rc).
+ * that belong to the wide stream.  Output capacity: one key per window, two with rc = 1 (strand
+ * rule above; KMG_CANONICAL emits one key per window in position order).
  * d_hist_out (optional, narrow stream, k >= 4): uint64[16][256] digit histograms of the emitted
  * keys for kmg_radix_sort's pass plan over bits [0, 2k), derived from one 4-mer histogram of
  * the bases; hand it to kmg_radix_sort(d_hist_in) to skip the sort's own histogram sweep.
  * For 8-byte keys and k >= 12, rows 13..15 additionally hold the histograms of the three top
- * key bytes (bits [2k-24, 2k)), which the hybrid sort's prefix passes use. */
+ * key bytes (bits [2k-24, 2k)), which the hybrid sort's prefix passes use.  KMG_ERR_ARG with
+ * rc = KMG_CANONICAL: the 4-mer histograms describe window offsets, not canonical keys (pass NULL
+ * and let the sort run its own histogram sweep). */
 size_t kmg_extract_workspace_bytes(uint64_t n_windows);
 int kmg_extract(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
                 int wide, const uint8_t* d_lut256, const uint8_t* d_comp16, void* d_keys_out, int key_bytes,
@@ -116,14 +132,16 @@ int kmg_wide_part_table(int rna, int n_parts, uint8_t* h_table65536);
  * of keys in the range (kmg_extract_dest_counts, kmg_extract_wide_part_counts).  d_wide_parts: device
  * copy of kmg_wide_part_table's table (required for wide = 1).  d_hist_out must be NULL (KMG_ERR_ARG):
  * the 4-mer-derived histograms describe every key, not the kept ones.  Workspace:
- * kmg_extract_workspace_bytes(win_end - win_begin). */
+ * kmg_extract_workspace_bytes(win_end - win_begin).  `rc` as in kmg_extract (the strand rule above); a
+ * canonical key's part is that of the canonical key. */
 int kmg_extract_parts(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
                       int wide, const uint8_t* d_lut256, const uint8_t* d_comp16, int n_parts, int part_lo, int part_hi,
                       const uint8_t* d_wide_parts, void* d_keys_out, int key_bytes, void* d_vals_out, int val_bytes,
                       uint64_t pos_offset, uint64_t* d_counts, uint64_t* d_hist_out, void* d_ws, size_t ws_bytes,
                       void* stream);
 /* Keys of the wide stream per part (count-only launch of the filtered wide extraction, k >= 4):
- * d_counts[0..n_parts).  d_comp16 is required with rc (the '-' key has its own part). */
+ * d_counts[0..n_parts).  d_comp16 is required with rc = 1 (the '-' key has its own part) and with
+ * rc = KMG_CANONICAL (the part of the smaller key). */
 int kmg_extract_wide_part_counts(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k,
                                  int rc, const uint8_t* d_lut256, const uint8_t* d_comp16, int n_parts,
                                  const uint8_t* d_wide_parts, uint64_t* d_counts, void* stream);
@@ -222,7 +240,9 @@ int kmg_count_histogram(const uint32_t* d_counts, uint64_t n, uint64_t* d_hist, 
  * yields the histograms of the top key bytes, then every key is written once, straight into the region
  * of its digit -- the keys are never stored in extraction order.  Two host synchronisations per call
  * (32 + 56 bytes read back).
- * d_keys / d_keys_alt (and d_vals / d_vals_alt): capacity (win_end-win_begin)*(1+rc) items each.
+ * `rc`: the strand rule above (0, 1 or KMG_CANONICAL) for all four calls and both workspace queries.
+ * d_keys / d_keys_alt (and d_vals / d_vals_alt): capacity (win_end-win_begin) items each, twice that
+ * with rc = 1.
  * h_result[4] (host): [0] rows of the result ((k-mer, count) pairs / singletons), [1] keys that were
  * sorted, [2] windows that belong to the WIDE stream (the caller runs those through the stage
  * API), [3] selector: 0 = result keys in d_keys (payload in d_vals), 1 = in the alt buffers.
@@ -268,7 +288,8 @@ int kmg_range_partition(const void* d_keys, const void* d_vals, uint64_t n, int 
  * count_only != 0 nothing is written: d_counts[0..n_parts) receives the number of keys per
  * destination and d_counts[n_parts] the number of windows that belong to the wide stream.
  * As in kmg_extract, val_bytes = 4 with ((pos_offset + n_bases) << 1) >= 2^32 is KMG_ERR_RANGE (the
- * payload would not hold the position); this holds for all three kmg_extract_scatter* calls. */
+ * payload would not hold the position); this holds for all three kmg_extract_scatter* calls.
+ * rc must be 0 or 1 in all three: rc = KMG_CANONICAL is KMG_ERR_ARG. */
 int kmg_extract_scatter(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
                         const uint8_t* d_lut256, int n_parts, void* const* d_dest_keys, void* const* d_dest_vals,
                         int key_bytes, int val_bytes, uint64_t pos_offset, uint64_t* d_cursors, uint64_t* d_counts,
@@ -294,7 +315,8 @@ int kmg_extract_scatter_checked(const uint8_t* d_bases, uint64_t n_bases, uint64
 /* What kmg_extract_scatter's count-only launch computes, from the 4-mer histogram of the BASES instead
  * of a second key-building pass (power-of-two n_parts <= 256, k >= 12): the top log2(n_parts) bits of a
  * key are its first bases.  d_counts[0..n_parts) keys per destination, d_counts[n_parts] windows of
- * the wide stream. */
+ * the wide stream.  With rc = KMG_CANONICAL the counts are those of the canonical keys (the top byte of
+ * the smaller key is the smaller of the two top bytes; one count per window). */
 size_t kmg_dest_counts_workspace_bytes(void);
 int kmg_extract_dest_counts(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
                             const uint8_t* d_lut256, int n_parts, uint64_t* d_counts, void* d_ws, size_t ws_bytes,
@@ -383,7 +405,7 @@ int kmg_sort256(const void* d_keys, void* d_keys_out, const void* d_vals, void* 
  * h_bases is the flat buffer (records joined by '\n'), narrow stream only: the call
  * fails with KMG_ERR_STATE if the input holds wide windows (use the stage API then).
  * count: h_keys_out/h_counts_out capacity `cap` entries; *h_n_out = number of distinct
- * k-mers.  uniq: singletons with payload. */
+ * k-mers.  uniq: singletons with payload.  `rc`: the strand rule above (0, 1 or KMG_CANONICAL). */
 typedef struct kmg_ctx kmg_ctx;
 int kmg_ctx_create(int device, kmg_ctx** out);
 void kmg_ctx_destroy(kmg_ctx* ctx);

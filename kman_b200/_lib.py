@@ -12,6 +12,7 @@ LIB_PATH = os.path.join(_HERE, "libkmg.so")
 KMG_OK = 0
 KMG_ERR_ARG, KMG_ERR_CUDA, KMG_ERR_WS, KMG_ERR_RANGE, KMG_ERR_STATE = -1, -2, -3, -4, -5
 KMG_HISTO_BINS = 4096  # include/kmg.h
+KMG_CANONICAL = 2  # include/kmg.h: `rc` of the canonical strand rule
 
 u8p = C.POINTER(C.c_uint8)
 u32p = C.POINTER(C.c_uint32)

@@ -231,20 +231,24 @@ class BatchAppendable(Batch):
 class DeviceBatch:
     """All k-mers of one FASTA input, resident on the GPU.
 
-    Holds the flat base buffer in HBM plus (k, reverse, alphabet).  Extraction and sorting are
+    Holds the flat base buffer in HBM plus (k, reverse, canonical, alphabet).  Extraction and sorting are
     run lazily by whoever needs them: `KJoiner.join` asks for key-only sorted streams in count
     mode and for keys + coordinates in uniq mode; `record_gen` / `sorted` / `write` decode
-    records for callers that want the reference's record view."""
+    records for callers that want the reference's record view.  `canonical`: one k-mer per window, the
+    smaller of it and its reverse complement (`--canonical`; never together with `reverse`)."""
 
     isFasta = True
     suffix = ".fa"
 
     def __init__(self, engine, device_input, k: int, reverse: bool, natype: NATYPES, tmp_dir: str,
-                 size: int = 1_000_000):
+                 size: int = 1_000_000, canonical: bool = False):
+        if canonical and reverse:
+            raise AssertionError("canonical k-mers already cover both strands: not together with reverse")
         self._eng = engine
         self.device_input = device_input
         self.k = k
         self.reverse = reverse
+        self.canonical = canonical
         self.natype = natype
         self._tmp_dir = tmp_dir
         self._size = int(size)
@@ -254,15 +258,27 @@ class DeviceBatch:
 
     type = property(lambda self: KMer)
     size = property(lambda self: max(self._size, self.current_size))
+
+    @property
+    def strand_rule(self):
+        """The engine's `rc` for this batch: engine.CANONICAL, or `reverse`."""
+        if self.canonical:
+            from kman_b200.engine import CANONICAL
+
+            return CANONICAL
+        return self.reverse
     remaining = property(lambda self: 0)
     is_written = property(lambda self: self._written)
 
     @property
     def current_size(self) -> int:
-        """Number of k-mer records (valid windows, x2 with reverse complement)."""
+        """Number of k-mer records (valid windows, x2 with reverse complement; one per window when canonical)."""
         if self._n is None:
-            n, n_other = self._eng.count_windows(self.device_input, self.k, self.reverse)
-            self._n = n + n_other * (2 if self.reverse else 1)
+            from kman_b200.engine import keys_per_window
+
+            rc = self.strand_rule
+            n, n_other = self._eng.count_windows(self.device_input, self.k, rc)
+            self._n = n + n_other * keys_per_window(rc)
         return self._n
 
     @property
@@ -282,7 +298,7 @@ class DeviceBatch:
         flat = d.flat
         streams = []
         for wide in (False, True):
-            a = self._eng.extract(d, self.k, self.reverse, wide=wide, val_bytes=8)
+            a = self._eng.extract(d, self.k, self.strand_rule, wide=wide, val_bytes=8)
             if wide is False and a.n_other == 0:
                 streams.append(a)
                 break
@@ -319,7 +335,7 @@ class DeviceBatch:
         if not self._written or force:
             if doSort:
                 with open(self.tmp, "wb") as th:
-                    self._eng.write_batch(self.device_input, self.k, self.reverse, th)
+                    self._eng.write_batch(self.device_input, self.k, self.strand_rule, th)
             else:
                 with open(self.tmp, "w+") as th:
                     for r in self._records(do_sort=False):

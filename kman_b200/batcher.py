@@ -144,10 +144,13 @@ class FastaBatcher(BatcherThreading):
 
     def __init__(self, scan_mode: "FastaBatcher.MODE" = MODE.KMERS, reverse: bool = False, threads: int = 1,
                  size: int = BatcherThreading.DEFAULT_BATCH_SIZE, natype: NATYPES = BatcherThreading.DEFAULT_NATYPE,
-                 tmp: str = tempfile.gettempdir(), alphabet: Optional[str] = None):
+                 tmp: str = tempfile.gettempdir(), alphabet: Optional[str] = None, canonical: bool = False):
         super().__init__(size, threads, natype, tmp)
         self.mode = scan_mode
         self.doReverseComplement = reverse
+        if type(canonical) is not bool or (canonical and reverse):
+            raise AssertionError("canonical is a bool and excludes reverse (canonical k-mers cover both strands)")
+        self.canonical = canonical  # one k-mer per window: the smaller of it and its reverse complement
         self.alphabet = alphabet or ab.default_alphabet()
 
     @property
@@ -184,7 +187,7 @@ class FastaBatcher(BatcherThreading):
             d = eng.load_fasta(fasta_path, self.alphabet, self.natype)  # text -> flat buffer on the GPU
         else:
             d = eng.upload(fasta.read_fasta(fasta_path), self.alphabet, self.natype)
-        batch = DeviceBatch(eng, d, k, self.doReverseComplement, self.natype, self.tmp, self.size)
+        batch = DeviceBatch(eng, d, k, self.doReverseComplement, self.natype, self.tmp, self.size, self.canonical)
         self.feed_collection([batch], feedMode)
         return self
 

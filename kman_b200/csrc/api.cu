@@ -279,7 +279,7 @@ static int run_host(kmg_ctx* c, int mode, const uint8_t* h_bases, uint64_t n_bas
     const int vb = mode == 1 ? 8 : 0;
     const uint64_t n_win = n_bases >= (uint64_t)k ? n_bases - k + 1 : 0;
     if (n_win == 0) return KMG_OK;
-    const uint64_t n_max = n_win * (rc ? 2 : 1);
+    const uint64_t n_max = n_win * keys_per_window(rc);
     const size_t ws_bytes = kmg_pipeline_workspace_bytes(n_win, k, rc, vb);
 
     Carver cv{nullptr, 0};

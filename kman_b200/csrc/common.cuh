@@ -115,6 +115,11 @@ size_t top_hist_workspace_bytes();
 int extract_top_hist(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
                      const uint8_t* d_lut256, uint64_t* d_counts, unsigned long long* d_top, unsigned long long* d_plan,
                      void* d_ws, size_t ws_bytes, cudaStream_t st);
+// histogram of the canonical keys' top byte (d_top_row[256]) and d_counts = valid narrow windows, wide-stream
+// windows, both zeroed by the call (12 <= k <= 64)
+int extract_canonical_top(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k,
+                          const uint8_t* d_lut256, unsigned long long* d_top_row, unsigned long long* d_counts,
+                          cudaStream_t st);
 // Pre-pass of the fused pipeline (histogram of the top 16 key bits over the valid narrow windows).
 // `zeroed` = spill [65536] | top [3][256] | plan [4], zeroed by the call; plan = keys, largest top-byte
 // count, valid narrow windows, wide-stream windows.
@@ -158,6 +163,10 @@ extern thread_local int64_t g_stat_last_n_out, g_stat_last_err;
 // 2 histogram pre-pass, 3 fused extraction pass)
 void timing_begin(cudaStream_t st);
 void timing_end(cudaStream_t st, int kind);
+
+// keys an extraction emits per valid window under the strand rule `rc` (kmg.h): two with the reverse
+// complement beside every key, one forward-only or canonical
+__host__ __device__ constexpr int keys_per_window(int rc) { return rc == KMG_CANONICAL ? 1 : (rc ? 2 : 1); }
 
 // ---- 128-bit key ------------------------------------------------------------------------
 struct __align__(16) u128 {

@@ -254,6 +254,7 @@ static int scatter_impl(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_b
                         int count_only, uint64_t* const* d_cursor_ptrs, uint64_t capacity, uint32_t* d_status,
                         void* stream) {
     cudaStream_t st = (cudaStream_t)stream;
+    KMG_REQUIRE(rc != KMG_CANONICAL, KMG_ERR_ARG, "the multi-GPU exchange has no canonical keys (rc must be 0 or 1)");
     KMG_REQUIRE(k >= 8, KMG_ERR_RANGE, "the multi-GPU range partition needs k >= 8 (16 key bits), got %d", k);
     KMG_REQUIRE(k <= 64, KMG_ERR_RANGE, "k=%d: this build supports k <= 64", k);
     KMG_REQUIRE(n_parts >= 1 && n_parts <= DX_MAX_PARTS, KMG_ERR_ARG, "n_parts must be in [1,%d]", DX_MAX_PARTS);

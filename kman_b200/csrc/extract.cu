@@ -127,14 +127,18 @@ struct DigitRuns {
 //         keys never make the extra round trip through HBM in extraction order.
 // FILTER (MODE 0 only): keep only the keys whose part lies in [p.part_lo, p.part_hi)
 // (kmg_extract_parts); the tile counts kept keys instead of valid windows, order is unchanged.
-template <typename KeyT, int PPT, bool RC, int VAL_BYTES, bool HIST, int MODE, int EX_BLOCK, bool FILTER = false>
+// STRAND (ST_FWD, ST_BOTH, ST_CANON): the strand rule; ST_CANON emits the canonical key of every window
+// with its strand bit in the payload (no digit histograms: they describe window offsets).
+template <typename KeyT, int PPT, int STRAND, int VAL_BYTES, bool HIST, int MODE, int EX_BLOCK, bool FILTER = false>
 __global__ void __launch_bounds__(EX_BLOCK) extract_narrow_kernel(const ExtractParams p) {
     static_assert(MODE != 1 || HIST, "the pre-pass exists for its histograms");
     static_assert(MODE != 2 || !HIST, "the fused pass takes its histograms from the pre-pass");
     static_assert(!FILTER || (MODE == 0 && !HIST), "the range filter is a variant of the position-ordered extraction");
+    static_assert(STRAND != ST_CANON || !HIST, "the 4-mer histograms do not describe canonical keys");
+    constexpr bool RC = STRAND == ST_BOTH;
     constexpr int TILE = EX_BLOCK * PPT;
     constexpr int WORDS = TILE / 16 + EX_HALO_WORDS;
-    constexpr int OUT_PER_WIN = RC ? 2 : 1;
+    constexpr int OUT_PER_WIN = keys_per_window(STRAND);
     using ValT = typename std::conditional<VAL_BYTES == 4, uint32_t, uint64_t>::type;
 
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -199,7 +203,8 @@ __global__ void __launch_bounds__(EX_BLOCK) extract_narrow_kernel(const ExtractP
 #pragma unroll
         for (int j = 0; j < PPT; ++j) {
             if (!(vf & (1u << j))) continue;
-            const KeyT key = build_key<KeyT>(X0, X1, X2, joff + j, k);
+            uint32_t sd;
+            const KeyT key = window_key<STRAND, KeyT>(X0, X1, X2, joff + j, k, sd);
             if (in_parts(key_digit(key, p.part_shift, p.part_mask), p)) kf |= 1u << (j * OUT_PER_WIN);
             if constexpr (RC) {
                 if (in_parts(key_digit(rc_key(key, k), p.part_shift, p.part_mask), p)) kf |= 1u << (j * 2 + 1);
@@ -270,7 +275,8 @@ __global__ void __launch_bounds__(EX_BLOCK) extract_narrow_kernel(const ExtractP
 #pragma unroll
         for (int j = 0; j < PPT; ++j) {
             if (!(vf & (1u << j))) continue;
-            const KeyT key = build_key<KeyT>(X0, X1, X2, joff + j, k);
+            uint32_t sd;
+            const KeyT key = window_key<STRAND, KeyT>(X0, X1, X2, joff + j, k, sd);
             wh[j * OUT_PER_WIN] = runs.rank(key_digit(key, dsh, 255u));
             if constexpr (RC) wh[j * 2 + 1] = runs.rank(key_digit(rc_key(key, k), dsh, 255u));
         }
@@ -279,11 +285,12 @@ __global__ void __launch_bounds__(EX_BLOCK) extract_narrow_kernel(const ExtractP
 #pragma unroll
         for (int j = 0; j < PPT; ++j) {
             if (!(vf & (1u << j))) continue;
-            const KeyT key = build_key<KeyT>(X0, X1, X2, joff + j, k);
+            uint32_t sd;
+            const KeyT key = window_key<STRAND, KeyT>(X0, X1, X2, joff + j, k, sd);
             const uint64_t pos = tile_pos + (uint64_t)t * PPT + j + p.pos_offset;
             const uint32_t i0 = runs.slot(wh[j * OUT_PER_WIN]);
             s_keys[i0] = key;
-            if constexpr (VAL_BYTES != 0) s_vals[i0] = make_val<ValT>(pos, 0);
+            if constexpr (VAL_BYTES != 0) s_vals[i0] = make_val<ValT>(pos, sd);
             if constexpr (RC) {
                 const uint32_t i1 = runs.slot(wh[j * 2 + 1]);
                 s_keys[i1] = rc_key(key, k);
@@ -301,12 +308,13 @@ __global__ void __launch_bounds__(EX_BLOCK) extract_narrow_kernel(const ExtractP
 #pragma unroll
     for (int j = 0; j < PPT; ++j) {
         if (!(vf & (1u << j))) continue;
-        const KeyT key = build_key<KeyT>(X0, X1, X2, joff + j, k);
+        uint32_t sd;
+        const KeyT key = window_key<STRAND, KeyT>(X0, X1, X2, joff + j, k, sd);
         const uint64_t pos = tile_pos + (uint64_t)t * PPT + j + p.pos_offset;
         if constexpr (FILTER) {
             if ((kf >> (j * OUT_PER_WIN)) & 1u) {
                 s_keys[pad_idx<KB>(r)] = key;
-                if constexpr (VAL_BYTES != 0) s_vals[pad_idx<VB>(r)] = make_val<ValT>(pos, 0);
+                if constexpr (VAL_BYTES != 0) s_vals[pad_idx<VB>(r)] = make_val<ValT>(pos, sd);
                 ++r;
             }
             if constexpr (RC) {
@@ -319,7 +327,7 @@ __global__ void __launch_bounds__(EX_BLOCK) extract_narrow_kernel(const ExtractP
             continue;
         }
         s_keys[pad_idx<KB>(r * OUT_PER_WIN)] = key;
-        if constexpr (VAL_BYTES != 0) s_vals[pad_idx<VB>(r * OUT_PER_WIN)] = make_val<ValT>(pos, 0);
+        if constexpr (VAL_BYTES != 0) s_vals[pad_idx<VB>(r * OUT_PER_WIN)] = make_val<ValT>(pos, sd);
         if constexpr (RC) {
             s_keys[pad_idx<KB>(r * 2 + 1)] = rc_key(key, k);
             if constexpr (VAL_BYTES != 0) s_vals[pad_idx<VB>(r * 2 + 1)] = make_val<ValT>(pos, 1);
@@ -371,6 +379,13 @@ struct WideKey {
     }
     __device__ __forceinline__ void set_nibble(int q, uint32_t c) { w[q >> 4] |= (uint64_t)c << (4 * (q & 15)); }
 };
+template <int LIMBS>
+__device__ __forceinline__ bool operator<(const WideKey<LIMBS>& a, const WideKey<LIMBS>& b) {
+#pragma unroll
+    for (int i = LIMBS - 1; i > 0; --i)
+        if (a.w[i] != b.w[i]) return a.w[i] < b.w[i];
+    return a.w[0] < b.w[0];
+}
 
 // first 4 symbols of a wide key (its top 16 bits; k >= 4)
 template <int LIMBS>
@@ -388,12 +403,14 @@ __device__ __forceinline__ uint32_t wide_top16(const WideKey<LIMBS>& key, int k)
 
 // FILTER 0: every wide key (kmg_extract).  1: only keys whose part lies in [p.part_lo, p.part_hi),
 // position order as in 0 (kmg_extract_parts).  2: count-only, keys per part into p.part_counts
-// (kmg_extract_wide_part_counts; p.part_hi = n_parts).
-template <bool RC, int VAL_BYTES, int LIMBS, int FILTER = 0>
+// (kmg_extract_wide_part_counts; p.part_hi = n_parts).  STRAND: the strand rule, as in extract_narrow_kernel
+// (ST_CANON: every window's key is replaced by the smaller of it and its reverse complement up front).
+template <int STRAND, int VAL_BYTES, int LIMBS, int FILTER = 0>
 __global__ void __launch_bounds__(EXW_BLOCK) extract_wide_kernel(const ExtractParams p) {
     using ValT = typename std::conditional<VAL_BYTES == 4, uint32_t, uint64_t>::type;
     using KeyT = WideKey<LIMBS>;  // same layout as u128 / u256
-    constexpr int OUT_PER_WIN = RC ? 2 : 1;
+    constexpr bool RC = STRAND == ST_BOTH;
+    constexpr int OUT_PER_WIN = keys_per_window(STRAND);
     __shared__ uint8_t s_e[EXW_TILE + 64];  // LUT entries of the tile bytes (+ halo: k <= 64)
     __shared__ uint8_t s_lut[256];
     __shared__ uint8_t s_comp[16];
@@ -444,6 +461,18 @@ __global__ void __launch_bounds__(EXW_BLOCK) extract_wide_kernel(const ExtractPa
         for (int q = k - 1; q >= 0; --q) rcv.set_nibble(q, s_comp[f.pop()]);
         return rcv;
     };
+    uint32_t sb = 0;  // ST_CANON: bit j set when window j's reverse complement is strictly smaller
+    if constexpr (STRAND == ST_CANON) {
+#pragma unroll
+        for (int j = 0; j < EXW_PPT; ++j) {
+            if (!(vf & (1u << j))) continue;
+            const KeyT r = make_rc(keys[j]);
+            if (r < keys[j]) {
+                keys[j] = r;
+                sb |= 1u << j;
+            }
+        }
+    }
     if constexpr (FILTER != 0) {
         // bit 2j: key of window j kept, bit 2j+1: its reverse complement kept
         KeyT rcs[RC ? EXW_PPT : 1];
@@ -481,7 +510,7 @@ __global__ void __launch_bounds__(EXW_BLOCK) extract_wide_kernel(const ExtractPa
             const uint64_t pos = tile_pos + t * EXW_PPT + j + p.pos_offset;
             if ((kf >> (2 * j)) & 1u) {
                 keys_out[r] = keys[j];
-                if constexpr (VAL_BYTES != 0) vals_out[r] = make_val<ValT>(pos, 0);
+                if constexpr (VAL_BYTES != 0) vals_out[r] = make_val<ValT>(pos, (sb >> j) & 1u);
                 ++r;
             }
             if constexpr (RC) {
@@ -512,7 +541,7 @@ __global__ void __launch_bounds__(EXW_BLOCK) extract_wide_kernel(const ExtractPa
         if (!(vf & (1u << j))) continue;
         const uint64_t pos = tile_pos + t * EXW_PPT + j + p.pos_offset;
         keys_out[r] = keys[j];
-        if constexpr (VAL_BYTES != 0) vals_out[r] = make_val<ValT>(pos, 0);
+        if constexpr (VAL_BYTES != 0) vals_out[r] = make_val<ValT>(pos, (sb >> j) & 1u);
         ++r;
         if constexpr (RC) {
             keys_out[r] = make_rc(keys[j]);
@@ -523,15 +552,15 @@ __global__ void __launch_bounds__(EXW_BLOCK) extract_wide_kernel(const ExtractPa
     if (t == 0 && tile == gridDim.x - 1) p.counts[0] = base + (uint64_t)total * OUT_PER_WIN;
 }
 
-template <typename KeyT, int PPT, bool RC, int VB, bool HIST, int MODE = 0, int BLOCK = EX_BLOCK_DEFAULT, bool FILTER = false>
+template <typename KeyT, int PPT, int STRAND, int VB, bool HIST, int MODE = 0, int BLOCK = EX_BLOCK_DEFAULT, bool FILTER = false>
 static int launch_narrow(const ExtractParams& p, uint32_t n_tiles, cudaStream_t st) {
     constexpr int TILE = BLOCK * PPT;
-    constexpr uint32_t STAGE = TILE * (RC ? 2 : 1);
+    constexpr uint32_t STAGE = TILE * keys_per_window(STRAND);
     constexpr uint32_t STAGE_PAD = STAGE + STAGE / 8 + 8;
     // (the pre-pass stages no keys: its dynamic shared memory only holds the correction tables)
     const size_t smem = MODE == 1 ? (size_t)8 * 256 * sizeof(uint32_t)
                                   : (sizeof(KeyT) + (VB == 4 ? 4 : (VB == 8 ? 8 : 0))) * (size_t)STAGE_PAD;
-    auto kern = extract_narrow_kernel<KeyT, PPT, RC, VB, HIST, MODE, BLOCK, FILTER>;
+    auto kern = extract_narrow_kernel<KeyT, PPT, STRAND, VB, HIST, MODE, BLOCK, FILTER>;
     KMG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<n_tiles, BLOCK, smem, st>>>(p);
     KMG_LAUNCH_CHECK();
@@ -541,14 +570,21 @@ static int launch_narrow(const ExtractParams& p, uint32_t n_tiles, cudaStream_t 
 template <typename KeyT, int PPT, bool HIST, bool FILTER = false>
 static int dispatch_narrow2(const ExtractParams& p, uint32_t n_tiles, int rc, int vb, cudaStream_t st) {
     constexpr int B = EX_BLOCK_DEFAULT;
-    if (rc) {
-        if (vb == 0) return launch_narrow<KeyT, PPT, true, 0, HIST, 0, B, FILTER>(p, n_tiles, st);
-        if (vb == 4) return launch_narrow<KeyT, PPT, true, 4, HIST, 0, B, FILTER>(p, n_tiles, st);
-        return launch_narrow<KeyT, PPT, true, 8, HIST, 0, B, FILTER>(p, n_tiles, st);
+    if constexpr (!HIST) {  // (extract_impl rejects canonical keys with histograms)
+        if (rc == ST_CANON) {
+            if (vb == 0) return launch_narrow<KeyT, PPT, ST_CANON, 0, HIST, 0, B, FILTER>(p, n_tiles, st);
+            if (vb == 4) return launch_narrow<KeyT, PPT, ST_CANON, 4, HIST, 0, B, FILTER>(p, n_tiles, st);
+            return launch_narrow<KeyT, PPT, ST_CANON, 8, HIST, 0, B, FILTER>(p, n_tiles, st);
+        }
     }
-    if (vb == 0) return launch_narrow<KeyT, PPT, false, 0, HIST, 0, B, FILTER>(p, n_tiles, st);
-    if (vb == 4) return launch_narrow<KeyT, PPT, false, 4, HIST, 0, B, FILTER>(p, n_tiles, st);
-    return launch_narrow<KeyT, PPT, false, 8, HIST, 0, B, FILTER>(p, n_tiles, st);
+    if (rc) {
+        if (vb == 0) return launch_narrow<KeyT, PPT, ST_BOTH, 0, HIST, 0, B, FILTER>(p, n_tiles, st);
+        if (vb == 4) return launch_narrow<KeyT, PPT, ST_BOTH, 4, HIST, 0, B, FILTER>(p, n_tiles, st);
+        return launch_narrow<KeyT, PPT, ST_BOTH, 8, HIST, 0, B, FILTER>(p, n_tiles, st);
+    }
+    if (vb == 0) return launch_narrow<KeyT, PPT, ST_FWD, 0, HIST, 0, B, FILTER>(p, n_tiles, st);
+    if (vb == 4) return launch_narrow<KeyT, PPT, ST_FWD, 4, HIST, 0, B, FILTER>(p, n_tiles, st);
+    return launch_narrow<KeyT, PPT, ST_FWD, 8, HIST, 0, B, FILTER>(p, n_tiles, st);
 }
 template <typename KeyT, int PPT>
 static int dispatch_narrow(const ExtractParams& p, uint32_t n_tiles, int rc, int vb, bool hist, cudaStream_t st) {
@@ -556,19 +592,24 @@ static int dispatch_narrow(const ExtractParams& p, uint32_t n_tiles, int rc, int
                 : dispatch_narrow2<KeyT, PPT, false>(p, n_tiles, rc, vb, st);
 }
 
-// fused first prefix pass (MODE 2).  Key-only forward extraction stages 8192 keys per tile in 512
-// threads (digit runs of ~32 keys = 256 bytes); with payload or reverse complements 256 threads
+// fused first prefix pass (MODE 2).  Key-only forward or canonical extraction stages 8192 keys per tile
+// in 512 threads (digit runs of ~32 keys = 256 bytes); with payload or reverse complements 256 threads
 // keep the staging buffer at 64 KB.
 template <typename KeyT, int PPT>
 static int dispatch_scatter_digit(const ExtractParams& p, uint64_t n_win_tiles_256, int rc, int vb, cudaStream_t st) {
     const uint32_t t256 = (uint32_t)n_win_tiles_256;
-    if (rc) {
-        if (vb == 0) return launch_narrow<KeyT, PPT, true, 0, false, 2, 256>(p, t256, st);
-        if (vb == 4) return launch_narrow<KeyT, PPT, true, 4, false, 2, 256>(p, t256, st);
-        return launch_narrow<KeyT, PPT, true, 8, false, 2, 256>(p, t256, st);
+    if (rc == ST_CANON) {
+        if (vb == 4) return launch_narrow<KeyT, PPT, ST_CANON, 4, false, 2, 256>(p, t256, st);
+        if (vb == 8) return launch_narrow<KeyT, PPT, ST_CANON, 8, false, 2, 256>(p, t256, st);
+        return KMG_ERR_ARG;  // (key-only canonical: 512 threads, see extract_digit_scatter)
     }
-    if (vb == 4) return launch_narrow<KeyT, PPT, false, 4, false, 2, 256>(p, t256, st);
-    if (vb == 8) return launch_narrow<KeyT, PPT, false, 8, false, 2, 256>(p, t256, st);
+    if (rc) {
+        if (vb == 0) return launch_narrow<KeyT, PPT, ST_BOTH, 0, false, 2, 256>(p, t256, st);
+        if (vb == 4) return launch_narrow<KeyT, PPT, ST_BOTH, 4, false, 2, 256>(p, t256, st);
+        return launch_narrow<KeyT, PPT, ST_BOTH, 8, false, 2, 256>(p, t256, st);
+    }
+    if (vb == 4) return launch_narrow<KeyT, PPT, ST_FWD, 4, false, 2, 256>(p, t256, st);
+    if (vb == 8) return launch_narrow<KeyT, PPT, ST_FWD, 8, false, 2, 256>(p, t256, st);
     return KMG_ERR_ARG;  // (key-only forward: 512 threads, see extract_digit_scatter)
 }
 
@@ -739,8 +780,11 @@ __device__ __forceinline__ void count16(uint32_t* s_h, unsigned long long* spill
     }
 }
 
-template <bool RC>
+// STRAND: the strand rule.  ST_CANON needs no key either: a prefix is monotone in the key, so the top bits of
+// the smaller key are the smaller of the two keys' top bits -- one count16 per window, as forward-only.
+template <int STRAND>
 __global__ void __launch_bounds__(P16_BLOCK, 1) prefix16_hist_kernel(const Prefix16Params p) {
+    constexpr bool RC = STRAND == ST_BOTH;
     constexpr int WORDS = (int)(P16_TILE / 16) + EX_HALO_WORDS;
     extern __shared__ __align__(16) uint32_t s_h[];  // [P16_WORDS]: counter b is half (b & 1) of word b >> 1
     __shared__ uint32_t s_codes[WORDS];
@@ -773,6 +817,16 @@ __global__ void __launch_bounds__(P16_BLOCK, 1) prefix16_hist_kernel(const Prefi
 #pragma unroll
         for (int j = 0; j < P16_PPT; ++j) {
             if (!(vf & (1u << j))) continue;
+            if constexpr (STRAND == ST_CANON) {
+                // 16-bit prefixes of the key (8-mer at 0) and of its rc (rc of the 8-mer at k-8); byte 3 = the
+                // low byte of the smaller 24-bit prefix (fwd: + 4-mer at 8, rc: + rc of the 4-mer at k-12)
+                const uint32_t f8 = mer8_at(X0, X1, X2, j), r8 = rc8(mer8_at(X0, X1, X2, j + k - 8));
+                count16(s_h, p.spill, min(f8, r8));
+                const uint32_t f12 = (f8 << 8) | mer4_at(X0, X1, X2, j + 8);
+                const uint32_t r12 = (r8 << 8) | rc4(mer4_at(X0, X1, X2, j + k - 12));
+                atomicAdd(&s_b3[min(f12, r12) & 0xFFu], 1u);
+                continue;
+            }
             count16(s_h, p.spill, mer8_at(X0, X1, X2, j));
             atomicAdd(&s_b3[mer4_at(X0, X1, X2, j + 8)], 1u);
             if constexpr (RC) {
@@ -952,19 +1006,21 @@ static int launch_region_partition(const RegionPartParams& p, uint64_t n, cudaSt
     return KMG_OK;
 }
 
-template <bool RC, int LIMBS, int FILTER = 0>
+template <int STRAND, int LIMBS, int FILTER = 0>
 static int dispatch_wide(const ExtractParams& p, uint32_t n_tiles, int vb, cudaStream_t st) {
-    if (vb == 0) extract_wide_kernel<RC, 0, LIMBS, FILTER><<<n_tiles, EXW_BLOCK, 0, st>>>(p);
-    else if (vb == 4) extract_wide_kernel<RC, 4, LIMBS, FILTER><<<n_tiles, EXW_BLOCK, 0, st>>>(p);
-    else extract_wide_kernel<RC, 8, LIMBS, FILTER><<<n_tiles, EXW_BLOCK, 0, st>>>(p);
+    if (vb == 0) extract_wide_kernel<STRAND, 0, LIMBS, FILTER><<<n_tiles, EXW_BLOCK, 0, st>>>(p);
+    else if (vb == 4) extract_wide_kernel<STRAND, 4, LIMBS, FILTER><<<n_tiles, EXW_BLOCK, 0, st>>>(p);
+    else extract_wide_kernel<STRAND, 8, LIMBS, FILTER><<<n_tiles, EXW_BLOCK, 0, st>>>(p);
     KMG_LAUNCH_CHECK();
     return KMG_OK;
 }
 // FILTER 2 stores nothing: the payload width does not matter
 template <int FILTER>
 static int dispatch_wide_any(const ExtractParams& p, uint32_t n_tiles, int k, int rc, int vb, cudaStream_t st) {
-    if (k <= 32) return rc ? dispatch_wide<true, 2, FILTER>(p, n_tiles, vb, st) : dispatch_wide<false, 2, FILTER>(p, n_tiles, vb, st);
-    return rc ? dispatch_wide<true, 4, FILTER>(p, n_tiles, vb, st) : dispatch_wide<false, 4, FILTER>(p, n_tiles, vb, st);
+    if (rc == ST_CANON) return k <= 32 ? dispatch_wide<ST_CANON, 2, FILTER>(p, n_tiles, vb, st)
+                                       : dispatch_wide<ST_CANON, 4, FILTER>(p, n_tiles, vb, st);
+    if (k <= 32) return rc ? dispatch_wide<ST_BOTH, 2, FILTER>(p, n_tiles, vb, st) : dispatch_wide<ST_FWD, 2, FILTER>(p, n_tiles, vb, st);
+    return rc ? dispatch_wide<ST_BOTH, 4, FILTER>(p, n_tiles, vb, st) : dispatch_wide<ST_FWD, 4, FILTER>(p, n_tiles, vb, st);
 }
 
 static void fill_common(ExtractParams& p, const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end,
@@ -1009,7 +1065,7 @@ int extract_top_hist(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begi
         KMG_REQUIRE(n_tiles < (1ull << 31), KMG_ERR_RANGE, "too many tiles");
         // (the histograms do not depend on the key width; one window per lane and 16 per thread
         // span at most 79 bases, which the 96-base code words cover for every k <= 64)
-        const int rcode = launch_narrow<uint64_t, 16, false, 0, true, 1, EX_BLOCK_DEFAULT>(p, (uint32_t)n_tiles, st);
+        const int rcode = launch_narrow<uint64_t, 16, ST_FWD, 0, true, 1, EX_BLOCK_DEFAULT>(p, (uint32_t)n_tiles, st);
         if (rcode != KMG_OK) return rcode;
         hist_edges_kernel<<<1, 256, 0, st>>>(p);
         KMG_LAUNCH_CHECK();
@@ -1019,12 +1075,79 @@ int extract_top_hist(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begi
     return KMG_OK;
 }
 
+// Top-byte histogram of the canonical keys (kmg_extract_dest_counts with rc = KMG_CANONICAL).  The 4-mer shift
+// trick of extract_top_hist does not describe the smaller of two keys, but the top byte of the smaller key is
+// the smaller of the two top bytes: one shared atomic per window on min(4-mer at 0, rc4(4-mer at k-4)).
+constexpr int CT_BLOCK = 256;
+constexpr int CT_PPT = 16;  // one 16-base word per thread, as in prefix16_hist_kernel
+
+__global__ void __launch_bounds__(CT_BLOCK) canonical_top_kernel(const ExtractParams p) {
+    constexpr int TILE = CT_BLOCK * CT_PPT;
+    constexpr int WORDS = TILE / 16 + EX_HALO_WORDS;
+    __shared__ uint32_t s_codes[WORDS];
+    __shared__ uint16_t s_bad[WORDS];
+    __shared__ uint16_t s_inv[WORDS];
+    __shared__ uint8_t s_lut[256];
+    __shared__ uint32_t s_top[256];
+    __shared__ uint32_t s_n[2];
+    const int t = threadIdx.x;
+    s_lut[t] = p.lut[t];
+    s_top[t] = 0;
+    if (t < 2) s_n[t] = 0;
+    __syncthreads();
+    const uint64_t tile_pos = (p.first_tile + blockIdx.x) * (uint64_t)TILE;
+    encode_tile_words<CT_BLOCK, WORDS>(p.bases, p.n_bases, t, tile_pos, s_lut, s_codes, s_bad, s_inv);
+    __syncthreads();
+    const int k = p.k;
+    const auto [X0, X1, X2, B0, B1, I0, I1] = load_tile_words(s_codes, s_bad, s_inv, t);
+    uint32_t in_range_mask, nwide;
+    bool span_clean;
+    const uint32_t vf = narrow_window_flags<CT_PPT>(tile_pos + (uint64_t)t * CT_PPT, p.win_begin, p.win_end, k, 0, B0, B1,
+                                                    I0, I1, in_range_mask, span_clean, nwide);
+#pragma unroll
+    for (int j = 0; j < CT_PPT; ++j)
+        if (vf & (1u << j)) atomicAdd(&s_top[min(mer4_at(X0, X1, X2, j), rc4(mer4_at(X0, X1, X2, j + k - 4)))], 1u);
+    uint32_t n_valid = __popc(vf);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        n_valid += __shfl_xor_sync(0xffffffffu, n_valid, o);
+        nwide += __shfl_xor_sync(0xffffffffu, nwide, o);
+    }
+    if ((t & 31) == 0) {
+        if (n_valid) atomicAdd(&s_n[0], n_valid);
+        if (nwide) atomicAdd(&s_n[1], nwide);
+    }
+    __syncthreads();
+    if (s_top[t]) atomicAdd(&p.hs[t], (unsigned long long)s_top[t]);
+    if (t < 2 && s_n[t]) atomicAdd(&p.counts[t], (unsigned long long)s_n[t]);
+}
+
+// see common.cuh
+int extract_canonical_top(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k,
+                          const uint8_t* d_lut256, unsigned long long* d_top_row, unsigned long long* d_counts,
+                          cudaStream_t st) {
+    KMG_REQUIRE(k >= 12 && k <= 64, KMG_ERR_ARG, "the top-byte histogram needs 12 <= k <= 64");
+    KMG_CUDA(cudaMemsetAsync(d_top_row, 0, 256 * sizeof(uint64_t), st));
+    KMG_CUDA(cudaMemsetAsync(d_counts, 0, 2 * sizeof(uint64_t), st));
+    if (win_end == win_begin) return KMG_OK;
+    constexpr uint64_t TILE = (uint64_t)CT_BLOCK * CT_PPT;
+    ExtractParams p;
+    fill_common(p, d_bases, n_bases, win_begin, win_end, TILE, k, d_lut256);
+    p.hs = d_top_row;
+    p.counts = d_counts;
+    const uint64_t n_tiles = (win_end + TILE - 1) / TILE - p.first_tile;
+    KMG_REQUIRE(n_tiles < (1ull << 31), KMG_ERR_RANGE, "too many tiles");
+    canonical_top_kernel<<<(uint32_t)n_tiles, CT_BLOCK, 0, st>>>(p);
+    KMG_LAUNCH_CHECK();
+    return KMG_OK;
+}
+
 int extract_digit_scatter(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
                           const uint8_t* d_lut256, void* d_keys_out, int key_bytes, void* d_vals_out, int val_bytes,
                           uint64_t pos_offset, unsigned long long* d_cursors, int digit_shift, cudaStream_t st) {
     if (win_end == win_begin) return KMG_OK;
     const int ppt = key_bytes == 8 ? 16 : 8;
-    const bool big = !rc && val_bytes == 0;  // 512-thread tiles
+    const bool big = (!rc || rc == ST_CANON) && val_bytes == 0;  // 512-thread tiles
     const uint64_t tile = (uint64_t)(big ? 512 : 256) * ppt;
     ExtractParams p;
     fill_common(p, d_bases, n_bases, win_begin, win_end, tile, k, d_lut256);
@@ -1035,9 +1158,13 @@ int extract_digit_scatter(const uint8_t* d_bases, uint64_t n_bases, uint64_t win
     p.digit_shift = digit_shift;
     const uint64_t n_tiles = (win_end + tile - 1) / tile - p.first_tile;
     KMG_REQUIRE(n_tiles < (1ull << 31), KMG_ERR_RANGE, "too many tiles");
+    if (big && rc == ST_CANON) {
+        if (key_bytes == 8) return launch_narrow<uint64_t, 16, ST_CANON, 0, false, 2, 512>(p, (uint32_t)n_tiles, st);
+        return launch_narrow<u128, 8, ST_CANON, 0, false, 2, 512>(p, (uint32_t)n_tiles, st);
+    }
     if (big) {
-        if (key_bytes == 8) return launch_narrow<uint64_t, 16, false, 0, false, 2, 512>(p, (uint32_t)n_tiles, st);
-        return launch_narrow<u128, 8, false, 0, false, 2, 512>(p, (uint32_t)n_tiles, st);
+        if (key_bytes == 8) return launch_narrow<uint64_t, 16, ST_FWD, 0, false, 2, 512>(p, (uint32_t)n_tiles, st);
+        return launch_narrow<u128, 8, ST_FWD, 0, false, 2, 512>(p, (uint32_t)n_tiles, st);
     }
     if (key_bytes == 8) return dispatch_scatter_digit<uint64_t, 16>(p, n_tiles, rc, val_bytes, st);
     return dispatch_scatter_digit<u128, 8>(p, n_tiles, rc, val_bytes, st);
@@ -1076,7 +1203,7 @@ int extract_prefix16_hist(const uint8_t* d_bases, uint64_t n_bases, uint64_t win
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
         n_rows = (int)std::min<uint64_t>(n_tiles, (uint64_t)std::min(sms, P16_MAX_CTAS));
         const size_t smem = P16_WORDS * sizeof(uint32_t);
-        auto kern = rc ? prefix16_hist_kernel<true> : prefix16_hist_kernel<false>;
+        auto kern = rc == ST_CANON ? prefix16_hist_kernel<ST_CANON> : rc ? prefix16_hist_kernel<ST_BOTH> : prefix16_hist_kernel<ST_FWD>;
         KMG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         kern<<<n_rows, P16_BLOCK, smem, st>>>(p);
         KMG_LAUNCH_CHECK();
@@ -1154,6 +1281,8 @@ static int extract_impl(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_b
         KMG_REQUIRE(((pos_offset + n_bases) << 1) < (1ull << 32), KMG_ERR_RANGE, "val_bytes=4 needs < 2^31 positions");
     KMG_REQUIRE(ws_bytes >= kmg_extract_workspace_bytes(win_end - win_begin), KMG_ERR_WS, "extract workspace too small");
     KMG_REQUIRE(!d_hist_out || (!wide && k >= 4), KMG_ERR_ARG, "fused digit histograms need the narrow stream and k >= 4");
+    KMG_REQUIRE(!d_hist_out || rc != ST_CANON, KMG_ERR_ARG,
+                "fused digit histograms describe window offsets, not canonical keys (d_hist_out must be NULL)");
 
     KMG_CUDA(cudaMemsetAsync(d_counts, 0, 2 * sizeof(uint64_t), st));
     KMG_CUDA(cudaMemsetAsync(d_ws, 0, sizeof(WsHeader), st));
@@ -1214,10 +1343,7 @@ static int extract_impl(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_b
         }
     }
 
-    if (wide && k <= 32) return rc ? dispatch_wide<true, 2>(p, (uint32_t)n_tiles, val_bytes, st)
-                                   : dispatch_wide<false, 2>(p, (uint32_t)n_tiles, val_bytes, st);
-    if (wide) return rc ? dispatch_wide<true, 4>(p, (uint32_t)n_tiles, val_bytes, st)
-                        : dispatch_wide<false, 4>(p, (uint32_t)n_tiles, val_bytes, st);
+    if (wide) return dispatch_wide_any<0>(p, (uint32_t)n_tiles, k, rc, val_bytes, st);
     int rcode;
     if (key_bytes == 8) rcode = dispatch_narrow<uint64_t, 16>(p, (uint32_t)n_tiles, rc, val_bytes, d_hist_out != nullptr, st);
     else rcode = dispatch_narrow<u128, 8>(p, (uint32_t)n_tiles, rc, val_bytes, d_hist_out != nullptr, st);

@@ -32,6 +32,19 @@ __device__ __forceinline__ u128 rc_key(const u128& key, int k) {
     return r;
 }
 
+// Strand rule of an extraction kernel (the `rc` argument of kmg.h): the window's key only, the key and its
+// reverse complement (two keys per window), or the canonical key (one per window).
+constexpr int ST_FWD = 0, ST_BOTH = 1, ST_CANON = KMG_CANONICAL;
+
+// the canonical key: the smaller of the key and its reverse complement (integer order is the string order);
+// strand 1 when the reverse complement is strictly smaller, so a palindrome keeps strand 0
+template <typename KeyT>
+__device__ __forceinline__ KeyT canonical_key(const KeyT& key, int k, uint32_t& strand) {
+    const KeyT r = rc_key(key, k);
+    strand = r < key ? 1u : 0u;
+    return strand ? r : key;
+}
+
 template <typename ValT>
 __device__ __forceinline__ ValT make_val(uint64_t pos, uint32_t strand) {
     return (ValT)((pos << 1) | strand);
@@ -160,6 +173,16 @@ __device__ __forceinline__ KeyT build_key(uint64_t X0, uint64_t X1, uint64_t X2,
             key.hi = hi >> s;
         }
     }
+    return key;
+}
+
+// The first key of the window at base je under strand rule STRAND: the window's own key (strand 0), or with
+// ST_CANON the canonical key and its strand.
+template <int STRAND, typename KeyT>
+__device__ __forceinline__ KeyT window_key(uint64_t X0, uint64_t X1, uint64_t X2, int je, int k, uint32_t& strand) {
+    const KeyT key = build_key<KeyT>(X0, X1, X2, je, k);
+    strand = 0;
+    if constexpr (STRAND == ST_CANON) return canonical_key(key, k, strand);
     return key;
 }
 

@@ -58,7 +58,7 @@ PipeWs carve_pipe(void* ws, uint64_t n_windows, int k, int rc, int val_bytes, in
         return r;
     };
     const int kb = k <= 32 ? 8 : 16;
-    const uint64_t cap = std::max<uint64_t>(n_windows * (rc ? 2 : 1), 1);
+    const uint64_t cap = std::max<uint64_t>(n_windows * keys_per_window(rc), 1);
     w.zeroed = (unsigned long long*)take(P16_ZEROED_WORDS * sizeof(uint64_t));
     w.top = p16_top(w.zeroed);
     w.plan = p16_plan(w.zeroed);
@@ -98,7 +98,7 @@ int status_from_err(int64_t err) {
 }
 
 // mode 0: (k-mer, count) table, restricted to `range`; mode 1: singletons with payload; mode 2: the multiplicity
-// histogram, added to *histo.  h_result: [0] rows of the result, [1] keys sorted (valid narrow windows, x2 with rc),
+// histogram, added to *histo.  h_result: [0] rows of the result, [1] keys sorted (valid narrow windows, x2 with rc = 1),
 // [2] windows that belong to the wide stream, [3] selector (0: result in d_keys / d_vals, 1: in the alt
 // buffers); mode 2 has no table: [0] and [3] stay 0
 int run_pipeline(int mode, const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
@@ -125,7 +125,7 @@ int run_pipeline(int mode, const uint8_t* d_bases, uint64_t n_bases, uint64_t wi
         KMG_REQUIRE(((pos_offset + n_bases) << 1) < (1ull << 32), KMG_ERR_RANGE, "val_bytes=4 needs < 2^31 positions");
     const PipeWs w = carve_pipe(d_ws, n_win, k, rc, val_bytes, mode);
     KMG_REQUIRE(ws_bytes >= w.total, KMG_ERR_WS, "pipeline workspace too small: %zu < %zu", ws_bytes, w.total);
-    const uint64_t cap = n_win * (rc ? 2 : 1);
+    const uint64_t cap = n_win * keys_per_window(rc);
     int sel = 0;
     int rcode;
 
@@ -143,9 +143,9 @@ int run_pipeline(int mode, const uint8_t* d_bases, uint64_t n_bases, uint64_t wi
         n = h_plan[0];
         h_result[1] = n;
         h_result[2] = h_plan[3];
-        KMG_REQUIRE(h_plan[2] * (rc ? 2 : 1) == n, KMG_ERR_STATE,
+        KMG_REQUIRE(h_plan[2] * keys_per_window(rc) == n, KMG_ERR_STATE,
                     "prefix histogram (%llu keys) disagrees with the window count (%llu)", h_plan[0],
-                    h_plan[2] * (rc ? 2 : 1));
+                    h_plan[2] * keys_per_window(rc));
         if (n == 0) return KMG_OK;
         fused = hybrid_sort_applies(n, kb, val_bytes, 2 * k, true);  // (most windows skipped: small after all)
         if (fused) {
@@ -183,8 +183,9 @@ int run_pipeline(int mode, const uint8_t* d_bases, uint64_t n_bases, uint64_t wi
         }
     }
     if (!fused) {
-        // stage path: position-ordered extraction with every pass' histogram, then the sort
-        uint64_t* hist = k >= 4 ? w.hist16 : nullptr;
+        // stage path: position-ordered extraction with every pass' histogram (canonical keys: the sort's own
+        // histogram sweep), then the sort
+        uint64_t* hist = k >= 4 && rc != KMG_CANONICAL ? w.hist16 : nullptr;
         rcode = kmg_extract(d_bases, n_bases, win_begin, win_end, k, rc, 0, d_lut256, nullptr, d_keys, kb, d_vals, val_bytes,
                             pos_offset, reinterpret_cast<uint64_t*>(w.plan), hist, w.ex_ws, w.ex_ws_bytes, st);
         if (rcode != KMG_OK) return rcode;
@@ -255,8 +256,11 @@ extern "C" int kmg_extract_dest_counts(const uint8_t* d_bases, uint64_t n_bases,
     KMG_REQUIRE(win_begin <= win_end, KMG_ERR_ARG, "win_begin > win_end");
     unsigned long long* top = reinterpret_cast<unsigned long long*>((char*)d_ws + align_up(top_hist_workspace_bytes(), 256));
     unsigned long long* plan = top + 3 * 256;  // [0..1] plan, [2..3] window counts
-    const int rcode = extract_top_hist(d_bases, n_bases, win_begin, win_end, k, rc, d_lut256,
-                                       reinterpret_cast<uint64_t*>(plan + 2), top, plan, d_ws, top_hist_workspace_bytes(), st);
+    const int rcode = rc == KMG_CANONICAL
+                          ? extract_canonical_top(d_bases, n_bases, win_begin, win_end, k, d_lut256, top + 2 * 256, plan + 2, st)
+                          : extract_top_hist(d_bases, n_bases, win_begin, win_end, k, rc, d_lut256,
+                                             reinterpret_cast<uint64_t*>(plan + 2), top, plan, d_ws,
+                                             top_hist_workspace_bytes(), st);
     if (rcode != KMG_OK) return rcode;
     int g = 0;
     while ((1 << g) < n_parts) ++g;

@@ -550,7 +550,11 @@ class DistributedCounter:
 
     def count_streams(self, d, k: int, rc: bool = False, reuse: Optional[str] = "p2p_"):
         """This rank's slice (key range `rank`) of the global count table: [narrow] or [narrow, wide]
-        CountTables; rank-order concatenation per stream is globally sorted, counts are final."""
+        CountTables; rank-order concatenation per stream is globally sorted, counts are final.  rc = CANONICAL:
+        AssertionError (the exchange has no canonical keys)."""
+        from kman_b200.engine import per_strand
+
+        per_strand(rc)
         r, any_wide = self._narrow(d, k, rc, with_vals=False)
         tab = self.eng.sort_count(r, sort_bits_after_partition(r.key_bits, self.world), reuse=reuse)
         tab.keys = self._own(tab.keys, tab.n * tab.key_bytes)
@@ -567,7 +571,11 @@ class DistributedCounter:
         return self.count_streams(d, k, rc)[0]
 
     def uniq_streams(self, d, k: int, rc: bool = False):
-        """This rank's slice of the global singleton list (keys + (pos<<1|strand) payload) per stream."""
+        """This rank's slice of the global singleton list (keys + (pos<<1|strand) payload) per stream.  rc = CANONICAL:
+        AssertionError."""
+        from kman_b200.engine import per_strand
+
+        per_strand(rc)
         r, any_wide = self._narrow(d, k, rc, with_vals=True)
         s = self.eng.sort_uniq(r, sort_bits_after_partition(r.key_bits, self.world))
         s.keys, s.vals = self._own(s.keys, s.n * s.key_bytes), self._own(s.vals, s.n * s.val_bytes)

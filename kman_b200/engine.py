@@ -16,6 +16,10 @@ Stage -> reference mapping (see DESIGN.md):
                    the device, gzipped on host threads (abundance() returns the same vectors as host arrays)
   histogram()      `kmer histo`: the spectrum of count()'s count column, summed on the device pass by pass
                    (write_histogram() writes it as text)
+
+Strand rule: every method's `rc` is False / 0 (forward k-mers), True / 1 (`-r`: each k-mer and its reverse
+complement, two keys per window) or CANONICAL (`--canonical`: one key per window, the smaller of the k-mer and its
+reverse complement; see kmg.h).  Abundance vectors, batch files and the multi-GPU path take 0 / 1 only.
 """
 from __future__ import annotations
 
@@ -31,6 +35,20 @@ import torch
 
 from kman_b200 import _lib, alphabet as ab
 from kman_b200.fasta import FlatInput
+
+CANONICAL = _lib.KMG_CANONICAL  # `rc` of the canonical strand rule
+
+
+def keys_per_window(rc) -> int:
+    """Keys an extraction emits per valid window under the strand rule `rc`: 2 with `-r`, else 1."""
+    return 1 if rc == CANONICAL else (2 if rc else 1)
+
+
+def per_strand(rc) -> None:
+    """AssertionError for CANONICAL where the output is defined per strand (vectors, batch files) or the path
+    has no canonical keys (the multi-GPU exchange)."""
+    if rc == CANONICAL:
+        raise AssertionError("canonical k-mers are not available here: use rc = False / True")
 
 
 def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
@@ -517,15 +535,16 @@ class Engine:
         win_begin, win_end = window_range(d, k, win_begin, win_end)
         n_win = win_end - win_begin
         kb = key_bytes(k, wide)
-        cap = max(n_win * (2 if rc else 1), 1)
+        cap = max(n_win * keys_per_window(rc), 1)
         keys = self._out(reuse, "keys", cap * kb)
         keys_alt = self._out(reuse, "keys_alt", cap * kb)
         vals = self._out(reuse, "vals", cap * val_bytes) if val_bytes else None
         vals_alt = self._out(reuse, "vals_alt", cap * val_bytes) if val_bytes else None
         ws_bytes = self.lib.kmg_extract_workspace_bytes(n_win)
         ws = self._buf("ws_extract", ws_bytes)
-        # fused digit histograms for the sort that follows (narrow stream only)
-        hist = self._out(reuse, "hist", 16 * 256 * 8) if want_hist and not wide and k >= 4 else None
+        # fused digit histograms for the sort that follows (narrow stream only; they describe window offsets, not
+        # canonical keys)
+        hist = self._out(reuse, "hist", 16 * 256 * 8) if want_hist and not wide and k >= 4 and rc != CANONICAL else None
         _lib.check(
             self.lib.kmg_extract(
                 d.bases.data_ptr(), d.n_bases, win_begin, win_end, k, int(rc), int(wide), d.lut.data_ptr(),
@@ -788,7 +807,7 @@ class Engine:
                           win_begin: int, win_end: Optional[int]):
         win_begin, win_end = window_range(d, k, win_begin, win_end)
         kb = key_bytes(k, False)
-        cap = max((win_end - win_begin) * (2 if rc else 1), 1)
+        cap = max((win_end - win_begin) * keys_per_window(rc), 1)
         keys, keys_alt = self._out(reuse, "keys", cap * kb), self._out(reuse, "keys_alt", cap * kb)
         vals = self._out(reuse, "vals", cap * val_bytes) if val_bytes else None
         vals_alt = self._out(reuse, "vals_alt", cap * val_bytes) if val_bytes else None
@@ -921,20 +940,20 @@ class Engine:
         pipeline, then those of the wide stream while the narrow result is held."""
         lib = self.lib
         n_win = max(0, d.n_bases - k + 1)
-        cap = max(n_win * (2 if rc else 1), 1)
+        cap = max(n_win * keys_per_window(rc), 1)
         if mode == "vec":  # extract() with window-sized buffers, one stream at a time
             return pass_bytes(k, mode, cap, cap if n_other else 0, val_bytes, text_bytes, n_win)
         if mode == "histo":  # the fused pipeline, then the wide stream beside the (kept) pipeline workspace
             ws_pipe = lib.kmg_pipeline_histo_workspace_bytes(n_win, k, int(rc))
             need = 2 * cap * key_bytes(k, False) + ws_pipe + lib.kmg_extract_workspace_bytes(n_win)
             if n_other:
-                need = max(need, ws_pipe + pass_bytes(k, mode, 0, n_other * (2 if rc else 1), 0, 0, n_win))
+                need = max(need, ws_pipe + pass_bytes(k, mode, 0, n_other * keys_per_window(rc), 0, 0, n_win))
             return int(need)
         kb, kw = key_bytes(k, False), key_bytes(k, True)
         item = kb +(4 if mode == "count" else val_bytes)
         narrow = 2 * cap * item + lib.kmg_pipeline_workspace_bytes(n_win, k, int(rc), 0 if mode == "count" else val_bytes)
         if n_other:
-            m = n_other * (2 if rc else 1)
+            m = n_other * keys_per_window(rc)
             witem = kw + (4 if mode == "count" else val_bytes)
             wide = cap * item + 2 * cap * witem + pass_bytes(k, mode, 0, m, val_bytes, 0, n_win) + 8 * (cap + m)
             narrow = max(narrow, wide)
@@ -988,7 +1007,7 @@ class Engine:
         n, n_other = self.count_windows(d, k, rc)
         one = self._one_pass_bytes(d, k, rc, mode, n_other, vb, text_bytes)
         n_win = max(0, d.n_bases - k + 1)
-        return make_plan(k, budget, one, (n, n_other * (2 if rc else 1)), lambda: self.part_counts(d, k, rc, PASS_PARTS),
+        return make_plan(k, budget, one, (n, n_other * keys_per_window(rc)), lambda: self.part_counts(d, k, rc, PASS_PARTS),
                          lambda a, b: pass_bytes(k, mode, a, b, vb, text_bytes, n_win))
 
     def write_count(self, d: DeviceInput, k: int, rc: bool, fh: BinaryIO, budget_bytes: Optional[int] = None,
@@ -1007,7 +1026,8 @@ class Engine:
         """Write the text of the reference's batch files (batch.py:281-296: every k-mer as
         ">ref:start-end:strand\\nSEQ\\n", stably sorted by sequence, batch.py:156-168) to `fh` as one sorted
         batch; how the reference splits records over files is not part of its contract (SURVEY.md f-3).  The
-        payload sorts are stable, so equal sequences keep their emission order."""
+        payload sorts are stable, so equal sequences keep their emission order.  rc = CANONICAL: AssertionError."""
+        per_strand(rc)
         self._write_text(d, k, "uniq", fh, [self.sorted_streams(d, k, rc, d.payload_bytes)], chunk_rows)
 
     def count_text(self, d: DeviceInput, k: int, rc: bool = False, min_count: int = 1,
@@ -1145,7 +1165,8 @@ class Engine:
         """VEC_COUNT / VEC_COUNT_MASKED (join.py:287-335): per flat position the number of occurrences of the
         k-mer that starts there ('+' vector) / of its reverse complement ('-' vector); masked: occurrences
         in other records only.  Computed by the pass loop of write_vectors (_fill_vectors) under
-        plan_passes(mode="vec").  Returns host uint32 arrays over the flat buffer."""
+        plan_passes(mode="vec").  Returns host uint32 arrays over the flat buffer.  rc = CANONICAL: AssertionError."""
+        per_strand(rc)
         if d.rec_starts is None:
             self._upload_names(d)
         out, _ = self._fill_vectors(d, k, rc, masked, self.plan_passes(d, k, rc, "vec", budget_bytes, text=False))
@@ -1229,7 +1250,8 @@ class Engine:
         kmg_vector_extents trims it, and each vector leaves as device text in chunks of `chunk_rows` entries
         through pinned buffers.  Files are gzip-compressed (one stream each, level 9 as gzip.open) on a pool of
         host threads while the GPU formats the next chunks: host memory is O(threads x chunk).  Returns the plan
-        with pass_ms and text_ms filled in."""
+        with pass_ms and text_ms filled in.  rc = CANONICAL: AssertionError (the vectors are per strand)."""
+        per_strand(rc)
         import gzip
         from collections import deque
 
@@ -1288,7 +1310,7 @@ class Engine:
         that belong to the wide stream."""
         win_begin, win_end = window_range(d, k)
         kb = key_bytes(k, False)
-        cap = max((win_end - win_begin) * (2 if rc else 1), 1)
+        cap = max((win_end - win_begin) * keys_per_window(rc), 1)
         keys, keys_alt = self._out(reuse, "keys", cap * kb), self._out(reuse, "keys_alt", cap * kb)
         ws_bytes = self.lib.kmg_pipeline_histo_workspace_bytes(win_end - win_begin, k, int(rc))
         ws = self._buf("ws_pipeline", ws_bytes)

@@ -175,9 +175,9 @@ class KJoiner:
         if len(batches) == 1:
             return batches[0].device_input
         b0 = batches[0]
-        if any((b.k, b.reverse, b.natype, b.device_input.alphabet) != (b0.k, b0.reverse, b0.natype, b0.device_input.alphabet)
-               for b in batches):
-            raise AssertionError("batches were built with different k / reverse / alphabet settings")
+        if any((b.k, b.reverse, b.canonical, b.natype, b.device_input.alphabet)
+               != (b0.k, b0.reverse, b0.canonical, b0.natype, b0.device_input.alphabet) for b in batches):
+            raise AssertionError("batches were built with different k / reverse / canonical / alphabet settings")
         flats = [b.device_input.flat for b in batches]
         bases = np.concatenate([f.bases for f in flats])
         starts, names, titles, off = [], [], [], 0
@@ -197,6 +197,8 @@ class KJoiner:
 
             if any(isinstance(b, LoadedKmerBatch) for b in batches):
                 raise AssertionError("abundance vectors need the FASTA input, not re-imported batch files")
+            if any(b.canonical for b in batches):
+                raise AssertionError("abundance vectors are per strand: not with canonical k-mers")
             d = self._merged_device_input(batches)
             # join.py:370-372 -> abundance.py:148-172, in key-range passes with device text (KMG_DEVICE_BUDGET applies)
             b0._eng.write_vectors(d, b0.k, b0.reverse, self.mode == self.MODE.VEC_COUNT_MASKED, outpath)
@@ -215,13 +217,14 @@ class KJoiner:
                     oh.write(b0.uniq_text())
             return
         d = self._merged_device_input(batches)
+        rc = b0.strand_rule  # (engine.CANONICAL for --canonical batches)
         # key-range passes and chunked text: device memory is bounded by the largest pass, host memory by a
         # text chunk (KMG_DEVICE_BUDGET overrides the device budget)
         with open(outpath, "wb") as oh:  # join.py:351 opens "w+": the file exists even when empty
             if self.mode == self.MODE.SEQ_COUNT:
-                b0._eng.write_count(d, b0.k, b0.reverse, oh, min_count=lo, max_count=hi)
+                b0._eng.write_count(d, b0.k, rc, oh, min_count=lo, max_count=hi)
             else:
-                b0._eng.write_uniq(d, b0.k, b0.reverse, oh)
+                b0._eng.write_uniq(d, b0.k, rc, oh)
 
     def join(self, batches: List[Any], outpath: str) -> None:
         rng = self._check_range(*self.count_range)

@@ -24,6 +24,25 @@ def reverse():
     return click.option("--reverse", "-r", is_flag=True, help="Include also reverse-complemented sequences")
 
 
+def canonical():
+    # long option only: -C is the reference's --compress
+    return click.option("--canonical", is_flag=True,
+                        help="Count each k-mer together with its reverse complement, as the smaller of the two "
+                             "(canonical k-mers, one per window). Not with -r, -B or the VEC count modes.")
+
+
+def check_canonical(canonical: bool, reverse: bool = False, previous_batches=None, count_mode: str = "") -> None:
+    """AssertionError, before any work, for --canonical with an option it cannot go with."""
+    if not canonical:
+        return
+    if reverse:
+        raise AssertionError("--canonical already covers both strands: do not combine it with -r")
+    if previous_batches is not None:
+        raise AssertionError("--canonical needs the FASTA input: -B batch files fixed their strands when written")
+    if count_mode.startswith("VEC_"):
+        raise AssertionError(f"--canonical does not apply to {count_mode}: the vectors are per strand")
+
+
 def scan_mode():
     return click.option("--scan-mode", "-s", type=click.Choice([m.name for m in FastaBatcher.MODE], case_sensitive=True),
                         default=FastaBatcher.MODE.KMERS.name,

@@ -17,6 +17,7 @@ from kman_b200.scripts import arguments as args
 @args.output_path(file_okay=True)
 @args.k()
 @args.reverse()
+@args.canonical()
 @args.scan_mode()
 @args.batch_size()
 @args.batch_mode()
@@ -32,7 +33,8 @@ def run(input_path: str, output_path: str, k: int, reverse: bool = False, scan_m
         batch_size: int = 1000000, batch_mode: str = BatcherThreading.FEED_MODE.APPEND.name,
         previous_batches: Optional[str] = None, count_mode: str = KJoiner.MODE.SEQ_COUNT.name,
         memory_mode: str = KJoiner.MEMORY.NORMAL.name, threads: int = 1, tmp: str = tempfile.gettempdir(),
-        re_sort: bool = False, min_count: int = 1, max_count: Optional[int] = None) -> None:
+        re_sort: bool = False, min_count: int = 1, max_count: Optional[int] = None, canonical: bool = False) -> None:
+    args.check_canonical(canonical, reverse, previous_batches, count_mode)
     input_file_exists(input_path)
     set_tempdir(tmp)
     joiner = KJoinerThreading(KJoiner.MODE[count_mode], KJoiner.MEMORY[memory_mode])
@@ -40,7 +42,8 @@ def run(input_path: str, output_path: str, k: int, reverse: bool = False, scan_m
     if previous_batches is not None:
         batches = load_batches(previous_batches, threads, re_sort)
     else:
-        batches = (FastaBatcher(scan_mode=FastaBatcher.MODE[scan_mode], reverse=reverse, size=batch_size, threads=threads)
+        batches = (FastaBatcher(scan_mode=FastaBatcher.MODE[scan_mode], reverse=reverse, size=batch_size, threads=threads,
+                                canonical=canonical)
                    .do(input_path, k, BatcherThreading.FEED_MODE[batch_mode]).collection)
     prep_joiner(joiner, len(batches), threads).join(batches, output_path)
     logging.info("That's all! :smiley:")

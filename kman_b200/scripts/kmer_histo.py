@@ -16,14 +16,16 @@ from kman_b200.scripts import arguments as args
 @args.output_path(file_okay=True)
 @args.k()
 @args.reverse()
-def run(input_path: str, output_path: str, k: int, reverse: bool = False) -> None:
+@args.canonical()
+def run(input_path: str, output_path: str, k: int, reverse: bool = False, canonical: bool = False) -> None:
+    args.check_canonical(canonical, reverse)
     input_file_exists(input_path)
     if k <= 1:
         raise AssertionError(f"k must be >= 1, got {k} instead.")  # the check `kmer count` makes
-    from kman_b200.engine import get_engine
+    from kman_b200.engine import CANONICAL, get_engine
 
     eng = get_engine()
     d = eng.load_fasta(input_path, ab.default_alphabet(), ab.NATYPES.DNA, with_names=False)
     with open(output_path, "wb") as fh:  # (the file exists even when the spectrum is empty)
-        eng.write_histogram(d, k, reverse, fh)
+        eng.write_histogram(d, k, CANONICAL if canonical else reverse, fh)
     logging.info("That's all! :smiley:")

@@ -17,6 +17,7 @@ from kman_b200.scripts import arguments as args
 @args.output_path(file_okay=True)
 @args.k()
 @args.reverse()
+@args.canonical()
 @args.scan_mode()
 @args.batch_size()
 @args.batch_mode()
@@ -27,13 +28,15 @@ from kman_b200.scripts import arguments as args
 def run(input_path: str, output_path: str, k: int, reverse: bool = False, scan_mode: str = FastaBatcher.MODE.KMERS.name,
         batch_size: int = 1000000, batch_mode: str = BatcherThreading.FEED_MODE.APPEND.name,
         previous_batches: Optional[str] = None, threads: int = 1, tmp: str = tempfile.gettempdir(),
-        re_sort: bool = False) -> None:
+        re_sort: bool = False, canonical: bool = False) -> None:
+    args.check_canonical(canonical, reverse, previous_batches)
     input_file_exists(input_path)
     set_tempdir(tmp)
     if previous_batches is not None:
         batches = load_batches(previous_batches, threads, re_sort)
     else:
-        batches = (FastaBatcher(scan_mode=FastaBatcher.MODE[scan_mode], reverse=reverse, size=batch_size, threads=threads)
+        batches = (FastaBatcher(scan_mode=FastaBatcher.MODE[scan_mode], reverse=reverse, size=batch_size, threads=threads,
+                                canonical=canonical)
                    .do(input_path, k, BatcherThreading.FEED_MODE[batch_mode]).collection)
     joiner = KJoinerThreading()
     joiner.threads = threads
