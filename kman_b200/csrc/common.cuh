@@ -126,20 +126,30 @@ int extract_canonical_top(const uint8_t* d_bases, uint64_t n_bases, uint64_t win
 constexpr size_t P16_ZEROED_WORDS = 65536 + 3 * 256 + 4;
 static inline unsigned long long* p16_top(unsigned long long* zeroed) { return zeroed + 65536; }
 static inline unsigned long long* p16_plan(unsigned long long* zeroed) { return zeroed + 65536 + 3 * 256; }
+// one tile of region_partition: tile.n keys from tile.first on, all in top-byte region tile.region (n = 0: none)
+struct RpTile {
+    unsigned long long first;
+    uint32_t n, region;
+};
+// keys of one region_partition tile; the tile list of n keys has at most n / tile_keys + 257 entries
+uint32_t region_tile_keys(int key_bytes, int val_bytes);
 struct Prefix16Out {
     unsigned long long* zeroed;         // [P16_ZEROED_WORDS]
     unsigned long long* region_starts;  // [256] exclusive scan of the top-byte row
     unsigned long long* starts;         // [65537] first key of every 16-bit bucket, then the number of keys
     unsigned long long* cursors;        // [65536] copy of starts[0 .. 65536) (region_partition's cursors)
     uint32_t* rows;                     // prefix16_rows_bytes(): the per-CTA counts
+    RpTile* tiles;                      // region_partition's tile list
+    uint32_t tile_keys;                 // region_tile_keys() of the keys to come
 };
 size_t prefix16_rows_bytes();
 int extract_prefix16_hist(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
                           const uint8_t* d_lut256, const Prefix16Out& o, cudaStream_t st);
-// keys (+ payload) grouped by their top byte -> grouped by their top 16 bits (cursors: Prefix16Out::cursors)
+// keys (+ payload) grouped by their top byte -> grouped by their top 16 bits (cursors: Prefix16Out::cursors,
+// tiles: Prefix16Out::tiles)
 int region_partition(const void* d_keys_in, void* d_keys_out, const void* d_vals_in, void* d_vals_out, uint64_t n,
-                     int key_bytes, int val_bytes, const unsigned long long* d_region_counts, unsigned long long* d_cursors,
-                     int digit_shift, cudaStream_t st);
+                     int key_bytes, int val_bytes, const RpTile* d_tiles, unsigned long long* d_cursors, int digit_shift,
+                     cudaStream_t st);
 int extract_digit_scatter(const uint8_t* d_bases, uint64_t n_bases, uint64_t win_begin, uint64_t win_end, int k, int rc,
                           const uint8_t* d_lut256, void* d_keys_out, int key_bytes, void* d_vals_out, int val_bytes,
                           uint64_t pos_offset, unsigned long long* d_cursors, int digit_shift, cudaStream_t st);

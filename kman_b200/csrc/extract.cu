@@ -875,22 +875,41 @@ __global__ void __launch_bounds__(256) prefix16_reduce_kernel(const uint32_t* __
 // Makes the bucket starts absolute (starts[65536] = number of keys) and copies them into the cursors of
 // region_partition_kernel; region_starts = exclusive scan of the top-byte row (the cursors of the fused
 // top-byte scatter).  plan[0] = number of keys, plan[1] = largest top-byte count.
+// tiles: the region partition's tiles of tile_keys keys, region by region (region r owns ceil(count_r /
+// tile_keys) of them), then empty entries up to ceil(keys / tile_keys) + 256, the partition's grid.
 __global__ void __launch_bounds__(256) prefix16_starts_kernel(const unsigned long long* __restrict__ top,
                                                               unsigned long long* __restrict__ plan,
                                                               unsigned long long* __restrict__ region_starts,
                                                               unsigned long long* __restrict__ starts,
-                                                              unsigned long long* __restrict__ cursors) {
+                                                              unsigned long long* __restrict__ cursors,
+                                                              RpTile* __restrict__ tiles, uint32_t tile_keys) {
     __shared__ unsigned long long s_scan[256 / 32 + 1], s_max[8], s_base;
+    __shared__ uint32_t s_scan32[256 / 32 + 1], s_t0;
     const uint32_t r = blockIdx.x, t = threadIdx.x, b = r * 256 + t;
     const unsigned long long c = top[2 * 256 + t];
     unsigned long long total;
     const unsigned long long ex = block_excl_scan<256, unsigned long long>(c, s_scan, total);
-    if (t == r) s_base = ex;
+    const uint32_t nt = (uint32_t)((c + tile_keys - 1) / tile_keys);
+    uint32_t tiles_all;
+    const uint32_t t0 = block_excl_scan<256, uint32_t>(nt, s_scan32, tiles_all);
+    if (t == r) {
+        s_base = ex;
+        s_t0 = t0;
+    }
     __syncthreads();
     const unsigned long long s = starts[b] + s_base;
     starts[b] = s;
     cursors[b] = s;
     if (t == 0) region_starts[r] = s_base;
+    const unsigned long long c_r = top[2 * 256 + r];
+    for (uint32_t i = t; (unsigned long long)i * tile_keys < c_r; i += 256) {
+        const unsigned long long first = (unsigned long long)i * tile_keys;
+        tiles[s_t0 + i] = RpTile{s_base + first, (uint32_t)min((unsigned long long)tile_keys, c_r - first), r};
+    }
+    if (r == 255) {
+        const unsigned long long grid = (total + tile_keys - 1) / tile_keys + 256;
+        for (unsigned long long i = tiles_all + t; i < grid; i += 256) tiles[i] = RpTile{0, 0, 0};
+    }
     if (r == 0) {
         unsigned long long mx = c;
 #pragma unroll
@@ -909,23 +928,38 @@ __global__ void __launch_bounds__(256) prefix16_starts_kernel(const unsigned lon
 // ---- second prefix pass of the pb = 16 pipeline: split every top-byte region by byte 2 --------------------
 // The keys arrive grouped by their top byte (region r = [R_r, R_r + count_r)).  Every 16-bit bucket's start
 // is known from the pre-pass, so each region is split on its own with the order-free DigitRuns pass:
-// tiles never straddle a region (region r owns ceil(count_r / TILE) consecutive tiles), a tile ranks its
-// keys with shared-memory atomics, reserves its runs with one global atomic per digit on the bucket
-// cursors and writes them through shared-memory staging.
+// tiles never straddle a region (region r owns ceil(count_r / TILE) consecutive tiles, listed by
+// prefix16_starts_kernel), a tile ranks its keys with shared-memory atomics, reserves its runs with one
+// global atomic per digit on the bucket cursors and writes them through shared-memory staging.
+// A CTA first pulls the tile of the CTA that will start about one wave later into L2, so the DRAM reads
+// keep streaming while the resident CTAs rank, reserve and write.
 constexpr int RP_BLOCK = 512;
 // keys per thread: 48-80 KB of staging and at most 64 registers (two CTAs per SM) without spills
 template <typename KeyT, int VB>
 constexpr int rp_ipt() { return sizeof(KeyT) == 8 ? (VB == 0 ? 12 : 8) : (VB == 8 ? 6 : 8); }
+
+uint32_t region_tile_keys(int key_bytes, int val_bytes) {
+    if (key_bytes == 8) return RP_BLOCK * (val_bytes ? rp_ipt<uint64_t, 4>() : rp_ipt<uint64_t, 0>());
+    return RP_BLOCK * (val_bytes == 8 ? rp_ipt<u128, 8>() : rp_ipt<u128, 0>());
+}
 
 struct RegionPartParams {
     const void* keys_in;
     void* keys_out;
     const void* vals_in;
     void* vals_out;
-    const unsigned long long* counts;  // [256] keys per top-byte region
-    unsigned long long* cursors;       // [65536] next free slot of every 16-bit bucket
-    int digit_shift;                   // of byte 2
+    const RpTile* tiles;          // one entry per CTA (prefix16_starts_kernel)
+    unsigned long long* cursors;  // [65536] next free slot of every 16-bit bucket
+    int digit_shift;              // of byte 2
+    uint32_t ahead;               // the tile pulled into L2: this CTA's + ahead (about the CTAs resident at once)
 };
+
+// [a, a + bytes) into L2, trimmed to whole 16-byte units inside the range
+__device__ __forceinline__ void prefetch_l2_inside(const void* a, size_t bytes) {
+    const uintptr_t lo = (reinterpret_cast<uintptr_t>(a) + 15) & ~(uintptr_t)15;
+    const uintptr_t hi = (reinterpret_cast<uintptr_t>(a) + bytes) & ~(uintptr_t)15;
+    if (hi > lo) tma_prefetch_l2(reinterpret_cast<const void*>(lo), (uint32_t)(hi - lo));
+}
 
 template <typename KeyT, int VB>
 __global__ void __launch_bounds__(RP_BLOCK, 2) region_partition_kernel(const RegionPartParams p) {
@@ -938,28 +972,19 @@ __global__ void __launch_bounds__(RP_BLOCK, 2) region_partition_kernel(const Reg
     __shared__ uint32_t s_cnt[256], s_off[256];
     __shared__ unsigned long long s_gb[256];
     __shared__ uint32_t s_scan[RP_BLOCK / 32 + 1];
-    __shared__ unsigned long long s_scan64[RP_BLOCK / 32 + 1];
-    __shared__ uint32_t s_region;
-    __shared__ unsigned long long s_lo, s_hi;
 
     const int t = threadIdx.x;
-    const unsigned long long c = t < 256 ? p.counts[t] : 0ull;
-    const uint32_t nt = (uint32_t)((c + TILE - 1) / TILE);
-    uint32_t tiles_all;
-    unsigned long long keys_all;
-    const uint32_t t0 = block_excl_scan<RP_BLOCK, uint32_t>(nt, s_scan, tiles_all);
-    const unsigned long long k0 = block_excl_scan<RP_BLOCK, unsigned long long>(c, s_scan64, keys_all);
-    if (blockIdx.x >= tiles_all) return;  // surplus CTA (the grid is sized for the worst split)
-    if (t < 256) s_cnt[t] = 0;
-    if (blockIdx.x - t0 < nt) {  // the region this tile belongs to
-        s_region = t;
-        s_lo = k0 + (unsigned long long)(blockIdx.x - t0) * TILE;
-        s_hi = k0 + c;
+    const RpTile tile = p.tiles[blockIdx.x];
+    if (tile.n == 0) return;  // surplus CTA (the grid is sized for the worst split)
+    if (t == 0 && blockIdx.x + p.ahead < gridDim.x) {
+        const RpTile nx = p.tiles[blockIdx.x + p.ahead];
+        prefetch_l2_inside(reinterpret_cast<const KeyT*>(p.keys_in) + nx.first, (size_t)nx.n * sizeof(KeyT));
+        if constexpr (VB != 0)
+            prefetch_l2_inside(reinterpret_cast<const ValT*>(p.vals_in) + nx.first, (size_t)nx.n * sizeof(ValT));
     }
-    __syncthreads();
-    const uint32_t r = s_region;
-    const unsigned long long lo = s_lo;
-    const uint32_t n_in = (uint32_t)min((unsigned long long)TILE, s_hi - lo);
+    const uint32_t r = tile.region;
+    const unsigned long long lo = tile.first;
+    const uint32_t n_in = tile.n;
     const KeyT* keys_in = reinterpret_cast<const KeyT*>(p.keys_in) + lo;
     const ValT* vals_in = reinterpret_cast<const ValT*>(p.vals_in) + lo;
     const int dsh = p.digit_shift;
@@ -975,6 +1000,8 @@ __global__ void __launch_bounds__(RP_BLOCK, 2) region_partition_kernel(const Reg
             if constexpr (VB != 0) val[q] = vals_in[i];
         }
     }
+    if (t < 256) s_cnt[t] = 0;  // (after the loads: they are on their way while the CTA waits here)
+    __syncthreads();
 #pragma unroll
     for (int q = 0; q < IPT; ++q)
         if (q * RP_BLOCK + t < n_in) wh[q] = runs.rank(key_digit(key[q], dsh, 255u));
@@ -1001,7 +1028,12 @@ static int launch_region_partition(const RegionPartParams& p, uint64_t n, cudaSt
     const size_t smem = TILE * (sizeof(KeyT) + VB);
     auto kern = region_partition_kernel<KeyT, VB>;
     KMG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<(uint32_t)grid, RP_BLOCK, smem, st>>>(p);
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    RegionPartParams q = p;
+    q.ahead = 2 * (uint32_t)sms;  // (two CTAs per SM)
+    kern<<<(uint32_t)grid, RP_BLOCK, smem, st>>>(q);
     KMG_LAUNCH_CHECK();
     return KMG_OK;
 }
@@ -1210,21 +1242,21 @@ int extract_prefix16_hist(const uint8_t* d_bases, uint64_t n_bases, uint64_t win
     }
     prefix16_reduce_kernel<<<256, 256, 0, st>>>(o.rows, n_rows, spill, top, o.starts);
     KMG_LAUNCH_CHECK();
-    prefix16_starts_kernel<<<256, 256, 0, st>>>(top, plan, o.region_starts, o.starts, o.cursors);
+    prefix16_starts_kernel<<<256, 256, 0, st>>>(top, plan, o.region_starts, o.starts, o.cursors, o.tiles, o.tile_keys);
     KMG_LAUNCH_CHECK();
     return KMG_OK;
 }
 
 int region_partition(const void* d_keys_in, void* d_keys_out, const void* d_vals_in, void* d_vals_out, uint64_t n,
-                     int key_bytes, int val_bytes, const unsigned long long* d_region_counts, unsigned long long* d_cursors,
-                     int digit_shift, cudaStream_t st) {
+                     int key_bytes, int val_bytes, const RpTile* d_tiles, unsigned long long* d_cursors, int digit_shift,
+                     cudaStream_t st) {
     if (n == 0) return KMG_OK;
     RegionPartParams p;
     p.keys_in = d_keys_in;
     p.keys_out = d_keys_out;
     p.vals_in = d_vals_in;
     p.vals_out = d_vals_out;
-    p.counts = d_region_counts;
+    p.tiles = d_tiles;
     p.cursors = d_cursors;
     p.digit_shift = digit_shift;
     if (key_bytes == 8) {

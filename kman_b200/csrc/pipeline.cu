@@ -37,6 +37,8 @@ struct PipeWs {
     unsigned long long* cursors;  // [256] region starts of the fused scatter
     unsigned long long* starts;   // [65537] 16-bit bucket starts
     unsigned long long* cursors16;  // [65536] bucket cursors of the region partition
+    RpTile* rp_tiles;             // tile list of the region partition
+    uint32_t rp_tile_keys;
     uint32_t* rows;               // per-CTA rows of the pre-pass
     uint64_t* hist16;             // [16][256] digit histograms of the stage path
     uint64_t* n_out;              // device result count
@@ -65,6 +67,8 @@ PipeWs carve_pipe(void* ws, uint64_t n_windows, int k, int rc, int val_bytes, in
     w.cursors = (unsigned long long*)take(256 * sizeof(uint64_t));
     w.starts = (unsigned long long*)take(65537 * sizeof(uint64_t));
     w.cursors16 = (unsigned long long*)take(65536 * sizeof(uint64_t));
+    w.rp_tile_keys = region_tile_keys(kb, val_bytes);
+    w.rp_tiles = (RpTile*)take((cap / w.rp_tile_keys + 257) * sizeof(RpTile));
     w.rows = (uint32_t*)take(prefix16_rows_bytes());
     w.hist16 = (uint64_t*)take(16 * 256 * sizeof(uint64_t));
     w.n_out = (uint64_t*)take(sizeof(uint64_t));
@@ -133,7 +137,7 @@ int run_pipeline(int mode, const uint8_t* d_bases, uint64_t n_bases, uint64_t wi
     bool fused = k >= 16 && hybrid_sort_applies(cap, kb, val_bytes, 2 * k, true);
     if (fused) {
         timing_begin(st);
-        const Prefix16Out p16{w.zeroed, w.cursors, w.starts, w.cursors16, w.rows};
+        const Prefix16Out p16{w.zeroed, w.cursors, w.starts, w.cursors16, w.rows, w.rp_tiles, w.rp_tile_keys};
         rcode = extract_prefix16_hist(d_bases, n_bases, win_begin, win_end, k, rc, d_lut256, p16, st);
         timing_end(st, 2);
         if (rcode != KMG_OK) return rcode;
@@ -164,7 +168,7 @@ int run_pipeline(int mode, const uint8_t* d_bases, uint64_t n_bases, uint64_t wi
             if (rcode != KMG_OK) return rcode;
             if (msd) {
                 timing_begin(st);
-                rcode = region_partition(d_keys, d_keys_alt, d_vals, d_vals_alt, n, kb, val_bytes, w.top + 2 * 256, w.cursors16,
+                rcode = region_partition(d_keys, d_keys_alt, d_vals, d_vals_alt, n, kb, val_bytes, w.rp_tiles, w.cursors16,
                                          2 * k - 16, st);
                 timing_end(st, 0);
                 if (rcode != KMG_OK) return rcode;
