@@ -12,9 +12,10 @@
 //   * twice as many cells as keys (16-bit counters, two per word): a key shares its cell with another
 //     one with probability ~0.39 instead of 0.63, and -- the point -- a key ALONE in its cell is already
 //     in its final place after the placement;
-//   * the prefix pass sees every cell's count anyway and writes the cells that hold >= 2 keys to a compact
-//     list; the list (not the tile) is what gets sorted: entry by entry, a thread per cell (2..12 keys,
-//     the normal case: two), a warp per cell (<= 128), the block for the rest (bitonic);
+//   * the prefix pass sees every cell's count anyway and writes the cells that hold >= 2 keys to two compact
+//     lists; the lists (not the tile) are what gets sorted: the pairs (~84 % of them) with one
+//     compare-exchange each in a pass of their own, the larger cells a thread per cell (3..12 keys), a
+//     warp per cell (<= 128), the block for the rest (bitonic);
 //   * equal keys always share a cell, so duplicates are found right there and recorded in a bitmask of
 //     the tile's positions.  Run heads, run lengths (count) and singletons (uniq) then come from that
 //     bitmask with popcounts -- position-parallel, coalesced, no key is compared again; a tile without
@@ -44,6 +45,26 @@ __host__ __device__ constexpr size_t lsf_smem_bytes() {
            (PAIRS ? sizeof(uint16_t) * ls_cap<KeyT, PAIRS>() : 0);
 }
 
+// Rows [0, m) of a tile to out[0, m), where `out` is the table at the tile's first row: any multiple of
+// sizeof(T) (the running count of distinct keys decides it).  Single rows up to the first 16-byte
+// boundary, then one 16-byte store per 16 / sizeof(T) rows, then single rows; vec(i) gives rows i.. of one
+// such store, row(i) row i.  ITER: vector stores per thread that cover a full tile.
+template <typename T, int ITER, typename Row, typename Vec>
+__device__ __forceinline__ void lsf_store_rows(T* out, uint32_t m, Row row, Vec vec) {
+    constexpr uint32_t V = 16 / sizeof(T);
+    const uint32_t t = threadIdx.x;
+    const uint32_t head = min(m, (uint32_t)((16u - (reinterpret_cast<uintptr_t>(out) & 15u)) & 15u) / (uint32_t)sizeof(T));
+    const uint32_t nv = (m - head) / V, tail = head + nv * V;
+    uint4* vout = reinterpret_cast<uint4*>(out + head);
+#pragma unroll
+    for (int j = 0; j < ITER; ++j) {
+        const uint32_t i = t + j * LS_BLOCK;
+        if (i < nv) vout[i] = vec(head + V * i);
+    }
+    if (t < head) out[t] = row(t);
+    if (tail + t < m) out[tail + t] = row(tail + t);
+}
+
 template <typename KeyT, int EMIT, int VB>
 __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const HybridParams p) {
     constexpr bool PAIRS = VB != 0;
@@ -59,12 +80,13 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
     constexpr int CELL_BITS = 14;
     constexpr int NW = CAP / 32;                // bitmask words
     constexpr int MAX_BIG = CAP / (LS_WARP_RUN_MAX + 1) + 1;
+    constexpr uint32_t FIX_LIST = CAP / 2;     // entries of s_fix: pairs from the front, larger cells from the back
     static_assert(IPT % 4 == 0 && CHUNKS <= 4 && CAP == LS_BLOCK * IPT && CELLS <= (1 << CELL_BITS), "geometry");
     using ValT = typename ValType<VB == 0 ? 8 : VB>::type;
     extern __shared__ __align__(16) unsigned char ls_smem[];
     KeyT* s_stage = reinterpret_cast<KeyT*>(ls_smem);                                 // [CAP]
     uint32_t* s_cell = reinterpret_cast<uint32_t*>(ls_smem + sizeof(KeyT) * CAP);     // [CAP] two 16-bit counters per word
-    uint16_t* s_fix = reinterpret_cast<uint16_t*>(s_cell + CAP);                      // [CAP / 2] cells holding >= 2 keys
+    uint16_t* s_fix = reinterpret_cast<uint16_t*>(s_cell + CAP);                      // [FIX_LIST] cells holding >= 2 keys
     uint16_t* s_idx = reinterpret_cast<uint16_t*>(s_cell + lsf_cell_words<KeyT, PAIRS>());  // [CAP] (PAIRS)
     __shared__ uint64_t s_scan64[LS_BLOCK / 32 + 1];
     __shared__ uint32_t s_scan[LS_BLOCK / 32 + 1];
@@ -73,7 +95,8 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
     __shared__ uint32_t s_epre[NW];      // emitted positions before word w (HISTO: the CTA's shared bins)
     __shared__ int s_bad;
     __shared__ uint32_t s_has_mid, s_big_n, s_ndup;
-    __shared__ uint32_t s_nfix[2];       // list lengths: the tile in flight / the next one
+    __shared__ uint32_t s_nfix[2];       // pairs | larger cells << 16: the tile in flight / the next one
+    __shared__ CellMap<KeyT, CELLS> s_cm;  // the cell map of the tile whose placement comes next
     __shared__ uint64_t s_base;
     __shared__ uint32_t s_big[MAX_BIG][2];
     // what thread 0 learns about a ticket: kind 0 = no tile left, 1 = a tile to sort, 2 = a tile without
@@ -83,7 +106,6 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
     __shared__ uint64_t s_t_s;
     const int t = threadIdx.x;
     const uint32_t lane = t & 31u, warp = t >> 5;
-    const int sh_pref = p.key_bits - p.pb;
     // a fused table cannot be patched up afterwards: with oversize tiles around the host falls back to
     // sort + run-length stage, and this launch has nothing to do (every CTA takes the same exit)
     if (FUSED && p.over[0] != 0) return;
@@ -163,13 +185,26 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
             keys[j] = idx < x.m ? kin[idx] : KeyT{};
         }
     };
-    // FRONT of a tile: counting pass (needs zeroed counters), prefix + list of crowded cells.  Leaves in
-    // `meta` what every key remembers (cell | arrival order << 14); contains barriers.
-    auto front = [&](const Tile& x, const KeyT (&keys)[IPT], uint32_t (&meta)[IPT], int which) {
+    // the staged keys as rows of a copy-out (lsf_store_rows)
+    auto key_row = [&](uint32_t i) { return s_stage[i]; };
+    auto key_vec = [&](uint32_t i) -> uint4 {
+        if constexpr (sizeof(KeyT) == 8) {
+            if (i & 1u) {  // (block-uniform: the table starts at an odd row) two keys across a 16-byte boundary
+                const uint64_t a = s_stage[i], b = s_stage[i + 1];
+                return make_uint4((uint32_t)a, (uint32_t)(a >> 32), (uint32_t)b, (uint32_t)(b >> 32));
+            }
+        }
+        return *reinterpret_cast<const uint4*>(s_stage + i);
+    };
+    constexpr int KEY_ITER = (IPT * (int)sizeof(KeyT) + 15) / 16;
+    // FRONT of a tile: counting pass (needs zeroed counters), prefix + lists of crowded cells.  Leaves the
+    // tile's cell map in s_cm for the placement; contains barriers.
+    auto front = [&](const Tile& x, const KeyT (&keys)[IPT], int which) {
         // monotone map key -> cell (see local_sort_kernel), onto twice as many cells
         CellMap<KeyT, CELLS> cm;
         {
             const KeyT* kin = reinterpret_cast<const KeyT*>(p.keys_in) + x.s;
+            const int sh_pref = p.key_bits - p.pb;
             const uint64_t p_first = shr64(kin[0], sh_pref), p_last = shr64(kin[x.m - 1], sh_pref);
             const uint64_t R = p_last - p_first + 1;  // <= 2^24
             int w = min(CELL_BITS, sh_pref);
@@ -179,37 +214,40 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
             const uint64_t range = R << w;
             cm.inv = range <= (uint64_t)CELLS ? 0u : (uint32_t)((((uint64_t)CELLS) << 32) / range);
         }
+        if (t == 0) s_cm = cm;  // (the previous tile's placement is done: barriers since)
+        const int left = (int)x.m - t;  // (one register instead of IPT bounds)
 #pragma unroll
         for (int j = 0; j < IPT; ++j) {
-            meta[j] = 0;
-            if (t + j * LS_BLOCK < x.m) {
+            if (j * LS_BLOCK < left) {
                 const uint32_t c = cm(keys[j]);
-                const uint32_t sh = (c & 1u) << 4;
-                meta[j] = c | (((atomicAdd(&s_cell[c >> 1], 1u << sh) >> sh) & 0xFFFFu) << CELL_BITS);
+                atomicAdd(&s_cell[c >> 1], 1u << ((c & 1u) << 4));
             }
         }
         __syncthreads();
         // exclusive prefix over the counters; word = start of its even cell | count of the even cell << 16.
-        // Cells that hold two keys or more are listed (one bit per cell while scanning, then the set bits).
+        // Cells that hold two keys or more are listed (one bit per cell while scanning, then the set bits):
+        // the PAIRS (exactly two keys, most of them) from the front of s_fix, the larger cells from its back.
         uint4 q[CHUNKS];
         uint64_t packed = 0;
-        uint32_t crowd = 0;  // bit 8 i + 2 wi + half
+        uint32_t pair = 0, large = 0;  // bit 8 i + 2 wi + half
 #pragma unroll
         for (int i = 0; i < CHUNKS; ++i) {
             q[i] = reinterpret_cast<uint4*>(s_cell)[i * LS_BLOCK + t];
             uint32_t sum = 0;
 #define KMG_LSF_SUM(f, wi)                                                    \
     sum += (f & 0xFFFFu) + (f >> 16);                                         \
-    crowd |= ((f & 0xFFFEu) ? 1u : 0u) << (8 * i + 2 * wi);                   \
-    crowd |= ((f & 0xFFFE0000u) ? 1u : 0u) << (8 * i + 2 * wi + 1);
+    pair |= ((f & 0xFFFFu) == 2u ? 1u : 0u) << (8 * i + 2 * wi);              \
+    pair |= ((f >> 16) == 2u ? 1u : 0u) << (8 * i + 2 * wi + 1);              \
+    large |= ((f & 0xFFFFu) > 2u ? 1u : 0u) << (8 * i + 2 * wi);              \
+    large |= ((f >> 16) > 2u ? 1u : 0u) << (8 * i + 2 * wi + 1);
             KMG_LSF_SUM(q[i].x, 0) KMG_LSF_SUM(q[i].y, 1) KMG_LSF_SUM(q[i].z, 2) KMG_LSF_SUM(q[i].w, 3)
 #undef KMG_LSF_SUM
             packed |= (uint64_t)sum << (16 * i);
         }
         uint64_t total64;
         const uint64_t excl64 = block_excl_scan<LS_BLOCK, uint64_t>(packed, s_scan64, total64);
-        uint32_t fix_total;
-        uint32_t fat = block_excl_scan<LS_BLOCK, uint32_t>((uint32_t)__popc(crowd), s_scan, fix_total);
+        uint32_t fix_total;  // pairs | larger cells << 16 (at most CAP / 2 of either)
+        const uint32_t fat = block_excl_scan<LS_BLOCK, uint32_t>((uint32_t)__popc(pair) | (uint32_t)__popc(large) << 16, s_scan, fix_total);
         uint32_t chunk_base = 0;
 #pragma unroll
         for (int i = 0; i < CHUNKS; ++i) {
@@ -225,28 +263,30 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
 #undef KMG_LSF_STEP
             reinterpret_cast<uint4*>(s_cell)[i * LS_BLOCK + t] = q[i];
         }
-        while (crowd) {
-            const uint32_t b = (uint32_t)__ffs(crowd) - 1u;
-            crowd &= crowd - 1u;
-            // bit -> cell: chunk b >> 3, word (b >> 1) & 3 of this thread's four, half b & 1
-            s_fix[fat++] = (uint16_t)(2u * (((b >> 3) * LS_BLOCK + t) * 4u + ((b >> 1) & 3u)) + (b & 1u));
-        }
+        // bit -> cell: chunk b >> 3, word (b >> 1) & 3 of this thread's four, half b & 1
+        auto bit_cell = [&](uint32_t b) { return (uint16_t)(2u * (((b >> 3) * LS_BLOCK + t) * 4u + ((b >> 1) & 3u)) + (b & 1u)); };
+        for (uint32_t at = fat & 0xFFFFu; pair; pair &= pair - 1u) s_fix[at++] = bit_cell((uint32_t)__ffs(pair) - 1u);
+        for (uint32_t at = fat >> 16; large; large &= large - 1u) s_fix[FIX_LIST - 1u - at++] = bit_cell((uint32_t)__ffs(large) - 1u);
         if (t == 0) s_nfix[which] = fix_total;
         __syncthreads();
     };
-    // placement: start of the cell + arrival order.  A key alone in its cell is in its final place.
-    // The keys are read again (the tile's range is L2-resident), so that nothing but `meta` had to stay
-    // in registers since the counting pass.
-    auto placement = [&](const Tile& x, const uint32_t (&meta)[IPT]) {
+    // placement: the keys are read again (the tile's range is L2-resident) and mapped to their cells again,
+    // so that nothing per key stays in registers since the counting pass.  The slot comes from a second
+    // returning atomic on the counter word: an even cell takes lo and moves it on (+1 - (1 << 16)), an odd
+    // cell takes lo + hi and grows hi (+(1 << 16)); lo + hi, the odd cell's start, never moves while the even
+    // cell fills.  Afterwards the word holds the odd cell's start | its count << 16 (the even cell ends at
+    // lo).  A key alone in its cell is in its final place.
+    auto placement = [&](const Tile& x) {
         KeyT keys[IPT];
         load_keys(x, keys);
+        const CellMap<KeyT, CELLS> cm = s_cm;
 #pragma unroll
         for (int j = 0; j < IPT; ++j) {
             const uint32_t idx = t + j * LS_BLOCK;
             if (idx < x.m) {
-                const uint32_t c = meta[j] & ((1u << CELL_BITS) - 1u);
-                const uint32_t w = s_cell[c >> 1];
-                const uint32_t at = (w & 0xFFFFu) + ((c & 1u) ? (w >> 16) : 0u) + (meta[j] >> CELL_BITS);
+                const uint32_t c = cm(keys[j]);
+                const uint32_t w = atomicAdd(&s_cell[c >> 1], (c & 1u) ? 1u << 16 : 1u - (1u << 16));
+                const uint32_t at = (w & 0xFFFFu) + ((c & 1u) ? (w >> 16) : 0u);
                 s_stage[at] = keys[j];
                 if constexpr (PAIRS) s_idx[at] = (uint16_t)idx;
             }
@@ -256,43 +296,50 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
     // the crowded cells: sorted in place, duplicates recorded.  Returns false when a cell is beyond what the
     // block can sort (the tile is flagged for the fallback).  Contains barriers; leaves the total of
     // duplicates in s_ndup.
-    auto fixup = [&](const Tile& x, uint32_t n_fix) -> bool {
-        const uint32_t m = x.m;
+    auto fixup = [&](uint32_t n_fix) -> bool {
+        const uint32_t n_pair = n_fix & 0xFFFFu, n_large = n_fix >> 16;
         uint32_t my_dups = 0;
         auto mark_dup = [&](uint32_t pos) {
             atomicOr(&s_dup[pos >> 5], 1u << (pos & 31u));
             ++my_dups;
         };
-        // first position and size of a listed cell (the counter words stay intact until the block's pass)
+        auto large_cell = [&](uint32_t i) -> uint32_t { return s_fix[FIX_LIST - 1u - i]; };
+        // first position and size of a listed cell, from the counter words as the placement left them (intact
+        // until the block's pass): an odd cell is lo..lo + hi of its word, an even one ends at lo and starts
+        // where the word before ends
         auto cell_range = [&](uint32_t c, uint32_t& first, uint32_t& cnt) {
             const uint32_t w = s_cell[c >> 1];
             if (c & 1u) {
-                first = (w & 0xFFFFu) + (w >> 16);
-                cnt = ((c >> 1) + 1u < (uint32_t)CAP ? (s_cell[(c >> 1) + 1u] & 0xFFFFu) : m) - first;
-            } else {
                 first = w & 0xFFFFu;
                 cnt = w >> 16;
+            } else {
+                const uint32_t v = (c >> 1) ? s_cell[(c >> 1) - 1u] : 0u;
+                first = (v & 0xFFFFu) + (v >> 16);
+                cnt = (w & 0xFFFFu) - first;
             }
         };
-        // a thread per cell: two keys as a rule (one compare), else an insertion sort of up to 12
-        for (uint32_t i0 = t; i0 < n_fix; i0 += LS_BLOCK) {
-            uint32_t first, cnt;
-            cell_range(s_fix[i0], first, cnt);
-            if (cnt == 2u) {
-                const KeyT a = s_stage[first], b = s_stage[first + 1];
-                if (b < a) {
-                    s_stage[first] = b;
-                    s_stage[first + 1] = a;
-                    if constexpr (PAIRS) {
-                        const uint16_t ia = s_idx[first];
-                        s_idx[first] = s_idx[first + 1];
-                        s_idx[first + 1] = ia;
-                    }
-                } else if (a == b) {
-                    mark_dup(first + 1);
+        // the pairs: one compare-exchange each
+        for (uint32_t i0 = t; i0 < n_pair; i0 += LS_BLOCK) {
+            const uint32_t c = s_fix[i0];
+            const uint32_t lo = s_cell[c >> 1] & 0xFFFFu;
+            const uint32_t first = (c & 1u) ? lo : lo - 2u;
+            const KeyT a = s_stage[first], b = s_stage[first + 1];
+            if (b < a) {
+                s_stage[first] = b;
+                s_stage[first + 1] = a;
+                if constexpr (PAIRS) {
+                    const uint16_t ia = s_idx[first];
+                    s_idx[first] = s_idx[first + 1];
+                    s_idx[first + 1] = ia;
                 }
-                continue;
+            } else if (a == b) {
+                mark_dup(first + 1);
             }
+        }
+        // the larger cells: a thread per cell up to 12 keys (insertion sort), the rest is handed on
+        for (uint32_t i0 = t; i0 < n_large; i0 += LS_BLOCK) {
+            uint32_t first, cnt;
+            cell_range(large_cell(i0), first, cnt);
             if (cnt > (uint32_t)LSF_THREAD_MAX) {
                 if (cnt > (uint32_t)LS_WARP_RUN_MAX) {  // the block's share
                     const uint32_t b = atomicAdd(&s_big_n, 1u);
@@ -322,9 +369,9 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
         }
         __syncthreads();
         if (s_has_mid) {  // (block-uniform) cells of 13..128 keys: one warp each, rank sort with the keys in registers
-            for (uint32_t i0 = warp; i0 < n_fix; i0 += LS_BLOCK / 32) {
+            for (uint32_t i0 = warp; i0 < n_large; i0 += LS_BLOCK / 32) {
                 uint32_t rlo, rlen;
-                cell_range(s_fix[i0], rlo, rlen);
+                cell_range(large_cell(i0), rlo, rlen);
                 if (rlen <= (uint32_t)LSF_THREAD_MAX || rlen > (uint32_t)LS_WARP_RUN_MAX) continue;  // (warp-uniform)
                 constexpr int Q = LS_WARP_RUN_MAX / 32;
                 KeyT kq[Q];
@@ -434,10 +481,9 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
     if (A.kind == 0) return;
     {
         KeyT keys[IPT];
-        uint32_t meta[IPT];
         load_keys(A, keys);
-        front(A, keys, meta, 0);
-        placement(A, meta);
+        front(A, keys, 0);
+        placement(A);
     }
     for (;;) {
         // A sits in s_stage in cell order; its list has s_nfix[0] entries.  Take the next ticket and get its
@@ -462,30 +508,35 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
             tma_prefetch_l2(reinterpret_cast<const void*>(a0 & ~(uintptr_t)15), (uint32_t)(((a1 + 15) & ~(uintptr_t)15) - (a0 & ~(uintptr_t)15)));
         }
         if (N.kind == 2) publish_nothing(N.tile);  // (more of them in a row than the list holds)
-        const bool ok = fixup(A, s_nfix[0]);
-        const uint32_t ndup = s_ndup;
-        // A's aggregate: distinct keys (count), singletons (uniq; known here only without duplicates), kept
-        // rows (count in range: without duplicates all of them or none)
-        if (!ok && t == 0) {
-            atomicAdd(p.irregular, 1ull);
-            p.flag[A.tile] = 1;
-        }
-        if constexpr (FUSED) {
-            if (!ok) {
-                publish_nothing(A.tile);
-            } else if (COUNT || ndup == 0) {
-                if (t == 0) tile_prefix_publish(p.tile_state, A.tile, RANGE && p.min_count != 1u ? 0u : A.m - ndup);
+        {
+            const bool ok = fixup(s_nfix[0]);
+            const uint32_t ndup = s_ndup;
+            // A's aggregate: distinct keys (count), singletons (uniq; known here only without duplicates), kept
+            // rows (count in range: without duplicates all of them or none)
+            if (!ok && t == 0) {
+                atomicAdd(p.irregular, 1ull);
+                p.flag[A.tile] = 1;
+            }
+            if constexpr (FUSED) {
+                if (!ok) {
+                    publish_nothing(A.tile);
+                } else if (COUNT || ndup == 0) {
+                    if (t == 0) tile_prefix_publish(p.tile_state, A.tile, RANGE && p.min_count != 1u ? 0u : A.m - ndup);
+                }
             }
         }
         // the next tile's front, between A's publish and A's resolve
-        uint32_t meta_n[IPT];
         if (N.kind == 1) {
             KeyT keys[IPT];
             load_keys(N, keys);
             zero_cells();
             __syncthreads();
-            front(N, keys, meta_n, 1);
+            front(N, keys, 1);
         }
+        // A's outcome, read back from shared memory (unchanged since the fix-up): nothing of it stays in
+        // registers across the front
+        const bool ok = s_bad == 0;
+        const uint32_t ndup = s_ndup;
         // ---- emission of A ----
         if constexpr (HISTO) {
             // run lengths from the duplicate bitmask: a run head is a position without a mark, a singleton a
@@ -496,7 +547,7 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
                 if (t == 0) atomicAdd(&s_h[1], m);
             } else if (ok) {
                 uint32_t singles = 0;
-#pragma unroll
+#pragma unroll 1
                 for (int j = 0; j < IPT; ++j) {
                     const uint32_t pos = t + j * LS_BLOCK;
                     const uint32_t w = pos >> 5;
@@ -518,12 +569,7 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
             }
         } else if constexpr (!FUSED) {
             if (ok) {
-                KeyT* kout = reinterpret_cast<KeyT*>(p.keys_out) + A.s;
-#pragma unroll
-                for (int j = 0; j < IPT; ++j) {
-                    const uint32_t idx = t + j * LS_BLOCK;
-                    if (idx < A.m) kout[idx] = s_stage[idx];
-                }
+                lsf_store_rows<KeyT, KEY_ITER>(reinterpret_cast<KeyT*>(p.keys_out) + A.s, A.m, key_row, key_vec);
                 if constexpr (PAIRS) {
                     const ValT* vin = reinterpret_cast<const ValT*>(p.vals_in) + A.s;
                     ValT* vout = reinterpret_cast<ValT*>(p.vals_out) + A.s;
@@ -551,13 +597,15 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
                 }
                 __syncthreads();
                 const uint64_t base = s_base;
+                lsf_store_rows<KeyT, KEY_ITER>(kout_all + base, m, key_row, key_vec);
+                if constexpr (COUNT || RANGE) {
+                    lsf_store_rows<uint32_t, IPT / 4>(p.counts_out + base, m, [](uint32_t) { return 1u; },
+                                                      [](uint32_t) { return make_uint4(1u, 1u, 1u, 1u); });
+                } else {
 #pragma unroll
-                for (int j = 0; j < IPT; ++j) {
-                    const uint32_t pos = t + j * LS_BLOCK;
-                    if (pos < m) {
-                        kout_all[base + pos] = s_stage[pos];
-                        if constexpr (COUNT || RANGE) p.counts_out[base + pos] = 1u;
-                        else reinterpret_cast<ValT*>(p.vals_out)[base + pos] = (reinterpret_cast<const ValT*>(p.vals_in) + A.s)[s_idx[pos]];
+                    for (int j = 0; j < IPT; ++j) {
+                        const uint32_t pos = t + j * LS_BLOCK;
+                        if (pos < m) reinterpret_cast<ValT*>(p.vals_out)[base + pos] = (reinterpret_cast<const ValT*>(p.vals_in) + A.s)[s_idx[pos]];
                     }
                 }
             } else {
@@ -662,7 +710,7 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
             if (N.kind == 1) {
                 KeyT keys[IPT];
                 load_keys(N, keys);
-                front(N, keys, meta_n, 0);
+                front(N, keys, 0);
             }
         }
         if (N.kind == 0) {
@@ -670,7 +718,7 @@ __global__ void __launch_bounds__(LS_BLOCK, 2) local_sort_fine_kernel(const Hybr
             return;
         }
         __syncthreads();
-        placement(N, meta_n);
+        placement(N);
         A = N;
     }
 }
